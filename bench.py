@@ -12,6 +12,7 @@ at N = 1), each with its roofline fractions and a parity check against the commi
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torch.distributed.run)
   python bench.py --impl reference ...                      CPU restatement of the reference on the host cores
   python bench.py --only c3 --only-step --no-graph ...      one config, launch by launch (the ncu launch-list runs)
+  python bench.py --dump-outputs DIR ...                    also write the headline's last timed step to DIR/<name>.npy
 
 Prints ONE JSON line on rank 0.
 """
@@ -62,7 +63,8 @@ def parse():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch of the headline workload (0 = 64)")
-    ap.add_argument("--repeats", type=int, default=25, help="timed windows of --steps steps for the headline (median reported)")
+    ap.add_argument("--repeats", type=int, default=1,
+                    help="timed windows of --steps steps for the headline (median reported; the default times exactly --steps steps)")
     ap.add_argument("--config-repeats", type=int, default=9, help="timed windows per entry of `configs`")
     ap.add_argument("--only", default="", help="comma list out of c1,c2,c3,c4,c5: measure only these")
     ap.add_argument("--c5-global-batch", type=int, default=512, help="global batch of configs.c5 (512 = BASELINE configs[4])")
@@ -75,7 +77,11 @@ def parse():
     ap.add_argument("--verbose", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="issue every step launch by launch instead of replaying CUDA graphs")
     ap.add_argument("--only-step", action="store_true", help="skip phase timing / e2e / cpu baseline / parity (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the headline's last timed step returned (loss, sampled y_true) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or (args.only and "c2" not in args.only.split(","))):
+        ap.error("--dump-outputs writes the outputs of the headline (c2) on the GPU")
     args.graph_steps = auto_graph_steps(args.steps, args.graph_steps)
     return args
 
@@ -298,13 +304,13 @@ class Bench(object):
 
     def window(self, fn, steps, unit=1):
         """EXACTLY `steps` calls of fn bracketed by barrier + synchronize on both sides, CUDA events on the launching
-        stream, max over ranks.  Returns milliseconds for the window."""
+        stream, max over ranks.  Returns milliseconds for the window; self.last holds what the last call of fn returned."""
         torch = self.torch
         self.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps // unit):   # one call of fn = `unit` steps (a CUDA graph of several consecutive steps)
-            fn()
+            self.last = fn()
         for hook in self.tail_hooks:   # side streams whose work belongs to the timed region join before the stop event
             hook()
         e1.record()
@@ -446,12 +452,24 @@ def headline_c2(b, line):
     else:
         dev_step = b.runtime.capture(raw)
     ms_dev, windows = b.timed(dev_step, args.steps, args.warmup, args.repeats, unit=unit)
-    last = dev_step()
+    last = b.last
     torch.cuda.synchronize()
     loss_val = float(last.item())
     del b.tail_hooks[:]
     clocks = sampler.stop() if rank == 0 else None
     b.log("headline timed")
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results as a caller receives them: the loss and GetTargets' dense y_true.  The whole y_true
+        # is 495 MB at batch 64, so it is sampled: every layer of a fixed, seeded draw of 8 images (62 MB)
+        pick = np.sort(np.random.default_rng(SEED + 9).choice(batch, min(batch, 8), replace=False))
+        idx = torch.from_numpy(pick).to(dev)
+        outs = {"loss": last.cpu().numpy()}
+        for l, t in enumerate(y_true):
+            outs["y_true_%d" % l] = t.index_select(0, idx).cpu().numpy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+        line["dump"] = {"dir": args.dump_outputs, "files": sorted(n + ".npy" for n in outs), "y_true_images": pick.tolist()}
     n_fill = sum(int(t.numel()) for t in y_true)
     line.update({
         "metric": "images/sec", "value": global_batch / (ms_dev / 1e3), "unit": "images/s", "n_gpus": world,
