@@ -51,7 +51,7 @@ struct YlLevels {
 struct YlParams {
   YlLevels lv;
   int B, A, C, RF, n_img;
-  float img_w, img_h;
+  float img_w, img_h;  // divisors of the width / height channels (the variant decides the order, see yolo_loss_impl)
   float thr;
   int metric, variant;
   float* obj_compact;   // [B, n_img]
@@ -1143,7 +1143,12 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
   }
   unsigned char* wsb = static_cast<unsigned char*>(workspace);
   p.B = B; p.A = A; p.C = C; p.RF = 5 + C; p.n_img = n_img;
-  p.img_w = image_wh_host[0]; p.img_h = image_wh_host[1];
+  // GetLoss scales the width channel by image_wh[::-1] (tyu:48,57, SURVEY Q10): the target log takes tw*image_wh[1] and
+  // the predicted width is exp(tw)*anchor_w/image_wh[1].  Yolov4Loss's input_shape[::-1] really is (W, H).  The sparse
+  // target assignment (yt_fill_geometry) keeps image_wh in (w, h) order.
+  const bool wh_reversed = variant == YL_VARIANT_TF_YOLO_UTILS;
+  const float img_w = image_wh_host[wh_reversed ? 1 : 0], img_h = image_wh_host[wh_reversed ? 0 : 1];
+  p.img_w = img_w; p.img_h = img_h;
   p.thr = iou_thresh; p.metric = metric; p.variant = variant;
   p.obj_compact = reinterpret_cast<float*>(wsb + ws.obj);
   p.gt_box = reinterpret_cast<float4*>(wsb + ws.gt);
@@ -1152,10 +1157,10 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
   for (int l = 0; l < YL_LEVELS; ++l)
     for (int a = 0; a < A; ++a)
     {
-      p.logk[l][a] = (float)log(((double)p.lv.anc_w[l][a] * (double)p.lv.anc_h[l][a]) / ((double)image_wh_host[0] * (double)image_wh_host[1]));
+      p.logk[l][a] = (float)log(((double)p.lv.anc_w[l][a] * (double)p.lv.anc_h[l][a]) / ((double)img_w * (double)img_h));
       // width/height must stay >= 4e-5 (normalised) so that the rounding of x +- w/2 (<= 1.2e-7) is < 0.4 %
-      const double tw = log(4e-5 * (double)image_wh_host[0] / (double)p.lv.anc_w[l][a]);
-      const double th = log(4e-5 * (double)image_wh_host[1] / (double)p.lv.anc_h[l][a]);
+      const double tw = log(4e-5 * (double)img_w / (double)p.lv.anc_w[l][a]);
+      const double th = log(4e-5 * (double)img_h / (double)p.lv.anc_h[l][a]);
       p.tmin_w[l][a] = (float)(tw > -6.0 ? tw : -6.0);
       p.tmin_h[l][a] = (float)(th > -6.0 ? th : -6.0);
     }
