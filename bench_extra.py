@@ -31,6 +31,20 @@ def timed(fn, steps, warmup):
     return e0.elapsed_time(e1) / steps
 
 
+def _card():
+    """Name and power limit of cuda:0, read next to the measurement (a read-only nvidia-smi query)."""
+    import subprocess
+    import torch
+    out = {"gpu": torch.cuda.get_device_name(0)}
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=power.limit", "--format=csv,noheader"], capture_output=True,
+                           text=True, timeout=30)
+        out["power_limit"] = q.stdout.strip() or "unknown"
+    except (OSError, subprocess.SubprocessError):
+        out["power_limit"] = "unknown"
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--workload", default="all")
@@ -125,6 +139,57 @@ def main():
             ms = timed(fn, max(args.steps, 50), 10)
             report("n4_letterbox_%dx%d" % (w, h), "prepare_image: INTER_AREA letterbox to 416x416 + BGR->RGB + /255 (device-resident "
                    "uint8 frame; L2-resident after the first pass)", 1, ms, h * w * 3 + 416 * 416 * 3 * 4, {"latency_us": ms * 1e3})
+    if want("n4_letterbox_batch") or want("n4_serving_chain"):
+        from tfmv_b200.views.object_detection import prepare_image, prepare_images
+        card = _card()
+        mix_sizes = ((480, 640), (1080, 1920), (3024, 4032))
+        frames_mix = [torch.randint(0, 256, mix_sizes[i % 3] + (3,), device=dev, dtype=torch.uint8, generator=g) for i in range(64)]
+    if want("n4_letterbox_batch"):  # SURVEY 8f N4 batched: N frames per call against one call per frame
+        cases = [("1920x1080_n%d" % n, [torch.randint(0, 256, (1080, 1920, 3), device=dev, dtype=torch.uint8, generator=g)
+                                        for _ in range(n)]) for n in (1, 8, 64)] + [("mix_n64", frames_mix)]
+        for tag, frames in cases:
+            n = len(frames)
+            src = sum(f.numel() for f in frames)
+            steps = max(args.steps, 50)
+            ms_loop = timed(wrap(lambda: [prepare_image(f, (416, 416))[0] for f in frames]), steps, args.warmup)
+            ms = timed(wrap(lambda: prepare_images(frames, (416, 416))[0]), steps, args.warmup)
+            report("n4_letterbox_batch_" + tag, "prepare_images (one launch) vs a loop of prepare_image, %d device-resident frames "
+                   "to 416x416 + BGR->RGB + /255 (source %.0f MB: %s)" % (n, src / 1e6, "L2-resident" if src < 100e6 else
+                                                                          "exceeds the 126 MB L2"), n, ms,
+                   src / n + 416 * 416 * 3 * 4,
+                   dict(card, us_per_frame=ms * 1e3 / n, frames_per_s=n / ms * 1e3, l2_resident=src < 100e6,
+                        per_frame_loop_us_per_frame=ms_loop * 1e3 / n, per_frame_loop_frames_per_s=n / ms_loop * 1e3,
+                        speedup_vs_loop=ms_loop / ms))
+    if want("n4_serving_chain"):  # decoded frames -> network input ... NMS output -> pixel boxes, backbone not timed
+        from tfmv_b200.ai_models.utils import tf_yolo_utils as tyu
+        from tfmv_b200.views.object_detection import restore_predictions, restore_predictions_batch
+        frames = frames_mix
+        n = len(frames)
+        base = synth.yolo_heads_trained_like(np.random.default_rng(20261018 + 4), 16, 416)
+        heads = [torch.from_numpy(np.tile(h, (n // 16, 1, 1, 1))).to(dev) for h in base]   # the backbone's output, fixed
+
+        def batched():
+            _, _, _, geometry = prepare_images(frames, (416, 416))
+            nms = tyu.GetNMSBoxesBatch(*heads, anc, (416, 416), 80, 0.5, 0.3, 0.5, "iou")
+            return restore_predictions_batch(nms, (416, 416), geometry)
+
+        def per_frame():  # today's single-image calls; GetNMSBoxes and restore_predictions read counts on the host
+            out = []
+            for i, f in enumerate(frames):
+                _, padding, old = prepare_image(f, (416, 416))
+                y = tyu.GetNMSBoxes(*[h[i:i + 1] for h in heads], anc, (416, 416), 80, 0.5, 0.3, 0.5, "iou")
+                out.append(restore_predictions(*y, np.int32([416, 416]), padding, old))
+            return out
+        ms = timed(wrap(batched), args.steps, args.warmup)
+        ms_loop = timed(per_frame, args.steps, args.warmup)
+        kept = int(batched()["count"].sum().item())
+        report("n4_serving_chain_mix_n64", "prepare_images -> GetNMSBoxesBatch -> restore_predictions_batch on 64 device frames "
+               "(640x480 / 1920x1080 / 4032x3024 mix, source %.0f MB, exceeds the 126 MB L2) against a per-frame loop of prepare_image -> GetNMSBoxes -> "
+               "restore_predictions (always launch by launch: it syncs on the counts); trained-like heads stand in for the "
+               "backbone, outside the timed region" % (sum(f.numel() for f in frames) / 1e6), n, ms, sum(f.numel() for f in frames) / n + 416 * 416 * 3 * 4,
+               dict(card, us_per_frame=ms * 1e3 / n, frames_per_s=n / ms * 1e3, kept_boxes_total=kept,
+                    per_frame_loop_us_per_frame=ms_loop * 1e3 / n, per_frame_loop_frames_per_s=n / ms_loop * 1e3,
+                    speedup_vs_loop=ms_loop / ms))
     for name, cfgname, batch, with_loss in (("c3_d0_b128", "d0", 128, True), ("c4_d7_b16", "d7", 16, False)):
         if not want(name):
             continue

@@ -302,6 +302,25 @@ int b200_letterbox_image(const uint8_t* img, int height, int width, int channels
                          const uint8_t bg_color[3], uint8_t* out_u8, float* out_f32, int32_t padding_out[4],
                          int32_t resized_wh_out[2], void* stream);
 
+/* b200_letterbox_image for N frames of any sizes in one launch per 84 frames (a longer batch is split): slot i of
+ * out_u8 / out_f32 [N,out_height,out_width,3] is bit for bit what b200_letterbox_image gives for frame i alone.
+ * imgs (host array of N pointers) [hw[2i], hw[2i+1], 3] uint8 frames in device or pinned host memory; hw (host) [N,2]
+ * height,width; padding_out (host) [N,4]; resized_wh_out (host, optional) [N,2]; geometry_out (device, optional) [N,6]
+ * top,bottom,left,right,width,height of every frame, written by the kernel (what b200_unletterbox_boxes_batch reads).
+ * The per-frame plans travel in the kernel arguments (no workspace, no copy), so the call can be captured in a CUDA
+ * graph; a replay letterboxes frames of the captured sizes.  Every frame is checked before anything is launched: an
+ * invalid frame (empty resize, bad size, null pointer, channels != 3) fails the call and the message names its index.
+ * N == 0 does nothing. */
+int b200_letterbox_batch(int N, const uint8_t* const imgs[], const int32_t* hw, int channels, int out_width,
+                         int out_height, const uint8_t bg_color[3], uint8_t* out_u8, float* out_f32, int32_t* padding_out,
+                         int32_t* resized_wh_out, int32_t* geometry_out, void* stream);
+
+/* b200_unletterbox_boxes with per-image geometry (device [B,6]: padding top,bottom,left,right, then old_w, old_h, as
+ * b200_letterbox_batch writes it): frames of different sizes mapped back in one launch, same arithmetic. */
+int b200_unletterbox_boxes_batch(const float* boxes, const int32_t* counts, int B, int max_rows, const int32_t image_size[2],
+                                 const int32_t* geometry, int32_t* out_boxes, int32_t* out_index, int32_t* out_count,
+                                 void* stream);
+
 /* test_step of EfficientDetNetTrain (efficientnet/efficientdet_net_train.py:135-169) in ONE pass over the heads: focal +
  * Huber partial sums (:141-151; sums_out [2L+1] fp64 as b200_focal_box_partial_sums writes them -> b200_focal_box_finalize
  * / _dp), convert_outputs_boxes (:153, out_decoded[l] (B,H,W,A,4), entries may be NULL) and convert_outputs_one for every

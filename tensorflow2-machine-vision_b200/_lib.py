@@ -31,6 +31,8 @@ SIGNATURES = {
     "b200_yolo_loss": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_f, c_i, c_i, c_f, c_p, c_p, c_p, c_p, c_sz, c_p]),
     "b200_unletterbox_boxes": (c_i, [c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
     "b200_letterbox_image": (c_i, [c_p, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "b200_letterbox_batch": (c_i, [c_i, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "b200_unletterbox_boxes_batch": (c_i, [c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p]),
     "b200_yolo_loss_stages": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_f, c_i, c_i, c_f, c_p, c_p, c_p, c_sz, c_i, c_p]),
     "b200_yolo_loss_grad": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_f, c_i, c_i, c_f, c_p, c_p, c_p, c_p, c_sz, c_p]),
     "b200_yolo_loss_from_boxes_workspace_bytes": (c_sz, [c_p, c_i, c_i, c_i]),
