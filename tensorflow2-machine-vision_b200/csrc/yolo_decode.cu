@@ -49,7 +49,6 @@ struct YoloDecodeParams {
   int32_t* counts;     // [B]
   uint32_t* bitmap;    // [B, bitmap_words] or nullptr
   int bitmap_words;
-  int early_issue;     // refill a warp's slab before its append (atomic + stores) instead of after it
 };
 
 // ---- mbarrier / bulk-copy PTX -----------------------------------------------------------------
@@ -604,9 +603,8 @@ extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t h
   // Refilling a warp's slab before its append keeps one more copy in flight: -3 % for the call on its own at any size, and
   // for the fused evaluation step at 512 images; at 64 images per GPU the same step is 3 % SLOWER with it (the filter then
   // takes DRAM bandwidth from the loss chain that shares the GPU, and that chain is the longer one there).  Long streams
-  // (>= 32 tiles per warp) refill early, short ones late; B200_YD_EARLY_ISSUE=0/1 overrides (measurements only).
-  { const char* e = getenv("B200_YD_EARLY_ISSUE"); dp.early_issue = e ? atoi(e) : (n_tiles >= 32ll * grid * warps ? 1 : 0); }
-  if (dp.early_issue) {
+  // (>= 32 tiles per warp) refill early, short ones late.
+  if (n_tiles >= 32ll * grid * warps) {
     B200_CUDA(cudaFuncSetAttribute(yolo_decode_filter_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
     yolo_decode_filter_kernel<true><<<grid, warps * 32, smem1, stream>>>(dp);
   } else {

@@ -14,11 +14,14 @@
 //      the exact decode (tyu:57-75) and exact metric (iou / diou / ciou, tiu:5-65), and accumulates
 //      object_loss = obj*bce + (1-obj)*bce*ignore (tyu:111-114).  The trailing CTAs of its grid instead take a warp per
 //      object and produce the xy, wh and class terms (tyu:107-118) from the full y_true / y_pred records.
-//      Default (device-resident, 16-byte aligned y_pred, records of >= 8 floats): the pass is SPLIT.  K4b-lean
-//      (yolo_loss_ignore_lean_kernel, 48 registers, 10 CTAs per SM) streams, applies the rejects and only QUEUES the records
-//      that some GT might still hit (~1 % of them); K4b-exact resolves the queue (a warp per record) at the head of the
-//      widened K4c launch, its object-loss terms in 2^-32 fixed point so that the sum does not depend on the order.
-//      The launches of a dense call are then K4a (whose last CTA per (image, level) also does K4a'), K4b-lean, K4c.
+//      This single-kernel form runs when y_pred is in pinned host memory (read in place over PCIe), when a level of
+//      y_pred is not 16-byte aligned, or when a record holds fewer than 8 floats (C < 3).
+//      Every other call (device-resident y_pred, every level 16-byte aligned, records of >= 8 floats) SPLITS the pass.
+//      K4b-lean (yolo_loss_ignore_lean_kernel, 48 registers, 10 CTAs per SM) streams, applies the same rejects and only
+//      QUEUES the records that some GT might still hit (~1 % of them); K4b-exact resolves the queue (a warp per record) at
+//      the head of the widened K4c launch, its object-loss terms in 2^-32 fixed point so that the sum does not depend on
+//      the order.  The launches of a dense call are then K4a (whose last CTA per (image, level) also does K4a'),
+//      K4b-lean, K4c.
 //  K4c yolo_loss_finalize_kernel  fixed-order fp64 reduction of the per-CTA partials -> parts[3][4] / batch,
 //      loss = sum_l ((xy+wh)+obj)+cls in fp32 in the reference's order (tyu:120-125).  Deterministic run to run (the object lists are
 //      put into ascending record order by K4a' before anything is summed over them).
@@ -30,9 +33,7 @@
 
 #define YL_LEVELS 3
 #define YL_CHUNK 256
-#ifndef YL_ICHUNK
-#define YL_ICHUNK 128  // records (threads) per CTA of the ignore kernel
-#endif
+#define YL_ICHUNK 128  // records (threads) per CTA of the ignore kernels
 
 enum { YL_VARIANT_TF_YOLO_UTILS = 0, YL_VARIANT_KERAS_YOLO3 = 1 };
 
@@ -72,7 +73,6 @@ struct YlParams {
   const uint32_t* obj_bits;   // [B, bits_words]
   int bits_words;
   int32_t* gt_count;    // [B, 3]
-  int scan_reverse;           // scan CTAs walk y_true from its end: the part GetTargets wrote last is still in L2
   unsigned int* scan_ticket;  // [B, 3] scan CTAs done per (image, level): the last one prepares that GT list (null: K4a' runs as a launch)
   // split form of the ignore pass (K4b-lean + K4b-exact): records whose filter leaves a (record, GT) pair undecided
   uint32_t* pend_queue;            // [B * n_img] global record ids (img * n_img + anchor_base[l] + rin)
@@ -98,9 +98,7 @@ __device__ __forceinline__ bool yl_regular(const BoxT& b) {
          (dm_fabsf(b.c0) < 3.0e38f) && (dm_fabsf(b.c1) < 3.0e38f) && (dm_fabsf(b.c2) < 3.0e38f) && (dm_fabsf(b.c3) < 3.0e38f);
 }
 
-#ifndef YL_OBJ_PER_THREAD
 #define YL_OBJ_PER_THREAD 4
-#endif
 #define YL_OBJ_CHUNK (YL_CHUNK * YL_OBJ_PER_THREAD)
 
 #define YL_SORT_CAP 2048
@@ -155,9 +153,10 @@ __global__ void __launch_bounds__(YL_CHUNK) yolo_loss_scan_kernel(YlParams p) {
   __shared__ int s_idx[YL_SORT_CAP];
   __shared__ int s_n, s_base;
   __shared__ bool s_last;
-  // same (level, image, chunk) decomposition as the ignore kernel but with larger chunks
+  // same (level, image, chunk) decomposition as the ignore kernel but with larger chunks.  The CTAs walk y_true from its
+  // end: the part GetTargets wrote last is still in L2
   int l = 0;
-  const int bid = p.scan_reverse ? (int)(gridDim.x - 1 - blockIdx.x) : (int)blockIdx.x;
+  const int bid = (int)(gridDim.x - 1 - blockIdx.x);
 #pragma unroll
   for (int k = 1; k < YL_LEVELS; ++k) if (bid >= p.lv.obj_cta_base[k]) l = k;
   const int rcta = bid - p.lv.obj_cta_base[l];
@@ -208,9 +207,7 @@ __global__ void __launch_bounds__(YL_CHUNK) yolo_loss_scan_kernel(YlParams p) {
 // ignore kernel's grid (two dependent DRAM round trips and ~600 serial instructions per object: hidden under the
 // ignore pass instead of sitting on the critical path).  CTA (l, img, s) takes objects k = s*4 + warp, stepping by
 // 4*YL_TERM_SPLIT.
-#ifndef YL_TERM_SPLIT
 #define YL_TERM_SPLIT 16
-#endif
 
 __device__ __forceinline__ void yl_terms_body(const YlParams& p, int cta, double (*s_acc)[3]) {
   const int l = cta / (p.B * YL_TERM_SPLIT);
@@ -305,6 +302,150 @@ __device__ __forceinline__ int yl_fastdiv(int n, uint32_t magic) {
   return magic == 0u ? n : (int)__umulhi((uint32_t)n, magic);  // magic 0 encodes divisor 1
 }
 
+// obj of the record at flat anchor index `ain` of image `img`: one bit (sparse-target mode) or the scan's compact copy
+__device__ __forceinline__ float yl_obj(const YlParams& p, int img, int ain) {
+  if (p.obj_bits) return ((__ldg(p.obj_bits + (size_t)img * p.bits_words + (ain >> 5)) >> (ain & 31)) & 1u) ? 1.0f : 0.0f;
+  return p.obj_compact[(size_t)img * p.n_img + ain];
+}
+
+// tx, ty, tw, th, conf of a record that starts sh = 0..3 floats into the 8 loaded floats (lo, hi): rotate them left by sh
+// with two select stages
+__device__ __forceinline__ void yl_rotate5(const float4 lo, const float4 hi, int sh, float& tx, float& ty, float& tw, float& th,
+                                           float& pobj) {
+  const bool s1 = sh & 1, s2 = sh & 2;
+  const float a0 = s1 ? lo.y : lo.x, a1 = s1 ? lo.z : lo.y, a2 = s1 ? lo.w : lo.z, a3 = s1 ? hi.x : lo.w;
+  const float a4 = s1 ? hi.y : hi.x, a5 = s1 ? hi.z : hi.y, a6 = s1 ? hi.w : hi.z;
+  tx = s2 ? a2 : a0; ty = s2 ? a3 : a1; tw = s2 ? a4 : a2; th = s2 ? a5 : a3; pobj = s2 ? a6 : a4;
+}
+
+// One record's object_loss = obj*bce + (1-obj)*bce*ignore (tyu:114).  Also writes the record's ignore byte and
+// d loss / d conf logit = (sigmoid(p) - obj) * (obj + (1-obj)*ignore) / B (the mask has no gradient).  `filtered`: the
+// lean filter alone decided ignore = 1, and the gradient is taken as (sigmoid(p) - obj) / B.  The factor equals 1 in
+// exact arithmetic but not always in fp32 for a non-binary obj, so each form keeps its own bits.
+__device__ __forceinline__ float yl_record_term(const YlParams& p, int l, int img, int ain, float obj, float pobj, bool hit,
+                                                bool filtered) {
+  const float bc = yl_fast_bce(obj, pobj);
+  const float ign = hit ? 0.0f : 1.0f;
+  const float e = obj * bc + (1.0f - obj) * bc * ign;
+  if (p.out_ignore) p.out_ignore[(size_t)img * p.n_img + ain] = hit ? 0 : 1;
+  if (p.conf_grad) {
+    const float ex = __expf(-fabsf(pobj));
+    const float rr = 1.0f / (1.0f + ex);
+    const float sg = pobj >= 0.0f ? rr : ex * rr;
+    p.conf_grad[(size_t)p.B * p.lv.anchor_base[l] + (size_t)img * p.lv.rec_per_img[l] + (ain - p.lv.anchor_base[l])] =
+        filtered ? (sg - obj) * p.inv_div : (sg - obj) * (obj + (1.0f - obj) * ign) * p.inv_div;
+  }
+  return e;
+}
+
+// The CTA's object-loss partial: an fp32 sum of each warp's 32 terms, fp64 across the warps (and across the CTAs in K4c)
+__device__ __forceinline__ void yl_store_partial(const YlParams& p, int icta, float e, double* s_acc) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  e = warp_sum(e);
+  if (lane == 0) s_acc[warp] = (double)e;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double sum = 0;
+    for (int i = 0; i < YL_ICHUNK / 32; ++i) sum += s_acc[i];
+    p.partials[icta] = sum;
+  }
+}
+
+// The filter's per-record state, shared by both forms of the ignore pass.
+struct YlFilter {
+  bool nice;                         // logits in the range where the decode-free bounds are proven
+  bool fast_ok;                      // the approximate box may decide the IoU reject
+  bool any_rough;                    // some active lane of the warp is not nice: every GT is relevant
+  float sp;                          // tw + th + log(anchor area / image area)
+  float fx0, fy0, fx1, fy1, farea;   // approximate decoded box
+  float cx0, cy0, cx1, cy1;          // rectangle that certainly contains the decoded centre
+  float ux0, uy0, ux1, uy1;          // the warp's strip of cells
+  float lo_k, hi_k, thr_lo;
+};
+
+// Every lane of the warp calls this (it shuffles); inactive lanes are never nice.
+__device__ __forceinline__ YlFilter yl_filter_init(const YlParams& p, int l, int rin, bool active, float tx, float ty,
+                                                   float tw, float th) {
+  YlFilter f = {};
+  const int W = p.lv.w[l], H = p.lv.h[l];
+  const int cell = yl_fastdiv(rin, p.magic_a);
+  const int a = min(rin - cell * p.A, 7);
+  const int gy = yl_fastdiv(cell, p.lv.magic_w[l]);
+  const int gx = cell - gy * W;
+  const bool filter_ok = p.thr >= 0.5f;
+  f.nice = active && filter_ok && (tw >= p.tmin_w[l][a]) && (tw <= 4.0f) && (th >= p.tmin_h[l][a]) && (th <= 4.0f) &&
+           (tx == tx) && (ty == ty);
+  f.sp = tw + th + p.logk[l][a];
+  const float invW = 1.0f / (float)W, invH = 1.0f / (float)H;
+  // (c) approximate decode (MUFU exp / reciprocal; corner error < 2e-6 for boxes up to 2 image widths) for an
+  // IoU *upper-bound* reject: every metric of the family is <= IoU, so IoU_fast < thr - YL_IOU_EPS with both
+  // overlap extents >= YL_IOU_FLOOR (relative IoU error then < 3.2e-3, DESIGN.md) proves metric < thr.  Accepts
+  // are never decided here: pairs that survive go to the exact test.
+  if (f.nice) {
+    const float ex = __expf(-fabsf(tx)), ey = __expf(-fabsf(ty));
+    const float rx = __fdividef(1.0f, 1.0f + ex), ry = __fdividef(1.0f, 1.0f + ey);
+    const float fx = ((tx >= 0.0f ? rx : ex * rx) + (float)gx) * invW, fy = ((ty >= 0.0f ? ry : ey * ry) + (float)gy) * invH;
+    const float fw = __expf(tw) * __fdividef(p.lv.anc_w[l][a], p.img_w), fh = __expf(th) * __fdividef(p.lv.anc_h[l][a], p.img_h);
+    f.fx0 = fx - 0.5f * fw; f.fx1 = fx + 0.5f * fw; f.fy0 = fy - 0.5f * fh; f.fy1 = fy + 0.5f * fh;
+    f.farea = fw * fh;
+    f.fast_ok = (fw <= 2.0f) && (fh <= 2.0f);
+  }
+  f.thr_lo = p.thr - YL_IOU_EPS;
+  f.cx0 = (float)gx * invW - YL_CELL_MARGIN; f.cx1 = (float)(gx + 1) * invW + YL_CELL_MARGIN;
+  f.cy0 = (float)gy * invH - YL_CELL_MARGIN; f.cy1 = (float)(gy + 1) * invH + YL_CELL_MARGIN;
+  // the warp's 32 consecutive records cover a run of cells: rows gy(first)..gy(last); one row -> x range of
+  // the run, several rows -> full width.  (Superset of the nice lanes' cells: conservative.)
+  const uint32_t act = __ballot_sync(0xffffffffu, active);
+  if (act) {
+    const int first = __ffs(act) - 1, last = 31 - __clz(act);
+    const float first_x0 = __shfl_sync(0xffffffffu, f.cx0, first), first_y0 = __shfl_sync(0xffffffffu, f.cy0, first);
+    const float last_x1 = __shfl_sync(0xffffffffu, f.cx1, last), last_y1 = __shfl_sync(0xffffffffu, f.cy1, last);
+    const int gyf = __shfl_sync(0xffffffffu, gy, first), gyl = __shfl_sync(0xffffffffu, gy, last);
+    f.uy0 = first_y0; f.uy1 = last_y1;
+    f.ux0 = (gyf == gyl) ? first_x0 : -1.0f;
+    f.ux1 = (gyf == gyl) ? last_x1 : 2.0f;
+  }
+  f.any_rough = __any_sync(0xffffffffu, active && !f.nice);
+  f.lo_k = p.log_thr - YL_LOG_MARGIN; f.hi_k = -p.log_thr + YL_LOG_MARGIN;
+  return f;
+}
+
+// The filter proves metric < thr for this lane's record and the prepared GT (corners c; area, atan term, log area,
+// regular flag x).  All rejects as straight-line predicate arithmetic (bitwise, no short-circuit branches): the warp
+// executes the tests of every relevant GT anyway, and the divergence bookkeeping of early exits cost more than it saved.
+__device__ __forceinline__ bool yl_pair_rejected(const YlFilter& f, const float4 c, const float4 x) {
+  const float iw = fminf(f.fx1, c.z) - fmaxf(f.fx0, c.x), ih = fminf(f.fy1, c.w) - fmaxf(f.fy0, c.y);
+  const float inter = iw * ih;
+  const bool cell_rej = (f.cx1 < c.x) | (c.z < f.cx0) | (f.cy1 < c.y) | (c.w < f.cy0);
+  const bool win_rej = (f.sp < x.z + f.lo_k) | (f.sp > x.z + f.hi_k);
+  const bool dis_rej = (iw < -1e-5f) | (ih < -1e-5f);  // disjoint by far more than the decode error
+  const bool iou_rej = f.fast_ok & (iw >= YL_IOU_FLOOR) & (ih >= YL_IOU_FLOOR) & (inter < f.thr_lo * (f.farea + x.x - inter));
+  return f.nice & (x.w != 0.0f) & (cell_rej | win_rej | dis_rej | iou_rej);
+}
+
+// visit(g, c, x, rejected) for every GT g of the list that can touch the warp's strip of cells, in ascending order;
+// irregular GTs (x.w == 0) and warps with rough lanes take every GT.  The whole warp walks the same GTs.
+template <class Visit>
+__device__ __forceinline__ void yl_filter_gts(const YlFilter& f, const float4* gbox, const float4* gaux, int n_gt, Visit&& visit) {
+  const int lane = threadIdx.x & 31;
+  for (int j0 = 0; j0 < n_gt; j0 += 32) {
+    const int j = j0 + lane;
+    bool relevant = false;
+    if (j < n_gt) {
+      const float4 c = __ldg(gbox + j);
+      relevant = f.any_rough || (__ldg(gaux + j).w == 0.0f) || !((f.ux1 < c.x) || (c.z < f.ux0) || (f.uy1 < c.y) || (c.w < f.uy0));
+    }
+    uint32_t mask = __ballot_sync(0xffffffffu, relevant);
+    while (mask) {
+      const int g = j0 + __ffs(mask) - 1;
+      mask &= mask - 1u;
+      const float4 c = __ldg(gbox + g);
+      const float4 x = __ldg(gaux + g);
+      visit(g, c, x, yl_pair_rejected(f, c, x));
+    }
+  }
+}
+
 // Three phases per CTA of YL_ICHUNK (128) records:
 //  1. (all lanes, decode-free) each record tests the GTs that can touch its warp's strip of grid cells with the
 //     cell / logit-sum windows and pushes surviving (record, gt) pairs to a shared-memory queue;
@@ -314,9 +455,7 @@ __device__ __forceinline__ int yl_fastdiv(int n, uint32_t magic) {
 //  3. object_loss = obj*bce + (1-obj)*bce*ignore for every record.
 // The GT list is read straight from global memory (packed float4 pairs, L1-resident).
 #define YL_QCAP 1024
-#ifndef YL_IMINB
 #define YL_IMINB 8   // 64 registers: no spills; 10 (48 registers) spills and is 5 us slower
-#endif
 
 // exact decode of a record (tyu:57,61: xy = (sigmoid(t)+grid)/grid_wh ; wh = exp(t)*anchor/image_wh, no inf guard, Q7)
 __device__ __forceinline__ BoxT yl_decode_record(const YlParams& p, int l, int rin, float tx, float ty, float tw, float th) {
@@ -354,9 +493,9 @@ __device__ __forceinline__ bool yl_pair_hits(const YlParams& p, int l, int rin, 
   return yl_box_hits(p, pb, yl_regular(pb), c, x);
 }
 
-// PAIRED selects how the five logits of a record are fetched (see the load section): two lanes per record and one
-// request (y_pred in pinned host memory, read over PCIe) or two loads per lane (y_pred in HBM: 4 us faster there).
-template <bool PAIRED>
+// The single-kernel form.  Where a level is 16-byte aligned and a record holds at least 8 floats, two neighbouring lanes
+// fetch the five logits of a record with one request (see the load section): what bounds the kernel when y_pred is read
+// in place from pinned host memory over PCIe.  Other levels load the five floats one by one.
 __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(YlParams p) {
   __shared__ float4 s_t[YL_ICHUNK];
   __shared__ uint32_t s_q[YL_QCAP];
@@ -380,33 +519,12 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
   const int n_gt = p.gt_count[img * YL_LEVELS + l];
   const float4* gbox = p.gt_box + (size_t)img * p.n_img + p.lv.anchor_base[l];
   const float4* gaux = p.gt_aux + (size_t)img * p.n_img + p.lv.anchor_base[l];
-  const int W = p.lv.w[l], H = p.lv.h[l];
   float obj = 0.f, tx = 0.f, ty = 0.f, tw = 0.f, th = 0.f, pobj = 0.f;
   // block-uniform.  The two aligned 16-byte loads cover floats [f0 & ~3, (f0 & ~3) + 8): inside the tensor only when a
   // record holds at least 8 floats (C >= 3); narrower records take the scalar path
   const bool aligned = ((reinterpret_cast<uintptr_t>(p.lv.y_pred[l]) & 15) == 0) && (p.RF >= 8);
-  if (active) {
-    if (p.obj_bits) {
-      const int bit = p.lv.anchor_base[l] + rin;
-      obj = ((__ldg(p.obj_bits + (size_t)img * p.bits_words + (bit >> 5)) >> (bit & 31)) & 1u) ? 1.0f : 0.0f;
-    } else {
-      obj = p.obj_compact[(size_t)img * p.n_img + p.lv.anchor_base[l] + rin];
-    }
-  }
-  if (aligned && !PAIRED) {
-    if (active) {
-      // tx,ty,tw,th,conf sit at float offset f0; two aligned 16-byte loads cover them (L1 bypass)
-      const size_t f0 = ((size_t)img * rpi + rin) * p.RF;
-      const float4 lo = __ldcg(reinterpret_cast<const float4*>(p.lv.y_pred[l]) + (f0 >> 2));
-      const float4 hi = __ldcg(reinterpret_cast<const float4*>(p.lv.y_pred[l]) + (f0 >> 2) + 1);
-      // the record starts 0..3 floats into lo: rotate the 8 loaded floats left by sh with two select stages
-      const int sh = (int)(f0 & 3);
-      const bool s1 = sh & 1, s2 = sh & 2;
-      const float a0 = s1 ? lo.y : lo.x, a1 = s1 ? lo.z : lo.y, a2 = s1 ? lo.w : lo.z, a3 = s1 ? hi.x : lo.w;
-      const float a4 = s1 ? hi.y : hi.x, a5 = s1 ? hi.z : hi.y, a6 = s1 ? hi.w : hi.z;
-      tx = s2 ? a2 : a0; ty = s2 ? a3 : a1; tw = s2 ? a4 : a2; th = s2 ? a5 : a3; pobj = s2 ? a6 : a4;
-    }
-  } else if (aligned) {
+  if (active) obj = yl_obj(p, img, p.lv.anchor_base[l] + rin);
+  if (aligned) {
     // tx,ty,tw,th,conf of a record sit at float offset f0; the two aligned 16-byte chunks that cover them are fetched
     // by two neighbouring lanes of ONE load instruction (16 records per instruction, two instructions per warp), so a
     // record costs one memory request (one 128-byte line, 1-2 sectors) instead of two — this halves the request count,
@@ -422,30 +540,16 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
     }
     // lane r takes the pair loaded by lanes 2(r mod 16), 2(r mod 16)+1 of instruction r / 16
     const int src = (lane & 15) << 1;
-    const bool second = lane >= 16;
-    float4 lo, hi;
-    {
-      const float x0 = __shfl_sync(0xffffffffu, ld[0].x, src), x1 = __shfl_sync(0xffffffffu, ld[1].x, src);
-      const float y0 = __shfl_sync(0xffffffffu, ld[0].y, src), y1 = __shfl_sync(0xffffffffu, ld[1].y, src);
-      const float z0 = __shfl_sync(0xffffffffu, ld[0].z, src), z1 = __shfl_sync(0xffffffffu, ld[1].z, src);
-      const float w0 = __shfl_sync(0xffffffffu, ld[0].w, src), w1 = __shfl_sync(0xffffffffu, ld[1].w, src);
-      lo = second ? make_float4(x1, y1, z1, w1) : make_float4(x0, y0, z0, w0);
-    }
-    {
-      const float x0 = __shfl_sync(0xffffffffu, ld[0].x, src + 1), x1 = __shfl_sync(0xffffffffu, ld[1].x, src + 1);
-      const float y0 = __shfl_sync(0xffffffffu, ld[0].y, src + 1), y1 = __shfl_sync(0xffffffffu, ld[1].y, src + 1);
-      const float z0 = __shfl_sync(0xffffffffu, ld[0].z, src + 1), z1 = __shfl_sync(0xffffffffu, ld[1].z, src + 1);
-      const float w0 = __shfl_sync(0xffffffffu, ld[0].w, src + 1), w1 = __shfl_sync(0xffffffffu, ld[1].w, src + 1);
-      hi = second ? make_float4(x1, y1, z1, w1) : make_float4(x0, y0, z0, w0);
-    }
-    if (active) {
-      // the record starts 0..3 floats into lo: rotate the 8 loaded floats left by sh with two select stages
-      const int sh = (int)((((size_t)img * rpi + rin) * p.RF) & 3);
-      const bool s1 = sh & 1, s2 = sh & 2;
-      const float a0 = s1 ? lo.y : lo.x, a1 = s1 ? lo.z : lo.y, a2 = s1 ? lo.w : lo.z, a3 = s1 ? hi.x : lo.w;
-      const float a4 = s1 ? hi.y : hi.x, a5 = s1 ? hi.z : hi.y, a6 = s1 ? hi.w : hi.z;
-      tx = s2 ? a2 : a0; ty = s2 ? a3 : a1; tw = s2 ? a4 : a2; th = s2 ? a5 : a3; pobj = s2 ? a6 : a4;
-    }
+    auto take = [&](int from) {
+      float4 v[2];
+#pragma unroll
+      for (int t = 0; t < 2; ++t)
+        v[t] = make_float4(__shfl_sync(0xffffffffu, ld[t].x, from), __shfl_sync(0xffffffffu, ld[t].y, from),
+                           __shfl_sync(0xffffffffu, ld[t].z, from), __shfl_sync(0xffffffffu, ld[t].w, from));
+      return lane >= 16 ? v[1] : v[0];
+    };
+    const float4 lo = take(src), hi = take(src + 1);
+    if (active) yl_rotate5(lo, hi, (int)((((size_t)img * rpi + rin) * p.RF) & 3), tx, ty, tw, th, pobj);
   } else if (active) {
     const float* q = p.lv.y_pred[l] + ((size_t)img * rpi + rin) * p.RF;
     tx = __ldcg(q); ty = __ldcg(q + 1); tw = __ldcg(q + 2); th = __ldcg(q + 3); pobj = __ldcg(q + 4);
@@ -457,84 +561,18 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
     s_t[threadIdx.x] = make_float4(tx, ty, tw, th);
     __syncthreads();
     // ---------------- phase 1 ----------------
-    const int cell = yl_fastdiv(rin, p.magic_a);
-    const int a = min(rin - cell * p.A, 7);
-    const int gy = yl_fastdiv(cell, p.lv.magic_w[l]);
-    const int gx = cell - gy * W;
-    const bool filter_ok = p.thr >= 0.5f;
-    // lanes whose logits are in the range where the decode-free bounds are proven
-    const bool nice = active && filter_ok && (tw >= p.tmin_w[l][a]) && (tw <= 4.0f) && (th >= p.tmin_h[l][a]) &&
-                      (th <= 4.0f) && (tx == tx) && (ty == ty);
-    const float sp = tw + th + p.logk[l][a];
-    const float invW = 1.0f / (float)W, invH = 1.0f / (float)H;
-    // (c) approximate decode (MUFU exp / reciprocal; corner error < 2e-6 for boxes up to 2 image widths) for an
-    // IoU *upper-bound* reject: every metric of the family is <= IoU, so IoU_fast < thr - YL_IOU_EPS with both
-    // overlap extents >= YL_IOU_FLOOR (relative IoU error then < 3.2e-3, DESIGN.md) proves metric < thr.  Accepts
-    // are never decided here: pairs that survive go to the exact test.
-    float fx0 = 0.f, fy0 = 0.f, fx1 = 0.f, fy1 = 0.f, farea = 0.f;
-    bool fast_ok = false;
-    if (nice) {
-      const float ex = __expf(-fabsf(tx)), ey = __expf(-fabsf(ty));
-      const float rx = __fdividef(1.0f, 1.0f + ex), ry = __fdividef(1.0f, 1.0f + ey);
-      const float fx = ((tx >= 0.0f ? rx : ex * rx) + (float)gx) * invW, fy = ((ty >= 0.0f ? ry : ey * ry) + (float)gy) * invH;
-      const float fw = __expf(tw) * __fdividef(p.lv.anc_w[l][a], p.img_w), fh = __expf(th) * __fdividef(p.lv.anc_h[l][a], p.img_h);
-      fx0 = fx - 0.5f * fw; fx1 = fx + 0.5f * fw; fy0 = fy - 0.5f * fh; fy1 = fy + 0.5f * fh;
-      farea = fw * fh;
-      fast_ok = (fw <= 2.0f) && (fh <= 2.0f);
-    }
-    const float thr_lo = p.thr - YL_IOU_EPS;
-    // rectangle that certainly contains the decoded centre (grid cell grown by the margin)
-    const float cx0 = (float)gx * invW - YL_CELL_MARGIN, cx1 = (float)(gx + 1) * invW + YL_CELL_MARGIN;
-    const float cy0 = (float)gy * invH - YL_CELL_MARGIN, cy1 = (float)(gy + 1) * invH + YL_CELL_MARGIN;
-    // the warp's 32 consecutive records cover a run of cells: rows gy(first)..gy(last); one row -> x range of
-    // the run, several rows -> full width.  (Superset of the nice lanes' cells: conservative.)
-    const uint32_t act = __ballot_sync(0xffffffffu, active);
-    float ux0 = 0.f, ux1 = 0.f, uy0 = 0.f, uy1 = 0.f;
-    if (act) {
-      const int first = __ffs(act) - 1, last = 31 - __clz(act);
-      const float fx0 = __shfl_sync(0xffffffffu, cx0, first), fy0 = __shfl_sync(0xffffffffu, cy0, first);
-      const float lx1 = __shfl_sync(0xffffffffu, cx1, last), ly1 = __shfl_sync(0xffffffffu, cy1, last);
-      const int gyf = __shfl_sync(0xffffffffu, gy, first), gyl = __shfl_sync(0xffffffffu, gy, last);
-      uy0 = fy0; uy1 = ly1;
-      ux0 = (gyf == gyl) ? fx0 : -1.0f;
-      ux1 = (gyf == gyl) ? lx1 : 2.0f;
-    }
-    const bool any_rough = __any_sync(0xffffffffu, active && !nice);
-    const float lo_k = p.log_thr - YL_LOG_MARGIN, hi_k = -p.log_thr + YL_LOG_MARGIN;
-    for (int j0 = 0; j0 < n_gt; j0 += 32) {
-      const int j = j0 + lane;
-      bool relevant = false;
-      if (j < n_gt) {
-        const float4 c = __ldg(gbox + j);
-        // irregular GTs (aux.w == 0) and warps with rough lanes need every GT
-        relevant = any_rough || (__ldg(gaux + j).w == 0.0f) || !((ux1 < c.x) || (c.z < ux0) || (uy1 < c.y) || (c.w < uy0));
+    const YlFilter f = yl_filter_init(p, l, rin, active, tx, ty, tw, th);
+    yl_filter_gts(f, gbox, gaux, n_gt, [&](int g, const float4 c, const float4 x, bool rejected) {
+      if (!active | hit | rejected) return;
+      const int slot = atomicAdd(&s_nq, 1);
+      if (slot < YL_QCAP) s_q[slot] = (threadIdx.x << 24) | (uint32_t)g;            // drained in phase 2
+      else {  // queue full: exact test now.  The logits pass through an opaque asm so that the compiler cannot
+              // hoist the record decode in front of the filter loop (it did: ~200 instructions per warp, always).
+        float otx = tx, oty = ty, otw = tw, oth = th;
+        asm volatile("" : "+f"(otx), "+f"(oty), "+f"(otw), "+f"(oth));
+        if (yl_pair_hits(p, l, rin, otx, oty, otw, oth, c, x)) hit = true;
       }
-      uint32_t mask = __ballot_sync(0xffffffffu, relevant);
-      while (mask) {
-        const int g = j0 + __ffs(mask) - 1;
-        mask &= mask - 1u;
-        const float4 c = __ldg(gbox + g);
-        const float4 x = __ldg(gaux + g);  // area, atan term, log(area), regular flag
-        // all rejects as straight-line predicate arithmetic (bitwise, no short-circuit branches): the warp executes
-        // the tests of every relevant GT anyway, and the divergence bookkeeping of early exits cost more than it saved
-        const float iw = fminf(fx1, c.z) - fmaxf(fx0, c.x), ih = fminf(fy1, c.w) - fmaxf(fy0, c.y);
-        const float inter = iw * ih;
-        const bool cell_rej = (cx1 < c.x) | (c.z < cx0) | (cy1 < c.y) | (c.w < cy0);
-        const bool win_rej = (sp < x.z + lo_k) | (sp > x.z + hi_k);
-        const bool dis_rej = (iw < -1e-5f) | (ih < -1e-5f);  // disjoint by far more than the decode error
-        const bool iou_rej = fast_ok & (iw >= YL_IOU_FLOOR) & (ih >= YL_IOU_FLOOR) & (inter < thr_lo * (farea + x.x - inter));
-        const bool rejected = nice & (x.w != 0.0f) & (cell_rej | win_rej | dis_rej | iou_rej);
-        if (!active | hit | rejected) continue;
-        const int slot = atomicAdd(&s_nq, 1);
-        if (slot < YL_QCAP) s_q[slot] = (threadIdx.x << 24) | (uint32_t)g;            // drained in phase 2
-        else {  // queue full: exact test now.  The logits pass through an opaque asm so that the compiler cannot
-                // hoist the record decode in front of the filter loop (it did: ~200 instructions per warp, always).
-          float otx = tx, oty = ty, otw = tw, oth = th;
-          asm volatile("" : "+f"(otx), "+f"(oty), "+f"(otw), "+f"(oth));
-          if (yl_pair_hits(p, l, rin, otx, oty, otw, oth, c, x)) hit = true;
-        }
-      }
-    }
+    });
     if (hit) atomicOr(&s_hit[warp], 1u << lane);
     __syncthreads();
     // ---------------- phase 2 ----------------
@@ -552,35 +590,17 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
   }
   // ---------------- phase 3 ----------------
   float e = 0.f;
-  if (active) {
-    const float bc = yl_fast_bce(obj, pobj);
-    const float ign = hit ? 0.0f : 1.0f;
-    if (p.out_ignore) p.out_ignore[(size_t)img * p.n_img + p.lv.anchor_base[l] + rin] = hit ? 0 : 1;
-    e = obj * bc + (1.0f - obj) * bc * ign;  // tyu:114
-    if (p.conf_grad) {
-      // d/dp [obj*bce + (1-obj)*bce*ignore] = (sigmoid(p) - obj) * (obj + (1-obj)*ignore); the mask has no gradient
-      const float ex = __expf(-fabsf(pobj));
-      const float rr = 1.0f / (1.0f + ex);
-      const float sg = pobj >= 0.0f ? rr : ex * rr;
-      p.conf_grad[(size_t)p.B * p.lv.anchor_base[l] + (size_t)img * rpi + rin] = (sg - obj) * (obj + (1.0f - obj) * ign) * p.inv_div;
-    }
-  }
-  e = warp_sum(e);  // 32 fp32 terms; the cross-warp and cross-CTA sums are fp64
-  if (lane == 0) s_acc[warp] = (double)e;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double sum = 0;
-    for (int i = 0; i < YL_ICHUNK / 32; ++i) sum += s_acc[i];
-    p.partials[icta] = sum;
-  }
+  if (active) e = yl_record_term(p, l, img, p.lv.anchor_base[l] + rin, obj, pobj, hit, false);
+  yl_store_partial(p, icta, e, s_acc);
 }
 
-// ---- split form of K4b for predictions in device memory (the default there) ---------------------------------------
+// ---- split form of K4b: device-resident y_pred, every level 16-byte aligned, records of >= 8 floats ----------------
 // The filter of K4b rejects all but a few thousand (record, GT) pairs per batch; the exact decode + exact metric those few
 // need is what makes K4b a 64-register kernel (8 CTAs per SM, ~45 % of the warp slots).  Here the stream is split:
-//   K4b-lean   the same loads, the same decode-free / approximate-IoU rejects, BCE of every DECIDED record (no surviving
-//              pair => ignore = 1); a record with a surviving pair is only queued (one global id per record).  No
-//              shared-memory queue, no exact code: far fewer registers, no mid-kernel CTA barriers.
+//   K4b-lean   two aligned 16-byte loads per record, the same decode-free / approximate-IoU rejects (the filter helpers
+//              above), BCE of every DECIDED record (no surviving pair => ignore = 1); a record with a surviving pair is
+//              only queued (one global id per record).  No shared-memory queue, no exact code: far fewer registers, no
+//              mid-kernel CTA barriers.
 //   K4b-exact  a warp per queued record: the exact test (yl_pair_hits, with its own exact rejects) against EVERY ground
 //              truth of the record's (image, level), lanes <-> GTs; writes the record's ignore bit / gradient and adds its
 //              object-loss term to a 2^-32 fixed-point accumulator (integer atomics: the sum is order independent, so
@@ -589,8 +609,8 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
 // the ignore mask is bit-identical to K4b's.
 #define YL_FIXED_ONE 4294967296.0  // 2^32
 
-template <int MINB>
-__global__ void __launch_bounds__(YL_ICHUNK, MINB) yolo_loss_ignore_lean_kernel(YlParams p) {
+// 10 CTAs per SM (48 registers, no spills): the fastest headline step of 8, 10, 12 and 16 (profiles/r02_ab_measurements.txt)
+__global__ void __launch_bounds__(YL_ICHUNK, 10) yolo_loss_ignore_lean_kernel(YlParams p) {
   __shared__ double s_acc[YL_ICHUNK / 32];
   const int n_term_cta = YL_LEVELS * p.B * YL_TERM_SPLIT;
   const int n_icta = (int)gridDim.x - n_term_cta;
@@ -604,90 +624,24 @@ __global__ void __launch_bounds__(YL_ICHUNK, MINB) yolo_loss_ignore_lean_kernel(
   yl_locate(p.lv, icta, l, img, chunk);
   const int rpi = p.lv.rec_per_img[l];
   const int rin = chunk * YL_ICHUNK + (int)threadIdx.x;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31;
   const bool active = rin < rpi;
   const int n_gt = p.gt_count[img * YL_LEVELS + l];
   const float4* gbox = p.gt_box + (size_t)img * p.n_img + p.lv.anchor_base[l];
   const float4* gaux = p.gt_aux + (size_t)img * p.n_img + p.lv.anchor_base[l];
-  const int W = p.lv.w[l], H = p.lv.h[l];
   float obj = 0.f, tx = 0.f, ty = 0.f, tw = 0.f, th = 0.f, pobj = 0.f;
   if (active) {
-    if (p.obj_bits) {
-      const int bit = p.lv.anchor_base[l] + rin;
-      obj = ((__ldg(p.obj_bits + (size_t)img * p.bits_words + (bit >> 5)) >> (bit & 31)) & 1u) ? 1.0f : 0.0f;
-    } else {
-      obj = p.obj_compact[(size_t)img * p.n_img + p.lv.anchor_base[l] + rin];
-    }
+    obj = yl_obj(p, img, p.lv.anchor_base[l] + rin);
+    // tx,ty,tw,th,conf sit at float offset f0; two aligned 16-byte loads cover them (L1 bypass)
     const size_t f0 = ((size_t)img * rpi + rin) * p.RF;
     const float4 lo = __ldcg(reinterpret_cast<const float4*>(p.lv.y_pred[l]) + (f0 >> 2));
     const float4 hi = __ldcg(reinterpret_cast<const float4*>(p.lv.y_pred[l]) + (f0 >> 2) + 1);
-    const int sh = (int)(f0 & 3);
-    const bool s1 = sh & 1, s2 = sh & 2;
-    const float a0 = s1 ? lo.y : lo.x, a1 = s1 ? lo.z : lo.y, a2 = s1 ? lo.w : lo.z, a3 = s1 ? hi.x : lo.w;
-    const float a4 = s1 ? hi.y : hi.x, a5 = s1 ? hi.z : hi.y, a6 = s1 ? hi.w : hi.z;
-    tx = s2 ? a2 : a0; ty = s2 ? a3 : a1; tw = s2 ? a4 : a2; th = s2 ? a5 : a3; pobj = s2 ? a6 : a4;
+    yl_rotate5(lo, hi, (int)(f0 & 3), tx, ty, tw, th, pobj);
   }
   bool pending = false;  // some (record, GT) pair survives the rejects: K4b-exact decides
   if (n_gt > 0) {        // block-uniform
-    const int cell = yl_fastdiv(rin, p.magic_a);
-    const int a = min(rin - cell * p.A, 7);
-    const int gy = yl_fastdiv(cell, p.lv.magic_w[l]);
-    const int gx = cell - gy * W;
-    const bool filter_ok = p.thr >= 0.5f;
-    const bool nice = active && filter_ok && (tw >= p.tmin_w[l][a]) && (tw <= 4.0f) && (th >= p.tmin_h[l][a]) &&
-                      (th <= 4.0f) && (tx == tx) && (ty == ty);
-    const float sp = tw + th + p.logk[l][a];
-    const float invW = 1.0f / (float)W, invH = 1.0f / (float)H;
-    float fx0 = 0.f, fy0 = 0.f, fx1 = 0.f, fy1 = 0.f, farea = 0.f;
-    bool fast_ok = false;
-    if (nice) {
-      const float ex = __expf(-fabsf(tx)), ey = __expf(-fabsf(ty));
-      const float rx = __fdividef(1.0f, 1.0f + ex), ry = __fdividef(1.0f, 1.0f + ey);
-      const float fx = ((tx >= 0.0f ? rx : ex * rx) + (float)gx) * invW, fy = ((ty >= 0.0f ? ry : ey * ry) + (float)gy) * invH;
-      const float fw = __expf(tw) * __fdividef(p.lv.anc_w[l][a], p.img_w), fh = __expf(th) * __fdividef(p.lv.anc_h[l][a], p.img_h);
-      fx0 = fx - 0.5f * fw; fx1 = fx + 0.5f * fw; fy0 = fy - 0.5f * fh; fy1 = fy + 0.5f * fh;
-      farea = fw * fh;
-      fast_ok = (fw <= 2.0f) && (fh <= 2.0f);
-    }
-    const float thr_lo = p.thr - YL_IOU_EPS;
-    const float cx0 = (float)gx * invW - YL_CELL_MARGIN, cx1 = (float)(gx + 1) * invW + YL_CELL_MARGIN;
-    const float cy0 = (float)gy * invH - YL_CELL_MARGIN, cy1 = (float)(gy + 1) * invH + YL_CELL_MARGIN;
-    const uint32_t act = __ballot_sync(0xffffffffu, active);
-    float ux0 = 0.f, ux1 = 0.f, uy0 = 0.f, uy1 = 0.f;
-    if (act) {
-      const int first = __ffs(act) - 1, last = 31 - __clz(act);
-      const float f_x0 = __shfl_sync(0xffffffffu, cx0, first), f_y0 = __shfl_sync(0xffffffffu, cy0, first);
-      const float l_x1 = __shfl_sync(0xffffffffu, cx1, last), l_y1 = __shfl_sync(0xffffffffu, cy1, last);
-      const int gyf = __shfl_sync(0xffffffffu, gy, first), gyl = __shfl_sync(0xffffffffu, gy, last);
-      uy0 = f_y0; uy1 = l_y1;
-      ux0 = (gyf == gyl) ? f_x0 : -1.0f;
-      ux1 = (gyf == gyl) ? l_x1 : 2.0f;
-    }
-    const bool any_rough = __any_sync(0xffffffffu, active && !nice);
-    const float lo_k = p.log_thr - YL_LOG_MARGIN, hi_k = -p.log_thr + YL_LOG_MARGIN;
-    for (int j0 = 0; j0 < n_gt; j0 += 32) {
-      const int j = j0 + lane;
-      bool relevant = false;
-      if (j < n_gt) {
-        const float4 cg = __ldg(gbox + j);
-        relevant = any_rough || (__ldg(gaux + j).w == 0.0f) || !((ux1 < cg.x) || (cg.z < ux0) || (uy1 < cg.y) || (cg.w < uy0));
-      }
-      uint32_t mask = __ballot_sync(0xffffffffu, relevant);
-      while (mask) {
-        const int g = j0 + __ffs(mask) - 1;
-        mask &= mask - 1u;
-        const float4 cg = __ldg(gbox + g);
-        const float4 xg = __ldg(gaux + g);  // area, atan term, log(area), regular flag
-        const float iw = fminf(fx1, cg.z) - fmaxf(fx0, cg.x), ih = fminf(fy1, cg.w) - fmaxf(fy0, cg.y);
-        const float inter = iw * ih;
-        const bool cell_rej = (cx1 < cg.x) | (cg.z < cx0) | (cy1 < cg.y) | (cg.w < cy0);
-        const bool win_rej = (sp < xg.z + lo_k) | (sp > xg.z + hi_k);
-        const bool dis_rej = (iw < -1e-5f) | (ih < -1e-5f);
-        const bool iou_rej = fast_ok & (iw >= YL_IOU_FLOOR) & (ih >= YL_IOU_FLOOR) & (inter < thr_lo * (farea + xg.x - inter));
-        const bool rejected = nice & (xg.w != 0.0f) & (cell_rej | win_rej | dis_rej | iou_rej);
-        pending |= active & !rejected;
-      }
-    }
+    const YlFilter f = yl_filter_init(p, l, rin, active, tx, ty, tw, th);
+    yl_filter_gts(f, gbox, gaux, n_gt, [&](int, const float4, const float4, bool rejected) { pending |= active & !rejected; });
   }
   // queue the undecided records (warp-aggregated append), account for the decided ones
   {
@@ -700,25 +654,8 @@ __global__ void __launch_bounds__(YL_ICHUNK, MINB) yolo_loss_ignore_lean_kernel(
     }
   }
   float e = 0.f;
-  if (active && !pending) {
-    const float bc = yl_fast_bce(obj, pobj);
-    if (p.out_ignore) p.out_ignore[(size_t)img * p.n_img + p.lv.anchor_base[l] + rin] = 1;
-    e = obj * bc + (1.0f - obj) * bc;  // tyu:114 with ignore = 1
-    if (p.conf_grad) {
-      const float ex = __expf(-fabsf(pobj));
-      const float rr = 1.0f / (1.0f + ex);
-      const float sg = pobj >= 0.0f ? rr : ex * rr;
-      p.conf_grad[(size_t)p.B * p.lv.anchor_base[l] + (size_t)img * rpi + rin] = (sg - obj) * p.inv_div;   // obj + (1 - obj) * 1 = 1
-    }
-  }
-  e = warp_sum(e);  // 32 fp32 terms; the cross-warp and cross-CTA sums are fp64
-  if (lane == 0) s_acc[warp] = (double)e;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double sum = 0;
-    for (int i = 0; i < YL_ICHUNK / 32; ++i) sum += s_acc[i];
-    p.partials[icta] = sum;
-  }
+  if (active && !pending) e = yl_record_term(p, l, img, p.lv.anchor_base[l] + rin, obj, pobj, false, true);
+  yl_store_partial(p, icta, e, s_acc);
 }
 
 // the exact pass over the queued records: HALF a warp per record (two records in flight per warp: the pass is a chain of
@@ -741,9 +678,7 @@ __device__ __forceinline__ void yl_exact_pass(const YlParams& p, unsigned int gw
     const int rpi = p.lv.rec_per_img[l];
     const float* rec = p.lv.y_pred[l] + ((size_t)img * rpi + rin) * p.RF;
     const float tx = __ldg(rec), ty = __ldg(rec + 1), tw = __ldg(rec + 2), th = __ldg(rec + 3), pobj = __ldg(rec + 4);
-    float obj;
-    if (p.obj_bits) obj = ((__ldg(p.obj_bits + (size_t)img * p.bits_words + (ain >> 5)) >> (ain & 31)) & 1u) ? 1.0f : 0.0f;
-    else obj = p.obj_compact[(size_t)img * p.n_img + ain];
+    const float obj = yl_obj(p, img, ain);
     const int n_gt = valid ? p.gt_count[img * YL_LEVELS + l] : 0;
     const float4* gbox = p.gt_box + (size_t)img * p.n_img + p.lv.anchor_base[l];
     const float4* gaux = p.gt_aux + (size_t)img * p.n_img + p.lv.anchor_base[l];
@@ -762,19 +697,10 @@ __device__ __forceinline__ void yl_exact_pass(const YlParams& p, unsigned int gw
       hit = hit || ((bal >> (16 * half)) & 0xffffu) != 0u;
     }
     if (valid && sub == 0) {
-      const float bc = yl_fast_bce(obj, pobj);
-      const float ign = hit ? 0.0f : 1.0f;
-      if (p.out_ignore) p.out_ignore[(size_t)img * p.n_img + ain] = hit ? 0 : 1;
-      const float e = obj * bc + (1.0f - obj) * bc * ign;  // tyu:114
+      const float e = yl_record_term(p, l, img, ain, obj, pobj, hit, false);
       // non-finite terms (NaN / inf logits) cannot be carried in fixed point: they poison the sum through the top bit pattern
       if (e == e && e < 1.0e9f) atomicAdd(p.obj_fixed + l, (unsigned long long)((double)e * YL_FIXED_ONE + 0.5));
       else atomicOr(p.obj_fixed + l, 0x8000000000000000ull);
-      if (p.conf_grad) {
-        const float ex = __expf(-fabsf(pobj));
-        const float rr = 1.0f / (1.0f + ex);
-        const float sg = pobj >= 0.0f ? rr : ex * rr;
-        p.conf_grad[(size_t)p.B * p.lv.anchor_base[l] + (size_t)img * rpi + rin] = (sg - obj) * (obj + (1.0f - obj) * ign) * p.inv_div;
-      }
     }
   }
 }
@@ -786,12 +712,8 @@ __global__ void __launch_bounds__(128) yolo_loss_ignore_exact_kernel(YlParams p)
 // K4c: YL_FIN_CTAS CTAs each reduce an interleaved share of the per-CTA partials in fp64 (fixed assignment, fixed
 // order); the CTA that takes the last ticket adds the YL_FIN_CTAS slices in index order and writes parts / loss.
 // Deterministic run to run, and shorter than a single CTA walking all partials (shapes measured in DESIGN.md section 9).
-#ifndef YL_FIN_CTAS
 #define YL_FIN_CTAS 32
-#endif
-#ifndef YL_FIN_THREADS
 #define YL_FIN_THREADS 256
-#endif
 
 struct YlFinalize {
   const double* partials; const double* partials_obj;
@@ -1178,8 +1100,7 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
   p.pend_count = reinterpret_cast<unsigned int*>(wsb + ws.cnt) + (size_t)B * YL_LEVELS + 1;
   p.obj_fixed = reinterpret_cast<unsigned long long*>(wsb + ws.cnt + b200_align_up(sizeof(int32_t) * ((size_t)B * YL_LEVELS + 2), 8));
   // full dense call: the scan's last CTA per (image, level) prepares the GT list (stage hooks keep K4a' as its own launch)
-  { const char* e = getenv("B200_YL_SCAN_REV"); p.scan_reverse = e ? atoi(e) : 1; }
-  p.scan_ticket = (!sparse && (stages & 3) == 3 && !getenv("B200_YL_GTPREP_LAUNCH")) ? reinterpret_cast<unsigned int*>(p.obj_fixed + 3) : nullptr;
+  p.scan_ticket = (!sparse && (stages & 3) == 3) ? reinterpret_cast<unsigned int*>(p.obj_fixed + 3) : nullptr;
   p.sp_t = nullptr; p.sp_cls = nullptr; p.obj_bits = nullptr; p.bits_words = 0;
   if (sparse) {
     B200_REQUIRE(sparse->total_boxes >= 0 && sparse->offsets && sparse->assign_anchors_wh_host, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: null box arrays");
@@ -1208,7 +1129,8 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
   }
   bool use_split = false;
   if (stages & 4) {
-    // predictions in pinned host memory are read in place over PCIe: one request per record instead of two
+    // The split form needs device-resident y_pred, every level 16-byte aligned, and records of >= 8 floats.  Everything
+    // else takes the single kernel K4b, which reads pinned host predictions in place over PCIe with one request per record.
     cudaPointerAttributes attr;
     bool host_pred = false;
     if (cudaPointerGetAttributes(&attr, y_pred[YL_LEVELS - 1]) == cudaSuccess) host_pred = attr.type == cudaMemoryTypeHost;
@@ -1216,26 +1138,21 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
     const int grid = YL_LEVELS * B * YL_TERM_SPLIT + ws.n_cta;
     bool aligned16 = true;
     for (int l = 0; l < YL_LEVELS; ++l) aligned16 &= (reinterpret_cast<uintptr_t>(y_pred[l]) & 15) == 0;
-    // B200_YL_SPLIT = 0 selects the single kernel K4b, 8/10/12/16 the split form (CTAs per SM K4b-lean is compiled for;
-    // default 10).  Measured at 608x608 batch 64: K4b 71 us; K4b-lean 53.7 us (48 registers, 10 CTAs per SM); the exact pass
-    // over the ~12 k undecided records costs 15.6 us as a launch of its own and rides in the widened finalize launch instead.
-    const char* split_env = getenv("B200_YL_SPLIT");
-    const int split = split_env ? atoi(split_env) : 10;
-    use_split = !host_pred && aligned16 && p.RF >= 8 && split > 0;
+    // Measured at 608x608 batch 64: K4b 71 us; K4b-lean 53.7 us (48 registers, 10 CTAs per SM); the exact pass over the
+    // ~12 k undecided records costs 15.6 us as a launch of its own and rides in the widened finalize launch instead.
+    use_split = !host_pred && aligned16 && p.RF >= 8;
     if (use_split) {
       // the queue counter and the fixed-point sums are zeroed with the object counts (stage 1); the stage hook may run this
       // pass on its own, repeatedly
       if (!(stages & 1)) B200_CUDA(cudaMemsetAsync(p.pend_count, 0, (size_t)(reinterpret_cast<unsigned char*>(p.obj_fixed + 3) - reinterpret_cast<unsigned char*>(p.pend_count)), stream));
-      if (split >= 16) yolo_loss_ignore_lean_kernel<16><<<grid, YL_ICHUNK, 0, stream>>>(p);
-      else if (split >= 12) yolo_loss_ignore_lean_kernel<12><<<grid, YL_ICHUNK, 0, stream>>>(p);
-      else if (split >= 10) yolo_loss_ignore_lean_kernel<10><<<grid, YL_ICHUNK, 0, stream>>>(p);
-      else yolo_loss_ignore_lean_kernel<8><<<grid, YL_ICHUNK, 0, stream>>>(p);
+      yolo_loss_ignore_lean_kernel<<<grid, YL_ICHUNK, 0, stream>>>(p);
       if (!(stages & 8)) {   // no finalize in this call: the exact pass as a launch of its own (the finalize launch carries it otherwise)
         B200_LAUNCH_CHECK();
         yolo_loss_ignore_exact_kernel<<<1024, 128, 0, stream>>>(p);
       }
-    } else if (host_pred) yolo_loss_ignore_kernel<true><<<grid, YL_ICHUNK, 0, stream>>>(p);
-    else yolo_loss_ignore_kernel<false><<<grid, YL_ICHUNK, 0, stream>>>(p);
+    } else {
+      yolo_loss_ignore_kernel<<<grid, YL_ICHUNK, 0, stream>>>(p);
+    }
     B200_LAUNCH_CHECK();
   }
   if (!(stages & 8)) return B200_OK;
@@ -1249,13 +1166,10 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
   f.obj_fixed = p.obj_fixed;   // zero unless K4b-exact ran
   if (xchg) f.xchg = *xchg;
   else { f.xchg.rank = 0; f.xchg.world = 1; for (int r = 0; r < B200_XCHG_MAX_WORLD; ++r) f.xchg.mailbox[r] = nullptr; }
-  {
-    // split form: the finalize launch is widened and resolves the queued records first (default 4 CTAs per SM)
-    const char* fx = getenv("B200_YL_FINX_CTAS");
-    int wide = fx ? atoi(fx) : 4 * b200_sm_count();
-    if (wide < YL_FIN_CTAS) wide = YL_FIN_CTAS;
-    yolo_loss_finalize_kernel<<<use_split ? wide : YL_FIN_CTAS, YL_FIN_THREADS, 0, stream>>>(f, p, use_split ? 1 : 0);
-  }
+  // split form: the finalize launch is widened to 4 CTAs per SM and resolves the queued records first
+  int wide = 4 * b200_sm_count();
+  if (wide < YL_FIN_CTAS) wide = YL_FIN_CTAS;
+  yolo_loss_finalize_kernel<<<use_split ? wide : YL_FIN_CTAS, YL_FIN_THREADS, 0, stream>>>(f, p, use_split ? 1 : 0);
   B200_LAUNCH_CHECK();
   if (out_grad) {
     YlGradDense g;

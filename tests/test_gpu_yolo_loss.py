@@ -318,10 +318,32 @@ def test_get_loss_gradient_matches_oracle(lib, cuda, image, batch, iou_type):
         assert np.count_nonzero(np.delete(g[nobj], 4, axis=-1)) == 0
 
 
-def test_split_ignore_pass_is_bit_identical(lib, cuda, monkeypatch):
-    """The split form of the ignore pass (B200_YL_SPLIT: K4b-lean streams and filters, K4b-exact resolves the undecided
-    records) must give the ignore mask of the single kernel bit for bit and the same loss (the undecided records' terms go
-    through a 2^-32 fixed-point sum)."""
+def _offset_copy(t):
+    """The values of device tensor t in a new device buffer, 4 bytes past a 16-byte boundary.  GetLoss reads such a y_pred
+    with the single ignore kernel's scalar loads."""
+    import torch
+    buf = torch.empty(t.numel() + 4, dtype=t.dtype, device=t.device)
+    v = buf[1:1 + t.numel()].view(t.shape)
+    v.copy_(t)
+    assert v.data_ptr() % 16 == 4
+    return v
+
+
+def _ignore_layouts(heads):
+    """The same y_pred in the three layouts that select the forms of the ignore pass: 16-byte aligned device tensors (the
+    split form), device tensors at a 4-byte offset (the single kernel, scalar loads) and pinned host tensors (the single
+    kernel, paired loads)."""
+    assert all(h.is_cuda and h.data_ptr() % 16 == 0 for h in heads)
+    pinned = [h.cpu().pin_memory() for h in heads]
+    assert all(h.is_pinned() and h.data_ptr() % 16 == 0 for h in pinned)
+    return {"split": heads, "offset": [_offset_copy(h) for h in heads], "pinned": pinned}
+
+
+def test_split_ignore_pass_is_bit_identical(lib, cuda):
+    """The split form of the ignore pass (K4b-lean streams and filters, K4b-exact resolves the undecided records) must
+    give the ignore mask of the single kernel bit for bit and the same loss (the undecided records' terms go through a
+    2^-32 fixed-point sum).  The single kernel is reached through its real triggers: an unaligned y_pred and a pinned
+    host y_pred."""
     import torch
     from tfmv_b200 import synth
     from tfmv_b200.ai_models.datasets.coco_dataset import DataGenerator
@@ -350,17 +372,15 @@ def test_split_ignore_pass_is_bit_identical(lib, cuda, monkeypatch):
             hp[b, yy, xx, a, 3] = float(np.log(max(float(t[3]) * image / anc[l][a][1], 1e-6)))
     n_img = sum(int(t.shape[1] * t.shape[2] * 3) for t in y_true)
     out = {}
-    for mode in ("0", "10", "16"):
-        monkeypatch.setenv("B200_YL_SPLIT", mode)
+    for form, hp in _ignore_layouts(heads).items():
         ign = torch.zeros((batch, n_img), dtype=torch.uint8, device=cuda)
-        loss, parts = _loss_call(y_true, heads, (image, image), anc, 0.5, "ciou", 0, return_parts=True, ignore_out=ign)
-        out[mode] = (float(loss), parts.cpu().numpy(), ign.cpu().numpy())
-    assert out["0"][2].min() == 0 and out["0"][2].max() == 1          # the mask has both values
-    for mode in ("10", "16"):
-        assert np.array_equal(out[mode][2], out["0"][2]), mode
-        assert abs(out[mode][0] - out["0"][0]) <= 2e-6 * abs(out["0"][0]), (mode, out[mode][0], out["0"][0])
+        loss, parts = _loss_call(y_true, hp, (image, image), anc, 0.5, "ciou", 0, return_parts=True, ignore_out=ign)
+        out[form] = (float(loss), parts.cpu().numpy(), ign.cpu().numpy())
+    assert out["split"][2].min() == 0 and out["split"][2].max() == 1          # the mask has both values
+    for form in ("offset", "pinned"):
+        assert np.array_equal(out[form][2], out["split"][2]), form
+        assert abs(out[form][0] - out["split"][0]) <= 2e-6 * abs(out["split"][0]), (form, out[form][0], out["split"][0])
     # a NaN logit reaches the loss in both forms
     heads[2].view(y_true[2].shape)[0, 1, 1, 0, 4] = float("nan")
-    for mode in ("0", "10"):
-        monkeypatch.setenv("B200_YL_SPLIT", mode)
-        assert np.isnan(float(_loss_call(y_true, heads, (image, image), anc, 0.5, "ciou", 0))), mode
+    for form, hp in _ignore_layouts(heads).items():
+        assert np.isnan(float(_loss_call(y_true, hp, (image, image), anc, 0.5, "ciou", 0))), form

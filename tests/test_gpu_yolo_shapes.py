@@ -13,6 +13,7 @@ import pytest
 
 from test_gpu_core import _t, assert_bits_equal
 from test_gpu_yolo_decode import _check_image
+from test_gpu_yolo_loss import _offset_copy
 
 F = np.float32
 LOSS_RTOL = 1e-4
@@ -138,21 +139,22 @@ def _box_inputs(case):
 
 
 @gpu
-@pytest.mark.parametrize("split", ["0", "10"])
+@pytest.mark.parametrize("layout", ["aligned", "offset"])
 @pytest.mark.parametrize("case", LOSS_CASES, ids=_case_id)
-def test_get_loss_shapes(lib, cuda, monkeypatch, case, split):
-    """GetLoss in both ignore-pass forms (B200_YL_SPLIT 0: single kernel; 10: lean filter + exact pass, taken when
-    RF >= 8): ignore mask bit-exact, loss parts within 1e-4."""
+def test_get_loss_shapes(lib, cuda, case, layout):
+    """GetLoss in both ignore-pass forms: a 16-byte aligned device y_pred takes the lean filter + exact pass when
+    RF >= 8, the same values at a 4-byte offset take the single kernel.  Ignore mask bit-exact, loss parts within 1e-4."""
     import torch
     from oracle import yolo as oy
     from tfmv_b200.ai_models.utils.tf_yolo_utils import GetLoss, _loss_call
-    monkeypatch.setenv("B200_YL_SPLIT", split)
     image_wh, A, C, B, iou_type, thr = case
     y_true, y_pred, anc = _loss_inputs(case, 2.5)
     want, want_parts, want_ign = oy.get_loss(y_true, y_pred, image_wh, anc, thr, iou_type, return_ignore=True)
     assert 0 < int(want_ign.sum()) < want_ign.size
     ign = torch.full(want_ign.shape, 7, dtype=torch.uint8, device=cuda)
     dt, dp = [_t(t, cuda) for t in y_true], [_t(t, cuda) for t in y_pred]
+    if layout == "offset":
+        dp = [_offset_copy(t) for t in dp]
     got, parts = _loss_call(dt, dp, image_wh, anc, thr, iou_type, 0, return_parts=True, ignore_out=ign)
     g = ign.cpu().numpy()
     assert np.array_equal(g, want_ign), "%d ignore bits differ" % int((g != want_ign).sum())
@@ -320,11 +322,11 @@ def test_get_ground_truth_shapes(lib, cuda, image_wh, A, C):
 
 
 @gpu
-@pytest.mark.parametrize("early", ["0", "1"])
-def test_decode_filter_refill_forms(lib, cuda, monkeypatch, early):
-    """B200_YD_EARLY_ISSUE selects when a warp of the persistent decode filter refills its slab (before or after its
-    append).  The batch is large enough that the default picks the early refill (>= 32 tiles per warp: 4 warps per CTA
-    at C = 80, one CTA per SM); both forms must give the oracle's per-image results."""
+@pytest.mark.parametrize("refill", ["late", "early"])
+def test_decode_filter_refill_forms(lib, cuda, refill):
+    """A warp of the persistent decode filter refills its slab before its append on long streams (>= 32 tiles per warp:
+    4 warps per CTA at C = 80, one CTA per SM) and after it on short ones.  A batch large enough for the early refill and
+    its first 8 images, which take the late one, must both give the oracle's per-image results."""
     import torch
     from oracle import yolo as oy
     from tfmv_b200 import synth
@@ -335,9 +337,12 @@ def test_decode_filter_refill_forms(lib, cuda, monkeypatch, early):
     B = 8
     while tiles(B) < 32 * 4 * sms:
         B += 8
-    monkeypatch.setenv("B200_YD_EARLY_ISSUE", early)
     rng = _rng("refill", image)
     heads = synth.yolo_heads(rng, B, image)
+    if refill == "late":
+        B = 8
+        heads = [h[:B] for h in heads]
+        assert tiles(B) < 32 * 2 * sms   # short even if the filter ran 2 warps per CTA
     anc = synth.yolo_anchors()
     r = GetNMSBoxesBatch(*[_t(h, cuda) for h in heads], anc, (image, image), 80, *NMS_THR, "diou", with_indices=True)
     r = {k: v.cpu().numpy() for k, v in r.items()}
