@@ -6,6 +6,9 @@
 //   efficientnet/utils/anchors.py:161-202  convert_outputs_one            -> effdet_filter_kernel + effdet_nms_finalize_kernel
 //   efficientnet/utils/anchors.py:91-138, 219-243   generate_targets / _boxes_encoder -> effdet_assign_kernel
 //
+// The filter streams its class logits through the per-warp WarpSlabRing of bulkcopy.cuh, the same ring as the YOLO filter;
+// the filter and the fused eval-step stream share the candidate append (nms.cuh) and one box decode (ef_decode_box).
+//
 // Anchors are never read from HBM: every kernel rebuilds an anchor box from a tiny per-level table
 // (row centres yc[H], column centres xc[W], half extents hy[A], hx[A]; built on the host with the reference's own
 // double-precision Python arithmetic) exactly as the reference does — box = [yc-hy, xc-hx, yc+hy, xc+hx] in fp32,
@@ -45,6 +48,16 @@ __device__ __forceinline__ void ef_split(const EfLevels& lv, int l, int rin, int
   x = cell - y * lv.w[l];
 }
 
+// _boxes_decoder (anc:245-274): the box of anchor `an` from its head offsets rel = (ty, tx, th, tw)
+__device__ __forceinline__ float4 ef_decode_box(const AnchorBox& an, float4 rel) {
+  const float yca = DM_DIV(DM_ADD(an.y2, an.y1), 2.0f), xca = DM_DIV(DM_ADD(an.x2, an.x1), 2.0f);
+  const float ha = DM_SUB(an.y2, an.y1), wa = DM_SUB(an.x2, an.x1);
+  const float w = DM_MUL(dm_expf(rel.w), wa), h = DM_MUL(dm_expf(rel.z), ha);
+  const float yc = DM_ADD(DM_MUL(rel.x, ha), yca), xc = DM_ADD(DM_MUL(rel.y, wa), xca);
+  const float hh = DM_DIV(h, 2.0f), hw = DM_DIV(w, 2.0f);
+  return make_float4(DM_SUB(yc, hh), DM_SUB(xc, hw), DM_ADD(yc, hh), DM_ADD(xc, hw));
+}
+
 // ---- anchors -------------------------------------------------------------------------------------
 __global__ void effdet_anchors_kernel(EfLevels lv, int l, float4* __restrict__ out) {
   const int n = lv.anc_per_img[l];
@@ -78,13 +91,9 @@ __global__ void __launch_bounds__(256) effdet_decode_kernel(EfDecodeParams p) {
     int y, x, a;
     ef_split(p.lv, l, rin, y, x, a);
     const AnchorBox an = ef_anchor(p.lv, l, y, x, a);
-    const float yca = DM_DIV(DM_ADD(an.y2, an.y1), 2.0f), xca = DM_DIV(DM_ADD(an.x2, an.x1), 2.0f);
-    const float ha = DM_SUB(an.y2, an.y1), wa = DM_SUB(an.x2, an.x1);
-    const float4 r = __ldcs(p.rel[l] + e);  // ty, tx, th, tw
-    const float w = DM_MUL(dm_expf(r.w), wa), h = DM_MUL(dm_expf(r.z), ha);
-    const float yc = DM_ADD(DM_MUL(r.x, ha), yca), xc = DM_ADD(DM_MUL(r.y, wa), xca);
-    const float hh = DM_DIV(h, 2.0f), hw = DM_DIV(w, 2.0f);
-    __stcs(p.out[l] + e, make_float4(DM_SUB(yc, hh), DM_SUB(xc, hw), DM_ADD(yc, hh), DM_ADD(xc, hw)));
+    const float4 r = __ldcs(p.rel[l] + e);
+    const float4 b = ef_decode_box(an, r);
+    __stcs(p.out[l] + e, b);
   }
 }
 
@@ -104,22 +113,11 @@ struct EfFilterParams {
   uint32_t* bitmap; int bitmap_words;
 };
 
-__device__ __forceinline__ uint32_t ef_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
 __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p) {
   extern __shared__ __align__(128) unsigned char ef_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
   const int C = p.C;
-  const uint32_t slab_bytes = 128u * (uint32_t)C;
-  float* slab0 = reinterpret_cast<float*>(ef_smem) + (size_t)(warp * EF_STAGES) * (slab_bytes / 4);
-  uint64_t* bar0 = reinterpret_cast<uint64_t*>(ef_smem + (size_t)wpc * EF_STAGES * slab_bytes) + warp * EF_STAGES;
-  if (lane == 0) {
-#pragma unroll
-    for (int s = 0; s < EF_STAGES; ++s)
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(ef_smem_u32(bar0 + s)), "r"(1));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncwarp();
+  WarpSlabRing<EF_STAGES> ring(ef_smem, C);
   const long long n_tiles = p.tile_base[p.lv.num_levels];
   const long long gwarp = (long long)blockIdx.x * wpc + warp, gstride = (long long)gridDim.x * wpc;
 
@@ -134,34 +132,16 @@ __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p)
   auto issue = [&](long long tile, int s) {
     int l, nrec; long long rec0;
     locate(tile, l, rec0, nrec);
-    const float* src = p.cls[l] + ((long long)p.B0 * p.lv.anc_per_img[l] + rec0) * C;
-    const uint32_t bytes = (uint32_t)nrec * (uint32_t)C * 4u;
-    float* dst = slab0 + (size_t)s * (slab_bytes / 4);
-    if ((bytes & 15u) == 0u && (reinterpret_cast<uintptr_t>(src) & 15) == 0) {
-      if (lane == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(ef_smem_u32(bar0 + s)), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(ef_smem_u32(dst)),
-                     "l"(src), "r"(bytes), "r"(ef_smem_u32(bar0 + s)) : "memory");
-      }
-    } else {
-      for (int i = lane; i < nrec * C; i += 32) dst[i] = __ldg(src + i);
-      __syncwarp();
-      if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(ef_smem_u32(bar0 + s)) : "memory");
-    }
+    ring.issue(s, p.cls[l] + ((long long)p.B0 * p.lv.anc_per_img[l] + rec0) * C, nrec, C);
   };
   long long t_issue = gwarp;
 #pragma unroll
   for (int s = 0; s < EF_STAGES; ++s) { if (t_issue < n_tiles) issue(t_issue, s); t_issue += gstride; }
-  uint32_t phase = 0;
-  int stage = 0;
   for (long long tile = gwarp; tile < n_tiles; tile += gstride) {
-    {
-      const uint32_t bar = ef_smem_u32(bar0 + stage);
-      asm volatile("{\n.reg .pred p;\nEF_WAIT:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra EF_DONE;\nbra EF_WAIT;\nEF_DONE:\n}\n" ::"r"(bar), "r"(phase) : "memory");
-    }
+    ring.wait();
     int l, nrec; long long rec0;
     locate(tile, l, rec0, nrec);
-    const float* r = slab0 + (size_t)stage * (slab_bytes / 4) + lane * C;
+    const float* r = ring.slab(ring.stage) + lane * C;
     bool pass = false;
     int img = 0, cls = 0;
     float score = 0.f;
@@ -186,20 +166,14 @@ __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p)
     }
     // the class scan was the last read of the slab: its refill is in flight during the decode and the append below
     __syncwarp();
-    if (t_issue < n_tiles) issue(t_issue, stage);
+    if (t_issue < n_tiles) issue(t_issue, ring.stage);
     t_issue += gstride;
     if (lane < nrec) {
       if (fused_decode) {
-        // convert_outputs_boxes (_boxes_decoder, anc:245-274) for every anchor: the dense decoded tensor is an output
+        // convert_outputs_boxes for every anchor: the dense decoded tensor is an output
         int y, x, an_i;
         ef_split(p.lv, l, rin, y, x, an_i);
-        const AnchorBox an = ef_anchor(p.lv, l, y, x, an_i);
-        const float yca = DM_DIV(DM_ADD(an.y2, an.y1), 2.0f), xca = DM_DIV(DM_ADD(an.x2, an.x1), 2.0f);
-        const float ha = DM_SUB(an.y2, an.y1), wa = DM_SUB(an.x2, an.x1);
-        const float w = DM_MUL(dm_expf(r4.w), wa), h = DM_MUL(dm_expf(r4.z), ha);
-        const float yc = DM_ADD(DM_MUL(r4.x, ha), yca), xc = DM_ADD(DM_MUL(r4.y, wa), xca);
-        const float hh = DM_DIV(h, 2.0f), hw = DM_DIV(w, 2.0f);
-        box = make_float4(DM_SUB(yc, hh), DM_SUB(xc, hw), DM_ADD(yc, hh), DM_ADD(xc, hw));
+        box = ef_decode_box(ef_anchor(p.lv, l, y, x, an_i), r4);
         if (p.dec[l]) __stcs(p.dec[l] + grec, box);
       }
       if (mi != 0) {  // classes_mask = classes_id != 0 (anc:179)
@@ -208,22 +182,10 @@ __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p)
         if (!fused_decode) box = __ldg(p.boxes[l] + grec);
       }
     }
-    uint32_t todo = __ballot_sync(0xffffffffu, pass);
-    while (todo) {
-      const int leader = __ffs(todo) - 1;
-      const int limg = __shfl_sync(0xffffffffu, img, leader);
-      const uint32_t grp = __ballot_sync(0xffffffffu, pass && img == limg);
-      int base = 0;
-      if (lane == leader) base = atomicAdd(&p.counts[limg], __popc(grp));
-      base = __shfl_sync(0xffffffffu, base, leader);
-      if (pass && img == limg) {
-        const size_t slot = (size_t)limg * p.n_img + base + __popc(grp & ((1u << lane) - 1u));
-        p.cand_box[slot] = box; p.cand_score[slot] = score; p.cand_cls[slot] = cls; p.cand_aidx[slot] = aidx;
-        if (p.bitmap) atomicOr(&p.bitmap[(size_t)limg * p.bitmap_words + (aidx >> 5)], 1u << (aidx & 31u));
-      }
-      todo &= ~grp;
-    }
-    if (++stage == EF_STAGES) { stage = 0; phase ^= 1u; }
+    warp_append_by_image(pass, img, p.counts, p.n_img, p.bitmap, p.bitmap_words, aidx, [&](size_t slot) {
+      p.cand_box[slot] = box; p.cand_score[slot] = score; p.cand_cls[slot] = cls; p.cand_aidx[slot] = aidx;
+    });
+    ring.advance();
   }
 }
 
@@ -658,14 +620,12 @@ static int ef_post_impl(int num_levels, const int32_t* hw, int A, const float* t
   fp.bitmap = out_sel_idx ? reinterpret_cast<uint32_t*>(wsb + ws.bitmap) : nullptr;
   fp.bitmap_words = ws.bitmap_words;
   B200_CUDA(cudaMemsetAsync(wsb, 0, out_sel_idx ? ws.box : ws.bitmap, stream));
-  const uint32_t slab = 128u * (uint32_t)C;
+  using Ring = WarpSlabRing<EF_STAGES>;
   int warps = 8;
-  while (warps > 1 && (size_t)warps * EF_STAGES * slab + 256 > 200 * 1024) warps >>= 1;
-  const size_t smem1 = (size_t)warps * EF_STAGES * slab + sizeof(uint64_t) * warps * EF_STAGES + 16;
+  while (warps > 1 && Ring::smem_bytes(warps, C) > 200 * 1024) warps >>= 1;
+  const size_t smem1 = Ring::smem_bytes(warps, C);
   B200_CUDA(cudaFuncSetAttribute(effdet_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-  long long want = (tb + warps - 1) / warps;
-  int grid = (int)(want < (long long)b200_sm_count() ? want : (long long)b200_sm_count());
-  if (grid < 1) grid = 1;
+  const int grid = Ring::grid(tb, warps, b200_sm_count());
   effdet_filter_kernel<<<grid, warps * 32, smem1, stream>>>(fp);
   B200_LAUNCH_CHECK();
 
@@ -770,8 +730,8 @@ struct EfFusedParams {
 
 // Warp roles inside a CTA (tile = 64 anchors):
 //   warps 2-7 (CLASS stream, 192 threads): the tile's logits (and one-hot targets) arrive in shared memory by 1-D bulk
-//     asynchronous copies (cp.async.bulk + mbarrier, two stages: the copy of the CTA's next tile is in flight while this
-//     one is processed); focal terms from flat 128-bit shared-memory reads, then the per-anchor argmax with three lanes
+//     asynchronous copies (bulkcopy.cuh; two stages: the copy of the CTA's next tile is in flight while this one is
+//     processed); focal terms from flat 128-bit shared-memory reads, then the per-anchor argmax with three lanes
 //     per anchor (partial (max, first index) per third of the C logits -> shared memory);
 //   warps 0-1 (BOX half, lane <-> anchor): head offsets / box targets / mask straight from global memory, decode, Huber,
 //     and — behind the tile's single CTA barrier — the fold of the three argmax partials and the candidate append.
@@ -881,14 +841,7 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
         else { img = (int)(rec / api); rin = (int)(rec - (long long)img * api); }
         int y, x, an_i;
         ef_split(p.lv, l, rin, y, x, an_i);
-        const AnchorBox an = ef_anchor(p.lv, l, y, x, an_i);
-        // _boxes_decoder, anc:245-274 (the arithmetic of effdet_decode_kernel)
-        const float yca = DM_DIV(DM_ADD(an.y2, an.y1), 2.0f), xca = DM_DIV(DM_ADD(an.x2, an.x1), 2.0f);
-        const float ha = DM_SUB(an.y2, an.y1), wa = DM_SUB(an.x2, an.x1);
-        const float w = DM_MUL(dm_expf(r4.w), wa), h = DM_MUL(dm_expf(r4.z), ha);
-        const float yc = DM_ADD(DM_MUL(r4.x, ha), yca), xc = DM_ADD(DM_MUL(r4.y, wa), xca);
-        const float hh = DM_DIV(h, 2.0f), hw = DM_DIV(w, 2.0f);
-        d4 = make_float4(DM_SUB(yc, hh), DM_SUB(xc, hw), DM_ADD(yc, hh), DM_ADD(xc, hw));
+        d4 = ef_decode_box(ef_anchor(p.lv, l, y, x, an_i), r4);
         if (p.dec[l]) __stcs(p.dec[l] + rec, d4);
         if (WITH_LOSS) {
           hub += el_huber(t4.x, r4.x, p.delta) + el_huber(t4.y, r4.y, p.delta) + el_huber(t4.z, r4.z, p.delta) + el_huber(t4.w, r4.w, p.delta);
@@ -961,21 +914,9 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
 #pragma unroll
       for (int k = 1; k < 3; ++k) { const float vk = s_m[pb][tid][k]; if (vk > m) { m = vk; mi = s_mi[pb][tid][k]; } }
       const bool pass = (tid < nrec) && (mi != 0);   // classes_mask = classes_id != 0 (anc:179)
-      uint32_t todo = __ballot_sync(0xffffffffu, pass);
-      while (todo) {
-        const int leader = __ffs(todo) - 1;
-        const int limg = __shfl_sync(0xffffffffu, img, leader);
-        const uint32_t grp = __ballot_sync(0xffffffffu, pass && img == limg);
-        int base = 0;
-        if (lane == leader) base = atomicAdd(&p.counts[limg], __popc(grp));
-        base = __shfl_sync(0xffffffffu, base, leader);
-        if (pass && img == limg) {
-          const size_t slot = (size_t)limg * p.n_img + base + __popc(grp & ((1u << lane) - 1u));
-          p.cand_box[slot] = d4; p.cand_score[slot] = m; p.cand_cls[slot] = mi; p.cand_aidx[slot] = aidx;
-          if (p.bitmap) atomicOr(&p.bitmap[(size_t)limg * p.bitmap_words + (aidx >> 5)], 1u << (aidx & 31u));
-        }
-        todo &= ~grp;
-      }
+      warp_append_by_image(pass, img, p.counts, p.n_img, p.bitmap, p.bitmap_words, aidx, [&](size_t slot) {
+        p.cand_box[slot] = d4; p.cand_score[slot] = m; p.cand_cls[slot] = mi; p.cand_aidx[slot] = aidx;
+      });
     }
     // the partial buffers alternate by tile parity: the stream warps write buffer pb again only two tiles later, behind
     // the next tile's barrier, which the box warps reach after this append

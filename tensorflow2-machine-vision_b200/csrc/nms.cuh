@@ -64,6 +64,30 @@ struct NmsSegment {
   int n;
 };
 
+// Candidate store of a filter kernel: image i's candidates are slots [i * n_img, i * n_img + counts[i]) of every column,
+// in arbitrary order; bit aidx of the image's row of `bitmap` (when there is one) marks each appended flat anchor index.
+// warp_append_by_image appends the warp's lanes with `pass` set, grouped by image: one atomicAdd on counts[] per (warp,
+// image), a lane's slot from its rank among the lanes of its image.  store(slot) writes the caller's columns.
+template <class Store>
+__device__ __forceinline__ void warp_append_by_image(bool pass, int img, int32_t* counts, int n_img, uint32_t* bitmap,
+                                                     int bitmap_words, uint32_t aidx, Store store) {
+  const int lane = threadIdx.x & 31;
+  uint32_t todo = __ballot_sync(0xffffffffu, pass);
+  while (todo) {
+    const int leader = __ffs(todo) - 1;
+    const int limg = __shfl_sync(0xffffffffu, img, leader);
+    const uint32_t grp = __ballot_sync(0xffffffffu, pass && img == limg);
+    int base = 0;
+    if (lane == leader) base = atomicAdd(&counts[limg], __popc(grp));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (pass && img == limg) {
+      store((size_t)limg * n_img + base + __popc(grp & ((1u << lane) - 1u)));
+      if (bitmap) atomicOr(&bitmap[(size_t)limg * bitmap_words + (aidx >> 5)], 1u << (aidx & 31u));
+    }
+    todo &= ~grp;
+  }
+}
+
 // Optional pre-gathered first window of a segment (produced by nms_preselect_kernel with several CTAs per
 // segment, for segments too large for one CTA to scan quickly).  Ignored unless its counters show a valid window.
 struct NmsPre {

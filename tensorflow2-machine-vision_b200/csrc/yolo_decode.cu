@@ -5,21 +5,22 @@
 //
 // Kernel 1  yolo_decode_filter_kernel  (HBM-read bound: every head byte is read exactly once)
 //   * each level tensor is treated as a flat array of records of RF = 5+C floats; a warp owns tiles of 32
-//     records (32*RF*4 bytes, always a multiple of 16) staged into its own shared-memory ring by 1-D bulk
-//     async copies (cp.async.bulk + mbarrier, SASS UBLKCP); 16 warps per SM, each with its own tile in flight;
+//     records staged through its own WarpSlabRing (bulkcopy.cuh: one bulk copy per tile, a plain copy for a level's
+//     ragged tail); 16 warps per SM, each with its own tile in flight;
 //   * lane <-> record; the stride RF between lanes is odd for the 85-float COCO record so the column reads are
 //     bank-conflict free; conf is thresholded first, then the class maximum is found on raw logits and the
 //     sigmoid is evaluated only for logits inside a guard band of the maximum (max / first-argmax are taken
 //     in sigmoid space, exactly as tf.reduce_max / tf.argmax of sigmoid(classes) do; detmath's sigmoid is not
 //     monotone at ulp level, see oracle/DETMATH_REPORT.md);
 //   * survivors (valid box, conf > thr, score > thr: strict, tyu:163,191-192) are appended per image with
-//     warp-aggregated atomics.  Append order is arbitrary; each candidate carries its flat anchor index
-//     (level-major, then h, w, a) which is monotone in the reference's compaction order, so it serves as the
-//     NMS tie-break id and as the rank source for `sel_idx`.
+//     warp-aggregated atomics (warp_append_by_image, nms.cuh).  Append order is arbitrary; each candidate carries its
+//     flat anchor index (level-major, then h, w, a) which is monotone in the reference's compaction order, so it
+//     serves as the NMS tie-break id and as the rank source for `sel_idx`.
 // Kernel 2  yolo_nms_finalize_kernel  (one CTA per image): nms.cuh greedy NMS + gather of the five outputs,
 //   recomputing sigmoid(classes) for the <= max_out selected rows straight from the head tensors.
 #include <cmath>
 #include "nms.cuh"
+#include "bulkcopy.cuh"
 
 #define YD_MAX_LEVELS 3
 #define YD_STAGES 1
@@ -50,35 +51,6 @@ struct YoloDecodeParams {
   uint32_t* bitmap;    // [B, bitmap_words] or nullptr
   int bitmap_words;
 };
-
-// ---- mbarrier / bulk-copy PTX -----------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_LOOP:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE;\n"
-      "bra WAIT_LOOP;\n"
-      "DONE:\n"
-      "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
 
 // max and first-argmax of sigmoid(x_c), c in [0,C), for the warp's 32 records (lane <-> record, stride RF in shared
 // memory, conflict-free).  One pass per lane keeps the largest logit with its first index and the second largest
@@ -201,20 +173,7 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
   const int warp = threadIdx.x >> 5;
   const int warps_per_cta = blockDim.x >> 5;
   const int RF = p.RF;
-  const uint32_t slab_bytes = 128u * (uint32_t)RF;
-  // layout: [warps][stages] slabs, then barriers
-  float* slabs = reinterpret_cast<float*>(yd_smem);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(yd_smem + (size_t)warps_per_cta * YD_STAGES * slab_bytes);
-  float* const slab0 = slabs + (size_t)(warp * YD_STAGES) * (slab_bytes / 4);
-  uint64_t* const bar0 = bars + warp * YD_STAGES;
-#define my_slab(s) (slab0 + (size_t)(s) * (slab_bytes / 4))
-#define my_bar(s) (bar0 + (s))
-  if (lane == 0) {
-#pragma unroll
-    for (int s = 0; s < YD_STAGES; ++s) mbar_init(my_bar(s), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncwarp();
+  WarpSlabRing<YD_STAGES> ring(yd_smem, RF);
 
   const long long n_tiles = p.lv.tile_base[YD_MAX_LEVELS];
   const long long gwarp = (long long)blockIdx.x * warps_per_cta + warp;
@@ -227,19 +186,7 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
     for (int k = 1; k < YD_MAX_LEVELS; ++k) if (tile >= p.lv.tile_base[k]) l = k;
     const long long rec0 = (tile - p.lv.tile_base[l]) * 32;
     const long long remain = p.lv.total_rec[l] - rec0;
-    const int nrec = remain < 32 ? (int)remain : 32;
-    const float* src = p.lv.head[l] + rec0 * RF;
-    const uint32_t bytes = (uint32_t)nrec * (uint32_t)RF * 4u;
-    if ((bytes & 15u) == 0u) {
-      if (lane == 0) {
-        mbar_expect_tx(my_bar(s), bytes);
-        bulk_g2s(my_slab(s), src, bytes, my_bar(s));
-      }
-    } else {  // ragged tail of a level: plain copy, then a transaction-less arrive flips the same phase
-      for (int i = lane; i < nrec * RF; i += 32) my_slab(s)[i] = __ldg(src + i);
-      __syncwarp();
-      if (lane == 0) mbar_arrive(my_bar(s));
-    }
+    ring.issue(s, p.lv.head[l] + rec0 * RF, remain < 32 ? (int)remain : 32, RF);
   };
 
   long long t_issue = gwarp;
@@ -248,16 +195,15 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
     if (t_issue < n_tiles) issue(t_issue, s);
     t_issue += gstride;
   }
-  uint32_t phase = 0;
-  int stage = 0;
   for (long long tile = gwarp; tile < n_tiles; tile += gstride) {
-    mbar_wait(my_bar(stage), phase);
+    ring.wait();
+    const float* slab = ring.slab(ring.stage);
     int l = 0;
 #pragma unroll
     for (int k = 1; k < YD_MAX_LEVELS; ++k) if (tile >= p.lv.tile_base[k]) l = k;
     const long long rec = (tile - p.lv.tile_base[l]) * 32 + lane;
     const bool in_range = rec < p.lv.total_rec[l];
-    const float* r = my_slab(stage) + lane * RF;
+    const float* r = slab + lane * RF;
     bool pass = false;
     int img = 0;
     float score = 0.f, conf = 0.f;
@@ -270,7 +216,7 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
       if (conf > p.conf_hi) want = true;
       else if (conf >= p.conf_lo) want = dm_sigmoidf(conf) > p.conf_thr;  // NaN fails both comparisons: not wanted
     }
-    class_max_sigmoid_warp(my_slab(stage), RF, p.C, want, lane, score, cls);
+    class_max_sigmoid_warp(slab, RF, p.C, want, lane, score, cls);
     if (want && score > p.score_thr) {
       const int rpi = p.lv.rec_per_img[l];
       // 32-bit division when the level has fewer than 2^31 records (always, short of ~100k-image batches)
@@ -295,34 +241,21 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
     // below (an atomic round trip to L2 plus the stores — 9 % of the warp's cycle when the copy was issued after it).
     if (EARLY) {
       __syncwarp();
-      if (t_issue < n_tiles) issue(t_issue, stage);
+      if (t_issue < n_tiles) issue(t_issue, ring.stage);
       t_issue += gstride;
     }
-    // warp-aggregated append, one atomic per (warp, image)
-    uint32_t todo = __ballot_sync(0xffffffffu, pass);
-    while (todo) {
-      const int leader = __ffs(todo) - 1;
-      const int limg = __shfl_sync(0xffffffffu, img, leader);
-      const uint32_t grp = __ballot_sync(0xffffffffu, pass && img == limg);
-      int base = 0;
-      if (lane == leader) base = atomicAdd(&p.counts[limg], __popc(grp));
-      base = __shfl_sync(0xffffffffu, base, leader);
-      if (pass && img == limg) {
-        const size_t slot = (size_t)limg * p.n_img + base + __popc(grp & ((1u << lane) - 1u));
-        p.cand_score[slot] = score;
-        p.cand_cls[slot] = cls;
-        p.cand_conf[slot] = conf;  // the logit; the sigmoid is applied to the emitted rows only
-        p.cand_aidx[slot] = aidx;
-        if (p.bitmap) atomicOr(&p.bitmap[(size_t)limg * p.bitmap_words + (aidx >> 5)], 1u << (aidx & 31u));
-      }
-      todo &= ~grp;
-    }
+    warp_append_by_image(pass, img, p.counts, p.n_img, p.bitmap, p.bitmap_words, aidx, [&](size_t slot) {
+      p.cand_score[slot] = score;
+      p.cand_cls[slot] = cls;
+      p.cand_conf[slot] = conf;  // the logit; the sigmoid is applied to the emitted rows only
+      p.cand_aidx[slot] = aidx;
+    });
     if (!EARLY) {
       __syncwarp();  // every lane is done reading the slab before it is refilled
-      if (t_issue < n_tiles) issue(t_issue, stage);
+      if (t_issue < n_tiles) issue(t_issue, ring.stage);
       t_issue += gstride;
     }
-    if (++stage == YD_STAGES) { stage = 0; phase ^= 1u; }
+    ring.advance();
   }
 }
 
@@ -588,18 +521,16 @@ extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t h
   // counts and bitmap are adjacent at the front of the workspace: one memset
   B200_CUDA(cudaMemsetAsync(wsb, 0, out_sel_idx ? ws.box : ws.bitmap, stream));
 
-  const uint32_t slab = 128u * (uint32_t)dp.RF;
+  using Ring = WarpSlabRing<YD_STAGES>;
   int warps = 16;  // one tile in flight per warp; the warps of an SM overlap each other's loads
-  while (warps > 1 && (size_t)warps * YD_STAGES * slab + 256 > 200 * 1024) warps >>= 1;
+  while (warps > 1 && Ring::smem_bytes(warps, dp.RF) > 200 * 1024) warps >>= 1;
   // a single image has fewer tiles than the GPU has warp slots: spread them (one warp per scheduler finishes its tile sooner)
   while (warps > 2 && dp.lv.tile_base[YD_MAX_LEVELS] <= (long long)(warps / 2) * b200_sm_count()) warps >>= 1;
-  B200_REQUIRE((size_t)warps * YD_STAGES * slab + 256 <= 220 * 1024, B200_ERR_UNSUPPORTED, "b200_yolo_decode_nms: record too large (C=%d)", C);
-  const size_t smem1 = (size_t)warps * YD_STAGES * slab + sizeof(uint64_t) * warps * YD_STAGES + 16;
+  const size_t smem1 = Ring::smem_bytes(warps, dp.RF);
+  B200_REQUIRE(smem1 <= 220 * 1024, B200_ERR_UNSUPPORTED, "b200_yolo_decode_nms: record too large (C=%d)", C);
 
   const long long n_tiles = dp.lv.tile_base[YD_MAX_LEVELS];
-  long long want = (n_tiles + warps - 1) / warps;
-  int grid = (int)(want < (long long)b200_sm_count() ? want : (long long)b200_sm_count());
-  if (grid < 1) grid = 1;
+  const int grid = Ring::grid(n_tiles, warps, b200_sm_count());
   // Refilling a warp's slab before its append keeps one more copy in flight: -3 % for the call on its own at any size, and
   // for the fused evaluation step at 512 images; at 64 images per GPU the same step is 3 % SLOWER with it (the filter then
   // takes DRAM bandwidth from the loss chain that shares the GPU, and that chain is the longer one there).  Long streams
