@@ -45,8 +45,7 @@ def build(force=False, verbose=False):
     os.makedirs(os.path.join(HERE, "build"), exist_ok=True)
     for src in _sources():
         obj = os.path.join(HERE, "build", os.path.basename(src)[:-3] + ".o")
-        extra = os.environ.get("B200_EXTRA_NVCC_FLAGS", "").split()  # tuning builds (-DNMS_TRACE ...)
-        cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
+        cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
         objs.append(obj)
     failed = False

@@ -7,7 +7,9 @@
 //   efficientnet/utils/anchors.py:91-138, 219-243   generate_targets / _boxes_encoder -> effdet_assign_kernel
 //
 // The filter streams its class logits through the per-warp WarpSlabRing of bulkcopy.cuh, the same ring as the YOLO filter;
-// the filter and the fused eval-step stream share the candidate append (nms.cuh) and one box decode (ef_decode_box).
+// the filter and the fused eval-step stream share one box decode (ef_decode_box) and append to the candidate store of
+// nms.cuh (CandStore: workspace layout, append and NMS output tail, shared with yolo_decode.cu; EfficientDet adds the
+// buffers of the multi-CTA pre-selection).
 //
 // Anchors are never read from HBM: every kernel rebuilds an anchor box from a tiny per-level table
 // (row centres yc[H], column centres xc[W], half extents hy[A], hx[A]; built on the host with the reference's own
@@ -102,15 +104,12 @@ struct EfFilterParams {
   EfLevels lv;
   int B0, NB, C;                 // images [B0, B0+NB) of a batch of size B
   int B;
-  int n_img;                     // anchors per image
   const float* cls[EF_MAX_LEVELS];    // (B,H,W,A,C) logits
   const float4* boxes[EF_MAX_LEVELS]; // (B,H,W,A,4) decoded, or null: decode here from rel (lv.table must be set)
   const float4* rel[EF_MAX_LEVELS];   // (B,H,W,A,4) head offsets ty,tx,th,tw (fused decode mode)
   float4* dec[EF_MAX_LEVELS];         // fused decode mode: the dense decoded tensor is written here (may be null)
   long long tile_base[EF_MAX_LEVELS + 1];  // tiles of 32 anchors over the NB images of each level
-  float4* cand_box; float* cand_score; int32_t* cand_cls; uint32_t* cand_aidx;  // [NB, n_img]
-  int32_t* counts;               // [NB]
-  uint32_t* bitmap; int bitmap_words;
+  CandStore st;                  // [NB] images
 };
 
 __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p) {
@@ -182,82 +181,47 @@ __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p)
         if (!fused_decode) box = __ldg(p.boxes[l] + grec);
       }
     }
-    warp_append_by_image(pass, img, p.counts, p.n_img, p.bitmap, p.bitmap_words, aidx, [&](size_t slot) {
-      p.cand_box[slot] = box; p.cand_score[slot] = score; p.cand_cls[slot] = cls; p.cand_aidx[slot] = aidx;
+    warp_append_by_image(p.st, pass, img, aidx, [&](size_t slot) {
+      p.st.box[slot] = box; p.st.score[slot] = score; p.st.cls[slot] = cls;
     });
     ring.advance();
   }
 }
 
 struct EfFinalizeParams {
-  int NB, n_img;
   NmsConfig cfg;
-  const float4* cand_box; const float* cand_score; const int32_t* cand_cls; const uint32_t* cand_aidx;
-  const int32_t* counts; const uint32_t* bitmap; int bitmap_words;
-  int32_t* nms_pos;
-  const unsigned long long* pre_keys; const uint32_t* pre_pos; const int* pre_count; const int* pre_elig;
-  const unsigned long long* pre_khi;  // all nullptr when the pre-selection kernel was not run
+  CandStore st;
   float* out_boxes; long long* out_cls; float* out_score; int32_t* out_sel_idx; int32_t* out_sel_anchor; int32_t* out_count;
 };
 
 template <int METRIC>
 __global__ void __launch_bounds__(NMS_THREADS, 1) effdet_nms_finalize_kernel(EfFinalizeParams p) {
   extern __shared__ __align__(16) unsigned char nms_smem[];
-  NMS_T(13);
   const int img = blockIdx.x;
-  const size_t cbase = (size_t)img * p.n_img;
-  NmsSegment seg;
-  seg.boxes = reinterpret_cast<const float*>(p.cand_box + cbase);
-  seg.scores = p.cand_score + cbase;
-  seg.classes = nullptr;
-  seg.order_id = p.cand_aidx + cbase;
-  seg.n = p.counts[img];
-  int32_t* pos = p.nms_pos + (size_t)img * p.cfg.max_out;
+  const size_t cbase = (size_t)img * p.st.n_img;
+  int32_t* pos = p.st.pos + (size_t)img * p.cfg.max_out;
   NmsPre pre;
-  if (p.pre_keys) {
-    pre.keys = p.pre_keys + (size_t)img * NMS_PRE_CAP; pre.pos = p.pre_pos + (size_t)img * NMS_PRE_CAP;
-    pre.count = p.pre_count + img; pre.eligible = p.pre_elig + img; pre.khi = p.pre_khi + img;
+  if (p.st.pre_keys) {
+    pre.keys = p.st.pre_keys + (size_t)img * NMS_PRE_CAP; pre.pos = p.st.pre_pos + (size_t)img * NMS_PRE_CAP;
+    pre.count = p.st.pre_count + img; pre.eligible = p.st.pre_elig + img; pre.khi = p.st.pre_khi + img;
   }
-  const int kept = nms_run_segment<METRIC, NmsLoadDirectAgnostic>(seg, p.cfg, pos, nms_smem, p.pre_keys ? &pre : nullptr);
+  const int kept = nms_run_segment<METRIC, NmsLoadDirectAgnostic>(cand_segment(p.st, img, false), p.cfg, pos, nms_smem,
+                                                                  p.st.pre_keys ? &pre : nullptr);
   __syncthreads();
-  NMS_T(11);
   if (threadIdx.x == 0) p.out_count[img] = kept;
   const size_t obase = (size_t)img * p.cfg.max_out;
   uint32_t* wprefix = reinterpret_cast<uint32_t*>(nms_smem);
-  if (p.out_sel_idx && p.bitmap) {
-    const uint32_t* bm = p.bitmap + (size_t)img * p.bitmap_words;
-    if (threadIdx.x < 32) {
-      uint32_t run = 0;
-      for (int w0 = 0; w0 < p.bitmap_words; w0 += 32) {
-        const int w = w0 + (int)threadIdx.x;
-        const int c = (w < p.bitmap_words) ? __popc(bm[w]) : 0;
-        const int inc = warp_scan_incl(c);
-        if (w < p.bitmap_words) wprefix[w] = run + (uint32_t)(inc - c);
-        run += (uint32_t)__shfl_sync(0xffffffffu, inc, 31);
-      }
-    }
-    __syncthreads();
-  }
+  cand_word_prefix(p.st, img, wprefix);
   for (int k = threadIdx.x; k < kept; k += blockDim.x) {
     const int q = pos[k];
-    reinterpret_cast<float4*>(p.out_boxes)[obase + k] = p.cand_box[cbase + q];
-    p.out_cls[obase + k] = (long long)p.cand_cls[cbase + q];               // tf.argmax -> int64 (anc:172)
-    p.out_score[obase + k] = dm_sigmoidf(p.cand_score[cbase + q]);          // sigmoid only on survivors (anc:200)
-    const uint32_t a = p.cand_aidx[cbase + q];
+    reinterpret_cast<float4*>(p.out_boxes)[obase + k] = p.st.box[cbase + q];
+    p.out_cls[obase + k] = (long long)p.st.cls[cbase + q];               // tf.argmax -> int64 (anc:172)
+    p.out_score[obase + k] = dm_sigmoidf(p.st.score[cbase + q]);          // sigmoid only on survivors (anc:200)
+    const uint32_t a = p.st.aidx[cbase + q];
     if (p.out_sel_anchor) p.out_sel_anchor[obase + k] = (int32_t)a;
-    if (p.out_sel_idx && p.bitmap) {
-      const uint32_t wv = p.bitmap[(size_t)img * p.bitmap_words + (a >> 5)];
-      p.out_sel_idx[obase + k] = (int32_t)(wprefix[a >> 5] + __popc(wv & ((1u << (a & 31u)) - 1u)));
-    }
+    if (p.out_sel_idx) p.out_sel_idx[obase + k] = cand_sel_idx(p.st, img, wprefix, a);
   }
-  NMS_T(12);
 }
-
-#ifdef NMS_TRACE
-extern "C" int b200_debug_nms_trace_effdet(long long* out_host64) {
-  return cudaMemcpyFromSymbol(out_host64, g_nms_trace, sizeof(long long) * (64 + 4 * 32)) == cudaSuccess ? 0 : -1;
-}
-#endif
 
 // ---- target assignment (anc:91-138) ------------------------------------------------------------------
 struct EfAssignParams {
@@ -491,27 +455,6 @@ extern "C" int b200_effdet_decode(int num_levels, const int32_t* hw, int A, cons
   return B200_OK;
 }
 
-struct EfWs { size_t counts, pre_count, pre_elig, bitmap, box, score, cls, aidx, pos, pre_khi, pre_keys, pre_pos, total; int bitmap_words; };
-static EfWs ef_ws_layout(int NB, int n_img, int max_out) {
-  EfWs w;
-  size_t o = 0;
-  w.bitmap_words = (n_img + 31) / 32;
-  w.counts = o; o = b200_align_up(o + sizeof(int32_t) * NB, 256);
-  w.pre_count = o; o = b200_align_up(o + sizeof(int32_t) * NB, 256);   // zeroed together with counts
-  w.pre_elig = o; o = b200_align_up(o + sizeof(int32_t) * NB, 256);
-  w.bitmap = o; o = b200_align_up(o + sizeof(uint32_t) * (size_t)NB * w.bitmap_words, 256);
-  w.box = o; o = b200_align_up(o + sizeof(float4) * (size_t)NB * n_img, 256);
-  w.score = o; o = b200_align_up(o + sizeof(float) * (size_t)NB * n_img, 256);
-  w.cls = o; o = b200_align_up(o + sizeof(int32_t) * (size_t)NB * n_img, 256);
-  w.aidx = o; o = b200_align_up(o + sizeof(uint32_t) * (size_t)NB * n_img, 256);
-  w.pos = o; o = b200_align_up(o + sizeof(int32_t) * (size_t)NB * max_out, 256);
-  w.pre_khi = o; o = b200_align_up(o + sizeof(unsigned long long) * NB, 256);
-  w.pre_keys = o; o = b200_align_up(o + sizeof(unsigned long long) * (size_t)NB * NMS_PRE_CAP, 256);
-  w.pre_pos = o; o = b200_align_up(o + sizeof(uint32_t) * (size_t)NB * NMS_PRE_CAP, 256);
-  w.total = o;
-  return w;
-}
-
 __global__ void __launch_bounds__(NMS_THREADS, 1) effdet_nms_pivot_kernel(NmsPreselectParams p) {
   extern __shared__ __align__(16) unsigned char pre_smem[];
   nms_pivot_body(p, pre_smem);
@@ -520,42 +463,32 @@ __global__ void __launch_bounds__(256) effdet_nms_pregather_kernel(NmsPreselectP
 
 // The NMS tail shared by b200_effdet_postprocess and the fused entry points: (large segments) pivot + multi-CTA
 // pre-gather of the first window, then one CTA per image.
-static int ef_launch_nms(const EfFilterParams& fp, const EfWs& ws, unsigned char* wsb, int num_images, int n_img, int max_out,
-                         float iou_thr, float score_thr, int metric, float* out_boxes, long long* out_class_id, float* out_score,
-                         int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count, cudaStream_t stream) {
+static int ef_launch_nms(const CandStore& st, int num_images, int max_out, float iou_thr, float score_thr, int metric,
+                         float* out_boxes, long long* out_class_id, float* out_score, int32_t* out_sel_idx,
+                         int32_t* out_sel_anchor, int32_t* out_count, cudaStream_t stream) {
   EfFinalizeParams np;
-  np.NB = num_images; np.n_img = n_img;
   np.cfg.metric = metric; np.cfg.mode = B200_NMS_AGNOSTIC; np.cfg.iou_thr = iou_thr; np.cfg.score_thr = score_thr;
   np.cfg.use_score_thr = 1; np.cfg.max_out = max_out;
-  np.cand_box = fp.cand_box; np.cand_score = fp.cand_score; np.cand_cls = fp.cand_cls; np.cand_aidx = fp.cand_aidx;
-  np.counts = fp.counts; np.bitmap = fp.bitmap; np.bitmap_words = ws.bitmap_words;
-  np.nms_pos = reinterpret_cast<int32_t*>(wsb + ws.pos);
-  np.pre_keys = nullptr; np.pre_pos = nullptr; np.pre_count = nullptr; np.pre_elig = nullptr; np.pre_khi = nullptr;
-  if (n_img > NMS_PRE_MIN_N) {
+  np.st = st;
+  if (st.pre_keys) {
     // large segments: several CTAs per image gather the first NMS window so the single NMS CTA does not have to
     // scan hundreds of thousands of scores alone
     NmsPreselectParams pp;
     int slices = (5 * b200_sm_count() + num_images - 1) / num_images;   // ~5 CTAs of 256 threads (46 registers) per SM: one wave
     if (slices < 1) slices = 1;
     if (slices > 64) slices = 64;
-    pp.scores = fp.cand_score; pp.order_id = fp.cand_aidx; pp.counts = fp.counts; pp.stride = n_img; pp.slices = slices;
+    pp.scores = st.score; pp.order_id = st.aidx; pp.counts = st.counts; pp.stride = st.n_img; pp.slices = slices;
     pp.use_score_thr = 1; pp.score_thr = score_thr;
-    pp.keys = reinterpret_cast<unsigned long long*>(wsb + ws.pre_keys);
-    pp.pos = reinterpret_cast<uint32_t*>(wsb + ws.pre_pos);
-    pp.count = reinterpret_cast<int*>(wsb + ws.pre_count);
-    pp.eligible = reinterpret_cast<int*>(wsb + ws.pre_elig);
-    pp.khi = reinterpret_cast<unsigned long long*>(wsb + ws.pre_khi);
+    pp.keys = st.pre_keys; pp.pos = st.pre_pos; pp.count = st.pre_count; pp.eligible = st.pre_elig; pp.khi = st.pre_khi;
     B200_CUDA(cudaFuncSetAttribute(effdet_nms_pivot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NMS_PIVOT_SMEM));
     effdet_nms_pivot_kernel<<<num_images, NMS_THREADS, NMS_PIVOT_SMEM, stream>>>(pp);
     B200_LAUNCH_CHECK();
     effdet_nms_pregather_kernel<<<num_images * slices, 256, 0, stream>>>(pp);
     B200_LAUNCH_CHECK();
-    np.pre_keys = pp.keys; np.pre_pos = pp.pos; np.pre_count = pp.count; np.pre_elig = pp.eligible; np.pre_khi = pp.khi;
   }
   np.out_boxes = out_boxes; np.out_cls = out_class_id; np.out_score = out_score; np.out_sel_idx = out_sel_idx;
   np.out_sel_anchor = out_sel_anchor; np.out_count = out_count;
-  size_t smem2 = nms_smem_bytes(max_out);
-  if (smem2 < (size_t)ws.bitmap_words * 4) smem2 = (size_t)ws.bitmap_words * 4;
+  const size_t smem2 = cand_finalize_smem_bytes(st, max_out);
   B200_REQUIRE(smem2 <= 220 * 1024, B200_ERR_UNSUPPORTED, "b200_effdet_postprocess: too many anchors per image for the rank table");
 #define EF_LAUNCH(M)                                                                                                     \
   B200_CUDA(cudaFuncSetAttribute(effdet_nms_finalize_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2)); \
@@ -569,7 +502,7 @@ static int ef_launch_nms(const EfFilterParams& fp, const EfWs& ws, unsigned char
 extern "C" size_t b200_effdet_postprocess_workspace_bytes(int num_levels, const int32_t* hw, int A, int num_images, int max_out) {
   int n_img = 0;
   for (int l = 0; l < num_levels; ++l) n_img += hw[2 * l] * hw[2 * l + 1] * A;
-  return ef_ws_layout(num_images, n_img, max_out).total;
+  return cand_layout(num_images, n_img, max_out, false, true).total;
 }
 
 // boxes: decoded boxes (the drop-in convert_outputs_one), or null with rel / table_dev given: decode inside the filter
@@ -591,11 +524,11 @@ static int ef_post_impl(int num_levels, const int32_t* hw, int A, const float* t
   B200_REQUIRE(max_out >= 1 && max_out <= NMS_MAX_OUT_LIMIT, B200_ERR_UNSUPPORTED, "b200_effdet_postprocess: max_out %d outside [1,%d]", max_out, NMS_MAX_OUT_LIMIT);
   if (num_images == 0) return B200_OK;
   B200_REQUIRE(out_boxes && out_class_id && out_score && out_count, B200_ERR_BAD_ARG, "b200_effdet_postprocess: null output");
-  EfWs ws = ef_ws_layout(num_images, n_img, max_out);
+  const CandLayout ws = cand_layout(num_images, n_img, max_out, false, true);
   B200_REQUIRE(workspace && workspace_bytes >= ws.total, B200_ERR_WORKSPACE, "b200_effdet_postprocess: workspace %zu < required %zu", workspace_bytes, ws.total);
   B200_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, B200_ERR_BAD_ARG, "b200_effdet_postprocess: workspace not 256-byte aligned");
   unsigned char* wsb = static_cast<unsigned char*>(workspace);
-  fp.B0 = first_image; fp.NB = num_images; fp.C = C; fp.B = B; fp.n_img = n_img;
+  fp.B0 = first_image; fp.NB = num_images; fp.C = C; fp.B = B;
   long long tb = 0;
   for (int l = 0; l < EF_MAX_LEVELS; ++l) {
     fp.tile_base[l] = tb;
@@ -612,14 +545,8 @@ static int ef_post_impl(int num_levels, const int32_t* hw, int A, const float* t
     } else { fp.cls[l] = nullptr; fp.boxes[l] = nullptr; fp.rel[l] = nullptr; fp.dec[l] = nullptr; }
   }
   for (int l = num_levels; l <= EF_MAX_LEVELS; ++l) fp.tile_base[l] = tb;
-  fp.cand_box = reinterpret_cast<float4*>(wsb + ws.box);
-  fp.cand_score = reinterpret_cast<float*>(wsb + ws.score);
-  fp.cand_cls = reinterpret_cast<int32_t*>(wsb + ws.cls);
-  fp.cand_aidx = reinterpret_cast<uint32_t*>(wsb + ws.aidx);
-  fp.counts = reinterpret_cast<int32_t*>(wsb + ws.counts);
-  fp.bitmap = out_sel_idx ? reinterpret_cast<uint32_t*>(wsb + ws.bitmap) : nullptr;
-  fp.bitmap_words = ws.bitmap_words;
-  B200_CUDA(cudaMemsetAsync(wsb, 0, out_sel_idx ? ws.box : ws.bitmap, stream));
+  fp.st = cand_bind(ws, wsb, out_sel_idx != nullptr);
+  B200_CUDA(cudaMemsetAsync(wsb, 0, ws.zeroed(out_sel_idx != nullptr), stream));
   using Ring = WarpSlabRing<EF_STAGES>;
   int warps = 8;
   while (warps > 1 && Ring::smem_bytes(warps, C) > 200 * 1024) warps >>= 1;
@@ -629,8 +556,8 @@ static int ef_post_impl(int num_levels, const int32_t* hw, int A, const float* t
   effdet_filter_kernel<<<grid, warps * 32, smem1, stream>>>(fp);
   B200_LAUNCH_CHECK();
 
-  return ef_launch_nms(fp, ws, wsb, num_images, n_img, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id, out_score,
-                       out_sel_idx, out_sel_anchor, out_count, stream);
+  return ef_launch_nms(fp.st, num_images, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx,
+                       out_sel_anchor, out_count, stream);
 }
 
 extern "C" int b200_effdet_postprocess(int num_levels, const int32_t* hw, int A, int C, int B, int first_image,
@@ -708,22 +635,18 @@ extern "C" int b200_effdet_assign_targets_indexed(int num_levels, const int32_t*
 // stream and takes the decode along: b200_effdet_decode_postprocess.)
 #define EFU_TILE 64      // anchors per tile
 #define EFU_THREADS 256
-#ifndef EFU_INFLIGHT
-#define EFU_INFLIGHT 4   // float4 of each class tensor a stream thread has in flight
-#endif
 
 struct EfFusedParams {
   EfLevels lv;
-  int B, C, n_img;
+  int B, C;
   const float* cls[EF_MAX_LEVELS];        // (B,H,W,A,C) logits
-  const float* cls_true[EF_MAX_LEVELS];   // (B,H,W,A,C) targets (WITH_LOSS)
+  const float* cls_true[EF_MAX_LEVELS];   // (B,H,W,A,C) targets
   const float4* rel[EF_MAX_LEVELS];       // (B,H,W,A,4) head offsets ty,tx,th,tw
-  const float4* box_true[EF_MAX_LEVELS];  // (WITH_LOSS)
+  const float4* box_true[EF_MAX_LEVELS];
   const unsigned char* mask[EF_MAX_LEVELS];
   float4* dec[EF_MAX_LEVELS];             // decoded boxes out
   long long tile_base[EF_MAX_LEVELS + 1];
-  float4* cand_box; float* cand_score; int32_t* cand_cls; uint32_t* cand_aidx; int32_t* counts;
-  uint32_t* bitmap; int bitmap_words;
+  CandStore st;
   float alpha, gamma, delta, label_smoothing;
   double* partials;                       // [gridDim.x][num_levels][3] focal, huber, positives
 };
@@ -740,14 +663,14 @@ struct EfFusedParams {
 #define EFU_STREAM_THREADS (EFU_THREADS - 32 * EFU_BOX_WARPS)
 #define EFU_STAGES 2
 
-template <bool WITH_LOSS, bool G15>
-__global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_kernel(EfFusedParams p) {
+template <bool G15>
+__global__ void __launch_bounds__(EFU_THREADS, 2) effdet_stream_kernel(EfFusedParams p) {
   extern __shared__ __align__(128) unsigned char efu_smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int C = p.C;
   const uint32_t tile_bytes = (uint32_t)EFU_TILE * (uint32_t)C * 4u;
-  // stage s: [x tile][y tile (WITH_LOSS)]
-  const uint32_t stage_bytes = tile_bytes * (WITH_LOSS ? 2u : 1u);
+  // stage s: [x tile][y tile]
+  const uint32_t stage_bytes = tile_bytes * 2u;
   __shared__ __align__(8) uint64_t s_bar[EFU_STAGES];
   __shared__ double s_part[EF_MAX_LEVELS][3];
   __shared__ double s_red[EFU_THREADS / 32][3];
@@ -788,7 +711,7 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
   };
   auto bulk_ok = [&](int l, long long rec0, int nrec) {
     const uintptr_t ax = reinterpret_cast<uintptr_t>(p.cls[l] + rec0 * C);
-    const uintptr_t ay = WITH_LOSS ? reinterpret_cast<uintptr_t>(p.cls_true[l] + rec0 * C) : 0;
+    const uintptr_t ay = reinterpret_cast<uintptr_t>(p.cls_true[l] + rec0 * C);
     return (((ax | ay) & 15) == 0) && ((((uint32_t)nrec * (uint32_t)C * 4u) & 15u) == 0u);
   };
   auto issue = [&](long long t, int s) {   // one thread: start the copies of tile t into stage s
@@ -798,9 +721,9 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
     const uint32_t bytes = (uint32_t)nrec * (uint32_t)C * 4u;
     unsigned char* dst = efu_smem + (size_t)s * stage_bytes;
     bc_fence_proxy_async();
-    bc_mbar_expect_tx(&s_bar[s], bytes * (WITH_LOSS ? 2u : 1u));
+    bc_mbar_expect_tx(&s_bar[s], bytes * 2u);
     bc_bulk_g2s(dst, p.cls[l] + rec0 * C, bytes, &s_bar[s]);
-    if (WITH_LOSS) bc_bulk_g2s(dst + tile_bytes, p.cls_true[l] + rec0 * C, bytes, &s_bar[s]);
+    bc_bulk_g2s(dst + tile_bytes, p.cls_true[l] + rec0 * C, bytes, &s_bar[s]);
   };
   const bool box_warp = warp < EFU_BOX_WARPS;
   const int st = tid - 32 * EFU_BOX_WARPS;   // index among the stream threads
@@ -818,7 +741,7 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
     const int s = j & (EFU_STAGES - 1), pb = j & 1;
     int l, nrec; long long rec0;
     locate(t, l, rec0, nrec);
-    if (WITH_LOSS && l != cur_level) {
+    if (l != cur_level) {
       if (cur_level >= 0) flush(cur_level);
       cur_level = l;
     }
@@ -833,9 +756,8 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
       if (tid < nrec) {
         const long long rec = rec0 + tid;
         const float4 r4 = __ldcs(p.rel[l] + rec);
-        float4 t4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        unsigned char mk = 0;
-        if (WITH_LOSS) { t4 = __ldcs(p.box_true[l] + rec); mk = p.mask[l][rec]; }
+        const float4 t4 = __ldcs(p.box_true[l] + rec);
+        const unsigned char mk = p.mask[l][rec];
         int rin;
         if (total < 0x7fffffffLL) { img = (int)((uint32_t)rec / (uint32_t)api); rin = (int)((uint32_t)rec - (uint32_t)img * (uint32_t)api); }
         else { img = (int)(rec / api); rin = (int)(rec - (long long)img * api); }
@@ -843,10 +765,8 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
         ef_split(p.lv, l, rin, y, x, an_i);
         d4 = ef_decode_box(ef_anchor(p.lv, l, y, x, an_i), r4);
         if (p.dec[l]) __stcs(p.dec[l] + rec, d4);
-        if (WITH_LOSS) {
-          hub += el_huber(t4.x, r4.x, p.delta) + el_huber(t4.y, r4.y, p.delta) + el_huber(t4.z, r4.z, p.delta) + el_huber(t4.w, r4.w, p.delta);
-          pos += mk ? 1u : 0u;
-        }
+        hub += el_huber(t4.x, r4.x, p.delta) + el_huber(t4.y, r4.y, p.delta) + el_huber(t4.z, r4.z, p.delta) + el_huber(t4.w, r4.w, p.delta);
+        pos += mk ? 1u : 0u;
         aidx = (uint32_t)(p.lv.anchor_base[l] + rin);
       }
     } else {
@@ -857,28 +777,26 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
       float f0 = 0.f, f1 = 0.f;
       if (bulk) {
         bc_mbar_wait(&s_bar[s], (phase_bits >> s) & 1u);
-        if (WITH_LOSS) {
-          const int n_vec = n_el >> 2;
+        const int n_vec = n_el >> 2;
 #pragma unroll 2
-          for (int i = st; i < n_vec; i += EFU_STREAM_THREADS) {
-            const float4 x = reinterpret_cast<const float4*>(xs)[i];
-            const float4 y = reinterpret_cast<const float4*>(ys)[i];
-            f0 += el_focal<G15>(y.x, x.x, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.y, x.y, p.alpha, p.gamma, p.label_smoothing);
-            f1 += el_focal<G15>(y.z, x.z, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.w, x.w, p.alpha, p.gamma, p.label_smoothing);
-          }
+        for (int i = st; i < n_vec; i += EFU_STREAM_THREADS) {
+          const float4 x = reinterpret_cast<const float4*>(xs)[i];
+          const float4 y = reinterpret_cast<const float4*>(ys)[i];
+          f0 += el_focal<G15>(y.x, x.x, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.y, x.y, p.alpha, p.gamma, p.label_smoothing);
+          f1 += el_focal<G15>(y.z, x.z, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.w, x.w, p.alpha, p.gamma, p.label_smoothing);
         }
       } else {
         // ragged tail of a level or an unaligned tensor: plain loads; the logits still go to the stage for the argmax
         const float* xg = p.cls[l] + rec0 * C;
-        const float* yg = WITH_LOSS ? p.cls_true[l] + rec0 * C : nullptr;
+        const float* yg = p.cls_true[l] + rec0 * C;
         for (int e = st; e < n_el; e += EFU_STREAM_THREADS) {
           const float xv = __ldg(xg + e);
           xs[e] = xv;
-          if (WITH_LOSS) f0 += el_focal<G15>(__ldg(yg + e), xv, p.alpha, p.gamma, p.label_smoothing);
+          f0 += el_focal<G15>(__ldg(yg + e), xv, p.alpha, p.gamma, p.label_smoothing);
         }
         asm volatile("bar.sync 1, %0;" ::"n"(EFU_STREAM_THREADS) : "memory");   // stream warps only: the tile is complete
       }
-      if (WITH_LOSS) focal += (double)f0 + (double)f1;
+      focal += (double)f0 + (double)f1;
       // per-anchor argmax, three lanes per anchor: tf.argmax (first maximal index) / reduce_max over a third of the C
       // logits each; the box warps fold the three partials in ascending index order
       const int a = st / 3, part = st - a * 3;
@@ -914,19 +832,17 @@ __global__ void __launch_bounds__(EFU_THREADS, WITH_LOSS ? 2 : 4) effdet_stream_
 #pragma unroll
       for (int k = 1; k < 3; ++k) { const float vk = s_m[pb][tid][k]; if (vk > m) { m = vk; mi = s_mi[pb][tid][k]; } }
       const bool pass = (tid < nrec) && (mi != 0);   // classes_mask = classes_id != 0 (anc:179)
-      warp_append_by_image(pass, img, p.counts, p.n_img, p.bitmap, p.bitmap_words, aidx, [&](size_t slot) {
-        p.cand_box[slot] = d4; p.cand_score[slot] = m; p.cand_cls[slot] = mi; p.cand_aidx[slot] = aidx;
+      warp_append_by_image(p.st, pass, img, aidx, [&](size_t slot) {
+        p.st.box[slot] = d4; p.st.score[slot] = m; p.st.cls[slot] = mi;
       });
     }
     // the partial buffers alternate by tile parity: the stream warps write buffer pb again only two tiles later, behind
     // the next tile's barrier, which the box warps reach after this append
   }
-  if (WITH_LOSS) {
-    if (cur_level >= 0) flush(cur_level);
-    __syncthreads();
-    if (tid < p.lv.num_levels * 3)
-      p.partials[((size_t)blockIdx.x * p.lv.num_levels + tid / 3) * 3 + tid % 3] = s_part[tid / 3][tid % 3];
-  }
+  if (cur_level >= 0) flush(cur_level);
+  __syncthreads();
+  if (tid < p.lv.num_levels * 3)
+    p.partials[((size_t)blockIdx.x * p.lv.num_levels + tid / 3) * 3 + tid % 3] = s_part[tid / 3][tid % 3];
 }
 
 // sums layout of effdet_loss.cu: [0..L) focal_l, [L..2L) huber_l, [2L] positives
@@ -961,7 +877,7 @@ extern "C" size_t b200_effdet_eval_workspace_bytes(int num_levels, const int32_t
   return b200_effdet_postprocess_workspace_bytes(num_levels, hw, A, num_images, max_out) + efu_partials_bytes(num_levels);
 }
 
-static int efu_impl(bool with_loss, int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
+static int efu_impl(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
                     const float* const true_boxes[], const float* const true_classes[], const unsigned char* const true_masks[],
                     const float* const pred_boxes[], const float* const pred_classes[], float alpha, float gamma, float delta,
                     float label_smoothing, double* sums_out, float* const out_decoded[], int max_out, float iou_thr,
@@ -969,10 +885,10 @@ static int efu_impl(bool with_loss, int num_levels, const int32_t* hw, int A, co
                     int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count, void* workspace, size_t workspace_bytes,
                     void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  const char* who = with_loss ? "b200_effdet_eval_step" : "b200_effdet_decode_postprocess";
+  const char* who = "b200_effdet_eval_step";
   EfFusedParams p;
   B200_REQUIRE(hw && table_dev && pred_boxes && pred_classes, B200_ERR_BAD_ARG, "%s: null argument", who);
-  B200_REQUIRE(!with_loss || (true_boxes && true_classes && true_masks && sums_out), B200_ERR_BAD_ARG, "%s: null target argument", who);
+  B200_REQUIRE(true_boxes && true_classes && true_masks && sums_out, B200_ERR_BAD_ARG, "%s: null target argument", who);
   const int n_img = ef_fill_levels(p.lv, num_levels, hw, A, table_dev);
   B200_REQUIRE(n_img >= 0, B200_ERR_BAD_ARG, "%s: bad level spec", who);
   B200_REQUIRE(C >= 1 && C <= 400, B200_ERR_UNSUPPORTED, "%s: classes_num %d outside [1,400]", who, C);
@@ -981,70 +897,54 @@ static int efu_impl(bool with_loss, int num_levels, const int32_t* hw, int A, co
   B200_REQUIRE(max_out >= 1 && max_out <= NMS_MAX_OUT_LIMIT, B200_ERR_UNSUPPORTED, "%s: max_out %d outside [1,%d]", who, max_out, NMS_MAX_OUT_LIMIT);
   if (B == 0) return B200_OK;
   B200_REQUIRE(out_boxes && out_class_id && out_score && out_count, B200_ERR_BAD_ARG, "%s: null output", who);
-  EfWs ws = ef_ws_layout(B, n_img, max_out);
+  const CandLayout ws = cand_layout(B, n_img, max_out, false, true);
   const size_t part_bytes = efu_partials_bytes(num_levels);
   B200_REQUIRE(workspace && workspace_bytes >= ws.total + part_bytes, B200_ERR_WORKSPACE, "%s: workspace %zu < required %zu", who, workspace_bytes, ws.total + part_bytes);
   B200_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, B200_ERR_BAD_ARG, "%s: workspace not 256-byte aligned", who);
   unsigned char* wsb = static_cast<unsigned char*>(workspace);
-  p.B = B; p.C = C; p.n_img = n_img;
+  p.B = B; p.C = C;
   long long tb = 0;
   for (int l = 0; l < EF_MAX_LEVELS; ++l) {
     p.tile_base[l] = tb;
     p.cls[l] = nullptr; p.cls_true[l] = nullptr; p.rel[l] = nullptr; p.box_true[l] = nullptr; p.mask[l] = nullptr; p.dec[l] = nullptr;
     if (l >= num_levels) continue;
     B200_REQUIRE(pred_boxes[l] && pred_classes[l], B200_ERR_BAD_ARG, "%s: null level %d", who, l);
-    B200_REQUIRE(!with_loss || (true_boxes[l] && true_classes[l] && true_masks[l]), B200_ERR_BAD_ARG, "%s: null target level %d", who, l);
-    uintptr_t al = reinterpret_cast<uintptr_t>(pred_boxes[l]) | (out_decoded && out_decoded[l] ? reinterpret_cast<uintptr_t>(out_decoded[l]) : 0);
-    if (with_loss) al |= reinterpret_cast<uintptr_t>(true_boxes[l]);
+    B200_REQUIRE(true_boxes[l] && true_classes[l] && true_masks[l], B200_ERR_BAD_ARG, "%s: null target level %d", who, l);
+    const uintptr_t al = reinterpret_cast<uintptr_t>(pred_boxes[l]) | reinterpret_cast<uintptr_t>(true_boxes[l]) |
+                         (out_decoded && out_decoded[l] ? reinterpret_cast<uintptr_t>(out_decoded[l]) : 0);
     B200_REQUIRE((al & 15) == 0, B200_ERR_BAD_ARG, "%s: box tensors of level %d must be 16-byte aligned", who, l);
     p.cls[l] = pred_classes[l];
     p.rel[l] = reinterpret_cast<const float4*>(pred_boxes[l]);
     p.dec[l] = out_decoded ? reinterpret_cast<float4*>(out_decoded[l]) : nullptr;
-    if (with_loss) {
-      p.cls_true[l] = true_classes[l];
-      p.box_true[l] = reinterpret_cast<const float4*>(true_boxes[l]);
-      p.mask[l] = true_masks[l];
-    }
+    p.cls_true[l] = true_classes[l];
+    p.box_true[l] = reinterpret_cast<const float4*>(true_boxes[l]);
+    p.mask[l] = true_masks[l];
     tb += ((long long)B * p.lv.anc_per_img[l] + EFU_TILE - 1) / EFU_TILE;
   }
   for (int l = num_levels; l <= EF_MAX_LEVELS; ++l) p.tile_base[l] = tb;
-  p.cand_box = reinterpret_cast<float4*>(wsb + ws.box);
-  p.cand_score = reinterpret_cast<float*>(wsb + ws.score);
-  p.cand_cls = reinterpret_cast<int32_t*>(wsb + ws.cls);
-  p.cand_aidx = reinterpret_cast<uint32_t*>(wsb + ws.aidx);
-  p.counts = reinterpret_cast<int32_t*>(wsb + ws.counts);
-  p.bitmap = out_sel_idx ? reinterpret_cast<uint32_t*>(wsb + ws.bitmap) : nullptr;
-  p.bitmap_words = ws.bitmap_words;
+  p.st = cand_bind(ws, wsb, out_sel_idx != nullptr);
   p.alpha = alpha; p.gamma = gamma; p.delta = delta; p.label_smoothing = label_smoothing;
   p.partials = reinterpret_cast<double*>(wsb + ws.total);
-  B200_CUDA(cudaMemsetAsync(wsb, 0, out_sel_idx ? ws.box : ws.bitmap, stream));
+  B200_CUDA(cudaMemsetAsync(wsb, 0, ws.zeroed(out_sel_idx != nullptr), stream));
   B200_REQUIRE(C <= 128, B200_ERR_UNSUPPORTED, "%s: the fused pass stages %d-anchor tiles in shared memory: classes_num %d > 128 (use the separate calls)", who, EFU_TILE, C);
-  const size_t smem = (size_t)EFU_STAGES * EFU_TILE * C * sizeof(float) * (with_loss ? 2 : 1);
+  const size_t smem = (size_t)EFU_STAGES * EFU_TILE * C * sizeof(float) * 2;
   long long want = tb;
   const long long cap = (long long)b200_sm_count() * EFU_GRID_PER_SM;
   const int grid = (int)(want < cap ? (want < 1 ? 1 : want) : cap);
-#define EFU_LAUNCH(WL, G)                                                                                                  \
-  do {                                                                                                                     \
-    B200_CUDA(cudaFuncSetAttribute(effdet_stream_kernel<WL, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    effdet_stream_kernel<WL, G><<<grid, EFU_THREADS, smem, stream>>>(p);                                                  \
+#define EFU_LAUNCH(G)                                                                                                   \
+  do {                                                                                                                  \
+    B200_CUDA(cudaFuncSetAttribute(effdet_stream_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    effdet_stream_kernel<G><<<grid, EFU_THREADS, smem, stream>>>(p);                                                  \
   } while (0)
-  B200_REQUIRE(with_loss, B200_ERR_BAD_ARG, "%s: the CTA-tiled stream needs targets (the target-free pass is the bulk-copy filter)", who);
-  if (gamma == 1.5f) EFU_LAUNCH(true, true);
-  else EFU_LAUNCH(true, false);
+  if (gamma == 1.5f) EFU_LAUNCH(true);
+  else EFU_LAUNCH(false);
 #undef EFU_LAUNCH
   B200_LAUNCH_CHECK();
-  if (with_loss) {
-    B200_CUDA(cudaMemsetAsync(sums_out, 0, sizeof(double) * (2 * num_levels + 1), stream));
-    effdet_stream_reduce_kernel<<<num_levels, 256, 0, stream>>>(p.partials, grid, num_levels, sums_out);
-    B200_LAUNCH_CHECK();
-  }
-  // the NMS tail reads the candidate store through the filter-parameter view
-  EfFilterParams fp;
-  fp.lv = p.lv; fp.B0 = 0; fp.NB = B; fp.C = C; fp.B = B; fp.n_img = n_img;
-  fp.cand_box = p.cand_box; fp.cand_score = p.cand_score; fp.cand_cls = p.cand_cls; fp.cand_aidx = p.cand_aidx;
-  fp.counts = p.counts; fp.bitmap = p.bitmap; fp.bitmap_words = p.bitmap_words;
-  return ef_launch_nms(fp, ws, wsb, B, n_img, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx,
-                       out_sel_anchor, out_count, stream);
+  B200_CUDA(cudaMemsetAsync(sums_out, 0, sizeof(double) * (2 * num_levels + 1), stream));
+  effdet_stream_reduce_kernel<<<num_levels, 256, 0, stream>>>(p.partials, grid, num_levels, sums_out);
+  B200_LAUNCH_CHECK();
+  return ef_launch_nms(p.st, B, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx, out_sel_anchor,
+                       out_count, stream);
 }
 
 // test_step in one call: sums_out [2L+1] fp64 (un-normalised focal_l, huber_l, positives: feed b200_focal_box_finalize or
@@ -1057,7 +957,7 @@ extern "C" int b200_effdet_eval_step(int num_levels, const int32_t* hw, int A, c
                                      float iou_thr, float score_thr, int metric, float* out_boxes, long long* out_class_id,
                                      float* out_score, int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
                                      void* workspace, size_t workspace_bytes, void* stream) {
-  return efu_impl(true, num_levels, hw, A, table_dev, C, B, true_boxes, true_classes, true_masks, pred_boxes, pred_classes, alpha,
+  return efu_impl(num_levels, hw, A, table_dev, C, B, true_boxes, true_classes, true_masks, pred_boxes, pred_classes, alpha,
                   gamma, delta, label_smoothing, sums_out, out_decoded, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id,
                   out_score, out_sel_idx, out_sel_anchor, out_count, workspace, workspace_bytes, stream);
 }

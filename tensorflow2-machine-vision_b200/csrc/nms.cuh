@@ -1,5 +1,6 @@
 // nms.cuh — exact greedy NMS for one segment (image) per CTA.  Included by nms.cu (generic C-ABI entry),
-// yolo_decode.cu and effdet.cu (fused post-processing).
+// yolo_decode.cu and effdet.cu (fused post-processing).  The candidate store those two share — its workspace layout, the
+// append of the filter kernels and the output tail of the finalize kernels — is at the end of this file (CandStore).
 //
 // Replaces the tf.while_loop NMS drivers of the reference:
 //   utils/tf_iou_utils.py:67-108   GetIOUNMS            (class-agnostic, survivor iff metric <  thr; NaN drops)
@@ -38,17 +39,6 @@
 #include "boxmath.cuh"
 #include "common.cuh"
 
-#ifdef NMS_TRACE   // tuning builds only: SM-clock time stamps of the phases of block 0 (read back by b200_debug_nms_trace)
-static __device__ long long g_nms_trace[64 + 4 * 32];
-#define NMS_T(i) do { if (threadIdx.x == 0 && blockIdx.x == 0) g_nms_trace[i] = clock64(); } while (0)
-#define NMS_TW(k) do { if ((threadIdx.x & 31) == 0 && blockIdx.x == 0) g_nms_trace[64 + (k) * 32 + (threadIdx.x >> 5)] = clock64(); } while (0)
-#define NMS_TA(i, t_prev) do { if (threadIdx.x == 0 && blockIdx.x == 0) { const long long now_ = clock64(); g_nms_trace[i] += now_ - (t_prev); (t_prev) = now_; } } while (0)
-#else
-#define NMS_TA(i, t_prev) do { } while (0)
-#define NMS_T(i) do { } while (0)
-#define NMS_TW(k) do { } while (0)
-#endif
-
 #define NMS_THREADS 1024
 #define NMS_CHUNK 1024
 #define NMS_WINDOW 4096
@@ -63,30 +53,6 @@ struct NmsSegment {
   const uint32_t* order_id;  // [n] unique tie-break ids (ascending = earlier) or nullptr -> position
   int n;
 };
-
-// Candidate store of a filter kernel: image i's candidates are slots [i * n_img, i * n_img + counts[i]) of every column,
-// in arbitrary order; bit aidx of the image's row of `bitmap` (when there is one) marks each appended flat anchor index.
-// warp_append_by_image appends the warp's lanes with `pass` set, grouped by image: one atomicAdd on counts[] per (warp,
-// image), a lane's slot from its rank among the lanes of its image.  store(slot) writes the caller's columns.
-template <class Store>
-__device__ __forceinline__ void warp_append_by_image(bool pass, int img, int32_t* counts, int n_img, uint32_t* bitmap,
-                                                     int bitmap_words, uint32_t aidx, Store store) {
-  const int lane = threadIdx.x & 31;
-  uint32_t todo = __ballot_sync(0xffffffffu, pass);
-  while (todo) {
-    const int leader = __ffs(todo) - 1;
-    const int limg = __shfl_sync(0xffffffffu, img, leader);
-    const uint32_t grp = __ballot_sync(0xffffffffu, pass && img == limg);
-    int base = 0;
-    if (lane == leader) base = atomicAdd(&counts[limg], __popc(grp));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (pass && img == limg) {
-      store((size_t)limg * n_img + base + __popc(grp & ((1u << lane) - 1u)));
-      if (bitmap) atomicOr(&bitmap[(size_t)limg * bitmap_words + (aidx >> 5)], 1u << (aidx & 31u));
-    }
-    todo &= ~grp;
-  }
-}
 
 // Optional pre-gathered first window of a segment (produced by nms_preselect_kernel with several CTAs per
 // segment, for segments too large for one CTA to scan quickly).  Ignored unless its counters show a valid window.
@@ -141,13 +107,7 @@ __device__ __forceinline__ bool nms_suppresses(const BoxT& kept, int kept_cls, c
     if (bm_surely_below(kept, cand, METRIC, thr)) return false;
     return bm_metric(kept, cand, METRIC) >= thr;
   }
-#ifdef NMS_TRACE
-  if (blockIdx.x == 0) atomicAdd(reinterpret_cast<unsigned long long*>(&g_nms_trace[30]), 1ull);
-#endif
   if (bm_surely_below(kept, cand, METRIC, thr)) return false;
-#ifdef NMS_TRACE
-  if (blockIdx.x == 0) atomicAdd(reinterpret_cast<unsigned long long*>(&g_nms_trace[31]), 1ull);
-#endif
   return !(bm_metric(kept, cand, METRIC) < thr);
 }
 
@@ -176,9 +136,7 @@ __device__ __forceinline__ void nms_bitonic(unsigned long long* sK, uint32_t* sP
 
 #define NMS_BINS 2048
 #define NMS_KC 8   // keys a thread keeps in registers for the selection passes of a small segment
-#ifndef NMS_LOADS
 #define NMS_LOADS 4   // independent loads a thread keeps in flight in a selection pass over a large segment (8: no faster, spills)
-#endif
 
 // bucket of a descending-score key inside [dmin, dmax]: monotone non-decreasing in d (int->float rounding, the
 // multiplication by a positive constant and the truncation all are), so bucket(a) < bucket(b) implies a < b
@@ -261,7 +219,6 @@ __device__ __forceinline__ void nms_bucket_order(const unsigned long long* keys,
   for (int b = threadIdx.x; b < NMS_BINS; b += THREADS) { hist[b] = 0; head[b] = -1; }
   if (have_range) { mn = mn_in; mx = mx_in < mn_in ? mn_in : mx_in; __syncthreads(); }
   else nms_block_minmaxsum<THREADS>(mn, mx, dummy, red);   // its barriers also publish the cleared bins
-  NMS_T(16);
   const float scale = nms_bin_scale(mn, mx);
   for (int t = threadIdx.x; t < n; t += THREADS) {
     const int b = nms_bin((uint32_t)(keys[t] >> 32), mn, scale);
@@ -269,9 +226,7 @@ __device__ __forceinline__ void nms_bucket_order(const unsigned long long* keys,
     nxt[t] = atomicExch(&head[b], t);
   }
   __syncthreads();
-  NMS_T(17);
   nms_block_scan_bins<THREADS>(hist, red, 0, nullptr);
-  NMS_T(18);
   int dst[PER];
 #pragma unroll
   for (int u = 0; u < PER; ++u) {
@@ -289,7 +244,6 @@ __device__ __forceinline__ void nms_bucket_order(const unsigned long long* keys,
     }
   }
   __syncthreads();   // every chain walk is finished: the bins may be overwritten by ord
-  NMS_T(19);
 #pragma unroll
   for (int u = 0; u < PER; ++u) {
     const int t = (int)threadIdx.x + u * THREADS;
@@ -356,7 +310,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
 
   if (tid < 256) sHead[tid] = -1;
   const int n = seg.n;
-  NMS_T(0);
   // window size goal: enough candidates to emit max_out boxes when little is suppressed, small enough that the
   // bitonic sort of the window (the dominant cost of a lightly suppressed image) stays cheap
   const int target = nms_window_target(cfg.max_out, n);
@@ -475,7 +428,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
         nms_block_minmaxsum<THREADS>(dmin, dmax, n_el, sRed);
         if (n_el == 0) { exhausted = true; break; }
       }
-      NMS_T(1);
       const float scale = nms_bin_scale(dmin, dmax);
       int cut = NMS_BINS - 1;
       if (sampled || n_el > NMS_WINDOW) {
@@ -484,9 +436,7 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
         __syncthreads();
         for_each_key([&](int, unsigned long long K) { atomicAdd(&sBins[nms_bin((uint32_t)(K >> 32), dmin, scale)], 1); });
         __syncthreads();
-        NMS_T(2);
         const int total = nms_block_scan_bins<THREADS>(sBins, sRed, target, &sScalar[3]);
-        NMS_T(3);
         if (sampled) n_el = total;      // (>= 16: the samples are among them)
         cut = sScalar[3];
         const int upto = (cut + 1 < NMS_BINS) ? sBins[cut + 1] : n_el;   // keys in buckets 0..cut
@@ -511,7 +461,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
         });
         __syncthreads();
         n_win = sScalar[0];
-        NMS_T(4);
         gathered = true;
         win_range = !sampled; win_mn = dmin; win_mx = dmax;   // (a sampled range would pile the best keys into one ordering bucket)
         if (cut < NMS_BINS - 1) {       // keys of buckets 0..cut lie below dmin + (cut + 1) / scale (an estimate is enough)
@@ -606,7 +555,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
       __syncthreads();
     } else {
       nms_bucket_order<THREADS>(sK, n_win, sBins, sNext, sRed, sOrd, win_range, win_mn, win_mx);
-      NMS_T(5);
       if (khi == 1ull) khi = sK[sOrd[n_win - 1]] + 1ull;   // everything not gathered has a larger key (bucket > cut)
     }
 
@@ -625,7 +573,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
       }
       if (tid < 2) sSupp[tid] = 0u;
       __syncthreads();
-      NMS_T(6);
       if (mode == B200_NMS_BY_CLASS) {
         // ---- per-class NMS: classes never interact, so the chunk is split by class bucket and every bucket is resolved
         // by its own warp (greedy in rank order inside the bucket); the survivors are then emitted in global rank order.
@@ -661,7 +608,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
         for (int i = tid; i < 32 * 256 / 2; i += THREADS) reinterpret_cast<uint32_t*>(sTab)[i] = 0u;
         for (int i = tid; i < 256; i += THREADS) sSet[i] = 0ull;
         __syncthreads();
-        NMS_T(7);
         // (2) stable split by bucket: 32-candidate blocks in rank order; intra-block rank by match_any, block counts in sTab
         const int n_blk = (n_chunk + 31) >> 5;
         for (int blk = warp; blk < n_blk; blk += NW) {
@@ -713,14 +659,12 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
           }
         }
         __syncthreads();
-        NMS_T(8);
         // (3) inside a bucket.  The pairs (i < j) of all buckets form one flat index space (bucket starts in sPB, a triangle
         // inside a bucket): every thread tests an equal share of them and ORs bit i into member j's word when i (same class)
         // suppresses j.  Then one thread per bucket walks its members in rank order with the alive set in a register: member
         // t stays iff it was alive and no ALIVE better-ranked mate suppresses it — the greedy recurrence itself, ~5 dependent
         // ALU steps per member.  (A warp per bucket walking shared-memory state took 14 us of the 36 us of a 416x416 image —
         // 10 members per class, three buckets per warp, the slowest warp decides; a thread per member 5 us.)
-        NMS_TW(0);
         {
           const int P = sPB[256];
           const int per = (P + THREADS - 1) / THREADS;
@@ -758,9 +702,7 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
             }
           }
         }
-        NMS_TW(1);
         __syncthreads();
-        NMS_TW(2);
         // (buckets spread over all warps: a warp waits for the largest of its buckets)
         for (int b = tid / (THREADS / 256); b < 256 && tid % (THREADS / 256) == 0; b += 256) {
           const int base = sBase[b], m = sBase[b + 1] - base;
@@ -791,9 +733,7 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
             __syncwarp();
           }
         }
-        NMS_TW(3);
         __syncthreads();
-        NMS_T(9);
         // (4) emit the survivors in rank order, up to the cap
         for (int c0 = 0; c0 < n_chunk && n_kept < cfg.max_out; c0 += THREADS) {
           const int ct = c0 + tid;
@@ -806,7 +746,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
           const uint32_t bal = __ballot_sync(0xffffffffu, a);
           if (lane == 0) sRed[warp] = (uint32_t)__popc(bal);
           __syncthreads();
-          NMS_T(14);
           int before = 0, total = 0;
 #pragma unroll
           for (int w = 0; w < NW; ++w) { const int t = (int)sRed[w]; if (w < warp) before += t; total += t; }
@@ -818,25 +757,13 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
             kNext[slot] = atomicExch(&sHead[(uint32_t)cCl[ct] & 255u], slot);
           }
           n_kept = min(cfg.max_out, n_kept + total);
-          NMS_T(15);
           __syncthreads();
         }
-        NMS_T(10);
         continue;
       }
       const int n_tiles = (n_chunk + 63) >> 6;
-#ifdef NMS_TRACE
-      if (tid == 0 && blockIdx.x == 0) g_nms_trace[21] = 0;
-#endif
       for (int T = 0; T < n_tiles && n_kept < cfg.max_out; ++T) {
-#ifdef NMS_TRACE
-        if (tid == 0 && blockIdx.x == 0) g_nms_trace[21] += 1;   // tiles consumed
-#endif
         const int t0 = T << 6;
-#ifdef NMS_TRACE
-        long long t_ph = clock64();
-        if (tid == 0 && blockIdx.x == 0 && T == 0) { g_nms_trace[24] = g_nms_trace[25] = g_nms_trace[26] = g_nms_trace[27] = 0; }
-#endif
         // phase 1: tile candidates vs the kept list.  warp w: candidates 32*(w&1)..+31, kept indices (w>>1) + (THREADS/64) j
         {
           const int c = ((warp & 1) << 5) + lane;
@@ -867,7 +794,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
         __syncthreads();
         unsigned long long tile_alive = ~((unsigned long long)sSupp[0] | ((unsigned long long)sSupp[1] << 32));
         if (n_chunk - t0 < 64) tile_alive &= (1ull << (n_chunk - t0)) - 1ull;
-        NMS_TA(24, t_ph);
         // phase 2: intra-tile mask via ballots: warp w owns rows (2048/THREADS) w ... (2 rows at 1024 threads)
 #pragma unroll
         for (int rr = 0; rr < 2048 / THREADS; ++rr) {
@@ -895,7 +821,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
           if (lane == 0) sMask[r] = (unsigned long long)bits[0] | ((unsigned long long)bits[1] << 32);
         }
         __syncthreads();
-        NMS_TA(25, t_ph);
         // one-warp sweep.  lane <-> columns lane and lane + 32: the warp first transposes the 64 x 64 bit matrix (64 broadcast
         // reads; by = the better-ranked rows that suppress the column), then iterates  kept' = alive & ~any(by & kept)  from
         // kept = alive until nothing changes.  The greedy solution is the unique fixed point and position j is final after
@@ -942,7 +867,6 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
         __syncthreads();
         const unsigned long long keptmask = *sKeptMask;
         const int nk = sScalar[2];
-        NMS_TA(26, t_ph);
         // emit: append to the kept list
         if (tid < 64 && ((keptmask >> tid) & 1ull)) {
           const int gi = t0 + tid;
@@ -953,15 +877,10 @@ static __device__ int nms_run_segment(const NmsSegment& seg, const NmsConfig& cf
           if (mode == B200_NMS_BY_CLASS) kNext[slot] = atomicExch(&sHead[(uint32_t)cCl[gi] & 255u], slot);
         }
         n_kept += nk;
-        NMS_TA(27, t_ph);
         __syncthreads();
       }
       __syncthreads();
-      NMS_T(20);
     }
-#ifdef NMS_TRACE
-    if (tid == 0 && blockIdx.x == 0) g_nms_trace[22] += 1;   // windows
-#endif
     if (khi == ~0ull) exhausted = true;
     klo = khi;
     __syncthreads();
@@ -1080,6 +999,146 @@ static __device__ void nms_pregather_body(const NmsPreselectParams& p) {
     const int g = s_base + t;
     if (g < NMS_PRE_CAP) { p.keys[(size_t)seg * NMS_PRE_CAP + g] = s_keys[t]; p.pos[(size_t)seg * NMS_PRE_CAP + g] = s_pos[t]; }
   }
+}
+
+// ---- candidate store of the fused post-processing (yolo_decode.cu, effdet.cu) --------------------------------------
+// A filter kernel appends the candidates of every image to the store; one finalize CTA per image then runs the NMS over its
+// image's row and gathers the kept rows.  Image i's candidates are slots [i * n_img, i * n_img + counts[i]) of every
+// column, in arbitrary order; bit aidx of the image's row of `bitmap` marks each appended flat anchor index.
+struct CandStore {
+  float4* box; float* score; int32_t* cls; uint32_t* aidx;  // [n_images, n_img]
+  float* conf;                  // [n_images, n_img] (YOLO: the conf logit) or nullptr
+  int32_t* counts;              // [n_images]
+  uint32_t* bitmap;             // [n_images, bitmap_words], only when sel_idx is wanted (else nullptr)
+  int bitmap_words, n_img;
+  int32_t* pos;                 // [n_images, max_out] NMS output positions
+  // first NMS window from the multi-CTA pre-selection (EfficientDet); nullptr unless an image can exceed NMS_PRE_MIN_N
+  unsigned long long* pre_keys; uint32_t* pre_pos;          // [n_images, NMS_PRE_CAP]
+  int* pre_count; int* pre_elig; unsigned long long* pre_khi;  // [n_images]
+};
+
+// Byte offsets of the store's blocks in a workspace.  Each block is 256-aligned on its own.  counts, the pre-selection
+// counters and the bitmap lead, so one memset of zeroed(sel_idx) bytes clears everything that is counted into.
+struct CandLayout {
+  size_t counts, pre_count, pre_elig, bitmap, box, score, cls, conf, aidx, pos, pre_khi, pre_keys, pre_pos, total;
+  int n_img, bitmap_words;
+  bool with_conf, with_preselect;
+  size_t zeroed(bool sel_idx) const { return sel_idx ? box : bitmap; }
+};
+
+static inline CandLayout cand_layout(int n_images, int n_img, int max_out, bool with_conf, bool with_preselect) {
+  CandLayout L = {};
+  L.n_img = n_img; L.bitmap_words = (n_img + 31) / 32;
+  L.with_conf = with_conf; L.with_preselect = with_preselect;
+  const size_t N = (size_t)n_images, NC = N * (size_t)n_img;
+  size_t o = 0;
+  auto block = [&o](size_t bytes) { const size_t at = o; o = b200_align_up(o + bytes, 256); return at; };
+  L.counts = block(sizeof(int32_t) * N);
+  if (with_preselect) { L.pre_count = block(sizeof(int) * N); L.pre_elig = block(sizeof(int) * N); }
+  L.bitmap = block(sizeof(uint32_t) * N * L.bitmap_words);
+  L.box = block(sizeof(float4) * NC);
+  L.score = block(sizeof(float) * NC);
+  L.cls = block(sizeof(int32_t) * NC);
+  if (with_conf) L.conf = block(sizeof(float) * NC);
+  L.aidx = block(sizeof(uint32_t) * NC);
+  L.pos = block(sizeof(int32_t) * N * (size_t)max_out);
+  if (with_preselect) {
+    L.pre_khi = block(sizeof(unsigned long long) * N);
+    L.pre_keys = block(sizeof(unsigned long long) * N * NMS_PRE_CAP);
+    L.pre_pos = block(sizeof(uint32_t) * N * NMS_PRE_CAP);
+  }
+  L.total = o;
+  return L;
+}
+
+// The store in workspace `ws` laid out by L.  The pre-selection buffers are always laid out when asked for, but bound
+// only when an image can have more than NMS_PRE_MIN_N candidates: a bound pre_keys is what runs the pre-selection.
+static inline CandStore cand_bind(const CandLayout& L, unsigned char* ws, bool sel_idx) {
+  const bool pre = L.with_preselect && L.n_img > NMS_PRE_MIN_N;
+  CandStore s;
+  s.box = reinterpret_cast<float4*>(ws + L.box);
+  s.score = reinterpret_cast<float*>(ws + L.score);
+  s.cls = reinterpret_cast<int32_t*>(ws + L.cls);
+  s.aidx = reinterpret_cast<uint32_t*>(ws + L.aidx);
+  s.conf = L.with_conf ? reinterpret_cast<float*>(ws + L.conf) : nullptr;
+  s.counts = reinterpret_cast<int32_t*>(ws + L.counts);
+  s.bitmap = sel_idx ? reinterpret_cast<uint32_t*>(ws + L.bitmap) : nullptr;
+  s.bitmap_words = L.bitmap_words; s.n_img = L.n_img;
+  s.pos = reinterpret_cast<int32_t*>(ws + L.pos);
+  s.pre_keys = pre ? reinterpret_cast<unsigned long long*>(ws + L.pre_keys) : nullptr;
+  s.pre_pos = pre ? reinterpret_cast<uint32_t*>(ws + L.pre_pos) : nullptr;
+  s.pre_count = pre ? reinterpret_cast<int*>(ws + L.pre_count) : nullptr;
+  s.pre_elig = pre ? reinterpret_cast<int*>(ws + L.pre_elig) : nullptr;
+  s.pre_khi = pre ? reinterpret_cast<unsigned long long*>(ws + L.pre_khi) : nullptr;
+  return s;
+}
+
+// Appends the warp's lanes with `pass` set, grouped by image: one atomicAdd on counts[] per (warp, image), a lane's slot
+// from its rank among the lanes of its image.  columns(slot) writes the caller's columns; the anchor index and the
+// bitmap bit are written here.
+template <class Columns>
+__device__ __forceinline__ void warp_append_by_image(const CandStore& s, bool pass, int img, uint32_t aidx, Columns columns) {
+  const int lane = threadIdx.x & 31;
+  uint32_t todo = __ballot_sync(0xffffffffu, pass);
+  while (todo) {
+    const int leader = __ffs(todo) - 1;
+    const int limg = __shfl_sync(0xffffffffu, img, leader);
+    const uint32_t grp = __ballot_sync(0xffffffffu, pass && img == limg);
+    int base = 0;
+    if (lane == leader) base = atomicAdd(&s.counts[limg], __popc(grp));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (pass && img == limg) {
+      const size_t slot = (size_t)limg * s.n_img + base + __popc(grp & ((1u << lane) - 1u));
+      columns(slot);
+      s.aidx[slot] = aidx;
+      if (s.bitmap) atomicOr(&s.bitmap[(size_t)limg * s.bitmap_words + (aidx >> 5)], 1u << (aidx & 31u));
+    }
+    todo &= ~grp;
+  }
+}
+
+// ---- NMS output tail of a finalize kernel (one CTA per image) ----
+// The NMS segment of image img: its row of the store, with the classes for per-class NMS only.
+__device__ __forceinline__ NmsSegment cand_segment(const CandStore& s, int img, bool with_classes) {
+  const size_t base = (size_t)img * s.n_img;
+  NmsSegment seg;
+  seg.boxes = reinterpret_cast<const float*>(s.box + base);
+  seg.scores = s.score + base;
+  seg.classes = with_classes ? s.cls + base : nullptr;
+  seg.order_id = s.aidx + base;
+  seg.n = s.counts[img];
+  return seg;
+}
+
+// After the NMS (wprefix reuses its shared memory): exclusive prefix popcount of image img's bitmap words, one pass by
+// warp 0 (a few thousand words at most).  Does nothing without a bitmap.
+__device__ __forceinline__ void cand_word_prefix(const CandStore& s, int img, uint32_t* wprefix) {
+  if (!s.bitmap) return;
+  const uint32_t* bm = s.bitmap + (size_t)img * s.bitmap_words;
+  if (threadIdx.x < 32) {
+    uint32_t run = 0;
+    for (int w0 = 0; w0 < s.bitmap_words; w0 += 32) {
+      const int w = w0 + (int)threadIdx.x;
+      const int c = (w < s.bitmap_words) ? __popc(bm[w]) : 0;
+      const int inc = warp_scan_incl(c);
+      if (w < s.bitmap_words) wprefix[w] = run + (uint32_t)(inc - c);
+      run += (uint32_t)__shfl_sync(0xffffffffu, inc, 31);
+    }
+  }
+  __syncthreads();
+}
+
+// sel_idx of anchor index a of image img: its rank among the image's candidates, which is its position in the
+// reference's compacted list
+__device__ __forceinline__ int32_t cand_sel_idx(const CandStore& s, int img, const uint32_t* wprefix, uint32_t a) {
+  const uint32_t wv = s.bitmap[(size_t)img * s.bitmap_words + (a >> 5)];
+  return (int32_t)(wprefix[a >> 5] + __popc(wv & ((1u << (a & 31u)) - 1u)));
+}
+
+// dynamic shared memory of a finalize kernel: the NMS, then the word prefix in the same bytes
+static inline size_t cand_finalize_smem_bytes(const CandStore& s, int max_out) {
+  const size_t nms = nms_smem_bytes(max_out), prefix = (size_t)s.bitmap_words * 4;
+  return nms < prefix ? prefix : nms;
 }
 
 // runs CALL(METRIC) with the runtime metric as a compile-time constant

@@ -12,8 +12,9 @@
 //     sigmoid is evaluated only for logits inside a guard band of the maximum (max / first-argmax are taken
 //     in sigmoid space, exactly as tf.reduce_max / tf.argmax of sigmoid(classes) do; detmath's sigmoid is not
 //     monotone at ulp level, see oracle/DETMATH_REPORT.md);
-//   * survivors (valid box, conf > thr, score > thr: strict, tyu:163,191-192) are appended per image with
-//     warp-aggregated atomics (warp_append_by_image, nms.cuh).  Append order is arbitrary; each candidate carries its
+//   * survivors (valid box, conf > thr, score > thr: strict, tyu:163,191-192) are appended per image to the candidate
+//     store (CandStore, nms.cuh: its workspace layout, the warp-aggregated append and the NMS output tail live there,
+//     shared with effdet.cu; YOLO adds the conf column).  Append order is arbitrary; each candidate carries its
 //     flat anchor index (level-major, then h, w, a) which is monotone in the reference's compaction order, so it
 //     serves as the NMS tie-break id and as the rank source for `sel_idx`.
 // Kernel 2  yolo_nms_finalize_kernel  (one CTA per image): nms.cuh greedy NMS + gather of the five outputs,
@@ -41,15 +42,10 @@ struct YoloLevels {
 struct YoloDecodeParams {
   YoloLevels lv;
   int B, A, C, RF;
-  int n_img;  // anchors per image over all levels
   float conf_thr, score_thr;
   float conf_lo, conf_hi;  // logits below / above which sigmoid(conf) > conf_thr is decided without the sigmoid
   uint32_t magic_a;        // floor(2^32/A)+1 (0 for A == 1): rin / A == umulhi(rin, magic_a) for rin * A < 2^32
-  // candidate store, stride n_img per image
-  float4* cand_box; float* cand_score; int32_t* cand_cls; float* cand_conf; uint32_t* cand_aidx;
-  int32_t* counts;     // [B]
-  uint32_t* bitmap;    // [B, bitmap_words] or nullptr
-  int bitmap_words;
+  CandStore st;            // box is left to the NMS pass (decode on demand)
 };
 
 // max and first-argmax of sigmoid(x_c), c in [0,C), for the warp's 32 records (lane <-> record, stride RF in shared
@@ -244,11 +240,10 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
       if (t_issue < n_tiles) issue(t_issue, ring.stage);
       t_issue += gstride;
     }
-    warp_append_by_image(pass, img, p.counts, p.n_img, p.bitmap, p.bitmap_words, aidx, [&](size_t slot) {
-      p.cand_score[slot] = score;
-      p.cand_cls[slot] = cls;
-      p.cand_conf[slot] = conf;  // the logit; the sigmoid is applied to the emitted rows only
-      p.cand_aidx[slot] = aidx;
+    warp_append_by_image(p.st, pass, img, aidx, [&](size_t slot) {
+      p.st.score[slot] = score;
+      p.st.cls[slot] = cls;
+      p.st.conf[slot] = conf;  // the logit; the sigmoid is applied to the emitted rows only
     });
     if (!EARLY) {
       __syncwarp();  // every lane is done reading the slab before it is refilled
@@ -261,12 +256,9 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
 
 struct YoloFinalizeParams {
   YoloLevels lv;
-  int B, A, C, RF, n_img;
+  int B, A, C, RF;
   NmsConfig cfg;
-  float4* cand_box;  // written by the NMS pass (decode on demand)
-  const float* cand_score; const int32_t* cand_cls; const float* cand_conf;
-  const uint32_t* cand_aidx; const int32_t* counts; const uint32_t* bitmap; int bitmap_words;
-  int32_t* nms_pos;  // [B, max_out] scratch
+  CandStore st;      // box is written by the NMS pass (decode on demand)
   // outputs, all [B, max_out, ...]
   float* out_boxes; int32_t* out_cls; float* out_score; float* out_classes; float* out_conf;
   int32_t* out_sel_idx; int32_t* out_sel_anchor; int32_t* out_count;
@@ -301,63 +293,29 @@ struct YoloLazyBox {
 template <int METRIC, int THREADS>
 __global__ void __launch_bounds__(THREADS, NMS_THREADS / THREADS) yolo_nms_finalize_kernel(YoloFinalizeParams p) {
   extern __shared__ __align__(16) unsigned char nms_smem[];
-  NMS_T(13);
   const int img = blockIdx.x;
-  const size_t cbase = (size_t)img * p.n_img;
-  NmsSegment seg;
-  seg.boxes = reinterpret_cast<const float*>(p.cand_box + cbase);
-  seg.scores = p.cand_score + cbase;
-  seg.classes = p.cand_cls + cbase;
-  seg.order_id = p.cand_aidx + cbase;
-  seg.n = p.counts[img];
-  int32_t* pos = p.nms_pos + (size_t)img * p.cfg.max_out;
+  const size_t cbase = (size_t)img * p.st.n_img;
+  int32_t* pos = p.st.pos + (size_t)img * p.cfg.max_out;
   YoloLazyBox lazy;
-  lazy.lv = &p.lv; lazy.img = img; lazy.A = p.A; lazy.RF = p.RF; lazy.cand_box = p.cand_box + cbase;
-  const int kept = nms_run_segment<METRIC, YoloLazyBox, THREADS>(seg, p.cfg, pos, nms_smem, nullptr, lazy);
+  lazy.lv = &p.lv; lazy.img = img; lazy.A = p.A; lazy.RF = p.RF; lazy.cand_box = p.st.box + cbase;
+  const int kept = nms_run_segment<METRIC, YoloLazyBox, THREADS>(cand_segment(p.st, img, true), p.cfg, pos, nms_smem, nullptr, lazy);
   __syncthreads();
-  NMS_T(11);
   if (threadIdx.x == 0) p.out_count[img] = kept;
   const size_t obase = (size_t)img * p.cfg.max_out;
-  // rank of an anchor index among the image's candidates = its position in the reference's compacted list
-  uint32_t* wprefix = reinterpret_cast<uint32_t*>(nms_smem);  // reuse (NMS is finished)
-  if (p.out_sel_idx && p.bitmap) {
-    const uint32_t* bm = p.bitmap + (size_t)img * p.bitmap_words;
-    // exclusive prefix popcount over words, single pass by warp 0 (<= a few thousand words)
-    if (threadIdx.x < 32) {
-      uint32_t run = 0;
-      for (int w0 = 0; w0 < p.bitmap_words; w0 += 32) {
-        int w = w0 + (int)threadIdx.x;
-        int c = (w < p.bitmap_words) ? __popc(bm[w]) : 0;
-        int inc = warp_scan_incl(c);
-        if (w < p.bitmap_words) wprefix[w] = run + (uint32_t)(inc - c);
-        run += (uint32_t)__shfl_sync(0xffffffffu, inc, 31);
-      }
-    }
-    __syncthreads();
-  }
+  uint32_t* wprefix = reinterpret_cast<uint32_t*>(nms_smem);
+  cand_word_prefix(p.st, img, wprefix);
   for (int k = threadIdx.x; k < kept; k += blockDim.x) {
     const int q = pos[k];
-    const float4 b = p.cand_box[cbase + q];
-    reinterpret_cast<float4*>(p.out_boxes)[obase + k] = b;
-    p.out_cls[obase + k] = p.cand_cls[cbase + q];
-    p.out_score[obase + k] = p.cand_score[cbase + q];
-    p.out_conf[obase + k] = dm_sigmoidf(p.cand_conf[cbase + q]);
-    const uint32_t a = p.cand_aidx[cbase + q];
+    reinterpret_cast<float4*>(p.out_boxes)[obase + k] = p.st.box[cbase + q];
+    p.out_cls[obase + k] = p.st.cls[cbase + q];
+    p.out_score[obase + k] = p.st.score[cbase + q];
+    p.out_conf[obase + k] = dm_sigmoidf(p.st.conf[cbase + q]);
+    const uint32_t a = p.st.aidx[cbase + q];
     pos[k] = (int32_t)a;   // from here on the scratch row holds flat anchor indices: yolo_classes_kernel needs no candidate lookup
     if (p.out_sel_anchor) p.out_sel_anchor[obase + k] = (int32_t)a;
-    if (p.out_sel_idx && p.bitmap) {
-      const uint32_t wv = p.bitmap[(size_t)img * p.bitmap_words + (a >> 5)];
-      p.out_sel_idx[obase + k] = (int32_t)(wprefix[a >> 5] + __popc(wv & ((1u << (a & 31u)) - 1u)));
-    }
+    if (p.out_sel_idx) p.out_sel_idx[obase + k] = cand_sel_idx(p.st, img, wprefix, a);
   }
-  NMS_T(12);
 }
-
-#ifdef NMS_TRACE
-extern "C" int b200_debug_nms_trace(long long* out_host64) {
-  return cudaMemcpyFromSymbol(out_host64, g_nms_trace, sizeof(long long) * (64 + 4 * 32)) == cudaSuccess ? 0 : -1;
-}
-#endif
 
 // sigmoid(classes) rows of the selected boxes, read back from the head tensors (tyu:140,265).  A separate launch
 // so the B*max_out*C sigmoids spread over the whole GPU instead of serialising inside the per-image NMS CTAs.
@@ -372,7 +330,7 @@ __global__ void __launch_bounds__(256) yolo_classes_kernel(YoloFinalizeParams p)
   if (row >= p.B * p.cfg.max_out) return;
   const int img = row / p.cfg.max_out, k = row - img * p.cfg.max_out;
   // flat anchor index, left by the NMS kernel; fetched together with the count (rows past the count hold stale values)
-  const uint32_t a = (uint32_t)__ldcg(p.nms_pos + (size_t)img * p.cfg.max_out + k);
+  const uint32_t a = (uint32_t)__ldcg(p.st.pos + (size_t)img * p.cfg.max_out + k);
   if (k >= __ldcg(p.out_count + img)) return;
   int l = 0;
 #pragma unroll
@@ -445,30 +403,10 @@ static int fill_levels(YoloLevels& lv, const float* const heads[3], const int32_
   return ab;
 }
 
-struct YoloWs {
-  size_t counts, bitmap, box, score, cls, conf, aidx, pos, total;
-  int bitmap_words;
-};
-static YoloWs yolo_ws_layout(int B, int n_img, int max_out) {
-  YoloWs w;
-  size_t o = 0;
-  w.bitmap_words = (n_img + 31) / 32;
-  w.counts = o; o = b200_align_up(o + sizeof(int32_t) * B, 256);
-  w.bitmap = o; o = b200_align_up(o + sizeof(uint32_t) * (size_t)B * w.bitmap_words, 256);
-  w.box = o; o = b200_align_up(o + sizeof(float4) * (size_t)B * n_img, 256);
-  w.score = o; o = b200_align_up(o + sizeof(float) * (size_t)B * n_img, 256);
-  w.cls = o; o = b200_align_up(o + sizeof(int32_t) * (size_t)B * n_img, 256);
-  w.conf = o; o = b200_align_up(o + sizeof(float) * (size_t)B * n_img, 256);
-  w.aidx = o; o = b200_align_up(o + sizeof(uint32_t) * (size_t)B * n_img, 256);
-  w.pos = o; o = b200_align_up(o + sizeof(int32_t) * (size_t)B * max_out, 256);
-  w.total = o;
-  return w;
-}
-
 extern "C" size_t b200_yolo_decode_nms_workspace_bytes(const int32_t hw[6], int B, int A, int max_out) {
   int n_img = 0;
   for (int l = 0; l < 3; ++l) n_img += hw[2 * l] * hw[2 * l + 1] * A;
-  return yolo_ws_layout(B, n_img, max_out).total;
+  return cand_layout(B, n_img, max_out, true, false).total;
 }
 
 extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t hw[6], int B, int A, int C,
@@ -493,12 +431,12 @@ extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t h
   B200_REQUIRE((reinterpret_cast<uintptr_t>(out_boxes) & 15) == 0, B200_ERR_BAD_ARG, "b200_yolo_decode_nms: out_boxes not 16-byte aligned");
   YoloDecodeParams dp;
   const int n_img = fill_levels(dp.lv, heads, hw, B, A, C, anchors_wh_host, image_wh_host);
-  YoloWs ws = yolo_ws_layout(B, n_img, max_out);
+  const CandLayout ws = cand_layout(B, n_img, max_out, true, false);
   B200_REQUIRE(workspace && workspace_bytes >= ws.total, B200_ERR_WORKSPACE,
                "b200_yolo_decode_nms: workspace %zu < required %zu", workspace_bytes, ws.total);
   B200_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, B200_ERR_BAD_ARG, "b200_yolo_decode_nms: workspace not 256-byte aligned");
   unsigned char* wsb = static_cast<unsigned char*>(workspace);
-  dp.B = B; dp.A = A; dp.C = C; dp.RF = 5 + C; dp.n_img = n_img;
+  dp.B = B; dp.A = A; dp.C = C; dp.RF = 5 + C;
   dp.conf_thr = conf_thr; dp.score_thr = score_thr;
   dp.magic_a = A == 1 ? 0u : (uint32_t)((1ull << 32) / (unsigned long long)A + 1ull);
   // sigmoid(x) > conf_thr is certain for x > logit(thr) + d and certainly false for x < logit(thr) - d, with d ten times
@@ -510,16 +448,8 @@ extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t h
     const double d = 3e-6 / ((double)conf_thr * (1.0 - (double)conf_thr)) + 1e-6 * fabs(t);
     dp.conf_lo = (float)(t - d); dp.conf_hi = (float)(t + d);
   }
-  dp.cand_box = reinterpret_cast<float4*>(wsb + ws.box);
-  dp.cand_score = reinterpret_cast<float*>(wsb + ws.score);
-  dp.cand_cls = reinterpret_cast<int32_t*>(wsb + ws.cls);
-  dp.cand_conf = reinterpret_cast<float*>(wsb + ws.conf);
-  dp.cand_aidx = reinterpret_cast<uint32_t*>(wsb + ws.aidx);
-  dp.counts = reinterpret_cast<int32_t*>(wsb + ws.counts);
-  dp.bitmap = out_sel_idx ? reinterpret_cast<uint32_t*>(wsb + ws.bitmap) : nullptr;
-  dp.bitmap_words = ws.bitmap_words;
-  // counts and bitmap are adjacent at the front of the workspace: one memset
-  B200_CUDA(cudaMemsetAsync(wsb, 0, out_sel_idx ? ws.box : ws.bitmap, stream));
+  dp.st = cand_bind(ws, wsb, out_sel_idx != nullptr);
+  B200_CUDA(cudaMemsetAsync(wsb, 0, ws.zeroed(out_sel_idx != nullptr), stream));
 
   using Ring = WarpSlabRing<YD_STAGES>;
   int warps = 16;  // one tile in flight per warp; the warps of an SM overlap each other's loads
@@ -545,19 +475,14 @@ extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t h
   B200_LAUNCH_CHECK();
 
   YoloFinalizeParams fp;
-  fp.lv = dp.lv; fp.B = B; fp.A = A; fp.C = C; fp.RF = dp.RF; fp.n_img = n_img;
+  fp.lv = dp.lv; fp.B = B; fp.A = A; fp.C = C; fp.RF = dp.RF; fp.st = dp.st;
   fp.cfg.metric = metric; fp.cfg.mode = B200_NMS_BY_CLASS; fp.cfg.iou_thr = iou_thr; fp.cfg.score_thr = 0.f;
   fp.cfg.use_score_thr = 0; fp.cfg.max_out = max_out;
-  fp.cand_box = dp.cand_box; fp.cand_score = dp.cand_score; fp.cand_cls = dp.cand_cls; fp.cand_conf = dp.cand_conf;
-  fp.cand_aidx = dp.cand_aidx; fp.counts = dp.counts; fp.bitmap = dp.bitmap; fp.bitmap_words = ws.bitmap_words;
-  fp.nms_pos = reinterpret_cast<int32_t*>(wsb + ws.pos);
   fp.out_boxes = out_boxes; fp.out_cls = out_class_id; fp.out_score = out_score; fp.out_classes = out_classes;
   fp.out_conf = out_conf; fp.out_sel_idx = out_sel_idx; fp.out_sel_anchor = out_sel_anchor; fp.out_count = out_count;
   // one 1024-thread CTA per SM gives the lowest latency; batches that need more than one wave use 512-thread CTAs,
   // two per SM (the shared-memory footprint allows it up to max_out ~ 500)
-  size_t smem2 = nms_smem_bytes(max_out);
-  const size_t need_prefix = (size_t)ws.bitmap_words * 4;
-  if (smem2 < need_prefix) smem2 = need_prefix;
+  const size_t smem2 = cand_finalize_smem_bytes(fp.st, max_out);
   const bool half_ctas = (B > b200_sm_count()) && (2 * (smem2 + 1024) <= 227 * 1024);
 #define YD_LAUNCH(M)                                                                                                   \
   if (half_ctas) {                                                                                                          \
