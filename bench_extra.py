@@ -131,6 +131,41 @@ def main():
         ms = timed(wrap(lambda: tyu.GetLossAndGrad(y_true, heads, (image, image), anc, 0.5, "ciou")), args.steps, args.warmup)
         report("c2_backward", "YOLOv4 608 B=64: GetLossAndGrad(ciou) = forward + dense d loss/d y_pred (y_true given)", batch, ms,
                3 * 7732620, {"forward_only_ms": ms_f, "note": "bytes: read y_true + read y_pred + write the gradient"})
+    if want("c2_sparse_backward"):  # SURVEY 8f N3 + N1: the training step from box lists against the drop-in one
+        card = _card()
+        batch, image = 64, 608
+        heads = yolo_heads(batch, image)
+        rng = np.random.default_rng(20261018 + 2)
+        boxes, classes, off = synth.gt_batch(rng, batch, (image, image), max_boxes=100)
+        boxes_d, classes_d, off_d = (torch.from_numpy(x).to(dev) for x in (boxes, classes, off))
+        gen = DataGenerator(80, anc, (image, image))
+        arms = {
+            "dense": lambda: tyu.GetLossAndGrad(gen.GetTargetsBatch(classes_d, boxes_d, off_d), heads, (image, image), anc, 0.5, "ciou"),
+            "sparse": lambda: tyu.GetLossFromBoxesAndGrad(classes_d, boxes_d, off_d, heads, (image, image), anc, 80, 0.5, "ciou"),
+            "sparse_forward": lambda: tyu.GetLossFromBoxes(classes_d, boxes_d, off_d, heads, (image, image), anc, 80, 0.5, "ciou"),
+        }
+        loss_a, grads_a = arms["dense"]()
+        loss_b, grads_b = arms["sparse"]()
+        assert all(torch.equal(x.view(torch.int32), y.view(torch.int32)) for x, y in zip(grads_a, grads_b)), \
+            "GetLossFromBoxesAndGrad and GetTargetsBatch + GetLossAndGrad disagree on the gradient bits"
+        loss_rel = abs(float(loss_b) - float(loss_a)) / abs(float(loss_a))
+        del grads_a, grads_b
+        fns = {k: wrap(f) for k, f in arms.items()}
+        # the arms alternate window by window (order rotated) so that drift of clocks and neighbours hits all of them
+        steps, n_win = max(args.steps, 50), 7
+        times = {k: [] for k in fns}
+        order = list(fns)
+        for w in range(n_win):
+            for k in order[w % 3:] + order[:w % 3]:
+                times[k].append(timed(fns[k], steps, args.warmup))
+        ms = {k: float(np.median(v)) for k, v in times.items()}
+        report("c2_sparse_backward", "YOLOv4 608 B=64 training step from box lists: GetLossFromBoxesAndGrad(ciou) against "
+               "GetTargetsBatch + GetLossAndGrad (gradients asserted bit-identical first) and GetLossFromBoxes alone; median of %d "
+               "alternating windows of %d steps" % (n_win, steps), batch, ms["sparse"], 2 * 7732620,
+               dict(card, dense_targets_and_grad_ms=ms["dense"], from_boxes_forward_ms=ms["sparse_forward"],
+                    speedup_vs_dense=ms["dense"] / ms["sparse"], window_ms={k: [round(t, 5) for t in v] for k, v in times.items()},
+                    grads_bit_identical=True, loss_rel_diff=loss_rel,
+                    note="bytes: read y_pred + write the gradient (dense equivalent; y_pred and the gradients exceed the 126 MB L2)"))
     if want("n4_letterbox"):  # SURVEY 8f N4: the serving view's image pre-processing, one image per call (latency)
         from tfmv_b200.views.object_detection import prepare_image
         for (h, w) in ((1080, 1920), (3024, 4032), (480, 640), (240, 320)):

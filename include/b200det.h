@@ -151,7 +151,7 @@ int b200_yolo_loss_grad(const float* const y_true[3], const float* const y_pred[
  * dense y_true.  boxes [total,4] pixel corners x1,y1,x2,y2 / classes [total] / offsets [B+1] as for
  * b200_yolo_assign_targets; assign_anchors_wh_host = the anchors GetTargets compares against (cds:209-217),
  * anchors_wh_host = the anchors of the loss.  Same result as assign + b200_yolo_loss up to fp64 summation order;
- * out_ignore as in b200_yolo_loss.  Forward only. */
+ * out_ignore as in b200_yolo_loss.  The backward is b200_yolo_loss_from_boxes_grad. */
 size_t b200_yolo_loss_from_boxes_workspace_bytes(const int32_t hw[6], int B, int A, int total_boxes);
 int b200_yolo_loss_from_boxes(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
                               const float* assign_anchors_wh_host, const float* const y_pred[3], const int32_t hw[6],
@@ -159,6 +159,18 @@ int b200_yolo_loss_from_boxes(const float* boxes, const int32_t* classes, const 
                               float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
                               float* out_loss, unsigned char* out_ignore, void* workspace, size_t workspace_bytes,
                               void* stream);
+
+/* b200_yolo_loss_from_boxes forward + the analytic backward of b200_yolo_loss_grad, still without a dense y_true:
+ * out_grad[l] (B,H_l,W_l,A*(5+C)), 16-byte aligned, = d loss / d y_pred[l] for an upstream gradient of 1, bit-identical
+ * to b200_yolo_loss_grad on the targets b200_yolo_assign_targets writes from the same boxes.  Same workspace size as
+ * b200_yolo_loss_from_boxes.  Data parallel: each rank passes its own images with batch_divisor = the global batch; the
+ * gradients need no exchange, out_parts go through any all-reduce + b200_yolo_loss_combine for the global loss. */
+int b200_yolo_loss_from_boxes_grad(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
+                                   const float* assign_anchors_wh_host, const float* const y_pred[3], const int32_t hw[6],
+                                   int B, int A, int C, const float* anchors_wh_host, const float* image_wh_host,
+                                   float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
+                                   float* out_loss, float* const out_grad[3], void* workspace, size_t workspace_bytes,
+                                   void* stream);
 
 /* DataGenerator.GetTargets (datasets/coco_dataset.py:185-285), batched: boxes [total,4] pixel corners
  * x1,y1,x2,y2, classes [total] int32, offsets [B+1] int32 (all device).  targets[l]: (B,H_l,W_l,A,5+C), zeroed

@@ -38,6 +38,8 @@ SIGNATURES = {
     "b200_yolo_loss_from_boxes_workspace_bytes": (c_sz, [c_p, c_i, c_i, c_i]),
     "b200_yolo_loss_from_boxes": (c_i, [c_p, c_p, c_p, c_i, c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_f, c_i, c_i, c_f, c_p, c_p,
                                         c_p, c_p, c_sz, c_p]),
+    "b200_yolo_loss_from_boxes_grad": (c_i, [c_p, c_p, c_p, c_i, c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_f, c_i, c_i, c_f, c_p,
+                                             c_p, c_p, c_p, c_sz, c_p]),
     "b200_yolo_assign_targets": (c_i, [c_p, c_p, c_p, c_i, c_i, c_p, c_i, c_p, c_i, c_p, c_p, c_i, c_p]),
     "b200_fill_zero": (c_i, [c_p, c_sz, c_p]),
     "b200_yolo_reset_targets": (c_i, [c_p, c_p, c_i, c_i, c_p, c_i, c_p, c_i, c_p, c_p, c_p]),

@@ -249,8 +249,33 @@ def GetLossFromBoxes(classes, boxes, offsets, y_pred, image_wh, anchors_wh, clas
     target_anchors: the anchors DataGenerator was constructed with (default: anchors_wh)
   '''
   assert iou_type in ['iou','diou','ciou']
+  loss, parts, _ = _boxes_call(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_num, iou_thresh, iou_type,
+                               target_anchors, batch_divisor, workspace, ignore_out=ignore_out)
+  return (loss, parts) if return_parts else loss
+
+
+def GetLossFromBoxesAndGrad(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_num, iou_thresh=0.5, iou_type='iou',
+                            target_anchors=None, batch_divisor=None, return_parts=False, workspace=None):
+  '''GetLossFromBoxes plus d loss / d y_pred (list of 3 tensors shaped like y_pred) for an upstream gradient of 1: the
+  training step of the sparse-target path.  Gradients bit-identical to
+  GetLossAndGrad(DataGenerator(classes_num, target_anchors, image_wh).GetTargetsBatch(classes, boxes, offsets), y_pred, ...).
+  Returns (loss, grads), or (loss, parts, grads) with return_parts.
+
+  Data parallel: each rank passes its own images with batch_divisor = the global batch.  The gradients need no exchange;
+  the (3,4) parts go through combine_loss_parts (or any all-reduce + b200_yolo_loss_combine) for the global loss.
+  Wrap with tf.custom_gradient (INTEGRATION.md §3).'''
+  assert iou_type in ['iou','diou','ciou']
+  loss, parts, grads = _boxes_call(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_num, iou_thresh, iou_type,
+                                   target_anchors, batch_divisor, workspace, with_grad=True)
+  return (loss, parts, grads) if return_parts else (loss, grads)
+
+
+def _boxes_call(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_num, iou_thresh, iou_type, target_anchors,
+                batch_divisor, workspace, ignore_out=None, with_grad=False):
+  '''Argument checks and marshalling of the sparse-target entries.  Returns (loss, parts, grads or None).'''
   lib = _lib.load()
-  yp = [t if T.is_pinned_host_f32(t) else T.to_cuda(t) for t in y_pred]  # pinned host predictions are read in place
+  # pinned host predictions are read in place by the forward; the backward needs device tensors
+  yp = [t if (not with_grad and T.is_pinned_host_f32(t)) else T.to_cuda(t) for t in y_pred]
   if len(yp) != 3:
     raise ValueError('y_pred must hold 3 levels')
   boxes = T.to_cuda(boxes).reshape(-1, 4)
@@ -279,12 +304,21 @@ def GetLossFromBoxes(classes, boxes, offsets, y_pred, image_wh, anchors_wh, clas
   if workspace is None or workspace.numel() < ws_bytes:
     workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
   div = float(B if batch_divisor is None else batch_divisor)
+  if with_grad:
+    grads = [torch.empty_like(t) for t in yp]
+    gp = (ctypes.c_void_p * 3)(*[t.data_ptr() for t in grads])
+    _lib.check(lib.b200_yolo_loss_from_boxes_grad(T.ptr(boxes), T.ptr(classes), T.ptr(offsets), total,
+                                                  tanc.ctypes.data_as(ctypes.c_void_p), pp, hw, B, A, RF - 5,
+                                                  anc.ctypes.data_as(ctypes.c_void_p), img.ctypes.data_as(ctypes.c_void_p),
+                                                  float(iou_thresh), _lib.METRIC_YOLO[iou_type], 0, div, T.ptr(parts), T.ptr(loss),
+                                                  gp, T.ptr(workspace), workspace.numel(), T.stream_ptr()), 'GetLossFromBoxesAndGrad')
+    return loss, parts, grads
   _lib.check(lib.b200_yolo_loss_from_boxes(T.ptr(boxes), T.ptr(classes), T.ptr(offsets), total,
                                            tanc.ctypes.data_as(ctypes.c_void_p), pp, hw, B, A, RF - 5,
                                            anc.ctypes.data_as(ctypes.c_void_p), img.ctypes.data_as(ctypes.c_void_p),
                                            float(iou_thresh), _lib.METRIC_YOLO[iou_type], 0, div, T.ptr(parts), T.ptr(loss),
                                            T.ptr(ignore_out), T.ptr(workspace), workspace.numel(), T.stream_ptr()), 'GetLossFromBoxes')
-  return (loss, parts) if return_parts else loss
+  return loss, parts, None
 
 
 _SIDE_STREAMS = {}

@@ -861,8 +861,12 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g
 }
 
 // YL_GRAD_SPLIT CTAs per (image, level): a warp per object record overwrites channels 0-3 and 5.. of that record
-// (each object is two dependent DRAM round trips and ~85 sigmoids: spread wide instead of looping in one CTA)
+// (each object is two dependent DRAM round trips and ~85 sigmoids: spread wide instead of looping in one CTA).
+// kSparse (b200_yolo_loss_from_boxes_grad): the targets of object slot k come from sp_t / sp_cls, i.e. the record the
+// dense scatter would have written (obj = 1, one-hot class row; an out-of-range class id gives an all-zero row, as
+// tf.one_hot); the arithmetic is the dense form's.
 #define YL_GRAD_SPLIT 8
+template <bool kSparse>
 __global__ void __launch_bounds__(256) yolo_loss_grad_objects_kernel(YlParams p, float* g0, float* g1, float* g2) {
   const int pair = blockIdx.x / YL_GRAD_SPLIT, split = blockIdx.x - pair * YL_GRAD_SPLIT;
   const int img = pair / YL_LEVELS, l = pair - img * YL_LEVELS;
@@ -871,16 +875,25 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_objects_kernel(YlParams p,
   const int rpi = p.lv.rec_per_img[l];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int W = p.lv.w[l], H = p.lv.h[l];
-  const float* yt = p.lv.y_true[l] + ((size_t)img * rpi) * p.RF;
+  const float* yt = kSparse ? nullptr : p.lv.y_true[l] + ((size_t)img * rpi) * p.RF;
   const float* yp = p.lv.y_pred[l] + ((size_t)img * rpi) * p.RF;
   float* gr = grad + ((size_t)img * rpi) * p.RF;
   for (int k = split * 8 + warp; k < n; k += 8 * YL_GRAD_SPLIT) {
-    const int r = p.obj_index[(size_t)img * p.n_img + p.lv.anchor_base[l] + k];
-    const float* t = yt + (size_t)r * p.RF;
+    const size_t slot = (size_t)img * p.n_img + p.lv.anchor_base[l] + k;
+    const int r = p.obj_index[slot];
+    const float* t = kSparse ? nullptr : yt + (size_t)r * p.RF;
     const float* q = yp + (size_t)r * p.RF;
     float* o = gr + (size_t)r * p.RF;
-    const float obj = __ldg(t + 4);
-    const float tx = __ldg(t), ty = __ldg(t + 1), tw = __ldg(t + 2), th = __ldg(t + 3);
+    float obj, tx, ty, tw, th;
+    int sp_class = -1;
+    if (kSparse) {
+      const float4 v = p.sp_t[slot];
+      obj = 1.0f; tx = v.x; ty = v.y; tw = v.z; th = v.w;
+      sp_class = p.sp_cls[slot];
+    } else {
+      obj = __ldg(t + 4);
+      tx = __ldg(t); ty = __ldg(t + 1); tw = __ldg(t + 2); th = __ldg(t + 3);
+    }
     const float os = (obj * (2.0f - tw * th)) * p.inv_div;
     if (lane < 2) {
       const int cell = r / p.A;
@@ -895,7 +908,8 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_objects_kernel(YlParams p,
       const float raw = dm_logf(num / (lane == 2 ? p.lv.anc_w[l][a] : p.lv.anc_h[l][a]));
       o[lane] = os * (__ldg(q + lane) - raw);
     }
-    for (int c = 5 + lane; c < p.RF; c += 32) o[c] = (obj * p.inv_div) * (dm_sigmoidf(__ldg(q + c)) - __ldg(t + c));
+    for (int c = 5 + lane; c < p.RF; c += 32)
+      o[c] = (obj * p.inv_div) * (dm_sigmoidf(__ldg(q + c)) - (kSparse ? ((c - 5 == sp_class) ? 1.0f : 0.0f) : __ldg(t + c)));
   }
 }
 
@@ -1046,6 +1060,10 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
                "b200_yolo_loss: iou_type must be iou/diou/ciou (metric %d)", metric);
   B200_REQUIRE(variant == YL_VARIANT_TF_YOLO_UTILS || variant == YL_VARIANT_KERAS_YOLO3, B200_ERR_BAD_ARG, "b200_yolo_loss: bad variant %d", variant);
   B200_REQUIRE(batch_divisor > 0.0f, B200_ERR_BAD_ARG, "b200_yolo_loss: batch_divisor must be positive");
+  if (out_grad)   // checked before anything is enqueued: a refused call leaves the stream untouched
+    for (int l = 0; l < YL_LEVELS; ++l)
+      B200_REQUIRE(out_grad[l] && (reinterpret_cast<uintptr_t>(out_grad[l]) & 15) == 0, B200_ERR_BAD_ARG, "%s: grad level %d null or not 16-byte aligned",
+                   sparse ? "b200_yolo_loss_from_boxes_grad" : "b200_yolo_loss_grad", l);
   YlParams p;
   int n_img = 0;
   YlWs ws = yl_layout(hw, B, A, &n_img, &p.lv);
@@ -1176,7 +1194,6 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
     g.RF = p.RF;
     unsigned long long cum = 0;
     for (int l = 0; l < YL_LEVELS; ++l) {
-      B200_REQUIRE(out_grad[l] && (reinterpret_cast<uintptr_t>(out_grad[l]) & 15) == 0, B200_ERR_BAD_ARG, "b200_yolo_loss_grad: grad level %d null or not 16-byte aligned", l);
       g.records[l] = (unsigned long long)B * p.lv.rec_per_img[l];
       g.grad[l] = out_grad[l];
       g.conf_grad[l] = p.conf_grad + (size_t)B * p.lv.anchor_base[l];
@@ -1189,7 +1206,8 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
     if (blocks < 1) blocks = 1;
     yolo_loss_grad_dense_kernel<<<(int)blocks, 256, 0, stream>>>(g);
     B200_LAUNCH_CHECK();
-    yolo_loss_grad_objects_kernel<<<B * YL_LEVELS * YL_GRAD_SPLIT, 256, 0, stream>>>(p, out_grad[0], out_grad[1], out_grad[2]);
+    if (sparse) yolo_loss_grad_objects_kernel<true><<<B * YL_LEVELS * YL_GRAD_SPLIT, 256, 0, stream>>>(p, out_grad[0], out_grad[1], out_grad[2]);
+    else yolo_loss_grad_objects_kernel<false><<<B * YL_LEVELS * YL_GRAD_SPLIT, 256, 0, stream>>>(p, out_grad[0], out_grad[1], out_grad[2]);
     B200_LAUNCH_CHECK();
   }
   return B200_OK;
@@ -1233,6 +1251,22 @@ extern "C" int b200_yolo_loss_from_boxes(const float* boxes, const int32_t* clas
   sp.assign_anchors_wh_host = assign_anchors_wh_host;
   return yolo_loss_impl(nullptr, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
                         batch_divisor, out_parts, out_loss, out_ignore, nullptr, workspace, workspace_bytes, stream_, &sp);
+}
+
+// b200_yolo_loss_from_boxes plus d loss / d y_pred, as b200_yolo_loss_grad is to b200_yolo_loss.  The workspace of
+// b200_yolo_loss_from_boxes_workspace_bytes already holds the per-record conf gradient the backward reads.
+extern "C" int b200_yolo_loss_from_boxes_grad(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
+                                              const float* assign_anchors_wh_host, const float* const y_pred[3], const int32_t hw[6],
+                                              int B, int A, int C, const float* anchors_wh_host, const float* image_wh_host,
+                                              float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
+                                              float* out_loss, float* const out_grad[3], void* workspace, size_t workspace_bytes,
+                                              void* stream_) {
+  B200_REQUIRE(out_grad, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes_grad: null out_grad");
+  YlSparseIn sp;
+  sp.boxes = boxes; sp.classes = classes; sp.offsets = offsets; sp.total_boxes = total_boxes;
+  sp.assign_anchors_wh_host = assign_anchors_wh_host;
+  return yolo_loss_impl(nullptr, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+                        batch_divisor, out_parts, out_loss, nullptr, out_grad, workspace, workspace_bytes, stream_, &sp);
 }
 
 extern "C" int b200_yolo_loss_grad(const float* const y_true[3], const float* const y_pred[3], const int32_t hw[6],
