@@ -166,6 +166,55 @@ def main():
                     speedup_vs_dense=ms["dense"] / ms["sparse"], window_ms={k: [round(t, 5) for t in v] for k, v in times.items()},
                     grads_bit_identical=True, loss_rel_diff=loss_rel,
                     note="bytes: read y_pred + write the gradient (dense equivalent; y_pred and the gradients exceed the 126 MB L2)"))
+    if want("c3_sparse_backward"):  # SURVEY 8f N3 + N1 for EfficientDet: the training step from box lists against the two-call ones
+        from tfmv_b200.ai_models.efficientnet.efficientdet_net_train import (get_loss_and_grad, get_loss_from_boxes,
+                                                                             get_loss_from_boxes_and_grad)
+        card = _card()
+        c = synth.EFFDET_CONFIGS["d0"]
+        batch, C = 128, 81
+        a = Anchors(c["min_level"], c["max_level"], c["image_size"], c["num_scales"], c["aspect_ratios"], c["anchor_scale"])
+        shapes = [tuple(b.shape) for b in a.boxes]
+        rel = [torch.randn((batch,) + s, device=dev, generator=g) * 0.25 for s in shapes]
+        cls = [torch.randn((batch,) + s[:-1] + (C,), device=dev, generator=g) for s in shapes]
+        n_anchor = sum(s[0] * s[1] * s[2] for s in shapes)
+        rng = np.random.default_rng(20261018 + 3)
+        boxes, classes, off = synth.gt_batch(rng, batch, (c["image_size"][1], c["image_size"][0]), max_boxes=100, order="yxyx")
+        d_boxes, d_cls, d_off = (torch.from_numpy(boxes).to(dev), torch.from_numpy((classes + 1).astype(np.int32)).to(dev),
+                                 torch.from_numpy(off).to(dev))
+        arms = {
+            "one_hot": lambda: get_loss_and_grad(*a.generate_targets_batch(d_boxes, d_cls, d_off, C), rel, cls),
+            "class_id": lambda: get_loss_and_grad(*a.generate_targets_batch(d_boxes, d_cls, d_off, C, class_index=True), rel, cls),
+            "from_boxes": lambda: get_loss_from_boxes_and_grad(a, d_boxes, d_cls, d_off, rel, cls),
+            "from_boxes_forward": lambda: get_loss_from_boxes(a, d_boxes, d_cls, d_off, rel, cls),
+        }
+        res = {k: arms[k]() for k in ("one_hot", "class_id", "from_boxes")}
+        same = lambda x, y: all(torch.equal(p.view(torch.int32), q.view(torch.int32)) for p, q in zip(x[1] + x[2], y[1] + y[2]))
+        assert same(res["one_hot"], res["from_boxes"]) and same(res["class_id"], res["from_boxes"]), \
+            "get_loss_from_boxes_and_grad and generate_targets_batch + get_loss_and_grad disagree on the gradient bits"
+        loss_ref = float(res["one_hot"][0])
+        loss_rel = abs(float(res["from_boxes"][0]) - loss_ref) / abs(loss_ref)
+        fwd_bits = float(arms["from_boxes_forward"]()) == float(res["from_boxes"][0])
+        del res
+        fns = {k: wrap(f) for k, f in arms.items()}
+        # the arms alternate window by window (order rotated) so that drift of clocks and neighbours hits all of them
+        steps, n_win = max(args.steps, 20), 7
+        times = {k: [] for k in fns}
+        order = list(fns)
+        for w in range(n_win):
+            for k in order[w % len(order):] + order[:w % len(order)]:
+                times[k].append(timed(fns[k], steps, args.warmup))
+        ms = {k: float(np.median(v)) for k, v in times.items()}
+        report("c3_sparse_backward", "EfficientDet-D0 512 B=128 C=81 training step from box lists: get_loss_from_boxes_and_grad "
+               "against generate_targets_batch (one-hot / class ids) + get_loss_and_grad (gradients asserted bit-identical "
+               "first) and get_loss_from_boxes alone; median of %d alternating windows of %d steps" % (n_win, steps), batch,
+               ms["from_boxes"], n_anchor * (C * 8 + 32 + 8),
+               dict(card, one_hot_targets_and_grad_ms=ms["one_hot"], class_id_targets_and_grad_ms=ms["class_id"],
+                    from_boxes_forward_ms=ms["from_boxes_forward"], speedup_vs_one_hot=ms["one_hot"] / ms["from_boxes"],
+                    speedup_vs_class_id=ms["class_id"] / ms["from_boxes"], window_ms={k: [round(t, 5) for t in v] for k, v in times.items()},
+                    grads_bit_identical=True, forward_loss_bit_identical=fwd_bits, loss_rel_diff_vs_one_hot=loss_rel,
+                    note="bytes: read logits + box outputs, write both gradients, write + read one int32 match per anchor"))
+        del rel, cls
+        torch.cuda.empty_cache()
     if want("n4_letterbox"):  # SURVEY 8f N4: the serving view's image pre-processing, one image per call (latency)
         from tfmv_b200.views.object_detection import prepare_image
         for (h, w) in ((1080, 1920), (3024, 4032), (480, 640), (240, 320)):

@@ -291,6 +291,30 @@ int b200_focal_box_grad_indexed(int num_levels, const unsigned long long* anchor
                                 const double* numel_per_level_host, float* const grad_boxes[],
                                 float* const grad_classes[], void* stream);
 
+/* generate_targets + _get_loss and its backward from box lists (SURVEY §8f N3 + N1; an API extension): no dense targets.
+ * gt_boxes [total,4] y1,x1,y2,x2 (16-byte aligned), gt_classes [total] int32, gt_offsets [B+1] as for
+ * b200_effdet_assign_targets.  Two stages, because num_pos scales every gradient and depends only on boxes and anchors:
+ *   _match: the matched GT row of every anchor (generate_targets' IoU, tie rule and iou_thr) into the workspace; zeroes
+ *     sums[2L+1] and sets sums[2L] = this call's matched anchors;
+ *   _grad: one pass over the heads: sums[0..2L) as b200_focal_box_partial_sums writes them (sums[2L] unchanged) and, when
+ *     the arrays are given, grad_boxes[l] / grad_classes[l] = d loss / d pred_*[l] for an upstream gradient of 1 with
+ *     num_pos = sums[2L] + 1 — bit-identical to b200_focal_box_grad on the targets b200_effdet_assign_targets writes.
+ *     NULL grad arrays give the loss terms only.  classes_num < 4 returns B200_ERR_UNSUPPORTED.
+ * Then b200_focal_box_finalize(sums, numel_per_level_host) gives the loss.  Both stages take the same workspace
+ * (b200_effdet_loss_from_boxes_workspace_bytes, 256-byte aligned; its size does not depend on the device).
+ * Data parallel, on every rank: _match; all-reduce sums[2L]; _grad with the GLOBAL numel; all-reduce sums[0..2L);
+ * b200_focal_box_finalize.  Not b200_focal_box_finalize_dp: sums[2L] is already global and would be added `world` times. */
+size_t b200_effdet_loss_from_boxes_workspace_bytes(int num_levels, const int32_t* hw, int A, int B);
+int b200_effdet_loss_from_boxes_match(int num_levels, const int32_t* hw, int A, const float* table_dev, int B,
+                                      const float* gt_boxes, const int32_t* gt_offsets, int total_boxes, float iou_thr,
+                                      double* sums, void* workspace, size_t workspace_bytes, void* stream);
+int b200_effdet_loss_from_boxes_grad(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
+                                     const float* gt_boxes, const int32_t* gt_classes, int total_boxes,
+                                     const float* const pred_boxes[], const float* const pred_classes[], float alpha,
+                                     float gamma, float delta, float label_smoothing, const double* numel_per_level_host,
+                                     double* sums, float* const grad_boxes[], float* const grad_classes[], void* workspace,
+                                     size_t workspace_bytes, void* stream);
+
 /* Serving-path box post-processing (SURVEY §8f N4; views/object_detection.py:70-85): boxes [B,max_rows,4] normalised
  * x1,y1,x2,y2 on the letterboxed image (image_size = (w,h) of the network input, padding = (top,bottom,left,right) of
  * opencvProportionalResize, image_size_old = (w,h) of the original image; host int32) -> pixel boxes on the original

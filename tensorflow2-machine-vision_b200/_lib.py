@@ -58,6 +58,10 @@ SIGNATURES = {
     "b200_focal_box_grad": (c_i, [c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_f, c_f, c_f, c_f, c_p, c_p, c_p, c_p, c_p]),
     "b200_focal_box_grad_indexed": (c_i, [c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_f, c_f, c_f, c_f, c_p, c_p, c_p, c_p, c_p]),
     "b200_focal_box_finalize": (c_i, [c_i, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "b200_effdet_loss_from_boxes_workspace_bytes": (c_sz, [c_i, c_p, c_i, c_i]),
+    "b200_effdet_loss_from_boxes_match": (c_i, [c_i, c_p, c_i, c_p, c_i, c_p, c_p, c_i, c_f, c_p, c_p, c_sz, c_p]),
+    "b200_effdet_loss_from_boxes_grad": (c_i, [c_i, c_p, c_i, c_p, c_i, c_i, c_p, c_p, c_i, c_p, c_p, c_f, c_f, c_f, c_f, c_p, c_p,
+                                               c_p, c_p, c_p, c_sz, c_p]),
     "b200_row_positions_workspace_bytes": (c_sz, [ctypes.c_longlong]),
     "b200_row_positions": (c_i, [c_p, ctypes.c_longlong, c_p, c_p, c_p, c_sz, c_p]),
     "b200_gather_rows": (c_i, [c_p, c_i, c_p, c_p, ctypes.c_longlong, c_p, c_p]),

@@ -75,6 +75,102 @@ def get_loss_and_grad(y_true_boxes, y_true_classes, y_true_masks, y_pred_boxes, 
                   with_grad=True)
 
 
+def _from_boxes_args(anchors, boxes, classes, offsets, y_pred_boxes, y_pred_classes):
+  '''Checks and device placement shared by get_loss_from_boxes and get_loss_from_boxes_and_grad.'''
+  L = anchors._num_levels
+  pb = [T.to_cuda(t) for t in y_pred_boxes]
+  pc = [T.to_cuda(t) for t in y_pred_classes]
+  if len(pb) != L or len(pc) != L:
+    raise ValueError('expected %d levels, got %d box / %d class outputs' % (L, len(pb), len(pc)))
+  gb = T.to_cuda(boxes).reshape(-1, 4)
+  if gb.data_ptr() % 16:
+    gb = gb.clone()   # the loss pass reads a GT box as one 16-byte load
+  gc = T.to_cuda(classes, torch.int32).reshape(-1)
+  go = T.to_cuda(offsets, torch.int32).reshape(-1)
+  if gc.numel() != gb.shape[0]:
+    raise ValueError('%d boxes but %d classes' % (gb.shape[0], gc.numel()))
+  B, C = go.numel() - 1, pc[0].shape[-1]
+  if B < 0:
+    raise ValueError('offsets must hold B + 1 entries')
+  for l, (h, w) in enumerate(anchors._level_hw):
+    if tuple(pb[l].shape) != (B, h, w, anchors._A, 4) or tuple(pc[l].shape) != (B, h, w, anchors._A, C):
+      raise ValueError('prediction shapes of level %d (%r / %r) do not match (%d,%d,%d,%d,4|C)' % (
+          l, tuple(pb[l].shape), tuple(pc[l].shape), B, h, w, anchors._A))
+  return gb, gc, go, pb, pc, B, C
+
+
+def _loss_from_boxes(anchors, boxes, classes, offsets, y_pred_boxes, y_pred_classes, iou_threshold, alpha, gamma, delta,
+                     global_batch_scale, group, exchange, return_parts, with_grad):
+  gb, gc, go, pb, pc, B, C = _from_boxes_args(anchors, boxes, classes, offsets, y_pred_boxes, y_pred_classes)
+  if C < 4:
+    # the one-pass kernel rebuilds one-hot rows a float4 at a time (a float4 may straddle at most two anchors):
+    # narrower heads take the dense targets — same results
+    tb, tc, tm = anchors.generate_targets_batch(gb, gc, go, C, iou_threshold)
+    return get_loss(tb, tc, tm, pb, pc, alpha, gamma, delta, global_batch_scale, group, return_parts, with_grad, exchange)
+  lib = _lib.load()
+  import torch.distributed as dist
+  allreduce = None
+  if exchange is not None:
+    allreduce, global_batch_scale = exchange.allreduce_, exchange.world
+  elif dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+    allreduce = lambda t: dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+    global_batch_scale = dist.get_world_size(group)
+  L, dev = anchors._num_levels, pc[0].device
+  tab = anchors._dev_table()
+  nm = (ctypes.c_double * L)(*[float(t.numel()) * global_batch_scale for t in pc])
+  sums = torch.empty((2 * L + 1,), dtype=torch.float64, device=dev)
+  ws_bytes = lib.b200_effdet_loss_from_boxes_workspace_bytes(L, anchors._hw, anchors._A, B)
+  ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+  n_boxes = gb.shape[0]
+  _lib.check(lib.b200_effdet_loss_from_boxes_match(L, anchors._hw, anchors._A, T.ptr(tab), B, T.ptr(gb), T.ptr(go), n_boxes,
+                                                   float(iou_threshold), T.ptr(sums), T.ptr(ws), ws_bytes, T.stream_ptr()),
+             'get_loss_from_boxes (match)')
+  if allreduce is not None:
+    allreduce(sums[2 * L:])   # num_positives over the global batch scales every gradient
+  arr = lambda ts: (ctypes.c_void_p * L)(*[t.data_ptr() for t in ts])
+  grad_b = [torch.empty_like(t) for t in pb] if with_grad else None
+  grad_c = [torch.empty_like(t) for t in pc] if with_grad else None
+  _lib.check(lib.b200_effdet_loss_from_boxes_grad(L, anchors._hw, anchors._A, T.ptr(tab), C, B, T.ptr(gb), T.ptr(gc), n_boxes,
+                                                  arr(pb), arr(pc), float(alpha), float(gamma), float(delta), 0.0, nm,
+                                                  T.ptr(sums), arr(grad_b) if with_grad else None,
+                                                  arr(grad_c) if with_grad else None, T.ptr(ws), ws_bytes, T.stream_ptr()),
+             'get_loss_from_boxes')
+  if allreduce is not None:
+    allreduce(sums[:2 * L])
+  parts = torch.empty((L, 2), dtype=torch.float32, device=dev)
+  loss = torch.empty((), dtype=torch.float32, device=dev)
+  npos = torch.empty((), dtype=torch.float32, device=dev)
+  # sums[2L] is global already: the plain finalize (the _dp form would add it once per rank)
+  _lib.check(lib.b200_focal_box_finalize(L, T.ptr(sums), nm, T.ptr(parts), T.ptr(loss), T.ptr(npos), T.stream_ptr()),
+             'get_loss_from_boxes (finalize)')
+  if with_grad:
+    return loss, tuple(grad_b), tuple(grad_c)
+  return (loss, parts, npos) if return_parts else loss
+
+
+def get_loss_from_boxes(anchors, boxes, classes, offsets, y_pred_boxes, y_pred_classes, iou_threshold=0.5, alpha=0.25,
+                        gamma=1.5, delta=0.1, global_batch_scale=1, group=None, exchange=None, return_parts=False):
+  '''Anchors.generate_targets_batch + get_loss without materialising the targets (SURVEY §8f N3).
+
+  anchors: utils.anchors.Anchors; boxes [total,4] y1,x1,y2,x2, classes [total], offsets [B+1] (image b owns rows
+  offsets[b]:offsets[b+1]).  The loss equals get_loss on the targets generate_targets_batch writes from the same boxes
+  (fp64 sums in another order).  Data parallel: every rank passes its own images; the matched-anchor count and then the
+  2L loss terms are all-reduced (exchange = runtime.PeerExchange / NcclExchange, or torch.distributed on `group`).  No
+  host synchronisation: the call can be captured with runtime.capture.  classes_num < 4 takes generate_targets_batch +
+  get_loss.'''
+  return _loss_from_boxes(anchors, boxes, classes, offsets, y_pred_boxes, y_pred_classes, iou_threshold, alpha, gamma, delta,
+                          global_batch_scale, group, exchange, return_parts, False)
+
+
+def get_loss_from_boxes_and_grad(anchors, boxes, classes, offsets, y_pred_boxes, y_pred_classes, iou_threshold=0.5,
+                                 alpha=0.25, gamma=1.5, delta=0.1, global_batch_scale=1, group=None, exchange=None):
+  '''get_loss_from_boxes plus (d loss / d y_pred_boxes[l], d loss / d y_pred_classes[l]) for an upstream gradient of 1,
+  in one pass over the heads: returns (loss, grad_boxes, grad_classes) as get_loss_and_grad does, with gradients
+  bit-identical to generate_targets_batch + get_loss_and_grad on the same boxes.'''
+  return _loss_from_boxes(anchors, boxes, classes, offsets, y_pred_boxes, y_pred_classes, iou_threshold, alpha, gamma, delta,
+                          global_batch_scale, group, exchange, False, True)
+
+
 class EfficientDetNetTrain(object):
   '''Only the head-loss part of the reference class: `_get_loss` with the reference's argument order.'''
 

@@ -11,44 +11,13 @@
 // nms.cuh (CandStore: workspace layout, append and NMS output tail, shared with yolo_decode.cu; EfficientDet adds the
 // buffers of the multi-CTA pre-selection).
 //
-// Anchors are never read from HBM: every kernel rebuilds an anchor box from a tiny per-level table
-// (row centres yc[H], column centres xc[W], half extents hy[A], hx[A]; built on the host with the reference's own
-// double-precision Python arithmetic) exactly as the reference does — box = [yc-hy, xc-hx, yc+hy, xc+hx] in fp32,
-// then centre/size re-derived from those corners (anc:204-217) — so results are bit-identical to reading
-// Anchors.boxes while saving 0.8 MB (D0) / 7 MB (D7) of reads per image.
+// Anchors are rebuilt in-kernel from the per-level table (effdet_anchor.cuh, shared with effdet_loss.cu).
 #include "nms.cuh"
 #include "effdet_focal.cuh"
+#include "effdet_anchor.cuh"
 #include "bulkcopy.cuh"
 
-#define EF_MAX_LEVELS 8
 #define EF_STAGES 2
-
-struct EfLevels {
-  int num_levels, A;
-  int h[EF_MAX_LEVELS], w[EF_MAX_LEVELS];
-  int anc_per_img[EF_MAX_LEVELS];   // h*w*A
-  int anchor_base[EF_MAX_LEVELS];   // flat anchor index of the level's first anchor within an image
-  const float* table;               // device
-  int tab_off[EF_MAX_LEVELS];       // float offset of the level's [yc(h) | xc(w) | hy(A) | hx(A)] block
-};
-
-struct AnchorBox { float y1, x1, y2, x2; };
-
-__device__ __forceinline__ AnchorBox ef_anchor(const EfLevels& lv, int l, int y, int x, int a) {
-  const float* t = lv.table + lv.tab_off[l];
-  const float yc = __ldg(t + y), xc = __ldg(t + lv.h[l] + x);
-  const float hy = __ldg(t + lv.h[l] + lv.w[l] + a), hx = __ldg(t + lv.h[l] + lv.w[l] + lv.A + a);
-  AnchorBox b;
-  b.y1 = DM_SUB(yc, hy); b.x1 = DM_SUB(xc, hx); b.y2 = DM_ADD(yc, hy); b.x2 = DM_ADD(xc, hx);  // anc:77-78
-  return b;
-}
-
-__device__ __forceinline__ void ef_split(const EfLevels& lv, int l, int rin, int& y, int& x, int& a) {
-  const int cell = rin / lv.A;
-  a = rin - cell * lv.A;
-  y = cell / lv.w[l];
-  x = cell - y * lv.w[l];
-}
 
 // _boxes_decoder (anc:245-274): the box of anchor `an` from its head offsets rel = (ty, tx, th, tw)
 __device__ __forceinline__ float4 ef_decode_box(const AnchorBox& an, float4 rel) {
@@ -236,6 +205,8 @@ struct EfAssignParams {
   float* out_onehot[EF_MAX_LEVELS];        // (B,H,W,A,C), or null when out_class is used
   int32_t* out_class[EF_MAX_LEVELS];       // (B,H,W,A): class id instead of the one-hot row (sparse-target mode)
   unsigned char* out_mask[EF_MAX_LEVELS];  // (B,H,W,A,1)
+  int32_t* out_match;                      // match mode: the matched row of gt_boxes (or -1) per anchor, level l at B*anchor_base[l]
+  double* positives;                       // match mode: += matched anchors
   int cta_base[EF_MAX_LEVELS + 1];         // CTAs of 256 anchors, per (level, image)
   int chunks_per_img[EF_MAX_LEVELS];
 };
@@ -331,23 +302,20 @@ __global__ void __launch_bounds__(256, 8) effdet_assign_kernel(EfAssignParams p)
   }
   // encode + outputs
   const bool matched = active && (n_gt > 0) && (best >= p.thr);  // iou_max >= thr (anc:121)
+  const size_t abase = (size_t)img * api;
+  if (p.out_match) {  // match mode (block-uniform): the GT row stands for the targets, the loss pass encodes them itself
+    if (active) p.out_match[(size_t)p.B * p.lv.anchor_base[l] + abase + rin] = matched ? g_beg + best_i : -1;
+    const int n = __syncthreads_count(matched);
+    if (threadIdx.x == 0 && n > 0) atomicAdd(p.positives, (double)n);  // integer-valued: exact and order-independent
+    return;
+  }
   int cls = 0;
   float4 enc = make_float4(0.f, 0.f, 0.f, 0.f);
   if (matched) {
     const float* q = p.gt_boxes + 4 * (size_t)(g_beg + best_i);
-    const float by1 = q[0], bx1 = q[1], by2 = q[2], bx2 = q[3];
     cls = p.gt_classes[g_beg + best_i];
-    // _boxes_encoder, anc:231-243
-    const float yca = DM_DIV(DM_ADD(an.c2, an.c0), 2.0f), xca = DM_DIV(DM_ADD(an.c3, an.c1), 2.0f);
-    const float ha = dm_max(1e-8f, DM_SUB(an.c2, an.c0)), wa = dm_max(1e-8f, DM_SUB(an.c3, an.c1));
-    const float yc = DM_DIV(DM_ADD(by2, by1), 2.0f), xc = DM_DIV(DM_ADD(bx2, bx1), 2.0f);
-    const float h = dm_max(1e-8f, DM_SUB(by2, by1)), w = dm_max(1e-8f, DM_SUB(bx2, bx1));
-    enc.x = DM_DIV(DM_SUB(yc, yca), ha);
-    enc.y = DM_DIV(DM_SUB(xc, xca), wa);
-    enc.z = dm_logf(DM_DIV(h, ha));
-    enc.w = dm_logf(DM_DIV(w, wa));
+    enc = ef_encode_box(an.c0, an.c1, an.c2, an.c3, q[0], q[1], q[2], q[3]);
   }
-  const size_t abase = (size_t)img * api;
   if (active) {
     p.out_boxes[l][abase + rin] = enc;
     p.out_mask[l][abase + rin] = matched ? 1 : 0;
@@ -388,24 +356,6 @@ __global__ void __launch_bounds__(256, 8) effdet_assign_kernel(EfAssignParams p)
 }
 
 // ---- host side ------------------------------------------------------------------------------------
-static int ef_fill_levels(EfLevels& lv, int num_levels, const int32_t* hw, int A, const float* table_dev) {
-  if (num_levels < 1 || num_levels > EF_MAX_LEVELS || A < 1) return -1;
-  lv.num_levels = num_levels; lv.A = A; lv.table = table_dev;
-  int base = 0, off = 0;
-  for (int l = 0; l < EF_MAX_LEVELS; ++l) {
-    if (l < num_levels) {
-      lv.h[l] = hw[2 * l]; lv.w[l] = hw[2 * l + 1];
-      if (lv.h[l] <= 0 || lv.w[l] <= 0) return -1;
-      lv.anc_per_img[l] = lv.h[l] * lv.w[l] * A;
-      lv.anchor_base[l] = base; base += lv.anc_per_img[l];
-      lv.tab_off[l] = off; off += lv.h[l] + lv.w[l] + 2 * A;
-    } else {
-      lv.h[l] = lv.w[l] = 1; lv.anc_per_img[l] = 0; lv.anchor_base[l] = base; lv.tab_off[l] = off;
-    }
-  }
-  return base;
-}
-
 extern "C" size_t b200_effdet_table_floats(int num_levels, const int32_t* hw, int A) {
   size_t n = 0;
   for (int l = 0; l < num_levels; ++l) n += (size_t)hw[2 * l] + hw[2 * l + 1] + 2 * (size_t)A;
@@ -572,6 +522,18 @@ extern "C" int b200_effdet_postprocess(int num_levels, const int32_t* hw, int A,
                       workspace_bytes, stream_);
 }
 
+// CTAs of 256 anchors per (level, image); returns the grid size
+static int ef_assign_plan(EfAssignParams& p) {
+  int cta = 0;
+  for (int l = 0; l < EF_MAX_LEVELS; ++l) {
+    p.cta_base[l] = cta;
+    p.chunks_per_img[l] = l < p.lv.num_levels ? (p.lv.anc_per_img[l] + 255) / 256 : 1;
+    if (l < p.lv.num_levels) cta += p.chunks_per_img[l] * p.B;
+  }
+  p.cta_base[EF_MAX_LEVELS] = cta;
+  return cta;
+}
+
 static int ef_assign_impl(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
                           const float* gt_boxes, const int32_t* gt_classes, const int32_t* gt_offsets, float iou_thr,
                           float* const out_boxes[], float* const out_onehot[], int32_t* const out_class[],
@@ -584,9 +546,8 @@ static int ef_assign_impl(int num_levels, const int32_t* hw, int A, const float*
   p.B = B; p.C = C; p.thr = iou_thr;
   p.magic_c = C == 1 ? 0u : (uint32_t)((1ull << 32) / (unsigned long long)C + 1ull);
   p.gt_boxes = gt_boxes; p.gt_classes = gt_classes; p.gt_offsets = gt_offsets;
-  int cta = 0;
+  p.out_match = nullptr; p.positives = nullptr;
   for (int l = 0; l < EF_MAX_LEVELS; ++l) {
-    p.cta_base[l] = cta;
     if (l < num_levels) {
       B200_REQUIRE(out_boxes[l] && (out_onehot ? out_onehot[l] != nullptr : out_class[l] != nullptr) && out_mask[l], B200_ERR_BAD_ARG,
                    "b200_effdet_assign_targets: null level %d", l);
@@ -595,11 +556,9 @@ static int ef_assign_impl(int num_levels, const int32_t* hw, int A, const float*
       p.out_onehot[l] = out_onehot ? out_onehot[l] : nullptr;
       p.out_class[l] = out_onehot ? nullptr : out_class[l];
       p.out_mask[l] = out_mask[l];
-      p.chunks_per_img[l] = (p.lv.anc_per_img[l] + 255) / 256;
-      cta += p.chunks_per_img[l] * B;
-    } else { p.out_boxes[l] = nullptr; p.out_onehot[l] = nullptr; p.out_class[l] = nullptr; p.out_mask[l] = nullptr; p.chunks_per_img[l] = 1; }
+    } else { p.out_boxes[l] = nullptr; p.out_onehot[l] = nullptr; p.out_class[l] = nullptr; p.out_mask[l] = nullptr; }
   }
-  for (int l = num_levels; l <= EF_MAX_LEVELS; ++l) p.cta_base[l] = cta;
+  const int cta = ef_assign_plan(p);
   effdet_assign_kernel<<<cta, 256, 0, (cudaStream_t)stream>>>(p);
   B200_LAUNCH_CHECK();
   return B200_OK;
@@ -621,6 +580,38 @@ extern "C" int b200_effdet_assign_targets_indexed(int num_levels, const int32_t*
   B200_REQUIRE(out_class, B200_ERR_BAD_ARG, "b200_effdet_assign_targets_indexed: null argument");
   return ef_assign_impl(num_levels, hw, A, table_dev, C, B, gt_boxes, gt_classes, gt_offsets, iou_thr, out_boxes, nullptr,
                         out_class, out_mask, stream);
+}
+
+// Stage 1 of the loss from box lists (effdet_loss.cu has stage 2): the anchor -> GT row of every anchor of the batch
+// into the workspace, sums zeroed and sums[2L] = this call's matched anchors.  The IoU, the culling, the tie rule and the
+// threshold are generate_targets' own (the same kernel in match mode).
+size_t efb_workspace_bytes(int num_levels, int anchors_per_image, int B);   // effdet_loss.cu
+
+extern "C" int b200_effdet_loss_from_boxes_match(int num_levels, const int32_t* hw, int A, const float* table_dev, int B,
+                                                 const float* gt_boxes, const int32_t* gt_offsets, int total_boxes,
+                                                 float iou_thr, double* sums, void* workspace, size_t workspace_bytes,
+                                                 void* stream) {
+  const char* who = "b200_effdet_loss_from_boxes_match";
+  EfAssignParams p;
+  B200_REQUIRE(hw && table_dev && gt_offsets && sums, B200_ERR_BAD_ARG, "%s: null argument", who);
+  const int n_img = ef_fill_levels(p.lv, num_levels, hw, A, table_dev);
+  B200_REQUIRE(n_img >= 0, B200_ERR_BAD_ARG, "%s: bad level spec", who);
+  B200_REQUIRE(B >= 0 && total_boxes >= 0, B200_ERR_BAD_ARG, "%s: negative batch or box count", who);
+  B200_REQUIRE(total_boxes == 0 || gt_boxes, B200_ERR_BAD_ARG, "%s: null gt_boxes", who);
+  const size_t need = efb_workspace_bytes(num_levels, n_img, B);
+  B200_REQUIRE(workspace && workspace_bytes >= need, B200_ERR_WORKSPACE, "%s: workspace %zu < required %zu", who, workspace_bytes, need);
+  B200_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, B200_ERR_BAD_ARG, "%s: workspace not 256-byte aligned", who);
+  B200_CUDA(cudaMemsetAsync(sums, 0, sizeof(double) * (2 * num_levels + 1), (cudaStream_t)stream));
+  if (B == 0) return B200_OK;
+  p.B = B; p.C = 1; p.magic_c = 0u; p.thr = iou_thr;
+  p.gt_boxes = gt_boxes; p.gt_classes = nullptr; p.gt_offsets = gt_offsets;
+  for (int l = 0; l < EF_MAX_LEVELS; ++l) { p.out_boxes[l] = nullptr; p.out_onehot[l] = nullptr; p.out_class[l] = nullptr; p.out_mask[l] = nullptr; }
+  p.out_match = static_cast<int32_t*>(workspace);
+  p.positives = sums + 2 * num_levels;
+  const int cta = ef_assign_plan(p);
+  effdet_assign_kernel<<<cta, 256, 0, (cudaStream_t)stream>>>(p);
+  B200_LAUNCH_CHECK();
+  return B200_OK;
 }
 
 // ---- fused eval-step stream (test_step, efficientnet/efficientdet_net_train.py:135-169) ----------------------------

@@ -16,6 +16,7 @@
 #include "detmath.h"
 #include "exchange.cuh"
 #include "effdet_focal.cuh"
+#include "effdet_anchor.cuh"
 
 #define EL_MAX_LEVELS 8
 #define EL_THREADS 256
@@ -181,7 +182,8 @@ struct ElGradParams {
   const double* sums;  // [2L+1], sums[2L] = positives
 };
 
-__device__ __forceinline__ float el_focal_grad(float y, float x, float alpha, float gamma, float ls) {
+// The focal derivative and, from the same intermediates, the focal value af*mod*ce (4 MUFU operations for both).
+__device__ __forceinline__ float el_focal_value_grad(float y, float x, float alpha, float gamma, float ls, float& value) {
   const float e = el_ex2(-1.4426950408889634f * fabsf(x));
   const float r = el_rcp(1.0f + e);
   const float p = (x >= 0.0f) ? r : e * r;
@@ -194,7 +196,13 @@ __device__ __forceinline__ float el_focal_grad(float y, float x, float alpha, fl
   const float ys = y * (1.0f - ls) + 0.5f * ls;
   const float ce = fmaxf(x, 0.0f) - x * ys - 0.6931471805599453f * el_lg2(r);
   const float dq = -(2.0f * y - 1.0f) * p * (1.0f - p);
+  value = af * mod * ce;
   return af * (dmod * dq * ce + mod * (p - ys));
+}
+
+__device__ __forceinline__ float el_focal_grad(float y, float x, float alpha, float gamma, float ls) {
+  float unused;
+  return el_focal_value_grad(y, x, alpha, gamma, ls, unused);
 }
 
 __device__ __forceinline__ float el_huber_grad(float t, float o, float delta) {
@@ -268,13 +276,11 @@ __global__ void __launch_bounds__(EL_THREADS) focal_box_grad_kernel(ElGradParams
 }
 
 // ---- host side ------------------------------------------------------------------------------------
-static int el_cta_plan(int num_levels, const unsigned long long* cls_elems, int* cta_base) {
-  // CTAs proportional to the class-tensor size of each level, ~64 per SM in total, at least 1 per level.  Measured on
-  // D0 B=128: 8 per SM 0.80 ms, 16 0.75, 32 0.71, 64 0.69 (92 % of the copy bandwidth), 96 0.69 — many short CTAs
-  // keep the tail of every level busy.
+// CTAs proportional to the class-tensor size of each level, `budget` in total (at most budget + num_levels after
+// rounding up), at least 1 per level.
+static int el_cta_plan_budget(int num_levels, const unsigned long long* cls_elems, int* cta_base, int budget) {
   unsigned long long tot = 0;
   for (int l = 0; l < num_levels; ++l) tot += cls_elems[l];
-  const int budget = b200_sm_count() * 64;
   int c = 0;
   for (int l = 0; l < num_levels; ++l) {
     cta_base[l] = c;
@@ -286,6 +292,12 @@ static int el_cta_plan(int num_levels, const unsigned long long* cls_elems, int*
   }
   for (int l = num_levels; l <= EL_MAX_LEVELS; ++l) cta_base[l] = c;
   return c;
+}
+
+static int el_cta_plan(int num_levels, const unsigned long long* cls_elems, int* cta_base) {
+  // ~64 CTAs per SM.  Measured on D0 B=128: 8 per SM 0.80 ms, 16 0.75, 32 0.71, 64 0.69 (92 % of the copy bandwidth),
+  // 96 0.69 — many short CTAs keep the tail of every level busy.
+  return el_cta_plan_budget(num_levels, cls_elems, cta_base, b200_sm_count() * 64);
 }
 
 // FocalLoss.call (focal_loss.py:26-52): the per-element tensor alpha*mod*ce/normalizer.
@@ -514,4 +526,202 @@ extern "C" int b200_focal_box_grad_indexed(int num_levels, const unsigned long l
   B200_REQUIRE(true_class_index, B200_ERR_BAD_ARG, "b200_focal_box_grad_indexed: null argument");
   return el_grad_impl(num_levels, anchors_per_level, C, true_boxes, nullptr, true_class_index, pred_boxes, pred_classes, alpha,
                       gamma, delta, label_smoothing, sums, numel_per_level_host, grad_boxes, grad_classes, stream);
+}
+
+// ---- loss and gradient from box lists, stage 2 (SURVEY §8f N3 + N1) --------------------------------------------------
+// One pass over the heads after b200_effdet_loss_from_boxes_match (effdet.cu) has left the matched GT row of every anchor
+// in the workspace: the class of an anchor is gt_classes[match] (0 = background when unmatched), its box target is
+// encoded in registers from the rebuilt anchor and the GT box.  The focal and Huber terms go to per-CTA partials
+// {focal_l, huber_l, 0} (the positives are the match stage's), the gradients — the arithmetic of focal_box_grad_kernel on
+// the same targets, so the same bits — are written when their pointers are given.
+#define EFB_MAX_CTAS 16384   // cap of the CTA plan: keeps the workspace size independent of the device
+
+struct EfbParams {
+  EfLevels lv;
+  int B, C;
+  const float* gt_boxes;       // [total,4] y1,x1,y2,x2
+  const int32_t* gt_classes;   // [total]
+  const int32_t* match;        // per anchor: row of gt_boxes or -1; level l at B*anchor_base[l]
+  const float4* cls_pred[EL_MAX_LEVELS]; float4* cls_grad[EL_MAX_LEVELS];
+  const float4* box_pred[EL_MAX_LEVELS]; float4* box_grad[EL_MAX_LEVELS];
+  unsigned long long cls_vec[EL_MAX_LEVELS];
+  int cls_tail[EL_MAX_LEVELS];
+  unsigned long long anchors[EL_MAX_LEVELS];   // B*H*W*A
+  double numel[EL_MAX_LEVELS];
+  int cta_base[EL_MAX_LEVELS + 1];
+  float alpha, gamma, delta, label_smoothing;
+  const double* sums;   // sums[2L] = positives (after the caller's all-reduce)
+  double* partials;     // [n_cta, 3]
+};
+
+// the class id whose one-hot row generate_targets writes for anchor a (anc:131-133: class 0 when unmatched)
+__device__ __forceinline__ int efb_class(const EfbParams& p, const int32_t* match, unsigned long long a) {
+  const int m = __ldg(match + a);
+  return m >= 0 ? __ldg(p.gt_classes + m) : 0;
+}
+
+__global__ void __launch_bounds__(EL_THREADS) effdet_loss_from_boxes_kernel(EfbParams p) {
+  __shared__ double s_red[EL_THREADS / 32][2];
+  int l = 0;
+#pragma unroll
+  for (int k = 1; k < EL_MAX_LEVELS; ++k) if (k < p.lv.num_levels && (int)blockIdx.x >= p.cta_base[k]) l = k;
+  const int ncta = p.cta_base[l + 1] - p.cta_base[l];
+  const int cta = blockIdx.x - p.cta_base[l];
+  const unsigned long long stride = (unsigned long long)ncta * EL_THREADS;
+  const float npos = (float)p.sums[2 * p.lv.num_levels] + 1.0f;
+  const float cs = (float)(1.0 / ((double)npos * p.numel[l]));
+  const float bs = 50.0f / (4.0f * npos);
+  const int32_t* __restrict__ match = p.match + (size_t)p.B * p.lv.anchor_base[l];
+  const int C = p.C;
+  // class half: flat float4 walk over the logits; a float4 straddles at most two anchors (C >= 4)
+  float f0 = 0.f, f1 = 0.f;
+  double focal = 0.0;
+  int it = 0;
+  const float4* __restrict__ cp = p.cls_pred[l];
+  float4* __restrict__ cg = p.cls_grad[l];
+  const unsigned long long nv = p.cls_vec[l];
+#pragma unroll 2
+  for (unsigned long long i = (unsigned long long)cta * EL_THREADS + threadIdx.x; i < nv; i += stride) {
+    const float4 x = __ldcs(cp + i);
+    const unsigned long long e = i * 4ull, a0 = e / (unsigned long long)C;
+    const int c0 = (int)(e - a0 * (unsigned long long)C);
+    const int id0 = efb_class(p, match, a0);
+    const int id1 = (c0 + 3 >= C) ? efb_class(p, match, a0 + 1) : 0;
+    float yy[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int c = c0 + k;
+      yy[k] = (c < C) ? ((c == id0) ? 1.0f : 0.0f) : ((c - C == id1) ? 1.0f : 0.0f);   // ids outside [0, C): zero row
+    }
+    float v0, v1, v2, v3;
+    float4 g;
+    g.x = cs * el_focal_value_grad(yy[0], x.x, p.alpha, p.gamma, p.label_smoothing, v0);
+    g.y = cs * el_focal_value_grad(yy[1], x.y, p.alpha, p.gamma, p.label_smoothing, v1);
+    g.z = cs * el_focal_value_grad(yy[2], x.z, p.alpha, p.gamma, p.label_smoothing, v2);
+    g.w = cs * el_focal_value_grad(yy[3], x.w, p.alpha, p.gamma, p.label_smoothing, v3);
+    if (cg) __stcs(cg + i, g);
+    f0 += v0 + v1;
+    f1 += v2 + v3;
+    if ((++it & 63) == 0) { focal += (double)f0 + (double)f1; f0 = f1 = 0.f; }
+  }
+  if (cta == 0 && (int)threadIdx.x < p.cls_tail[l]) {
+    const unsigned long long e = nv * 4ull + threadIdx.x, a = e / (unsigned long long)C;
+    const float yt = ((int)(e - a * (unsigned long long)C) == efb_class(p, match, a)) ? 1.0f : 0.0f;
+    float v;
+    const float g = cs * el_focal_value_grad(yt, reinterpret_cast<const float*>(cp)[e], p.alpha, p.gamma, p.label_smoothing, v);
+    if (cg) reinterpret_cast<float*>(cg)[e] = g;
+    f0 += v;
+  }
+  focal += (double)f0 + (double)f1;
+  // box half: one anchor per thread, the target encoded from the rebuilt anchor and the matched GT box
+  float hub = 0.f;
+  const unsigned long long na = p.anchors[l];
+  const unsigned int api = (unsigned int)p.lv.anc_per_img[l];
+  float4* __restrict__ bg = p.box_grad[l];
+  for (unsigned long long a = (unsigned long long)cta * EL_THREADS + threadIdx.x; a < na; a += stride) {
+    const float4 o = __ldcs(p.box_pred[l] + a);
+    const int m = __ldg(match + a);
+    float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (m >= 0) {
+      const int rin = (int)(a % api);
+      int y, x, an_i;
+      ef_split(p.lv, l, rin, y, x, an_i);
+      const AnchorBox an = ef_anchor(p.lv, l, y, x, an_i);
+      const float4 q = __ldg(reinterpret_cast<const float4*>(p.gt_boxes) + m);
+      t = ef_encode_box(an.y1, an.x1, an.y2, an.x2, q.x, q.y, q.z, q.w);
+    }
+    hub += el_huber(t.x, o.x, p.delta) + el_huber(t.y, o.y, p.delta) + el_huber(t.z, o.z, p.delta) + el_huber(t.w, o.w, p.delta);
+    if (bg) __stcs(bg + a, make_float4(bs * el_huber_grad(t.x, o.x, p.delta), bs * el_huber_grad(t.y, o.y, p.delta),
+                                       bs * el_huber_grad(t.z, o.z, p.delta), bs * el_huber_grad(t.w, o.w, p.delta)));
+  }
+  const double v0 = warp_sum_d(focal), v1 = warp_sum_d((double)hub);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (lane == 0) { s_red[warp][0] = v0; s_red[warp][1] = v1; }
+  __syncthreads();
+  if (threadIdx.x < 3) {
+    double s = 0.0;
+    if (threadIdx.x < 2)
+      for (int w = 0; w < EL_THREADS / 32; ++w) s += s_red[w][threadIdx.x];
+    p.partials[(size_t)blockIdx.x * 3 + threadIdx.x] = s;   // {focal_l, huber_l, 0}
+  }
+}
+
+// workspace: [match: int32 per anchor of the batch][partials: 3 doubles per CTA]
+static size_t efb_match_bytes(int anchors_per_image, int B) {
+  return b200_align_up(sizeof(int32_t) * (size_t)anchors_per_image * (size_t)B, 256);
+}
+
+size_t efb_workspace_bytes(int num_levels, int anchors_per_image, int B) {
+  return efb_match_bytes(anchors_per_image, B) + b200_align_up(sizeof(double) * 3 * (size_t)(EFB_MAX_CTAS + num_levels), 256);
+}
+
+extern "C" size_t b200_effdet_loss_from_boxes_workspace_bytes(int num_levels, const int32_t* hw, int A, int B) {
+  EfLevels lv;
+  if (!hw || B < 0) return 0;
+  const int n_img = ef_fill_levels(lv, num_levels, hw, A, nullptr);
+  return n_img < 0 ? 0 : efb_workspace_bytes(num_levels, n_img, B);
+}
+
+extern "C" int b200_effdet_loss_from_boxes_grad(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
+                                                const float* gt_boxes, const int32_t* gt_classes, int total_boxes,
+                                                const float* const pred_boxes[], const float* const pred_classes[], float alpha,
+                                                float gamma, float delta, float label_smoothing,
+                                                const double* numel_per_level_host, double* sums, float* const grad_boxes[],
+                                                float* const grad_classes[], void* workspace, size_t workspace_bytes,
+                                                void* stream_) {
+  const char* who = "b200_effdet_loss_from_boxes_grad";
+  cudaStream_t stream = (cudaStream_t)stream_;
+  EfbParams p;
+  B200_REQUIRE(hw && table_dev && pred_boxes && pred_classes && numel_per_level_host && sums, B200_ERR_BAD_ARG, "%s: null argument", who);
+  const int n_img = ef_fill_levels(p.lv, num_levels, hw, A, table_dev);
+  B200_REQUIRE(n_img >= 0, B200_ERR_BAD_ARG, "%s: bad level spec", who);
+  B200_REQUIRE(C >= 4, B200_ERR_UNSUPPORTED, "%s: needs classes_num >= 4 (got %d)", who, C);
+  B200_REQUIRE(B >= 0 && total_boxes >= 0, B200_ERR_BAD_ARG, "%s: negative batch or box count", who);
+  B200_REQUIRE(total_boxes == 0 || (gt_boxes && gt_classes), B200_ERR_BAD_ARG, "%s: null gt_boxes / gt_classes", who);
+  B200_REQUIRE((reinterpret_cast<uintptr_t>(gt_boxes) & 15) == 0, B200_ERR_BAD_ARG, "%s: gt_boxes not 16-byte aligned", who);
+  unsigned long long plan[EL_MAX_LEVELS];
+  for (int l = 0; l < EL_MAX_LEVELS; ++l) {
+    p.cls_pred[l] = nullptr; p.cls_grad[l] = nullptr; p.box_pred[l] = nullptr; p.box_grad[l] = nullptr;
+    p.cls_vec[l] = 0; p.cls_tail[l] = 0; p.anchors[l] = 0; p.numel[l] = 1.0; plan[l] = 0;
+    if (l >= num_levels) continue;
+    B200_REQUIRE(pred_boxes[l] && pred_classes[l], B200_ERR_BAD_ARG, "%s: null prediction at level %d", who, l);
+    B200_REQUIRE(!grad_boxes || grad_boxes[l], B200_ERR_BAD_ARG, "%s: null grad_boxes at level %d", who, l);
+    B200_REQUIRE(!grad_classes || grad_classes[l], B200_ERR_BAD_ARG, "%s: null grad_classes at level %d", who, l);
+    const uintptr_t al = reinterpret_cast<uintptr_t>(pred_boxes[l]) | reinterpret_cast<uintptr_t>(pred_classes[l]) |
+                         (grad_boxes ? reinterpret_cast<uintptr_t>(grad_boxes[l]) : 0) |
+                         (grad_classes ? reinterpret_cast<uintptr_t>(grad_classes[l]) : 0);
+    B200_REQUIRE((al & 15) == 0, B200_ERR_BAD_ARG, "%s: level %d tensors must be 16-byte aligned", who, l);
+    B200_REQUIRE(numel_per_level_host[l] > 0.0, B200_ERR_BAD_ARG, "%s: numel of level %d must be positive", who, l);
+    const unsigned long long na = (unsigned long long)B * (unsigned long long)p.lv.anc_per_img[l], n = na * (unsigned long long)C;
+    p.cls_pred[l] = reinterpret_cast<const float4*>(pred_classes[l]);
+    p.cls_grad[l] = grad_classes ? reinterpret_cast<float4*>(grad_classes[l]) : nullptr;
+    p.box_pred[l] = reinterpret_cast<const float4*>(pred_boxes[l]);
+    p.box_grad[l] = grad_boxes ? reinterpret_cast<float4*>(grad_boxes[l]) : nullptr;
+    p.cls_vec[l] = n / 4ull;
+    p.cls_tail[l] = (int)(n - p.cls_vec[l] * 4ull);
+    p.anchors[l] = na;
+    p.numel[l] = numel_per_level_host[l];
+    plan[l] = n > na * 4ull ? n : na * 4ull;
+    if (plan[l] == 0) plan[l] = 4;
+  }
+  const size_t need = efb_workspace_bytes(num_levels, n_img, B);
+  B200_REQUIRE(workspace && workspace_bytes >= need, B200_ERR_WORKSPACE, "%s: workspace %zu < required %zu", who, workspace_bytes, need);
+  B200_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, B200_ERR_BAD_ARG, "%s: workspace not 256-byte aligned", who);
+  if (B == 0) return B200_OK;   // the match stage left sums[0..2L) at zero
+  p.B = B; p.C = C;
+  p.gt_boxes = gt_boxes; p.gt_classes = gt_classes;
+  unsigned char* wsb = static_cast<unsigned char*>(workspace);
+  p.match = reinterpret_cast<const int32_t*>(wsb);
+  p.partials = reinterpret_cast<double*>(wsb + efb_match_bytes(n_img, B));
+  p.alpha = alpha; p.gamma = gamma; p.delta = delta; p.label_smoothing = label_smoothing; p.sums = sums;
+  const int budget = b200_sm_count() * 64;
+  const int n_cta = el_cta_plan_budget(num_levels, plan, p.cta_base, budget < EFB_MAX_CTAS ? budget : EFB_MAX_CTAS);
+  effdet_loss_from_boxes_kernel<<<n_cta, EL_THREADS, 0, stream>>>(p);
+  B200_LAUNCH_CHECK();
+  ElReduce r;
+  r.partials = p.partials; r.num_levels = num_levels; r.sums = sums;
+  for (int l = 0; l <= EL_MAX_LEVELS; ++l) r.cta_base[l] = p.cta_base[l];
+  focal_box_reduce_kernel<<<num_levels, 256, 0, stream>>>(r);   // sums[0..2L); adds the partials' 0 to sums[2L]
+  B200_LAUNCH_CHECK();
+  return B200_OK;
 }
