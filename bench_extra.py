@@ -215,6 +215,116 @@ def main():
                     note="bytes: read logits + box outputs, write both gradients, write + read one int32 match per anchor"))
         del rel, cls
         torch.cuda.empty_cache()
+    if want("c3_sparse_eval"):  # test_step of config 3 from box lists against the dense-target eval step
+        card = _card()
+        c = synth.EFFDET_CONFIGS["d0"]
+        batch, C = 128, 81
+        a = Anchors(c["min_level"], c["max_level"], c["image_size"], c["num_scales"], c["aspect_ratios"], c["anchor_scale"])
+        shapes = [tuple(b.shape) for b in a.boxes]
+        rel = [torch.randn((batch,) + s, device=dev, generator=g) * 0.25 for s in shapes]
+        cls = [torch.randn((batch,) + s[:-1] + (C,), device=dev, generator=g) for s in shapes]
+        n_anchor = sum(s[0] * s[1] * s[2] for s in shapes)
+        rng = np.random.default_rng(20261018 + 3)
+        boxes, classes, off = synth.gt_batch(rng, batch, (c["image_size"][1], c["image_size"][0]), max_boxes=100, order="yxyx")
+        d_boxes, d_cls, d_off = (torch.from_numpy(boxes).to(dev), torch.from_numpy((classes + 1).astype(np.int32)).to(dev),
+                                 torch.from_numpy(off).to(dev))
+        targets = a.generate_targets_batch(d_boxes, d_cls, d_off, C)
+        arms = {
+            "from_boxes": lambda: a.eval_step_from_boxes(d_boxes, d_cls, d_off, rel, cls),
+            "targets_and_eval": lambda: a.eval_step(*a.generate_targets_batch(d_boxes, d_cls, d_off, C), rel, cls),
+            "eval_precomputed": lambda: a.eval_step(*targets, rel, cls),
+        }
+        # the match stage alone (the same kernel and launch as the first stage of eval_step_from_boxes): separates its time
+        # from the stream's
+        import ctypes
+        from tfmv_b200 import _lib, _tensors as T
+        lib = _lib.load()
+        L = a._num_levels
+        m_sums = torch.empty((2 * L + 1,), dtype=torch.float64, device=dev)
+        m_ws = torch.empty((lib.b200_effdet_loss_from_boxes_workspace_bytes(L, a._hw, a._A, batch),), dtype=torch.uint8, device=dev)
+        arms["match_stage"] = lambda: lib.b200_effdet_loss_from_boxes_match(
+            L, a._hw, a._A, T.ptr(a._dev_table()), batch, T.ptr(d_boxes), T.ptr(d_off), d_boxes.shape[0], ctypes.c_float(0.5),
+            T.ptr(m_sums), T.ptr(m_ws), m_ws.numel(), T.stream_ptr())
+        got = a.eval_step_from_boxes(d_boxes, d_cls, d_off, rel, cls, with_indices=True, return_parts=True)
+        ref = a.eval_step(*targets, rel, cls, with_indices=True, return_parts=True)
+        bits = lambda x, y: x.shape == y.shape and torch.equal(x.reshape(-1).view(torch.uint8), y.reshape(-1).view(torch.uint8))
+        cnt = ref[2]["count"]
+        rows = torch.arange(ref[2]["boxes"].shape[1], device=dev)[None, :] < cnt[:, None]   # rows past count are not written
+        assert bits(got[0], ref[0]) and bits(got[3], ref[3]) and bits(got[4], ref[4]), "loss terms differ"
+        assert all(bits(x, y) for x, y in zip(got[1], ref[1])), "decoded boxes differ"
+        assert bits(got[2]["count"], cnt) and all(bits(got[2][k][rows], ref[2][k][rows]) for k in ref[2] if k != "count"), \
+            "NMS outputs differ"
+        del got, ref
+        fns = {k: wrap(f) for k, f in arms.items()}
+        # the arms alternate window by window (order rotated) so that drift of clocks and neighbours hits all of them
+        steps, n_win = max(args.steps, 20), 7
+        times = {k: [] for k in fns}
+        order = list(fns)
+        for w in range(n_win):
+            for k in order[w % len(order):] + order[:w % len(order)]:
+                times[k].append(timed(fns[k], steps, args.warmup))
+        ms = {k: float(np.median(v)) for k, v in times.items()}
+        report("c3_sparse_eval", "EfficientDet-D0 512 B=128 C=81 eval step from box lists: eval_step_from_boxes against "
+               "generate_targets_batch + eval_step and against eval_step on precomputed targets (loss terms, decoded boxes and "
+               "NMS outputs asserted bit-identical first); median of %d alternating windows of %d steps" % (n_win, steps), batch,
+               ms["from_boxes"], n_anchor * (C * 4 + 16 + 16 + 8),
+               dict(card, targets_and_eval_ms=ms["targets_and_eval"], eval_precomputed_targets_ms=ms["eval_precomputed"],
+                    match_stage_ms=ms["match_stage"], stream_reduce_nms_ms=ms["from_boxes"] - ms["match_stage"],
+                    speedup_vs_targets_and_eval=ms["targets_and_eval"] / ms["from_boxes"],
+                    speedup_vs_precomputed=ms["eval_precomputed"] / ms["from_boxes"],
+                    window_ms={k: [round(t, 5) for t in v] for k, v in times.items()}, outputs_bit_identical=True,
+                    note="bytes: read logits + box outputs, write the decoded boxes, write + read one int32 match per anchor"))
+        del rel, cls, targets, m_ws
+        torch.cuda.empty_cache()
+    if want("c5_sparse_eval"):  # test_step of config 5 from box lists against the dense targets + host-offset mAP
+        from tfmv_b200.ai_models.utils.mAP import Get_mAP_batch
+        card = _card()
+        batch, image, C = 64, 608, 80
+        heads = yolo_heads(batch, image)
+        rng = np.random.default_rng(20261018 + 5)
+        boxes, classes, off = synth.gt_batch(rng, batch, (image, image), max_boxes=100)
+        boxes_d, classes_d, off_d = (torch.from_numpy(x).to(dev) for x in (boxes, classes, off))
+        gen = DataGenerator(C, anc, (image, image))
+        wh = (image, image)
+
+        def dense():
+            y = gen.GetTargetsBatch(classes_d, boxes_d, off_d)
+            loss, r = tyu.LossAndNMSBoxesBatch(y, heads, wh, anc, C, 0.5, "ciou", nms_iou_type="diou")
+            # GetGroudTruth per level (batch-major) regrouped per image, the NMS rows compacted: host offsets for Get_mAP_batch
+            per_level = [tyu.GetGroudTruth(t) for t in y]
+            n_l = [(t[..., 4] != 0).reshape(batch, -1).sum(1).cpu().numpy() for t in y]
+            parts = [torch.split(g, n.tolist()) for g, n in zip(per_level, n_l)]
+            gt = torch.cat([p[b] for b in range(batch) for p in parts])
+            go = np.concatenate([[0], np.cumsum(sum(n_l))]).astype(np.int32)
+            cnt = r["count"].cpu().numpy()
+            pred = torch.cat([torch.cat([r["boxes"][b, :n], r["classes_id"][b, :n, None].float(), r["scores"][b, :n, None]], 1)
+                              for b, n in enumerate(cnt)])
+            return loss, r, Get_mAP_batch(gt, go, pred, np.concatenate([[0], np.cumsum(cnt)]).astype(np.int32), C)
+
+        arms = {
+            "from_boxes": lambda: tyu.EvalStepFromBoxes(classes_d, boxes_d, off_d, heads, wh, anc, C, 0.5, "ciou", nms_iou_type="diou"),
+            "dense": dense,
+        }
+        got, ref = arms["from_boxes"](), arms["dense"]()
+        loss_rel = abs(float(got[0]) - float(ref[0])) / abs(float(ref[0]))   # dense GetLoss sums in another order
+        assert loss_rel < 1e-4, "losses differ"
+        assert got[2].cpu().numpy().tobytes() == ref[2].cpu().numpy().tobytes(), "mAP differs"
+        assert torch.equal(got[1]["count"], ref[1]["count"])
+        m_ap = float(got[2].mean())
+        fns = {"from_boxes": wrap(arms["from_boxes"]), "dense": arms["dense"]}   # the dense arm synchronises: no graph
+        steps, n_win = max(args.steps, 20), 7
+        times = {k: [] for k in fns}
+        order = list(fns)
+        for w in range(n_win):
+            for k in order[w % len(order):] + order[:w % len(order)]:
+                times[k].append(timed(fns[k], steps, args.warmup))
+        ms = {k: float(np.median(v)) for k, v in times.items()}
+        report("c5_sparse_eval", "YOLOv4 608 B=64 eval step from box lists: EvalStepFromBoxes(ciou loss, diou NMS, mAP) against "
+               "GetTargetsBatch + LossAndNMSBoxesBatch + GetGroudTruth + Get_mAP_batch (host offsets; mAP asserted bit-identical "
+               "and the loss within 1e-4 first); median of %d alternating windows of %d steps" % (n_win, steps), batch, ms["from_boxes"],
+               7732620, dict(card, dense_targets_and_host_map_ms=ms["dense"], speedup_vs_dense=ms["dense"] / ms["from_boxes"],
+                             mean_map=m_ap, window_ms={k: [round(t, 5) for t in v] for k, v in times.items()},
+                             map_bit_identical=True, loss_rel_diff=loss_rel, note="bytes: read y_pred once (dense equivalent)"))
     if want("n4_letterbox"):  # SURVEY 8f N4: the serving view's image pre-processing, one image per call (latency)
         from tfmv_b200.views.object_detection import prepare_image
         for (h, w) in ((1080, 1920), (3024, 4032), (480, 640), (240, 320)):

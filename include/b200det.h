@@ -198,6 +198,20 @@ int b200_gather_rows(const float* src, int row_floats, const unsigned char* flag
  * y (…,5+C): rows[i] = [x-w/2, y-h/2, x+w/2, y+h/2, argmax(classes)], flags[i] = (conf != 0). */
 int b200_yolo_ground_truth_rows(const float* y, long long n_records, int C, float* rows, unsigned char* flags,
                                 void* stream);
+/* GetGroudTruth of the three levels DataGenerator.GetTargets would write, straight from the box lists (an API
+ * extension; no dense y_true): boxes [total,4] pixel corners x1,y1,x2,y2 (16-byte aligned), classes [total] int32,
+ * offsets [B+1] (device); hw, A, C, anchors_wh_host (the anchors DataGenerator takes) and image_wh_host as for
+ * b200_yolo_assign_targets.  The boxes that reach y_true (the same assignment; boxes colliding on a record are all
+ * dropped) give rows [total,5] x1,y1,x2,y2,class packed at the start of their image's range, level by level in record
+ * order, and count [B] (device) = rows per image; the rows of image b are bit-identical to GetGroudTruth of the three
+ * dense levels of that image (a class id outside [0,C) gives class 0).  Rows past the count are not written.  Every
+ * argument is checked before the launch.  Workspace: b200_yolo_ground_truth_from_boxes_workspace_bytes (one int32 per
+ * box; 0 for a bad spec). */
+size_t b200_yolo_ground_truth_from_boxes_workspace_bytes(const int32_t hw[6], int B, int A, int total_boxes);
+int b200_yolo_ground_truth_from_boxes(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
+                                      int B, const int32_t hw[6], int A, int C, const float* anchors_wh_host,
+                                      const float* image_wh_host, float* rows, int32_t* count, void* workspace,
+                                      size_t workspace_bytes, void* stream);
 
 /* Get_mAP_one (utils/mAP.py:114-125; SURVEY §8f N2), batched: gt [total_gt,5] x1,y1,x2,y2,class; pred [total_pred,6]
  * x1,y1,x2,y2,class,score (fp32, as test_step concatenates them); offsets [num_images+1] int32; out [num_images] fp64.
@@ -205,6 +219,19 @@ int b200_yolo_ground_truth_rows(const float* y, long long n_records, int C, floa
 int b200_map_per_image(const float* gt, const int32_t* gt_offsets, const float* pred, const int32_t* pred_offsets,
                        int num_images, int max_gt_per_image, int max_pred_per_image, int class_num, double thresh,
                        double* out, void* stream);
+/* The same mAP straight from the padded NMS output, with no host-known maxima (an API extension; the call never waits for
+ * the host and can be captured in a CUDA graph).  Predictions as the post-processing writes them: pred_boxes
+ * [num_images,max_out,4] x1,y1,x2,y2 (or any corner order shared with the ground truth), pred_classes [num_images,max_out]
+ * int32 (class_id_bytes = 4, YOLO) or int64 (8, EfficientDet), pred_scores [num_images,max_out], pred_count [num_images]
+ * (device).  Ground truth as box lists: gt_boxes [total_gt,4], gt_classes [total_gt] int32 (may be NULL when total_gt is
+ * 0), gt_offsets [num_images+1] (device, clamped to [0, total_gt]); image b uses rows gt_offsets[b] ..
+ * gt_offsets[b]+gt_count[b] (gt_count device [num_images], or NULL = the whole range).  Shared memory is sized from
+ * max_out (<= 4096); the ground truth is walked in chunks, so any number of boxes per image works.  Same arithmetic as
+ * b200_map_per_image. */
+int b200_map_padded(const float* pred_boxes, const void* pred_classes, int class_id_bytes, const float* pred_scores,
+                    const int32_t* pred_count, int num_images, int max_out, const float* gt_boxes, const int32_t* gt_classes,
+                    int total_gt, const int32_t* gt_offsets, const int32_t* gt_count, int class_num, double thresh, double* out,
+                    void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * EfficientDet (efficientnet/utils/anchors.py, iou.py, nms.py; losses/focal_loss.py, box_loss.py;
@@ -377,6 +404,24 @@ int b200_effdet_decode_postprocess(int num_levels, const int32_t* hw, int A, con
                                    float* out_boxes, long long* out_class_id, float* out_score, int32_t* out_sel_idx,
                                    int32_t* out_sel_anchor, int32_t* out_count, void* workspace, size_t workspace_bytes,
                                    void* stream);
+/* b200_effdet_eval_step from box lists (an API extension): no dense targets.  gt_boxes [total,4] y1,x1,y2,x2 (16-byte
+ * aligned), gt_classes [total] int32, gt_offsets [B+1] (device) as for b200_effdet_assign_targets; match_iou_thr is
+ * generate_targets' iou_threshold.  One call = the match stage of b200_effdet_loss_from_boxes_match (one int32 per anchor
+ * in the workspace), the one-pass stream reading only the logits of the class tensor (the one-hot row, box target and
+ * mask of every anchor rebuilt from its match), the reduce and the NMS tail.  Every output, sums_out included, is
+ * bit-identical to b200_effdet_assign_targets + b200_effdet_eval_step on the same boxes; sums_out feeds
+ * b200_focal_box_finalize or its _dp form unchanged.  classes_num < 4 and > 128 return B200_ERR_UNSUPPORTED (take
+ * b200_effdet_assign_targets + b200_effdet_eval_step, or the separate calls).  Every argument is checked before anything
+ * is enqueued.  Workspace: b200_effdet_eval_step_from_boxes_workspace_bytes (256-byte aligned). */
+size_t b200_effdet_eval_step_from_boxes_workspace_bytes(int num_levels, const int32_t* hw, int A, int num_images, int max_out);
+int b200_effdet_eval_step_from_boxes(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
+                                     const float* gt_boxes, const int32_t* gt_classes, const int32_t* gt_offsets,
+                                     int total_boxes, float match_iou_thr, const float* const pred_boxes[],
+                                     const float* const pred_classes[], float alpha, float gamma, float delta,
+                                     float label_smoothing, double* sums_out, float* const out_decoded[], int max_out,
+                                     float iou_thr, float score_thr, int metric, float* out_boxes, long long* out_class_id,
+                                     float* out_score, int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
+                                     void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- the collective of the path (SURVEY §8b b200_allreduce_loss, §8e) ------------------------------------------
  * Data parallel over images: the only inter-GPU traffic is the sum of a handful of per-GPU partial loss terms (YOLO:

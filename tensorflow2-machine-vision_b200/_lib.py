@@ -93,6 +93,12 @@ SIGNATURES = {
     "b200_effdet_decode_postprocess": (c_i, [c_i, c_p, c_i, c_p, c_i, c_i, c_p, c_p, c_p, c_i, c_f, c_f, c_i, c_p, c_p, c_p, c_p, c_p,
                                              c_p, c_p, c_sz, c_p]),
     "b200_map_per_image": (c_i, [c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, ctypes.c_double, c_p, c_p]),
+    "b200_map_padded": (c_i, [c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_i, c_p, c_p, c_i, ctypes.c_double, c_p, c_p]),
+    "b200_yolo_ground_truth_from_boxes_workspace_bytes": (c_sz, [c_p, c_i, c_i, c_i]),
+    "b200_yolo_ground_truth_from_boxes": (c_i, [c_p, c_p, c_p, c_i, c_i, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
+    "b200_effdet_eval_step_from_boxes_workspace_bytes": (c_sz, [c_i, c_p, c_i, c_i, c_i]),
+    "b200_effdet_eval_step_from_boxes": (c_i, [c_i, c_p, c_i, c_p, c_i, c_i, c_p, c_p, c_p, c_i, c_f, c_p, c_p, c_f, c_f, c_f, c_f,
+                                               c_p, c_p, c_i, c_f, c_f, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
 }
 
 METRIC_YOLO = {"iou": 0, "diou": 1, "ciou": 2}

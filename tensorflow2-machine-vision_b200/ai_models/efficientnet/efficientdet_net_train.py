@@ -76,7 +76,8 @@ def get_loss_and_grad(y_true_boxes, y_true_classes, y_true_masks, y_pred_boxes, 
 
 
 def _from_boxes_args(anchors, boxes, classes, offsets, y_pred_boxes, y_pred_classes):
-  '''Checks and device placement shared by get_loss_from_boxes and get_loss_from_boxes_and_grad.'''
+  '''Checks and device placement shared by get_loss_from_boxes, get_loss_from_boxes_and_grad and
+  Anchors.eval_step_from_boxes.'''
   L = anchors._num_levels
   pb = [T.to_cuda(t) for t in y_pred_boxes]
   pc = [T.to_cuda(t) for t in y_pred_classes]

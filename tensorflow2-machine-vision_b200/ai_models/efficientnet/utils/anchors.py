@@ -296,6 +296,12 @@ class Anchors(object):
                                          T.ptr(out['boxes']), T.ptr(out['classes_id']), T.ptr(out['scores']),
                                          T.ptr(out.get('sel_idx')), T.ptr(out.get('sel_anchor')), T.ptr(out['count']),
                                          T.ptr(ws), ws_bytes, T.stream_ptr()), 'eval_step')
+    return self._eval_finalize(sums, cl, dec, out, exchange, return_parts, 'eval_step')
+
+  def _eval_finalize(self, sums, cl, dec, out, exchange, return_parts, what):
+    '''The tail of the eval steps: the data-parallel sum of the 2L+1 terms and the loss normalisation.'''
+    lib = _lib.load()
+    L, dev = self._num_levels, sums.device
     scale = 1
     peer = exchange is not None and hasattr(exchange, 'mailboxes')
     if exchange is not None:
@@ -309,12 +315,52 @@ class Anchors(object):
     if peer:
       rank, world, boxes_ = exchange.args()
       _lib.check(lib.b200_focal_box_finalize_dp(L, T.ptr(sums), nm, T.ptr(parts), T.ptr(loss), T.ptr(npos), rank, world, boxes_,
-                                                T.stream_ptr()), 'eval_step (data parallel)')
+                                                T.stream_ptr()), what + ' (data parallel)')
     else:
-      _lib.check(lib.b200_focal_box_finalize(L, T.ptr(sums), nm, T.ptr(parts), T.ptr(loss), T.ptr(npos), T.stream_ptr()), 'eval_step')
+      _lib.check(lib.b200_focal_box_finalize(L, T.ptr(sums), nm, T.ptr(parts), T.ptr(loss), T.ptr(npos), T.stream_ptr()), what)
     if return_parts:
       return loss, tuple(dec), out, parts, npos
     return loss, tuple(dec), out
+
+  def eval_step_from_boxes(self, boxes, classes, offsets, y_pred_boxes, y_pred_classes, match_iou_threshold=0.5, alpha=0.25,
+                           gamma=1.5, delta=0.1, max_output_size=200, iou_threshold=0.5, score_threshold=0.0001,
+                           iou_type='diou', with_indices=False, exchange=None, return_parts=False):
+    '''eval_step with the ground truth as box lists instead of the dense targets: boxes [total,4] y1,x1,y2,x2, classes
+    [total], offsets [B+1] as generate_targets_batch takes them (match_iou_threshold is its iou_threshold).  Returns what
+    eval_step returns on generate_targets_batch's targets, bit for bit, without writing the targets: one call matches
+    the anchors to the boxes (one int32 per anchor) and streams the heads once, reading only the logits of the class
+    tensor.  The keyword arguments are eval_step's.  No host synchronisation (capturable with runtime.capture).
+    classes_num < 4 and > 128 take generate_targets_batch + eval_step.
+
+    The per-image mAP of test_step follows from the returned dict, e.g. with the box lists as ground truth:
+    utils.mAP.Get_mAP_padded(boxes, classes, offsets, out, classes_num).'''
+    assert iou_type in ('iou', 'giou', 'diou', 'ciou')
+    from ..efficientdet_net_train import _from_boxes_args
+    gb, gc, go, rel, cl, B, C = _from_boxes_args(self, boxes, classes, offsets, y_pred_boxes, y_pred_classes)
+    if C < 4 or C > 128:
+      # the one-pass stream rebuilds one-hot rows a float4 at a time (C >= 4) and stages 64-anchor tiles of logits in
+      # shared memory (C <= 128): other heads take the dense targets — same results
+      tb, tc, tm = self.generate_targets_batch(gb, gc, go, C, match_iou_threshold)
+      return self.eval_step(tb, tc, tm, rel, cl, alpha=alpha, gamma=gamma, delta=delta, max_output_size=max_output_size,
+                            iou_threshold=iou_threshold, score_threshold=score_threshold, iou_type=iou_type,
+                            with_indices=with_indices, exchange=exchange, return_parts=return_parts)
+    lib = _lib.load()
+    tab = self._dev_table()
+    L, K, dev = self._num_levels, int(max_output_size), cl[0].device
+    dec = [torch.empty_like(t) for t in rel]
+    out = self._post_outputs(B, K, dev, with_indices)
+    sums = torch.empty((2 * L + 1,), dtype=torch.float64, device=dev)
+    ws_bytes = lib.b200_effdet_eval_step_from_boxes_workspace_bytes(L, self._hw, self._A, B, K)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    arr = lambda ts: (ctypes.c_void_p * L)(*[t.data_ptr() for t in ts])
+    _lib.check(lib.b200_effdet_eval_step_from_boxes(L, self._hw, self._A, T.ptr(tab), C, B, T.ptr(gb), T.ptr(gc), T.ptr(go),
+                                                    gb.shape[0], float(match_iou_threshold), arr(rel), arr(cl), float(alpha),
+                                                    float(gamma), float(delta), 0.0, T.ptr(sums), arr(dec), K,
+                                                    float(iou_threshold), float(score_threshold), _lib.METRIC_EFF[iou_type],
+                                                    T.ptr(out['boxes']), T.ptr(out['classes_id']), T.ptr(out['scores']),
+                                                    T.ptr(out.get('sel_idx')), T.ptr(out.get('sel_anchor')), T.ptr(out['count']),
+                                                    T.ptr(ws), ws_bytes, T.stream_ptr()), 'eval_step_from_boxes')
+    return self._eval_finalize(sums, cl, dec, out, exchange, return_parts, 'eval_step_from_boxes')
 
   def convert_outputs_one(self, batch_index, outputs_boxes, outputs_classes):
     '''One image of the batch: (nms_boxes [K,4], nms_classes_id [K] int64, nms_scores [K]); K <= 200.'''

@@ -363,6 +363,73 @@ def LossAndNMSBoxesBatch(y_true, y_pred, image_wh, anchors_wh, classes_num, iou_
   return loss, r
 
 
+def GetGroudTruthFromBoxes(classes, boxes, offsets, image_wh, anchors_wh, classes_num):
+  '''GetGroudTruth of the three levels DataGenerator(classes_num, anchors_wh, image_wh).GetTargetsBatch(classes, boxes,
+  offsets) would write, without the dense targets (an API extension).  classes [total] int, boxes [total,4] pixel corners
+  x1,y1,x2,y2, offsets [B+1]; anchors_wh as DataGenerator takes them.  Returns (rows [total,5], count [B] int32): the rows
+  of image b are rows[offsets[b] : offsets[b] + count[b]], bit-identical to
+  torch.cat([GetGroudTruth(t[b]) for t in GetTargetsBatch(...)]); the rest of its range is zero.  No host
+  synchronisation.'''
+  lib = _lib.load()
+  boxes = T.to_cuda(boxes).reshape(-1, 4)
+  if boxes.data_ptr() % 16:
+    boxes = boxes.clone()   # one 16-byte load per box
+  classes = T.to_cuda(classes, torch.int32).reshape(-1)
+  offsets = T.to_cuda(offsets, torch.int32).reshape(-1)
+  if classes.numel() != boxes.shape[0]:
+    raise ValueError('%d boxes but %d classes' % (boxes.shape[0], classes.numel()))
+  anc = T.host_floats(anchors_wh)
+  if anc.size % 6 != 0:
+    raise ValueError('anchors_wh must be (3, anchors_num, 2)')
+  img = T.host_floats(image_wh, 2)
+  w, h = int(img[0]), int(img[1])
+  hw = (ctypes.c_int32 * 6)(*[d for s in (32, 16, 8) for d in (h // s, w // s)])   # DataGenerator.layers_hw
+  B, total, dev = offsets.numel() - 1, int(boxes.shape[0]), boxes.device
+  if B < 0:
+    raise ValueError('offsets must hold B + 1 entries')
+  rows = torch.zeros((total, 5), dtype=torch.float32, device=dev)
+  count = torch.empty((B,), dtype=torch.int32, device=dev)
+  ws_bytes = lib.b200_yolo_ground_truth_from_boxes_workspace_bytes(hw, B, anc.size // 6, total)
+  ws = torch.empty((max(ws_bytes, 1),), dtype=torch.uint8, device=dev)
+  _lib.check(lib.b200_yolo_ground_truth_from_boxes(T.ptr(boxes), T.ptr(classes), T.ptr(offsets), total, B, hw, anc.size // 6,
+                                                   int(classes_num), anc.ctypes.data_as(ctypes.c_void_p),
+                                                   img.ctypes.data_as(ctypes.c_void_p), T.ptr(rows), T.ptr(count), T.ptr(ws),
+                                                   ws_bytes, T.stream_ptr()), 'GetGroudTruthFromBoxes')
+  return rows, count
+
+
+def EvalStepFromBoxes(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_num, iou_thresh=0.5, iou_type='iou',
+                      confidence_thresh=0.5, scores_thresh=0.3, nms_iou_thresh=0.5, nms_iou_type='iou',
+                      max_output_size=NMS_MAX_OUTPUT, target_anchors=None, batch_divisor=None, map_thresh=0.5,
+                      with_classes=True, with_indices=False, return_parts=False, workspace=None):
+  '''test_step (yolo_v4/model.py:341-378) from box lists, with no dense y_true and no host synchronisation (an API
+  extension): GetLossFromBoxes and GetNMSBoxesBatch on the same y_pred as the two stream branches of LossAndNMSBoxesBatch
+  (the loss branch also builds GetGroudTruthFromBoxes' rows), then Get_mAP_padded of the NMS output against those rows.
+  Arguments: GetLossFromBoxes' (target_anchors = the anchors DataGenerator takes, default anchors_wh) and
+  LossAndNMSBoxesBatch's thresholds.  Returns (loss, dict as GetNMSBoxesBatch, mAP float64 [B]); with return_parts
+  (loss, parts, dict, mAP).  Data parallel: as GetLossFromBoxes — batch_divisor = the global batch, parts combined with
+  combine_loss_parts; the mAP is per image and needs no exchange.  CUDA-graph capturable.'''
+  from .mAP import Get_mAP_padded
+  assert iou_type in ['iou','diou','ciou'] and nms_iou_type in ['iou','diou','ciou']
+  heads = [T.to_cuda(t) for t in y_pred]
+  dev = heads[0].device
+  main = torch.cuda.current_stream(dev)
+  side = _side_stream(dev)
+  side.wait_stream(main)
+  with torch.cuda.stream(side):
+    r = GetNMSBoxesBatch(heads[0], heads[1], heads[2], anchors_wh, image_wh, classes_num, confidence_thresh, scores_thresh,
+                         nms_iou_thresh, nms_iou_type, max_output_size, with_classes, with_indices)
+  loss, parts, _ = _boxes_call(classes, boxes, offsets, heads, image_wh, anchors_wh, classes_num, iou_thresh, iou_type,
+                               target_anchors, batch_divisor, workspace)
+  rows, count = GetGroudTruthFromBoxes(classes, boxes, offsets, image_wh,
+                                       anchors_wh if target_anchors is None else target_anchors, classes_num)
+  main.wait_stream(side)
+  for t in r.values():
+    t.record_stream(main)   # allocated on the side stream, consumed on the current one
+  m_ap = Get_mAP_padded(rows[:, :4], rows[:, 4].to(torch.int32), offsets, r, classes_num, map_thresh, gt_count=count)
+  return (loss, parts, r, m_ap) if return_parts else (loss, r, m_ap)
+
+
 def GetLossAndGrad(y_true, y_pred, image_wh, anchors_wh, iou_thresh=0.5, iou_type='iou'):
   '''GetLoss plus d loss / d y_pred (list of 3 tensors shaped like y_pred) for an upstream gradient of 1 —
   what tf.GradientTape derives from the reference's GetLoss.  Wrap with tf.custom_gradient (INTEGRATION.md §3).'''

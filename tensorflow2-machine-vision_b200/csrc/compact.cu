@@ -6,6 +6,7 @@
 //   a [n, row_floats] array to their positions, one warp per row.
 #include "common.cuh"
 #include "detmath.h"
+#include "yolo_targets.cuh"
 
 #define CP_THREADS 256
 
@@ -85,12 +86,12 @@ __global__ void __launch_bounds__(CP_THREADS) yolo_ground_truth_rows_kernel(cons
   flags[i] = f ? 1 : 0;
   if (!f) return;
   const float x = __ldg(r), yy = __ldg(r + 1), w = __ldg(r + 2), h = __ldg(r + 3);
-  const float hw = DM_DIV(w, 2.0f), hh = DM_DIV(h, 2.0f);
   int best = 0;
   float bv = __ldg(r + 5);
   for (int c = 1; c < RF - 5; ++c) { const float v = __ldg(r + 5 + c); if (v > bv) { bv = v; best = c; } }  // first max
   float* o = rows + i * 5;
-  o[0] = DM_SUB(x, hw); o[1] = DM_SUB(yy, hh); o[2] = DM_ADD(x, hw); o[3] = DM_ADD(yy, hh); o[4] = (float)best;
+  yolo_gt_corners(x, yy, w, h, o);
+  o[4] = (float)best;
 }
 
 extern "C" size_t b200_row_positions_workspace_bytes(long long n) {

@@ -206,7 +206,7 @@ struct EfAssignParams {
   int32_t* out_class[EF_MAX_LEVELS];       // (B,H,W,A): class id instead of the one-hot row (sparse-target mode)
   unsigned char* out_mask[EF_MAX_LEVELS];  // (B,H,W,A,1)
   int32_t* out_match;                      // match mode: the matched row of gt_boxes (or -1) per anchor, level l at B*anchor_base[l]
-  double* positives;                       // match mode: += matched anchors
+  double* positives;                       // match mode: += matched anchors (may be null: not counted)
   int cta_base[EF_MAX_LEVELS + 1];         // CTAs of 256 anchors, per (level, image)
   int chunks_per_img[EF_MAX_LEVELS];
 };
@@ -306,7 +306,7 @@ __global__ void __launch_bounds__(256, 8) effdet_assign_kernel(EfAssignParams p)
   if (p.out_match) {  // match mode (block-uniform): the GT row stands for the targets, the loss pass encodes them itself
     if (active) p.out_match[(size_t)p.B * p.lv.anchor_base[l] + abase + rin] = matched ? g_beg + best_i : -1;
     const int n = __syncthreads_count(matched);
-    if (threadIdx.x == 0 && n > 0) atomicAdd(p.positives, (double)n);  // integer-valued: exact and order-independent
+    if (threadIdx.x == 0 && n > 0 && p.positives) atomicAdd(p.positives, (double)n);  // integer-valued: exact and order-independent
     return;
   }
   int cls = 0;
@@ -587,14 +587,31 @@ extern "C" int b200_effdet_assign_targets_indexed(int num_levels, const int32_t*
 // threshold are generate_targets' own (the same kernel in match mode).
 size_t efb_workspace_bytes(int num_levels, int anchors_per_image, int B);   // effdet_loss.cu
 
+// effdet_assign_kernel in match mode over B > 0 images: match[B*anchor_base[l] + anchor] = GT row or -1, positives += matches
+// (positives null: not counted)
+static int ef_launch_match(const EfLevels& lv, int B, const float* gt_boxes, const int32_t* gt_offsets, float iou_thr,
+                           int32_t* match, double* positives, cudaStream_t stream) {
+  EfAssignParams p;
+  p.lv = lv;
+  p.B = B; p.C = 1; p.magic_c = 0u; p.thr = iou_thr;
+  p.gt_boxes = gt_boxes; p.gt_classes = nullptr; p.gt_offsets = gt_offsets;
+  for (int l = 0; l < EF_MAX_LEVELS; ++l) { p.out_boxes[l] = nullptr; p.out_onehot[l] = nullptr; p.out_class[l] = nullptr; p.out_mask[l] = nullptr; }
+  p.out_match = match;
+  p.positives = positives;
+  const int cta = ef_assign_plan(p);
+  effdet_assign_kernel<<<cta, 256, 0, stream>>>(p);
+  B200_LAUNCH_CHECK();
+  return B200_OK;
+}
+
 extern "C" int b200_effdet_loss_from_boxes_match(int num_levels, const int32_t* hw, int A, const float* table_dev, int B,
                                                  const float* gt_boxes, const int32_t* gt_offsets, int total_boxes,
                                                  float iou_thr, double* sums, void* workspace, size_t workspace_bytes,
                                                  void* stream) {
   const char* who = "b200_effdet_loss_from_boxes_match";
-  EfAssignParams p;
+  EfLevels lv;
   B200_REQUIRE(hw && table_dev && gt_offsets && sums, B200_ERR_BAD_ARG, "%s: null argument", who);
-  const int n_img = ef_fill_levels(p.lv, num_levels, hw, A, table_dev);
+  const int n_img = ef_fill_levels(lv, num_levels, hw, A, table_dev);
   B200_REQUIRE(n_img >= 0, B200_ERR_BAD_ARG, "%s: bad level spec", who);
   B200_REQUIRE(B >= 0 && total_boxes >= 0, B200_ERR_BAD_ARG, "%s: negative batch or box count", who);
   B200_REQUIRE(total_boxes == 0 || gt_boxes, B200_ERR_BAD_ARG, "%s: null gt_boxes", who);
@@ -603,15 +620,8 @@ extern "C" int b200_effdet_loss_from_boxes_match(int num_levels, const int32_t* 
   B200_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, B200_ERR_BAD_ARG, "%s: workspace not 256-byte aligned", who);
   B200_CUDA(cudaMemsetAsync(sums, 0, sizeof(double) * (2 * num_levels + 1), (cudaStream_t)stream));
   if (B == 0) return B200_OK;
-  p.B = B; p.C = 1; p.magic_c = 0u; p.thr = iou_thr;
-  p.gt_boxes = gt_boxes; p.gt_classes = nullptr; p.gt_offsets = gt_offsets;
-  for (int l = 0; l < EF_MAX_LEVELS; ++l) { p.out_boxes[l] = nullptr; p.out_onehot[l] = nullptr; p.out_class[l] = nullptr; p.out_mask[l] = nullptr; }
-  p.out_match = static_cast<int32_t*>(workspace);
-  p.positives = sums + 2 * num_levels;
-  const int cta = ef_assign_plan(p);
-  effdet_assign_kernel<<<cta, 256, 0, (cudaStream_t)stream>>>(p);
-  B200_LAUNCH_CHECK();
-  return B200_OK;
+  return ef_launch_match(lv, B, gt_boxes, gt_offsets, iou_thr, static_cast<int32_t*>(workspace), sums + 2 * num_levels,
+                         (cudaStream_t)stream);
 }
 
 // ---- fused eval-step stream (test_step, efficientnet/efficientdet_net_train.py:135-169) ----------------------------
@@ -640,6 +650,11 @@ struct EfFusedParams {
   CandStore st;
   float alpha, gamma, delta, label_smoothing;
   double* partials;                       // [gridDim.x][num_levels][3] focal, huber, positives
+  // from-boxes mode (effdet_stream_kernel<G, true>): the targets are rebuilt from the match stage's output
+  const int32_t* match;                   // per anchor: row of gt_boxes or -1; level l at B*anchor_base[l]
+  const float4* gt_boxes;                 // [total] y1,x1,y2,x2
+  const int32_t* gt_classes;              // [total]
+  uint32_t magic_c;                       // floor(2^32/C)+1: e / C for the flat element e < 2^16 * C of a tile
 };
 
 // Warp roles inside a CTA (tile = 64 anchors):
@@ -650,18 +665,27 @@ struct EfFusedParams {
 //   warps 0-1 (BOX half, lane <-> anchor): head offsets / box targets / mask straight from global memory, decode, Huber,
 //     and — behind the tile's single CTA barrier — the fold of the three argmax partials and the candidate append.
 // Both halves are ~600-800 instructions per warp and tile and independent, so they run side by side.
+//
+// FROM_BOXES (b200_effdet_eval_step_from_boxes): no dense targets.  The match stage (effdet_assign_kernel in match mode)
+// has left the matched GT row of every anchor; only the logits are bulk-copied (the stage bytes halve), the class stream
+// rebuilds each one-hot element from the anchor's class (match < 0 ? 0 : gt_classes[match], an id outside [0, C) giving
+// an all-zero row, as generate_targets writes it) and calls the same el_focal, and the box warps encode the box target
+// with ef_encode_box and count the positives from match >= 0.  The box warps look up the classes of the CTA's next tile
+// during this one: flat one-hot positions in shared memory, double-buffered by tile parity like the argmax partials.
 #define EFU_BOX_WARPS 2
 #define EFU_STREAM_THREADS (EFU_THREADS - 32 * EFU_BOX_WARPS)
 #define EFU_STAGES 2
+#define EFU_HOT_INTS (2 * (EFU_TILE + 1))   // from boxes: [2][EFU_TILE + 1] one-hot positions after the stages
+static_assert(EFU_BOX_WARPS * 32 == EFU_TILE, "the box warps hold one anchor of the tile per thread");
 
-template <bool G15>
+template <bool G15, bool FROM_BOXES>
 __global__ void __launch_bounds__(EFU_THREADS, 2) effdet_stream_kernel(EfFusedParams p) {
   extern __shared__ __align__(128) unsigned char efu_smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int C = p.C;
   const uint32_t tile_bytes = (uint32_t)EFU_TILE * (uint32_t)C * 4u;
-  // stage s: [x tile][y tile]
-  const uint32_t stage_bytes = tile_bytes * 2u;
+  // stage s: [x tile][y tile]; from boxes: [x tile]
+  const uint32_t stage_bytes = FROM_BOXES ? tile_bytes : tile_bytes * 2u;
   __shared__ __align__(8) uint64_t s_bar[EFU_STAGES];
   __shared__ double s_part[EF_MAX_LEVELS][3];
   __shared__ double s_red[EFU_THREADS / 32][3];
@@ -702,7 +726,7 @@ __global__ void __launch_bounds__(EFU_THREADS, 2) effdet_stream_kernel(EfFusedPa
   };
   auto bulk_ok = [&](int l, long long rec0, int nrec) {
     const uintptr_t ax = reinterpret_cast<uintptr_t>(p.cls[l] + rec0 * C);
-    const uintptr_t ay = reinterpret_cast<uintptr_t>(p.cls_true[l] + rec0 * C);
+    const uintptr_t ay = FROM_BOXES ? 0 : reinterpret_cast<uintptr_t>(p.cls_true[l] + rec0 * C);
     return (((ax | ay) & 15) == 0) && ((((uint32_t)nrec * (uint32_t)C * 4u) & 15u) == 0u);
   };
   auto issue = [&](long long t, int s) {   // one thread: start the copies of tile t into stage s
@@ -712,13 +736,30 @@ __global__ void __launch_bounds__(EFU_THREADS, 2) effdet_stream_kernel(EfFusedPa
     const uint32_t bytes = (uint32_t)nrec * (uint32_t)C * 4u;
     unsigned char* dst = efu_smem + (size_t)s * stage_bytes;
     bc_fence_proxy_async();
-    bc_mbar_expect_tx(&s_bar[s], bytes * 2u);
+    bc_mbar_expect_tx(&s_bar[s], FROM_BOXES ? bytes : bytes * 2u);
     bc_bulk_g2s(dst, p.cls[l] + rec0 * C, bytes, &s_bar[s]);
-    bc_bulk_g2s(dst + tile_bytes, p.cls_true[l] + rec0 * C, bytes, &s_bar[s]);
+    if (!FROM_BOXES) bc_bulk_g2s(dst + tile_bytes, p.cls_true[l] + rec0 * C, bytes, &s_bar[s]);
   };
   const bool box_warp = warp < EFU_BOX_WARPS;
   const int st = tid - 32 * EFU_BOX_WARPS;   // index among the stream threads
   const int q3 = (C + 2) / 3;
+  int* s_hot = reinterpret_cast<int*>(efu_smem + (size_t)EFU_STAGES * stage_bytes);   // from boxes only
+  auto stage_hot = [&](long long t, int buf) {   // box warps: flat tile position of each anchor's 1.0 of tile t, or -1
+    int l, nrec; long long rec0;
+    locate(t, l, rec0, nrec);
+    int h = -1;
+    if (tid < nrec) {
+      const int m = __ldg(p.match + (size_t)p.B * p.lv.anchor_base[l] + rec0 + tid);
+      const int id = m >= 0 ? __ldg(p.gt_classes + m) : 0;   // class 0 = background when unmatched (anc:131-133)
+      if (id >= 0 && id < C) h = tid * C + id;                 // tf.one_hot: an id outside [0, C) gives a row of zeros
+    }
+    s_hot[buf * (EFU_TILE + 1) + tid] = h;
+  };
+  if (FROM_BOXES) {
+    if (box_warp && (long long)blockIdx.x < n_tiles) stage_hot(blockIdx.x, 0);
+    if (tid < 2) s_hot[tid * (EFU_TILE + 1) + EFU_TILE] = -1;   // the anchor after the last: a float4 may reach into it
+    __syncthreads();
+  }
   if (tid == 32 * EFU_BOX_WARPS) {
 #pragma unroll
     for (int s = 0; s < EFU_STAGES; ++s) {
@@ -747,34 +788,69 @@ __global__ void __launch_bounds__(EFU_THREADS, 2) effdet_stream_kernel(EfFusedPa
       if (tid < nrec) {
         const long long rec = rec0 + tid;
         const float4 r4 = __ldcs(p.rel[l] + rec);
-        const float4 t4 = __ldcs(p.box_true[l] + rec);
-        const unsigned char mk = p.mask[l][rec];
+        float4 t4;
+        unsigned char mk;
+        int m = -1;
+        if (FROM_BOXES) {
+          m = __ldg(p.match + (size_t)p.B * p.lv.anchor_base[l] + rec);
+        } else {
+          t4 = __ldcs(p.box_true[l] + rec);
+          mk = p.mask[l][rec];
+        }
         int rin;
         if (total < 0x7fffffffLL) { img = (int)((uint32_t)rec / (uint32_t)api); rin = (int)((uint32_t)rec - (uint32_t)img * (uint32_t)api); }
         else { img = (int)(rec / api); rin = (int)(rec - (long long)img * api); }
         int y, x, an_i;
         ef_split(p.lv, l, rin, y, x, an_i);
-        d4 = ef_decode_box(ef_anchor(p.lv, l, y, x, an_i), r4);
+        const AnchorBox an = ef_anchor(p.lv, l, y, x, an_i);
+        d4 = ef_decode_box(an, r4);
         if (p.dec[l]) __stcs(p.dec[l] + rec, d4);
+        if (FROM_BOXES) {   // the box target and mask generate_targets writes for this anchor (anc:121-130)
+          t4 = make_float4(0.f, 0.f, 0.f, 0.f);
+          if (m >= 0) {
+            const float4 q = __ldg(p.gt_boxes + m);
+            t4 = ef_encode_box(an.y1, an.x1, an.y2, an.x2, q.x, q.y, q.z, q.w);
+          }
+          mk = m >= 0 ? 1 : 0;
+        }
         hub += el_huber(t4.x, r4.x, p.delta) + el_huber(t4.y, r4.y, p.delta) + el_huber(t4.z, r4.z, p.delta) + el_huber(t4.w, r4.w, p.delta);
         pos += mk ? 1u : 0u;
         aidx = (uint32_t)(p.lv.anchor_base[l] + rin);
+      }
+      if (FROM_BOXES) {
+        const long long tn = t + gridDim.x;
+        if (tn < n_tiles) stage_hot(tn, pb ^ 1);   // read by the class stream after this tile's barrier
       }
     } else {
       // ---- class stream ----
       float* xs = reinterpret_cast<float*>(efu_smem + (size_t)s * stage_bytes);
       const float* ys = reinterpret_cast<const float*>(efu_smem + (size_t)s * stage_bytes + tile_bytes);
+      const int* hot = s_hot + pb * (EFU_TILE + 1);
       const int n_el = nrec * C;
       float f0 = 0.f, f1 = 0.f;
       if (bulk) {
         bc_mbar_wait(&s_bar[s], (phase_bits >> s) & 1u);
         const int n_vec = n_el >> 2;
+        if (FROM_BOXES) {
 #pragma unroll 2
-        for (int i = st; i < n_vec; i += EFU_STREAM_THREADS) {
-          const float4 x = reinterpret_cast<const float4*>(xs)[i];
-          const float4 y = reinterpret_cast<const float4*>(ys)[i];
-          f0 += el_focal<G15>(y.x, x.x, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.y, x.y, p.alpha, p.gamma, p.label_smoothing);
-          f1 += el_focal<G15>(y.z, x.z, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.w, x.w, p.alpha, p.gamma, p.label_smoothing);
+          for (int i = st; i < n_vec; i += EFU_STREAM_THREADS) {
+            const float4 x = reinterpret_cast<const float4*>(xs)[i];
+            const int e = 4 * i;
+            const int a = (int)__umulhi((uint32_t)e, p.magic_c);   // e / C
+            const int h0 = hot[a], h1 = hot[a + 1];                // a float4 spans at most anchors a and a + 1 (C >= 4)
+            const float y0 = (e == h0 || e == h1) ? 1.0f : 0.0f, y1 = (e + 1 == h0 || e + 1 == h1) ? 1.0f : 0.0f;
+            const float y2 = (e + 2 == h0 || e + 2 == h1) ? 1.0f : 0.0f, y3 = (e + 3 == h0 || e + 3 == h1) ? 1.0f : 0.0f;
+            f0 += el_focal<G15>(y0, x.x, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y1, x.y, p.alpha, p.gamma, p.label_smoothing);
+            f1 += el_focal<G15>(y2, x.z, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y3, x.w, p.alpha, p.gamma, p.label_smoothing);
+          }
+        } else {
+#pragma unroll 2
+          for (int i = st; i < n_vec; i += EFU_STREAM_THREADS) {
+            const float4 x = reinterpret_cast<const float4*>(xs)[i];
+            const float4 y = reinterpret_cast<const float4*>(ys)[i];
+            f0 += el_focal<G15>(y.x, x.x, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.y, x.y, p.alpha, p.gamma, p.label_smoothing);
+            f1 += el_focal<G15>(y.z, x.z, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.w, x.w, p.alpha, p.gamma, p.label_smoothing);
+          }
         }
       } else {
         // ragged tail of a level or an unaligned tensor: plain loads; the logits still go to the stage for the argmax
@@ -783,7 +859,8 @@ __global__ void __launch_bounds__(EFU_THREADS, 2) effdet_stream_kernel(EfFusedPa
         for (int e = st; e < n_el; e += EFU_STREAM_THREADS) {
           const float xv = __ldg(xg + e);
           xs[e] = xv;
-          f0 += el_focal<G15>(__ldg(yg + e), xv, p.alpha, p.gamma, p.label_smoothing);
+          const float yv = FROM_BOXES ? ((e == hot[(int)__umulhi((uint32_t)e, p.magic_c)]) ? 1.0f : 0.0f) : __ldg(yg + e);
+          f0 += el_focal<G15>(yv, xv, p.alpha, p.gamma, p.label_smoothing);
         }
         asm volatile("bar.sync 1, %0;" ::"n"(EFU_STREAM_THREADS) : "memory");   // stream warps only: the tile is complete
       }
@@ -868,29 +945,61 @@ extern "C" size_t b200_effdet_eval_workspace_bytes(int num_levels, const int32_t
   return b200_effdet_postprocess_workspace_bytes(num_levels, hw, A, num_images, max_out) + efu_partials_bytes(num_levels);
 }
 
+// from boxes: [eval workspace][match: int32 per anchor of the batch]
+static size_t efu_match_bytes(int anchors_per_image, int B) {
+  return b200_align_up(sizeof(int32_t) * (size_t)anchors_per_image * (size_t)B, 256);
+}
+
+extern "C" size_t b200_effdet_eval_step_from_boxes_workspace_bytes(int num_levels, const int32_t* hw, int A, int num_images,
+                                                                   int max_out) {
+  EfLevels lv;
+  if (!hw || num_images < 0) return 0;
+  const int n_img = ef_fill_levels(lv, num_levels, hw, A, nullptr);
+  if (n_img < 0) return 0;
+  return b200_effdet_eval_workspace_bytes(num_levels, hw, A, num_images, max_out) + efu_match_bytes(n_img, num_images);
+}
+
+// Ground truth as box lists (b200_effdet_eval_step_from_boxes) instead of the dense targets
+struct EfuBoxes {
+  const float* gt_boxes; const int32_t* gt_classes; const int32_t* gt_offsets;
+  int total_boxes;
+  float iou_thr;   // generate_targets' match threshold
+};
+
 static int efu_impl(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
                     const float* const true_boxes[], const float* const true_classes[], const unsigned char* const true_masks[],
-                    const float* const pred_boxes[], const float* const pred_classes[], float alpha, float gamma, float delta,
-                    float label_smoothing, double* sums_out, float* const out_decoded[], int max_out, float iou_thr,
-                    float score_thr, int metric, float* out_boxes, long long* out_class_id, float* out_score,
+                    const EfuBoxes* fb, const float* const pred_boxes[], const float* const pred_classes[], float alpha,
+                    float gamma, float delta, float label_smoothing, double* sums_out, float* const out_decoded[], int max_out,
+                    float iou_thr, float score_thr, int metric, float* out_boxes, long long* out_class_id, float* out_score,
                     int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count, void* workspace, size_t workspace_bytes,
                     void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  const char* who = "b200_effdet_eval_step";
+  const char* who = fb ? "b200_effdet_eval_step_from_boxes" : "b200_effdet_eval_step";
   EfFusedParams p;
-  B200_REQUIRE(hw && table_dev && pred_boxes && pred_classes, B200_ERR_BAD_ARG, "%s: null argument", who);
-  B200_REQUIRE(true_boxes && true_classes && true_masks && sums_out, B200_ERR_BAD_ARG, "%s: null target argument", who);
+  B200_REQUIRE(hw && table_dev && pred_boxes && pred_classes && sums_out, B200_ERR_BAD_ARG, "%s: null argument", who);
+  if (fb) {
+    B200_REQUIRE(fb->gt_offsets, B200_ERR_BAD_ARG, "%s: null gt_offsets", who);
+    B200_REQUIRE(fb->total_boxes >= 0, B200_ERR_BAD_ARG, "%s: negative total_boxes", who);
+    B200_REQUIRE(fb->total_boxes == 0 || (fb->gt_boxes && fb->gt_classes), B200_ERR_BAD_ARG, "%s: null gt_boxes / gt_classes", who);
+    B200_REQUIRE((reinterpret_cast<uintptr_t>(fb->gt_boxes) & 15) == 0, B200_ERR_BAD_ARG, "%s: gt_boxes not 16-byte aligned", who);
+  } else {
+    B200_REQUIRE(true_boxes && true_classes && true_masks, B200_ERR_BAD_ARG, "%s: null target argument", who);
+  }
   const int n_img = ef_fill_levels(p.lv, num_levels, hw, A, table_dev);
   B200_REQUIRE(n_img >= 0, B200_ERR_BAD_ARG, "%s: bad level spec", who);
   B200_REQUIRE(C >= 1 && C <= 400, B200_ERR_UNSUPPORTED, "%s: classes_num %d outside [1,400]", who, C);
+  // from boxes: a float4 of logits spans at most two anchors, whose one-hot rows are rebuilt from two class ids
+  B200_REQUIRE(!fb || C >= 4, B200_ERR_UNSUPPORTED, "%s: classes_num %d < 4 (use generate_targets + b200_effdet_eval_step)", who, C);
   B200_REQUIRE(B >= 0, B200_ERR_BAD_ARG, "%s: negative batch", who);
   B200_REQUIRE(metric >= B200_METRIC_EFF_IOU && metric <= B200_METRIC_EFF_CIOU, B200_ERR_BAD_ARG, "%s: iou_type must be iou/giou/diou/ciou", who);
   B200_REQUIRE(max_out >= 1 && max_out <= NMS_MAX_OUT_LIMIT, B200_ERR_UNSUPPORTED, "%s: max_out %d outside [1,%d]", who, max_out, NMS_MAX_OUT_LIMIT);
   if (B == 0) return B200_OK;
   B200_REQUIRE(out_boxes && out_class_id && out_score && out_count, B200_ERR_BAD_ARG, "%s: null output", who);
+  B200_REQUIRE(C <= 128, B200_ERR_UNSUPPORTED, "%s: the fused pass stages %d-anchor tiles in shared memory: classes_num %d > 128 (use the separate calls)", who, EFU_TILE, C);
   const CandLayout ws = cand_layout(B, n_img, max_out, false, true);
   const size_t part_bytes = efu_partials_bytes(num_levels);
-  B200_REQUIRE(workspace && workspace_bytes >= ws.total + part_bytes, B200_ERR_WORKSPACE, "%s: workspace %zu < required %zu", who, workspace_bytes, ws.total + part_bytes);
+  const size_t need = ws.total + part_bytes + (fb ? efu_match_bytes(n_img, B) : 0);
+  B200_REQUIRE(workspace && workspace_bytes >= need, B200_ERR_WORKSPACE, "%s: workspace %zu < required %zu", who, workspace_bytes, need);
   B200_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, B200_ERR_BAD_ARG, "%s: workspace not 256-byte aligned", who);
   unsigned char* wsb = static_cast<unsigned char*>(workspace);
   p.B = B; p.C = C;
@@ -900,35 +1009,57 @@ static int efu_impl(int num_levels, const int32_t* hw, int A, const float* table
     p.cls[l] = nullptr; p.cls_true[l] = nullptr; p.rel[l] = nullptr; p.box_true[l] = nullptr; p.mask[l] = nullptr; p.dec[l] = nullptr;
     if (l >= num_levels) continue;
     B200_REQUIRE(pred_boxes[l] && pred_classes[l], B200_ERR_BAD_ARG, "%s: null level %d", who, l);
-    B200_REQUIRE(true_boxes[l] && true_classes[l] && true_masks[l], B200_ERR_BAD_ARG, "%s: null target level %d", who, l);
-    const uintptr_t al = reinterpret_cast<uintptr_t>(pred_boxes[l]) | reinterpret_cast<uintptr_t>(true_boxes[l]) |
+    if (!fb) B200_REQUIRE(true_boxes[l] && true_classes[l] && true_masks[l], B200_ERR_BAD_ARG, "%s: null target level %d", who, l);
+    const uintptr_t al = reinterpret_cast<uintptr_t>(pred_boxes[l]) | (fb ? 0 : reinterpret_cast<uintptr_t>(true_boxes[l])) |
                          (out_decoded && out_decoded[l] ? reinterpret_cast<uintptr_t>(out_decoded[l]) : 0);
     B200_REQUIRE((al & 15) == 0, B200_ERR_BAD_ARG, "%s: box tensors of level %d must be 16-byte aligned", who, l);
     p.cls[l] = pred_classes[l];
     p.rel[l] = reinterpret_cast<const float4*>(pred_boxes[l]);
     p.dec[l] = out_decoded ? reinterpret_cast<float4*>(out_decoded[l]) : nullptr;
-    p.cls_true[l] = true_classes[l];
-    p.box_true[l] = reinterpret_cast<const float4*>(true_boxes[l]);
-    p.mask[l] = true_masks[l];
+    if (!fb) {
+      p.cls_true[l] = true_classes[l];
+      p.box_true[l] = reinterpret_cast<const float4*>(true_boxes[l]);
+      p.mask[l] = true_masks[l];
+    }
     tb += ((long long)B * p.lv.anc_per_img[l] + EFU_TILE - 1) / EFU_TILE;
   }
   for (int l = num_levels; l <= EF_MAX_LEVELS; ++l) p.tile_base[l] = tb;
   p.st = cand_bind(ws, wsb, out_sel_idx != nullptr);
+  B200_REQUIRE(cand_finalize_smem_bytes(p.st, max_out) <= 220 * 1024, B200_ERR_UNSUPPORTED, "%s: too many anchors per image for the rank table", who);
   p.alpha = alpha; p.gamma = gamma; p.delta = delta; p.label_smoothing = label_smoothing;
   p.partials = reinterpret_cast<double*>(wsb + ws.total);
+  p.match = nullptr; p.gt_boxes = nullptr; p.gt_classes = nullptr;
+  p.magic_c = (uint32_t)((1ull << 32) / (unsigned long long)C + 1ull);
+  if (fb) {
+    p.match = reinterpret_cast<const int32_t*>(wsb + ws.total + part_bytes);
+    p.gt_boxes = reinterpret_cast<const float4*>(fb->gt_boxes);
+    p.gt_classes = fb->gt_classes;
+  }
+  // ---- every argument is checked: enqueue ----
   B200_CUDA(cudaMemsetAsync(wsb, 0, ws.zeroed(out_sel_idx != nullptr), stream));
-  B200_REQUIRE(C <= 128, B200_ERR_UNSUPPORTED, "%s: the fused pass stages %d-anchor tiles in shared memory: classes_num %d > 128 (use the separate calls)", who, EFU_TILE, C);
-  const size_t smem = (size_t)EFU_STAGES * EFU_TILE * C * sizeof(float) * 2;
+  if (fb) {
+    // the stream counts the positives itself (match >= 0)
+    const int rc = ef_launch_match(p.lv, B, fb->gt_boxes, fb->gt_offsets, fb->iou_thr, const_cast<int32_t*>(p.match), nullptr,
+                                   stream);
+    if (rc != B200_OK) return rc;
+  }
+  const size_t smem = fb ? (size_t)EFU_STAGES * EFU_TILE * C * sizeof(float) + EFU_HOT_INTS * sizeof(int)
+                         : (size_t)EFU_STAGES * EFU_TILE * C * sizeof(float) * 2;
   long long want = tb;
   const long long cap = (long long)b200_sm_count() * EFU_GRID_PER_SM;
   const int grid = (int)(want < cap ? (want < 1 ? 1 : want) : cap);
-#define EFU_LAUNCH(G)                                                                                                   \
-  do {                                                                                                                  \
-    B200_CUDA(cudaFuncSetAttribute(effdet_stream_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    effdet_stream_kernel<G><<<grid, EFU_THREADS, smem, stream>>>(p);                                                  \
+#define EFU_LAUNCH(G, FB)                                                                                                    \
+  do {                                                                                                                       \
+    B200_CUDA(cudaFuncSetAttribute(effdet_stream_kernel<G, FB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    effdet_stream_kernel<G, FB><<<grid, EFU_THREADS, smem, stream>>>(p);                                                  \
   } while (0)
-  if (gamma == 1.5f) EFU_LAUNCH(true);
-  else EFU_LAUNCH(false);
+  if (fb) {
+    if (gamma == 1.5f) EFU_LAUNCH(true, true);
+    else EFU_LAUNCH(false, true);
+  } else {
+    if (gamma == 1.5f) EFU_LAUNCH(true, false);
+    else EFU_LAUNCH(false, false);
+  }
 #undef EFU_LAUNCH
   B200_LAUNCH_CHECK();
   B200_CUDA(cudaMemsetAsync(sums_out, 0, sizeof(double) * (2 * num_levels + 1), stream));
@@ -948,8 +1079,26 @@ extern "C" int b200_effdet_eval_step(int num_levels, const int32_t* hw, int A, c
                                      float iou_thr, float score_thr, int metric, float* out_boxes, long long* out_class_id,
                                      float* out_score, int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
                                      void* workspace, size_t workspace_bytes, void* stream) {
-  return efu_impl(num_levels, hw, A, table_dev, C, B, true_boxes, true_classes, true_masks, pred_boxes, pred_classes, alpha,
-                  gamma, delta, label_smoothing, sums_out, out_decoded, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id,
+  return efu_impl(num_levels, hw, A, table_dev, C, B, true_boxes, true_classes, true_masks, nullptr, pred_boxes, pred_classes,
+                  alpha, gamma, delta, label_smoothing, sums_out, out_decoded, max_out, iou_thr, score_thr, metric, out_boxes,
+                  out_class_id, out_score, out_sel_idx, out_sel_anchor, out_count, workspace, workspace_bytes, stream);
+}
+
+// test_step from box lists: the match stage of generate_targets (match_iou_thr), then the one-pass stream with the targets
+// rebuilt per anchor, the reduce and the NMS tail — the outputs of b200_effdet_eval_step on generate_targets' targets.
+extern "C" int b200_effdet_eval_step_from_boxes(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
+                                                const float* gt_boxes, const int32_t* gt_classes, const int32_t* gt_offsets,
+                                                int total_boxes, float match_iou_thr, const float* const pred_boxes[],
+                                                const float* const pred_classes[], float alpha, float gamma, float delta,
+                                                float label_smoothing, double* sums_out, float* const out_decoded[], int max_out,
+                                                float iou_thr, float score_thr, int metric, float* out_boxes, long long* out_class_id,
+                                                float* out_score, int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
+                                                void* workspace, size_t workspace_bytes, void* stream) {
+  EfuBoxes fb;
+  fb.gt_boxes = gt_boxes; fb.gt_classes = gt_classes; fb.gt_offsets = gt_offsets; fb.total_boxes = total_boxes;
+  fb.iou_thr = match_iou_thr;
+  return efu_impl(num_levels, hw, A, table_dev, C, B, nullptr, nullptr, nullptr, &fb, pred_boxes, pred_classes, alpha, gamma,
+                  delta, label_smoothing, sums_out, out_decoded, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id,
                   out_score, out_sel_idx, out_sel_anchor, out_count, workspace, workspace_bytes, stream);
 }
 

@@ -917,9 +917,15 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_objects_kernel(YlParams p,
 // GetTargets + GetLoss without the dense y_true: one CTA per image assigns every box (same arithmetic as the dense
 // scatter, yolo_targets.cuh), drops the boxes that collide on a record (scatter_nd would sum them and the whole
 // record is then zeroed, cds:279-284) and writes the object list the dense path's scan kernel would have found.
+// kRows (b200_yolo_ground_truth_from_boxes): instead of the object list, the GetGroudTruth row [x1,y1,x2,y2,class] of every
+// surviving box, at box index offsets[img] + (surviving boxes with a smaller key): keys are anchor_base[layer] + record,
+// so that is the prefix of the lower layers' counts plus the slot — level by level, in record order, as GetGroudTruth
+// emits the rows of the three dense levels — and rows_count[img] = the survivors.
+template <bool kRows>
 __global__ void __launch_bounds__(128) yolo_loss_assign_sparse_kernel(YtParams t, YlParams p, int* __restrict__ keys,
                                                                       float4* __restrict__ sp_t, int32_t* __restrict__ sp_cls,
-                                                                      uint32_t* __restrict__ obj_bits) {
+                                                                      uint32_t* __restrict__ obj_bits, float* __restrict__ rows,
+                                                                      int32_t* __restrict__ rows_count) {
   __shared__ int s_cnt[YL_LEVELS];
   const int img = blockIdx.x;
   const int beg = t.offsets[img], end = t.offsets[img + 1];
@@ -967,13 +973,20 @@ __global__ void __launch_bounds__(128) yolo_loss_assign_sparse_kernel(YtParams t
     yt_assign(t, i, layer, rin, nx, ny, nw, nh);
     // slot = number of surviving boxes of the same layer with a smaller record index (ascending record order, as the
     // dense path's sorted object list): deterministic run to run, no atomics on the slot
-    const int lo_key = p.lv.anchor_base[layer];
+    const int lo_key = kRows ? 0 : p.lv.anchor_base[layer];
     int slot = 0;
     for (int j = beg; j < end; ++j) {
       const int kj = keys[j];
       slot += (kj >= lo_key && kj < key) ? 1 : 0;
     }
     atomicAdd(&s_cnt[layer], 1);
+    if (kRows) {
+      float* o = rows + 5 * (size_t)(beg + slot);
+      yolo_gt_corners(nx, ny, nw, nh, o);
+      const int c = t.classes[i];
+      o[4] = (float)((c >= 0 && c < t.C) ? c : 0);   // first arg-max of the one-hot row; an id outside [0, C): a zero row
+      continue;
+    }
     const size_t gi = (size_t)img * p.n_img + p.lv.anchor_base[layer] + slot;
     p.obj_index[gi] = rin;
     sp_t[gi] = make_float4(nx, ny, nw, nh);
@@ -981,6 +994,10 @@ __global__ void __launch_bounds__(128) yolo_loss_assign_sparse_kernel(YtParams t
     atomicOr(obj_bits + (size_t)img * p.bits_words + (key >> 5), 1u << (key & 31));
   }
   __syncthreads();
+  if (kRows) {
+    if (threadIdx.x == 0) rows_count[img] = s_cnt[0] + s_cnt[1] + s_cnt[2];
+    return;
+  }
   if (threadIdx.x < YL_LEVELS) p.gt_count[img * YL_LEVELS + threadIdx.x] = s_cnt[threadIdx.x];
 }
 
@@ -1133,7 +1150,8 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
     uint32_t* bits = reinterpret_cast<uint32_t*>(wsb + sws.bits);
     if (stages & 1) {
       B200_CUDA(cudaMemsetAsync(bits, 0, sizeof(uint32_t) * (size_t)B * sws.bits_words, stream));
-      yolo_loss_assign_sparse_kernel<<<B, 128, 0, stream>>>(t, p, reinterpret_cast<int*>(wsb + sws.keys), sp_t, sp_cls, bits);
+      yolo_loss_assign_sparse_kernel<false><<<B, 128, 0, stream>>>(t, p, reinterpret_cast<int*>(wsb + sws.keys), sp_t, sp_cls, bits,
+                                                                   nullptr, nullptr);
       B200_LAUNCH_CHECK();
     }
     p.sp_t = sp_t; p.sp_cls = sp_cls; p.obj_bits = bits;
@@ -1251,6 +1269,44 @@ extern "C" int b200_yolo_loss_from_boxes(const float* boxes, const int32_t* clas
   sp.assign_anchors_wh_host = assign_anchors_wh_host;
   return yolo_loss_impl(nullptr, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
                         batch_divisor, out_parts, out_loss, out_ignore, nullptr, workspace, workspace_bytes, stream_, &sp);
+}
+
+// GetGroudTruth of the three levels GetTargets would write, straight from the box lists: rows [total,5], image b's
+// surviving rows packed at rows[offsets[b] .. offsets[b] + count[b]).  Workspace: one int32 key per box.
+static size_t yl_rows_workspace_bytes(int total_boxes) {
+  return b200_align_up(sizeof(int32_t) * (size_t)(total_boxes > 0 ? total_boxes : 1), 256);
+}
+
+extern "C" size_t b200_yolo_ground_truth_from_boxes_workspace_bytes(const int32_t hw[6], int B, int A, int total_boxes) {
+  if (!hw || B < 0 || A < 1 || A > 8 || total_boxes < 0) return 0;
+  for (int k = 0; k < 6; ++k) if (hw[k] <= 0) return 0;
+  return yl_rows_workspace_bytes(total_boxes);
+}
+
+extern "C" int b200_yolo_ground_truth_from_boxes(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
+                                                 int B, const int32_t hw[6], int A, int C, const float* anchors_wh_host,
+                                                 const float* image_wh_host, float* rows, int32_t* count, void* workspace,
+                                                 size_t workspace_bytes, void* stream) {
+  const char* who = "b200_yolo_ground_truth_from_boxes";
+  B200_REQUIRE(B >= 0, B200_ERR_BAD_ARG, "%s: negative batch", who);
+  B200_REQUIRE(total_boxes >= 0, B200_ERR_BAD_ARG, "%s: negative total_boxes", who);
+  B200_REQUIRE(offsets, B200_ERR_BAD_ARG, "%s: null offsets", who);
+  B200_REQUIRE(total_boxes == 0 || (boxes && classes && rows), B200_ERR_BAD_ARG, "%s: null boxes / classes / rows", who);
+  B200_REQUIRE((reinterpret_cast<uintptr_t>(boxes) & 15) == 0, B200_ERR_BAD_ARG, "%s: boxes not 16-byte aligned", who);
+  B200_REQUIRE(B == 0 || count, B200_ERR_BAD_ARG, "%s: null count", who);
+  YtParams t;
+  B200_REQUIRE(yt_fill_geometry(t, A, C, anchors_wh_host, image_wh_host, hw) == 0, B200_ERR_BAD_ARG,
+               "%s: bad geometry (anchors, image_wh, hw or A outside [1,8])", who);
+  const size_t need = yl_rows_workspace_bytes(total_boxes);
+  B200_REQUIRE(workspace && workspace_bytes >= need, B200_ERR_WORKSPACE, "%s: workspace %zu < required %zu", who, workspace_bytes, need);
+  if (B == 0) return B200_OK;
+  t.boxes = boxes; t.classes = classes; t.offsets = offsets; t.B = B; t.total = total_boxes;
+  YlParams p;
+  yl_layout(hw, B, A, &p.n_img, &p.lv);
+  yolo_loss_assign_sparse_kernel<true><<<B, 128, 0, (cudaStream_t)stream>>>(t, p, static_cast<int*>(workspace), nullptr, nullptr,
+                                                                            nullptr, rows, count);
+  B200_LAUNCH_CHECK();
+  return B200_OK;
 }
 
 // b200_yolo_loss_from_boxes plus d loss / d y_pred, as b200_yolo_loss_grad is to b200_yolo_loss.  The workspace of

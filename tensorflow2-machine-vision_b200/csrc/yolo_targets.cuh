@@ -6,6 +6,13 @@
 
 #define YT_LEVELS 3
 
+// GetGroudTruth's corners of a target record (x, y, w, h) (yolo_v4/model.py:380-395): [x - w/2, y - h/2, x + w/2, y + h/2],
+// shared by the rows of a dense target (compact.cu) and the rows built from box lists (yolo_loss.cu)
+__device__ __forceinline__ void yolo_gt_corners(float x, float y, float w, float h, float* o) {
+  const float hw = DM_DIV(w, 2.0f), hh = DM_DIV(h, 2.0f);
+  o[0] = DM_SUB(x, hw); o[1] = DM_SUB(y, hh); o[2] = DM_ADD(x, hw); o[3] = DM_ADD(y, hh);
+}
+
 struct YtParams {
   const float* boxes;       // [total,4] pixel corners x1,y1,x2,y2
   const int32_t* classes;   // [total]
