@@ -440,6 +440,93 @@ def main():
         del rel, cls
         torch.cuda.empty_cache()
 
+    if any(want(n) for n in ("c1_half", "c3_half_post", "c4_half")):
+        _half_heads(args, dev, g, anc, tyu, Anchors, synth, report, wrap, want)
+
+
+def _half_heads(args, dev, g, anc, tyu, Anchors, synth, report, wrap, want):
+    """Post-processing from bf16 / fp16 heads read in place, against fp32 heads holding the same values and against
+    "bf16 cast then fp32" (what a mixed-precision user gets from an fp32-only library: a cast pass and an fp32 copy).
+    The values are bf16 values that fp16 also holds exactly, so the four arms must give the same bits; that is asserted
+    before anything is timed.  The arms alternate window by window (order rotated)."""
+    import torch
+    card = _card()
+
+    def values(shape, scale=1.0):
+        x = (torch.randn(shape, device=dev, generator=g) * scale).to(torch.bfloat16).float()
+        x[x.abs() < 1e-4] = 0.0   # below fp16's normal range a bf16 value may not be exact in fp16
+        return x
+
+    def run(name, what, batch, fams, call, bytes_f32, bytes_half, same):
+        """fams: the fp32 head families; call(families) runs the post-processing."""
+        arms = {
+            "fp32": [list(f) for f in fams],
+            "bf16": [[t.to(torch.bfloat16) for t in f] for f in fams],
+            "fp16": [[t.to(torch.float16) for t in f] for f in fams],
+        }
+        assert all(torch.equal(a.float(), b) for k in ("bf16", "fp16") for fa, fb in zip(arms[k], arms["fp32"]) for a, b in zip(fa, fb))
+        fns = {k: (lambda v=v: call(v)) for k, v in arms.items()}
+        fns["bf16_cast_then_fp32"] = lambda: call([[t.float() for t in f] for f in arms["bf16"]])
+        ref = fns["fp32"]()
+        for k in ("bf16", "fp16", "bf16_cast_then_fp32"):
+            same(fns[k](), ref)
+        del ref
+        fns = {k: wrap(f) for k, f in fns.items()}
+        steps, n_win = max(args.steps, 20), 5
+        times = {k: [] for k in fns}
+        order = list(fns)
+        for w in range(n_win):
+            for k in order[w % len(order):] + order[:w % len(order)]:
+                times[k].append(timed(fns[k], steps, args.warmup))
+        ms = {k: float(np.median(v)) for k, v in times.items()}
+        report(name, what + "; arms bit-identical (asserted); median of %d alternating windows of %d steps" % (n_win, steps),
+               batch, ms["bf16"], bytes_half,
+               dict(card, arms_ms=ms, algorithmic_bytes_per_image_fp32=bytes_f32, algorithmic_bytes_per_image_half=bytes_half,
+                    speedup_bf16_vs_cast_then_fp32=ms["bf16_cast_then_fp32"] / ms["bf16"],
+                    speedup_bf16_vs_fp32=ms["fp32"] / ms["bf16"], speedup_fp16_vs_fp32=ms["fp32"] / ms["fp16"],
+                    window_ms={k: [round(t, 5) for t in v] for k, v in times.items()}, outputs_bit_identical=True))
+
+    def same_rows(a, b):
+        assert torch.equal(a["count"], b["count"])
+        cnt = a["count"].cpu().tolist()
+        for k in a:
+            if k != "count":
+                for i, n in enumerate(cnt):
+                    x, y = a[k][i, :n], b[k][i, :n]
+                    if x.dtype == torch.float32:
+                        x, y = x.view(torch.int32), y.view(torch.int32)
+                    assert torch.equal(x, y), "%s differs between arms" % k
+
+    if want("c1_half"):
+        rec = sum(s * s * 3 for s in synth.yolo_grids(416))
+        for batch in (1, 256):
+            heads = [values((batch, s, s, 255), 2.0) for s in synth.yolo_grids(416)]
+            call = lambda f: tyu.GetNMSBoxesBatch(*f[0], anc, (416, 416), 80, 0.5, 0.3, 0.5, "iou", with_indices=True)
+            run("c1_half_b%d" % batch, "YOLOv3 416 B=%d decode + per-class NMS ('iou') from half heads" % batch, batch, [heads], call,
+                rec * 85 * 4, rec * 85 * 2, same_rows)
+            del heads
+    for name, cfg, batch in (("c3_half_post", "d0", 128), ("c4_half", "d7", 16)):
+        if not want(name):
+            continue
+        c = synth.EFFDET_CONFIGS[cfg]
+        a = Anchors(c["min_level"], c["max_level"], c["image_size"], c["num_scales"], c["aspect_ratios"], c["anchor_scale"])
+        shapes = [tuple(b.shape) for b in a.boxes]
+        n_anchor = sum(s[0] * s[1] * s[2] for s in shapes)
+        rel = [values((batch,) + s, 0.25) for s in shapes]
+        cls = [values((batch,) + s[:-1] + (81,)) for s in shapes]
+
+        def call(f):
+            return a.decode_and_postprocess(f[0], f[1])
+
+        def same(x, y):
+            for p, q in zip(x[0], y[0]):
+                assert torch.equal(p.view(torch.int32), q.view(torch.int32)), "decoded boxes differ between arms"
+            same_rows(x[1], y[1])
+        run(name, "EfficientDet-%s B=%d decode_and_postprocess (NMS diou, cap 200) from half heads" % (cfg.upper(), batch), batch,
+            [rel, cls], call, n_anchor * (81 * 4 + 16 + 16), n_anchor * (81 * 2 + 8 + 16), same)
+        del rel, cls
+        torch.cuda.empty_cache()
+
 
 if __name__ == "__main__":
     main()

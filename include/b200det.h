@@ -45,6 +45,11 @@ enum {
   B200_METRIC_COUNT = 7
 };
 
+/* Element type of the head tensors that the *_typed post-processing entries read.  bf16 and fp16 heads (Keras
+ * mixed_bfloat16 / mixed_float16, torch autocast) are read in place and widened to fp32 exactly on load: every output
+ * is bit-identical to the fp32 entry on the widened tensors.  Outputs, decoded boxes and workspaces stay fp32. */
+enum { B200_DTYPE_F32 = 0, B200_DTYPE_BF16 = 1, B200_DTYPE_F16 = 2 };
+
 /* NMS survivor predicate. */
 enum {
   B200_NMS_AGNOSTIC = 0, /* survivor iff metric < thr (NaN drops): GetIOUNMS tiu:98, get_nms enms:51 */
@@ -106,6 +111,15 @@ int b200_yolo_decode_nms(const float* const heads[3], const int32_t hw[6], int B
                          float* out_score, float* out_classes, float* out_conf, int32_t* out_sel_idx,
                          int32_t* out_sel_anchor, int32_t* out_count, void* workspace, size_t workspace_bytes,
                          void* stream);
+/* b200_yolo_decode_nms on heads of element type head_dtype (B200_DTYPE_*; all three levels share it), 16-byte
+ * aligned.  Same workspace; b200_yolo_decode_nms is the B200_DTYPE_F32 case.  Every argument is checked before
+ * anything is enqueued. */
+int b200_yolo_decode_nms_typed(const void* const heads[3], int head_dtype, const int32_t hw[6], int B, int A, int C,
+                               const float* anchors_wh_host, const float* image_wh_host, float conf_thr, float score_thr,
+                               float iou_thr, int metric, int max_out, float* out_boxes, int32_t* out_class_id,
+                               float* out_score, float* out_classes, float* out_conf, int32_t* out_sel_idx,
+                               int32_t* out_sel_anchor, int32_t* out_count, void* workspace, size_t workspace_bytes,
+                               void* stream);
 
 /* GetBoxes (utils/tf_yolo_utils.py:129-167) without the final boolean_mask: dense decode of one level.
  * head (B,H,W,A*(5+C)); anchors_wh_norm_dev [A][2] = anchors/image_wh (device); outputs for all B*H*W*A
@@ -247,6 +261,9 @@ int b200_effdet_anchors(int num_levels, const int32_t* hw, int A, const float* t
 /* convert_outputs_boxes / _boxes_decoder anc:141-158,245-274: rel[l] (B,H,W,A,4) ty,tx,th,tw -> out[l] y1,x1,y2,x2. */
 int b200_effdet_decode(int num_levels, const int32_t* hw, int A, const float* table_dev, int B,
                        const float* const rel[], float* const out[], void* stream);
+/* b200_effdet_decode on offsets of element type rel_dtype (B200_DTYPE_*); out stays fp32. */
+int b200_effdet_decode_typed(int num_levels, const int32_t* hw, int A, const float* table_dev, int B,
+                             const void* const rel[], int rel_dtype, float* const out[], void* stream);
 /* convert_outputs_one anc:161-202 for images [first_image, first_image+num_images) of a batch of B:
  * per anchor argmax/max over the C class logits, background (id 0) dropped, class-agnostic get_nms (enms:5-61)
  * on the raw max logits with score_thr (reference: max_out 200, iou_thr 0.5, score_thr 1e-4, diou), sigmoid of the
@@ -260,6 +277,13 @@ int b200_effdet_postprocess(int num_levels, const int32_t* hw, int A, int C, int
                             float score_thr, int metric, float* out_boxes, long long* out_class_id, float* out_score,
                             int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count, void* workspace,
                             size_t workspace_bytes, void* stream);
+/* b200_effdet_postprocess on decoded boxes of element type box_dtype and logits of element type cls_dtype
+ * (B200_DTYPE_*, each shared by all levels); outputs and workspace as b200_effdet_postprocess. */
+int b200_effdet_postprocess_typed(int num_levels, const int32_t* hw, int A, int C, int B, int first_image, int num_images,
+                                  const void* const boxes[], int box_dtype, const void* const classes[], int cls_dtype,
+                                  int max_out, float iou_thr, float score_thr, int metric, float* out_boxes,
+                                  long long* out_class_id, float* out_score, int32_t* out_sel_idx, int32_t* out_sel_anchor,
+                                  int32_t* out_count, void* workspace, size_t workspace_bytes, void* stream);
 /* Anchors.generate_targets anc:91-138 + _boxes_encoder anc:219-243, batched: gt_boxes [total,4] y1,x1,y2,x2,
  * gt_classes [total] int32, gt_offsets [B+1].  Per level: out_boxes (B,H,W,A,4), out_onehot (B,H,W,A,C),
  * out_mask (B,H,W,A,1) bytes.  Anchor -> best GT (first max IoU), mask = max >= iou_thr; unmatched anchors get
@@ -404,6 +428,14 @@ int b200_effdet_decode_postprocess(int num_levels, const int32_t* hw, int A, con
                                    float* out_boxes, long long* out_class_id, float* out_score, int32_t* out_sel_idx,
                                    int32_t* out_sel_anchor, int32_t* out_count, void* workspace, size_t workspace_bytes,
                                    void* stream);
+/* b200_effdet_decode_postprocess on head offsets of element type rel_dtype and logits of element type cls_dtype
+ * (B200_DTYPE_*); out_decoded and every other output stay fp32. */
+int b200_effdet_decode_postprocess_typed(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
+                                         const void* const pred_boxes[], int rel_dtype, const void* const pred_classes[],
+                                         int cls_dtype, float* const out_decoded[], int max_out, float iou_thr,
+                                         float score_thr, int metric, float* out_boxes, long long* out_class_id,
+                                         float* out_score, int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
+                                         void* workspace, size_t workspace_bytes, void* stream);
 /* b200_effdet_eval_step from box lists (an API extension): no dense targets.  gt_boxes [total,4] y1,x1,y2,x2 (16-byte
  * aligned), gt_classes [total] int32, gt_offsets [B+1] (device) as for b200_effdet_assign_targets; match_iou_thr is
  * generate_targets' iou_threshold.  One call = the match stage of b200_effdet_loss_from_boxes_match (one int32 per anchor

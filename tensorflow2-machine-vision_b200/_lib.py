@@ -26,6 +26,8 @@ SIGNATURES = {
     "b200_yolo_decode_nms_workspace_bytes": (c_sz, [c_p, c_i, c_i, c_i]),
     "b200_yolo_decode_nms": (c_i, [c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_f, c_f, c_f, c_i, c_i,
                                    c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
+    "b200_yolo_decode_nms_typed": (c_i, [c_p, c_i, c_p, c_i, c_i, c_i, c_p, c_p, c_f, c_f, c_f, c_i, c_i,
+                                         c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
     "b200_yolo_decode_dense": (c_i, [c_p, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p]),
     "b200_yolo_loss_workspace_bytes": (c_sz, [c_p, c_i, c_i]),
     "b200_yolo_loss": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_f, c_i, c_i, c_f, c_p, c_p, c_p, c_p, c_sz, c_p]),
@@ -46,9 +48,12 @@ SIGNATURES = {
     "b200_effdet_table_floats": (c_sz, [c_i, c_p, c_i]),
     "b200_effdet_anchors": (c_i, [c_i, c_p, c_i, c_p, c_i, c_p, c_p]),
     "b200_effdet_decode": (c_i, [c_i, c_p, c_i, c_p, c_i, c_p, c_p, c_p]),
+    "b200_effdet_decode_typed": (c_i, [c_i, c_p, c_i, c_p, c_i, c_p, c_i, c_p, c_p]),
     "b200_effdet_postprocess_workspace_bytes": (c_sz, [c_i, c_p, c_i, c_i, c_i]),
     "b200_effdet_postprocess": (c_i, [c_i, c_p, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_i, c_f, c_f, c_i,
                                       c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
+    "b200_effdet_postprocess_typed": (c_i, [c_i, c_p, c_i, c_i, c_i, c_i, c_i, c_p, c_i, c_p, c_i, c_i, c_f, c_f, c_i,
+                                            c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
     "b200_effdet_assign_targets": (c_i, [c_i, c_p, c_i, c_p, c_i, c_i, c_p, c_p, c_p, c_f, c_p, c_p, c_p, c_p]),
     "b200_focal_elementwise": (c_i, [c_p, c_p, c_sz, c_f, c_f, c_f, c_f, c_p, c_p]),
     "b200_focal_box_workspace_bytes": (c_sz, [c_i, c_p, c_i]),
@@ -92,6 +97,8 @@ SIGNATURES = {
                                     c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
     "b200_effdet_decode_postprocess": (c_i, [c_i, c_p, c_i, c_p, c_i, c_i, c_p, c_p, c_p, c_i, c_f, c_f, c_i, c_p, c_p, c_p, c_p, c_p,
                                              c_p, c_p, c_sz, c_p]),
+    "b200_effdet_decode_postprocess_typed": (c_i, [c_i, c_p, c_i, c_p, c_i, c_i, c_p, c_i, c_p, c_i, c_p, c_i, c_f, c_f, c_i,
+                                                   c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_sz, c_p]),
     "b200_map_per_image": (c_i, [c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, ctypes.c_double, c_p, c_p]),
     "b200_map_padded": (c_i, [c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_i, c_p, c_p, c_i, ctypes.c_double, c_p, c_p]),
     "b200_yolo_ground_truth_from_boxes_workspace_bytes": (c_sz, [c_p, c_i, c_i, c_i]),

@@ -8,23 +8,42 @@ def require_cuda():
         raise RuntimeError("tensorflow2-machine-vision_b200 needs a CUDA device (B200); there is no CPU fallback")
 
 
+def _as_tensor(x):
+    """Anything tensor-like -> torch tensor in its own dtype and place (zero-copy for torch/DLPack inputs)."""
+    if isinstance(x, torch.Tensor):
+        return x
+    if hasattr(x, "__dlpack__") and not isinstance(x, np.ndarray):
+        return torch.from_dlpack(x)  # e.g. tf.experimental.dlpack / cupy
+    t = torch.from_numpy(np.ascontiguousarray(np.asarray(x)))
+    return t.pin_memory() if t.numel() > (1 << 16) else t
+
+
 def to_cuda(x, dtype=torch.float32):
     """Anything tensor-like -> contiguous CUDA tensor of `dtype` (zero-copy for CUDA/DLPack inputs)."""
     require_cuda()
-    if isinstance(x, torch.Tensor):
-        t = x
-    elif hasattr(x, "__dlpack__") and not isinstance(x, np.ndarray):
-        t = torch.from_dlpack(x)  # e.g. tf.experimental.dlpack / cupy
-    else:
-        a = np.ascontiguousarray(np.asarray(x))
-        t = torch.from_numpy(a)
-        if t.numel() > (1 << 16):
-            t = t.pin_memory()
+    t = _as_tensor(x)
     if t.dtype != dtype:
         t = t.to(dtype)
     if not t.is_cuda:
         t = t.cuda(non_blocking=True)
     return t.contiguous()
+
+
+# element-type codes of the C ABI (B200_DTYPE_*) for the head dtypes the post-processing reads in place
+DTYPE_F32 = 0
+_HALF_CODES = {torch.bfloat16: 1, torch.float16: 2}
+
+
+def to_cuda_heads(xs):
+    """The levels of one head family (YOLO heads, EfficientDet box tensors or class logits) -> (contiguous CUDA tensors,
+    B200_DTYPE_* code).  A family that is all bf16 or all fp16 stays in its type: the kernels widen each element to fp32
+    exactly, so the results are those of the fp32 call on the widened tensors, without a cast pass or an fp32 copy.
+    Any other family is cast to fp32 as to_cuda does."""
+    ts = [_as_tensor(x) for x in xs]
+    code = _HALF_CODES.get(ts[0].dtype) if ts else None
+    if code is not None and all(t.dtype == ts[0].dtype for t in ts):
+        return [to_cuda(t, t.dtype) for t in ts], code
+    return [to_cuda(t) for t in ts], DTYPE_F32
 
 
 def is_pinned_host_f32(x):

@@ -154,32 +154,35 @@ class Anchors(object):
 
   # -- decode -------------------------------------------------------------------------------------------
   def convert_outputs_boxes(self, outputs_boxes):
-    '''[level, [batch, h, w, anchors, [ty, tx, th, tw]]] -> [level, [batch, h, w, anchors, [y1, x1, y2, x2]]]'''
+    '''[level, [batch, h, w, anchors, [ty, tx, th, tw]]] -> [level, [batch, h, w, anchors, [y1, x1, y2, x2]]]
+    (float32; offsets that are all bfloat16 or all float16 are read in place).'''
     lib = _lib.load()
     tab = self._dev_table()
-    rel = [T.to_cuda(t) for t in outputs_boxes]
+    rel, rel_dtype = T.to_cuda_heads(outputs_boxes)
     if len(rel) != self._num_levels:
       raise ValueError('expected %d levels, got %d' % (self._num_levels, len(rel)))
     B = rel[0].shape[0]
     for t, (h, w) in zip(rel, self._level_hw):
       if tuple(t.shape) != (B, h, w, self._A, 4):
         raise ValueError('level shape %r != %r' % (tuple(t.shape), (B, h, w, self._A, 4)))
-    out = [torch.empty_like(t) for t in rel]
+    out = [torch.empty(t.shape, dtype=torch.float32, device=t.device) for t in rel]
     L = self._num_levels
     pr = (ctypes.c_void_p * L)(*[t.data_ptr() for t in rel])
     po = (ctypes.c_void_p * L)(*[t.data_ptr() for t in out])
-    _lib.check(lib.b200_effdet_decode(L, self._hw, self._A, T.ptr(tab), B, pr, po, T.stream_ptr()), 'convert_outputs_boxes')
+    _lib.check(lib.b200_effdet_decode_typed(L, self._hw, self._A, T.ptr(tab), B, pr, rel_dtype, po, T.stream_ptr()),
+               'convert_outputs_boxes')
     return tuple(out)
 
   # -- post-processing ----------------------------------------------------------------------------------
   def convert_outputs_batch(self, outputs_boxes, outputs_classes, first_image=0, num_images=None, max_output_size=200,
                             iou_threshold=0.5, score_threshold=0.0001, iou_type='diou', with_indices=False):
     '''convert_outputs_one for a range of images in one launch.  Returns a dict of padded tensors
-    [n, max_output_size, ...] (boxes, classes_id int64, scores) and `count` [n].'''
+    [n, max_output_size, ...] (boxes, classes_id int64, scores) and `count` [n].  Boxes or logits that are all bfloat16
+    or all float16 are read in place; the results are those of the float32 call on the widened tensors.'''
     assert iou_type in ('iou', 'giou', 'diou', 'ciou')
     lib = _lib.load()
-    bx = [T.to_cuda(t) for t in outputs_boxes]
-    cl = [T.to_cuda(t) for t in outputs_classes]
+    bx, box_dtype = T.to_cuda_heads(outputs_boxes)
+    cl, cls_dtype = T.to_cuda_heads(outputs_classes)
     L = self._num_levels
     if len(bx) != L or len(cl) != L:
       raise ValueError('expected %d levels' % L)
@@ -201,11 +204,11 @@ class Anchors(object):
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
     pb = (ctypes.c_void_p * L)(*[t.data_ptr() for t in bx])
     pc = (ctypes.c_void_p * L)(*[t.data_ptr() for t in cl])
-    _lib.check(lib.b200_effdet_postprocess(L, self._hw, self._A, C, B, int(first_image), n, pb, pc, K,
-                                           float(iou_threshold), float(score_threshold), _lib.METRIC_EFF[iou_type],
-                                           T.ptr(out['boxes']), T.ptr(out['classes_id']), T.ptr(out['scores']),
-                                           T.ptr(out.get('sel_idx')), T.ptr(out.get('sel_anchor')), T.ptr(out['count']),
-                                           T.ptr(ws), ws_bytes, T.stream_ptr()), 'convert_outputs_one')
+    _lib.check(lib.b200_effdet_postprocess_typed(L, self._hw, self._A, C, B, int(first_image), n, pb, box_dtype, pc, cls_dtype, K,
+                                                 float(iou_threshold), float(score_threshold), _lib.METRIC_EFF[iou_type],
+                                                 T.ptr(out['boxes']), T.ptr(out['classes_id']), T.ptr(out['scores']),
+                                                 T.ptr(out.get('sel_idx')), T.ptr(out.get('sel_anchor')), T.ptr(out['count']),
+                                                 T.ptr(ws), ws_bytes, T.stream_ptr()), 'convert_outputs_one')
     return out
 
   # -- fused passes (one read of the class logits) -----------------------------------------------------------
@@ -224,12 +227,13 @@ class Anchors(object):
   def decode_and_postprocess(self, outputs_boxes, outputs_classes, max_output_size=200, iou_threshold=0.5,
                              score_threshold=0.0001, iou_type='diou', with_indices=False):
     '''convert_outputs_boxes followed by convert_outputs_one for every image of the batch (anchors.py:141-202) in one
-    pass over the heads.  Returns (decoded boxes per level, dict as convert_outputs_batch).'''
+    pass over the heads.  Returns (decoded boxes per level (float32), dict as convert_outputs_batch).  Offsets or logits
+    that are all bfloat16 or all float16 are read in place; the results are those of the float32 call on the widened tensors.'''
     assert iou_type in ('iou', 'giou', 'diou', 'ciou')
     lib = _lib.load()
     tab = self._dev_table()
-    rel = [T.to_cuda(t) for t in outputs_boxes]
-    cl = [T.to_cuda(t) for t in outputs_classes]
+    rel, rel_dtype = T.to_cuda_heads(outputs_boxes)
+    cl, cls_dtype = T.to_cuda_heads(outputs_classes)
     L = self._num_levels
     if len(rel) != L or len(cl) != L:
       raise ValueError('expected %d levels' % L)
@@ -238,16 +242,16 @@ class Anchors(object):
       if tuple(t.shape) != (B, h, w, self._A, 4) or tuple(c.shape) != (B, h, w, self._A, C):
         raise ValueError('level shapes %r / %r do not match (B,%d,%d,%d,4|C)' % (tuple(t.shape), tuple(c.shape), h, w, self._A))
     dev = cl[0].device
-    dec = [torch.empty_like(t) for t in rel]
+    dec = [torch.empty(t.shape, dtype=torch.float32, device=t.device) for t in rel]
     out = self._post_outputs(B, K, dev, with_indices)
     ws_bytes = lib.b200_effdet_eval_workspace_bytes(L, self._hw, self._A, B, K)
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
     arr = lambda ts: (ctypes.c_void_p * L)(*[t.data_ptr() for t in ts])
-    _lib.check(lib.b200_effdet_decode_postprocess(L, self._hw, self._A, T.ptr(tab), C, B, arr(rel), arr(cl), arr(dec), K,
-                                                  float(iou_threshold), float(score_threshold), _lib.METRIC_EFF[iou_type],
-                                                  T.ptr(out['boxes']), T.ptr(out['classes_id']), T.ptr(out['scores']),
-                                                  T.ptr(out.get('sel_idx')), T.ptr(out.get('sel_anchor')), T.ptr(out['count']),
-                                                  T.ptr(ws), ws_bytes, T.stream_ptr()), 'decode_and_postprocess')
+    _lib.check(lib.b200_effdet_decode_postprocess_typed(L, self._hw, self._A, T.ptr(tab), C, B, arr(rel), rel_dtype, arr(cl),
+                                                        cls_dtype, arr(dec), K, float(iou_threshold), float(score_threshold),
+                                                        _lib.METRIC_EFF[iou_type], T.ptr(out['boxes']), T.ptr(out['classes_id']),
+                                                        T.ptr(out['scores']), T.ptr(out.get('sel_idx')), T.ptr(out.get('sel_anchor')),
+                                                        T.ptr(out['count']), T.ptr(ws), ws_bytes, T.stream_ptr()), 'decode_and_postprocess')
     return tuple(dec), out
 
   def eval_step(self, y_true_boxes, y_true_classes, y_true_masks, y_pred_boxes, y_pred_classes, alpha=0.25, gamma=1.5,

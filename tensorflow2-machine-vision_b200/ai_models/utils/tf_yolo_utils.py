@@ -82,12 +82,8 @@ def _levels(y1, y2, y3, anchors_wh):
   if anc.size % 6 != 0:
     raise ValueError('anchors_wh must be (3, anchors_num, 2)')
   A = anc.size // 6
-  heads = []
-  for y in (y1, y2, y3):
-    t = T.to_cuda(y)
-    if t.dim() == 5:
-      t = t.reshape(t.shape[0], t.shape[1], t.shape[2], -1)
-    heads.append(t)
+  heads, dtype = T.to_cuda_heads((y1, y2, y3))
+  heads = [t.reshape(t.shape[0], t.shape[1], t.shape[2], -1) if t.dim() == 5 else t for t in heads]
   B = heads[0].shape[0]
   ch = heads[0].shape[3]
   if ch % A != 0:
@@ -95,7 +91,7 @@ def _levels(y1, y2, y3, anchors_wh):
   for t in heads:
     if t.shape[0] != B or t.shape[3] != ch:
       raise ValueError('the three heads disagree on batch or channel size')
-  return heads, anc, A, B, ch // A
+  return heads, dtype, anc, A, B, ch // A
 
 
 def GetNMSBoxesBatch(y1, y2, y3, anchors_wh, image_wh, classes_num,
@@ -105,10 +101,12 @@ def GetNMSBoxesBatch(y1, y2, y3, anchors_wh, image_wh, classes_num,
 
   Returns a dict of padded tensors [B, max_output_size, ...] plus `count` [B] (int32):
   boxes, classes_id, scores, classes (optional), confidence, and with_indices -> sel_idx / sel_anchor.
+  Heads that are all bfloat16 or all float16 (mixed-precision networks) are read in place; the outputs are fp32 and
+  bit-identical to those of the fp32 heads y.float().
   '''
   assert iou_type in ['iou','diou','ciou']
   lib = _lib.load()
-  heads, anc, A, B, RF = _levels(y1, y2, y3, anchors_wh)
+  heads, dtype, anc, A, B, RF = _levels(y1, y2, y3, anchors_wh)
   C = int(classes_num)
   if RF != 5 + C:
     raise ValueError('head channels %d != anchors_num*(5+classes_num)' % (RF * A))
@@ -131,8 +129,8 @@ def GetNMSBoxesBatch(y1, y2, y3, anchors_wh, image_wh, classes_num,
     out['sel_anchor'] = torch.empty((B, K), dtype=torch.int32, device=dev)
   ws_bytes = lib.b200_yolo_decode_nms_workspace_bytes(hw, B, A, K)
   ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-  _lib.check(lib.b200_yolo_decode_nms(
-    hp, hw, B, A, C, anc.ctypes.data_as(ctypes.c_void_p), img.ctypes.data_as(ctypes.c_void_p),
+  _lib.check(lib.b200_yolo_decode_nms_typed(
+    hp, dtype, hw, B, A, C, anc.ctypes.data_as(ctypes.c_void_p), img.ctypes.data_as(ctypes.c_void_p),
     float(confidence_thresh), float(scores_thresh), float(iou_thresh), _lib.METRIC_YOLO[iou_type], K,
     T.ptr(out['boxes']), T.ptr(out['classes_id']), T.ptr(out['scores']), T.ptr(out.get('classes')),
     T.ptr(out['confidence']), T.ptr(out.get('sel_idx')), T.ptr(out.get('sel_anchor')), T.ptr(out['count']),

@@ -42,6 +42,41 @@ static inline size_t b200_align_up(size_t x, size_t a) { return (x + a - 1) / a 
 int b200_sm_count();
 
 #ifdef __CUDACC__
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
+// Head elements in their own type (float, __nv_bfloat16, __half), widened to fp32 on load.  Widening bf16 / fp16 is
+// exact, so every decision downstream sees the value that heads.float() would hold.
+__device__ __forceinline__ float elem_f32(float x) { return x; }
+__device__ __forceinline__ float elem_f32(__nv_bfloat16 x) { return __bfloat162float(x); }
+__device__ __forceinline__ float elem_f32(__half x) { return __half2float(x); }
+template <typename T>
+__device__ __forceinline__ float ldg_f32(const T* p) { return elem_f32(__ldg(p)); }
+// four consecutive elements (a box or its head offsets) at a 4-element boundary: one 16-byte load for fp32, one 8-byte
+// load for the 2-byte types; STREAM marks data read once (ld.global.cs)
+template <bool STREAM>
+__device__ __forceinline__ float4 ld4_f32(const float* p) {
+  return STREAM ? __ldcs(reinterpret_cast<const float4*>(p)) : __ldg(reinterpret_cast<const float4*>(p));
+}
+template <bool STREAM, typename H>
+__device__ __forceinline__ float4 ld4_f32(const H* p) {
+  const uint2 u = STREAM ? __ldcs(reinterpret_cast<const uint2*>(p)) : __ldg(reinterpret_cast<const uint2*>(p));
+  const H* h = reinterpret_cast<const H*>(&u);
+  return make_float4(elem_f32(h[0]), elem_f32(h[1]), elem_f32(h[2]), elem_f32(h[3]));
+}
+#endif
+
+// Runs the statements that follow `T` with T bound to the element type of a B200_DTYPE_* code (checked by the caller).
+#define B200_DISPATCH_DTYPE(code, T, ...)                                 \
+  switch (code) {                                                         \
+    case B200_DTYPE_BF16: { using T = __nv_bfloat16; __VA_ARGS__; } break; \
+    case B200_DTYPE_F16: { using T = __half; __VA_ARGS__; } break;        \
+    default: { using T = float; __VA_ARGS__; } break;                     \
+  }
+static inline bool b200_dtype_ok(int code) { return code == B200_DTYPE_F32 || code == B200_DTYPE_BF16 || code == B200_DTYPE_F16; }
+static inline int b200_dtype_bytes(int code) { return code == B200_DTYPE_F32 ? 4 : 2; }
+
+#ifdef __CUDACC__
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

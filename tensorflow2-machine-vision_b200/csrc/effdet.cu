@@ -12,6 +12,9 @@
 // buffers of the multi-CTA pre-selection).
 //
 // Anchors are rebuilt in-kernel from the per-level table (effdet_anchor.cuh, shared with effdet_loss.cu).
+//
+// The decode and the filter read the heads in their own element type (fp32, bf16 or fp16: a template parameter, each
+// element widened to fp32 exactly on load); decoded boxes, the candidate store and every NMS output are fp32.
 #include "nms.cuh"
 #include "effdet_focal.cuh"
 #include "effdet_anchor.cuh"
@@ -44,11 +47,12 @@ __global__ void effdet_anchors_kernel(EfLevels lv, int l, float4* __restrict__ o
 struct EfDecodeParams {
   EfLevels lv;
   int B;
-  const float4* rel[EF_MAX_LEVELS];
+  const void* rel[EF_MAX_LEVELS];   // (B,H,W,A,4) of the kernel's element type T
   float4* out[EF_MAX_LEVELS];
   long long elem_base[EF_MAX_LEVELS + 1];  // cumulative B*anc_per_img
 };
 
+template <typename T>
 __global__ void __launch_bounds__(256) effdet_decode_kernel(EfDecodeParams p) {
   const long long total = p.elem_base[p.lv.num_levels];
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -62,7 +66,7 @@ __global__ void __launch_bounds__(256) effdet_decode_kernel(EfDecodeParams p) {
     int y, x, a;
     ef_split(p.lv, l, rin, y, x, a);
     const AnchorBox an = ef_anchor(p.lv, l, y, x, a);
-    const float4 r = __ldcs(p.rel[l] + e);
+    const float4 r = ld4_f32<true>(static_cast<const T*>(p.rel[l]) + 4 * e);
     const float4 b = ef_decode_box(an, r);
     __stcs(p.out[l] + e, b);
   }
@@ -73,19 +77,21 @@ struct EfFilterParams {
   EfLevels lv;
   int B0, NB, C;                 // images [B0, B0+NB) of a batch of size B
   int B;
-  const float* cls[EF_MAX_LEVELS];    // (B,H,W,A,C) logits
-  const float4* boxes[EF_MAX_LEVELS]; // (B,H,W,A,4) decoded, or null: decode here from rel (lv.table must be set)
-  const float4* rel[EF_MAX_LEVELS];   // (B,H,W,A,4) head offsets ty,tx,th,tw (fused decode mode)
+  const void* cls[EF_MAX_LEVELS];     // (B,H,W,A,C) logits, element type TC
+  const void* boxes[EF_MAX_LEVELS];   // (B,H,W,A,4) decoded, element type TB, or null: decode here from rel (lv.table must be set)
+  const void* rel[EF_MAX_LEVELS];     // (B,H,W,A,4) head offsets ty,tx,th,tw, element type TB (fused decode mode)
   float4* dec[EF_MAX_LEVELS];         // fused decode mode: the dense decoded tensor is written here (may be null)
   long long tile_base[EF_MAX_LEVELS + 1];  // tiles of 32 anchors over the NB images of each level
   CandStore st;                  // [NB] images
 };
 
+// TC: element type of the class logits; TB: of the decoded boxes or head offsets
+template <typename TC, typename TB>
 __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p) {
   extern __shared__ __align__(128) unsigned char ef_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
   const int C = p.C;
-  WarpSlabRing<EF_STAGES> ring(ef_smem, C);
+  WarpSlabRing<EF_STAGES> ring(ef_smem, C * (int)sizeof(TC));
   const long long n_tiles = p.tile_base[p.lv.num_levels];
   const long long gwarp = (long long)blockIdx.x * wpc + warp, gstride = (long long)gridDim.x * wpc;
 
@@ -100,7 +106,7 @@ __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p)
   auto issue = [&](long long tile, int s) {
     int l, nrec; long long rec0;
     locate(tile, l, rec0, nrec);
-    ring.issue(s, p.cls[l] + ((long long)p.B0 * p.lv.anc_per_img[l] + rec0) * C, nrec, C);
+    ring.issue(s, static_cast<const TC*>(p.cls[l]) + ((long long)p.B0 * p.lv.anc_per_img[l] + rec0) * C, nrec, C);
   };
   long long t_issue = gwarp;
 #pragma unroll
@@ -109,7 +115,7 @@ __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p)
     ring.wait();
     int l, nrec; long long rec0;
     locate(tile, l, rec0, nrec);
-    const float* r = ring.slab(ring.stage) + lane * C;
+    const TC* r = ring.template slab<TC>(ring.stage) + lane * C;
     bool pass = false;
     int img = 0, cls = 0;
     float score = 0.f;
@@ -127,10 +133,11 @@ __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p)
       if (total < 0x7fffffffLL) { img = (int)((uint32_t)rec / (uint32_t)api); rin = (int)((uint32_t)rec - (uint32_t)img * (uint32_t)api); }
       else { img = (int)(rec / api); rin = (int)(rec - (long long)img * api); }
       grec = (long long)(p.B0 + img) * api + rin;
-      if (fused_decode) r4 = __ldcs(p.rel[l] + grec);   // issued before the class scan: coalesced, 16 bytes per lane
+      // issued before the class scan: coalesced, 16 bytes per lane (8 for 2-byte offsets)
+      if (fused_decode) r4 = ld4_f32<true>(static_cast<const TB*>(p.rel[l]) + 4 * grec);
       // tf.math.argmax: first maximal index; reduce_max: the maximum (anc:172-174)
-      m = r[0];
-      for (int c = 1; c < C; ++c) { const float v = r[c]; if (v > m) { m = v; mi = c; } }
+      m = elem_f32(r[0]);
+      for (int c = 1; c < C; ++c) { const float v = elem_f32(r[c]); if (v > m) { m = v; mi = c; } }
     }
     // the class scan was the last read of the slab: its refill is in flight during the decode and the append below
     __syncwarp();
@@ -147,7 +154,7 @@ __global__ void __launch_bounds__(256, 1) effdet_filter_kernel(EfFilterParams p)
       if (mi != 0) {  // classes_mask = classes_id != 0 (anc:179)
         pass = true; cls = mi; score = m;
         aidx = (uint32_t)(p.lv.anchor_base[l] + rin);
-        if (!fused_decode) box = __ldg(p.boxes[l] + grec);
+        if (!fused_decode) box = ld4_f32<false>(static_cast<const TB*>(p.boxes[l]) + 4 * grec);
       }
     }
     warp_append_by_image(p.st, pass, img, aidx, [&](size_t slot) {
@@ -375,9 +382,10 @@ extern "C" int b200_effdet_anchors(int num_levels, const int32_t* hw, int A, con
   return B200_OK;
 }
 
-extern "C" int b200_effdet_decode(int num_levels, const int32_t* hw, int A, const float* table_dev, int B,
-                                  const float* const rel[], float* const out[], void* stream) {
+extern "C" int b200_effdet_decode_typed(int num_levels, const int32_t* hw, int A, const float* table_dev, int B,
+                                        const void* const rel[], int rel_dtype, float* const out[], void* stream) {
   EfDecodeParams p;
+  B200_REQUIRE(b200_dtype_ok(rel_dtype), B200_ERR_BAD_ARG, "b200_effdet_decode: rel_dtype %d is not a B200_DTYPE_* code", rel_dtype);
   B200_REQUIRE(hw && table_dev && rel && out, B200_ERR_BAD_ARG, "b200_effdet_decode: null argument");
   B200_REQUIRE(ef_fill_levels(p.lv, num_levels, hw, A, table_dev) >= 0, B200_ERR_BAD_ARG, "b200_effdet_decode: bad level spec");
   B200_REQUIRE(B >= 0, B200_ERR_BAD_ARG, "b200_effdet_decode: negative batch");
@@ -390,7 +398,7 @@ extern "C" int b200_effdet_decode(int num_levels, const int32_t* hw, int A, cons
       B200_REQUIRE(rel[l] && out[l], B200_ERR_BAD_ARG, "b200_effdet_decode: null level %d", l);
       B200_REQUIRE(((reinterpret_cast<uintptr_t>(rel[l]) | reinterpret_cast<uintptr_t>(out[l])) & 15) == 0, B200_ERR_BAD_ARG,
                    "b200_effdet_decode: level %d not 16-byte aligned", l);
-      p.rel[l] = reinterpret_cast<const float4*>(rel[l]);
+      p.rel[l] = rel[l];
       p.out[l] = reinterpret_cast<float4*>(out[l]);
       cum += (long long)B * p.lv.anc_per_img[l];
     } else { p.rel[l] = nullptr; p.out[l] = nullptr; }
@@ -400,9 +408,15 @@ extern "C" int b200_effdet_decode(int num_levels, const int32_t* hw, int A, cons
   long long blocks = (cum + 255) / 256;
   const long long cap = (long long)b200_sm_count() * 64;  // many short CTAs: see el_cta_plan
   if (blocks > cap) blocks = cap;
-  effdet_decode_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(p);
+  B200_DISPATCH_DTYPE(rel_dtype, T, effdet_decode_kernel<T><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(p))
   B200_LAUNCH_CHECK();
   return B200_OK;
+}
+
+extern "C" int b200_effdet_decode(int num_levels, const int32_t* hw, int A, const float* table_dev, int B,
+                                  const float* const rel[], float* const out[], void* stream) {
+  return b200_effdet_decode_typed(num_levels, hw, A, table_dev, B, reinterpret_cast<const void* const*>(rel), B200_DTYPE_F32, out,
+                                  stream);
 }
 
 __global__ void __launch_bounds__(NMS_THREADS, 1) effdet_nms_pivot_kernel(NmsPreselectParams p) {
@@ -457,14 +471,32 @@ extern "C" size_t b200_effdet_postprocess_workspace_bytes(int num_levels, const 
 
 // boxes: decoded boxes (the drop-in convert_outputs_one), or null with rel / table_dev given: decode inside the filter
 // pass (convert_outputs_boxes + convert_outputs_one in one sweep; dec_out[l] receives the dense decoded tensor)
+// The filter launch for logits of element type TC and boxes / head offsets of element type TB.
+template <typename TC, typename TB>
+static int ef_filter_launch(const EfFilterParams& fp, long long n_tiles, cudaStream_t stream) {
+  using Ring = WarpSlabRing<EF_STAGES>;
+  const int rec_bytes = fp.C * (int)sizeof(TC);
+  int warps = 8;
+  while (warps > 1 && Ring::smem_bytes(warps, rec_bytes) > 200 * 1024) warps >>= 1;
+  const size_t smem1 = Ring::smem_bytes(warps, rec_bytes);
+  B200_CUDA(cudaFuncSetAttribute(effdet_filter_kernel<TC, TB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+  const int grid = Ring::grid(n_tiles, warps, b200_sm_count());
+  effdet_filter_kernel<TC, TB><<<grid, warps * 32, smem1, stream>>>(fp);
+  B200_LAUNCH_CHECK();
+  return B200_OK;
+}
+
+// box_dtype is the element type of `boxes` or of `rel`, whichever is given; cls_dtype that of `classes`
 static int ef_post_impl(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B, int first_image,
-                        int num_images, const float* const boxes[], const float* const rel[], float* const dec_out[],
-                        const float* const classes[], int max_out, float iou_thr, float score_thr, int metric, float* out_boxes,
+                        int num_images, const void* const boxes[], const void* const rel[], int box_dtype,
+                        float* const dec_out[], const void* const classes[], int cls_dtype, int max_out, float iou_thr, float score_thr, int metric, float* out_boxes,
                         long long* out_class_id, float* out_score, int32_t* out_sel_idx,
                         int32_t* out_sel_anchor, int32_t* out_count, void* workspace,
                         size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   EfFilterParams fp;
+  B200_REQUIRE(b200_dtype_ok(box_dtype) && b200_dtype_ok(cls_dtype), B200_ERR_BAD_ARG,
+               "b200_effdet_postprocess: dtype codes %d / %d are not B200_DTYPE_* codes", box_dtype, cls_dtype);
   B200_REQUIRE(hw && (boxes || (rel && table_dev)) && classes, B200_ERR_BAD_ARG, "b200_effdet_postprocess: null argument");
   const int n_img = ef_fill_levels(fp.lv, num_levels, hw, A, table_dev);
   B200_REQUIRE(n_img >= 0, B200_ERR_BAD_ARG, "b200_effdet_postprocess: bad level spec");
@@ -483,13 +515,13 @@ static int ef_post_impl(int num_levels, const int32_t* hw, int A, const float* t
   for (int l = 0; l < EF_MAX_LEVELS; ++l) {
     fp.tile_base[l] = tb;
     if (l < num_levels) {
-      const float* bl = boxes ? boxes[l] : rel[l];
+      const void* bl = boxes ? boxes[l] : rel[l];
       B200_REQUIRE(bl && classes[l], B200_ERR_BAD_ARG, "b200_effdet_postprocess: null level %d", l);
       B200_REQUIRE(((reinterpret_cast<uintptr_t>(bl) | (dec_out && dec_out[l] ? reinterpret_cast<uintptr_t>(dec_out[l]) : 0)) & 15) == 0, B200_ERR_BAD_ARG,
                    "b200_effdet_postprocess: boxes level %d not 16-byte aligned", l);
       fp.cls[l] = classes[l];
-      fp.boxes[l] = boxes ? reinterpret_cast<const float4*>(boxes[l]) : nullptr;
-      fp.rel[l] = boxes ? nullptr : reinterpret_cast<const float4*>(rel[l]);
+      fp.boxes[l] = boxes ? boxes[l] : nullptr;
+      fp.rel[l] = boxes ? nullptr : rel[l];
       fp.dec[l] = (!boxes && dec_out) ? reinterpret_cast<float4*>(dec_out[l]) : nullptr;
       tb += ((long long)num_images * fp.lv.anc_per_img[l] + 31) / 32;
     } else { fp.cls[l] = nullptr; fp.boxes[l] = nullptr; fp.rel[l] = nullptr; fp.dec[l] = nullptr; }
@@ -497,17 +529,24 @@ static int ef_post_impl(int num_levels, const int32_t* hw, int A, const float* t
   for (int l = num_levels; l <= EF_MAX_LEVELS; ++l) fp.tile_base[l] = tb;
   fp.st = cand_bind(ws, wsb, out_sel_idx != nullptr);
   B200_CUDA(cudaMemsetAsync(wsb, 0, ws.zeroed(out_sel_idx != nullptr), stream));
-  using Ring = WarpSlabRing<EF_STAGES>;
-  int warps = 8;
-  while (warps > 1 && Ring::smem_bytes(warps, C) > 200 * 1024) warps >>= 1;
-  const size_t smem1 = Ring::smem_bytes(warps, C);
-  B200_CUDA(cudaFuncSetAttribute(effdet_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-  const int grid = Ring::grid(tb, warps, b200_sm_count());
-  effdet_filter_kernel<<<grid, warps * 32, smem1, stream>>>(fp);
-  B200_LAUNCH_CHECK();
+  int st = B200_OK;
+  B200_DISPATCH_DTYPE(cls_dtype, TC, B200_DISPATCH_DTYPE(box_dtype, TB, st = ef_filter_launch<TC, TB>(fp, tb, stream)))
+  if (st != B200_OK) return st;
 
   return ef_launch_nms(fp.st, num_images, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx,
                        out_sel_anchor, out_count, stream);
+}
+
+extern "C" int b200_effdet_postprocess_typed(int num_levels, const int32_t* hw, int A, int C, int B, int first_image,
+                                             int num_images, const void* const boxes[], int box_dtype,
+                                             const void* const classes[], int cls_dtype, int max_out, float iou_thr,
+                                             float score_thr, int metric, float* out_boxes, long long* out_class_id,
+                                             float* out_score, int32_t* out_sel_idx, int32_t* out_sel_anchor,
+                                             int32_t* out_count, void* workspace, size_t workspace_bytes, void* stream_) {
+  B200_REQUIRE(boxes, B200_ERR_BAD_ARG, "b200_effdet_postprocess: null argument");
+  return ef_post_impl(num_levels, hw, A, nullptr, C, B, first_image, num_images, boxes, nullptr, box_dtype, nullptr, classes,
+                      cls_dtype, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx,
+                      out_sel_anchor, out_count, workspace, workspace_bytes, stream_);
 }
 
 extern "C" int b200_effdet_postprocess(int num_levels, const int32_t* hw, int A, int C, int B, int first_image,
@@ -516,10 +555,10 @@ extern "C" int b200_effdet_postprocess(int num_levels, const int32_t* hw, int A,
                                        long long* out_class_id, float* out_score, int32_t* out_sel_idx,
                                        int32_t* out_sel_anchor, int32_t* out_count, void* workspace,
                                        size_t workspace_bytes, void* stream_) {
-  B200_REQUIRE(boxes, B200_ERR_BAD_ARG, "b200_effdet_postprocess: null argument");
-  return ef_post_impl(num_levels, hw, A, nullptr, C, B, first_image, num_images, boxes, nullptr, nullptr, classes, max_out, iou_thr,
-                      score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx, out_sel_anchor, out_count, workspace,
-                      workspace_bytes, stream_);
+  return b200_effdet_postprocess_typed(num_levels, hw, A, C, B, first_image, num_images, reinterpret_cast<const void* const*>(boxes),
+                                       B200_DTYPE_F32, reinterpret_cast<const void* const*>(classes), B200_DTYPE_F32, max_out,
+                                       iou_thr, score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx, out_sel_anchor,
+                                       out_count, workspace, workspace_bytes, stream_);
 }
 
 // CTAs of 256 anchors per (level, image); returns the grid size
@@ -1103,16 +1142,30 @@ extern "C" int b200_effdet_eval_step_from_boxes(int num_levels, const int32_t* h
 }
 
 // convert_outputs_boxes + convert_outputs_one of the whole batch in one pass over the heads (no targets, no loss).
+extern "C" int b200_effdet_decode_postprocess_typed(int num_levels, const int32_t* hw, int A, const float* table_dev, int C,
+                                                    int B, const void* const pred_boxes[], int rel_dtype,
+                                                    const void* const pred_classes[], int cls_dtype,
+                                                    float* const out_decoded[], int max_out, float iou_thr, float score_thr,
+                                                    int metric, float* out_boxes, long long* out_class_id, float* out_score,
+                                                    int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
+                                                    void* workspace, size_t workspace_bytes, void* stream) {
+  // without targets the per-warp bulk-copy filter (lane <-> anchor, no CTA barriers) is the faster stream: the decode rides
+  // on it (one coalesced 16-byte load and store per lane); the CTA-tiled kernel above pays off only with the focal terms
+  B200_REQUIRE(pred_boxes && table_dev, B200_ERR_BAD_ARG, "b200_effdet_decode_postprocess: null argument");
+  return ef_post_impl(num_levels, hw, A, table_dev, C, B, 0, B, nullptr, pred_boxes, rel_dtype, out_decoded, pred_classes,
+                      cls_dtype, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx,
+                      out_sel_anchor, out_count, workspace, workspace_bytes, stream);
+}
+
 extern "C" int b200_effdet_decode_postprocess(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
                                               const float* const pred_boxes[], const float* const pred_classes[],
                                               float* const out_decoded[], int max_out, float iou_thr, float score_thr, int metric,
                                               float* out_boxes, long long* out_class_id, float* out_score, int32_t* out_sel_idx,
                                               int32_t* out_sel_anchor, int32_t* out_count, void* workspace, size_t workspace_bytes,
                                               void* stream) {
-  // without targets the per-warp bulk-copy filter (lane <-> anchor, no CTA barriers) is the faster stream: the decode rides
-  // on it (one coalesced 16-byte load and store per lane); the CTA-tiled kernel above pays off only with the focal terms
-  B200_REQUIRE(pred_boxes && table_dev, B200_ERR_BAD_ARG, "b200_effdet_decode_postprocess: null argument");
-  return ef_post_impl(num_levels, hw, A, table_dev, C, B, 0, B, nullptr, pred_boxes, out_decoded, pred_classes, max_out, iou_thr,
-                      score_thr, metric, out_boxes, out_class_id, out_score, out_sel_idx, out_sel_anchor, out_count, workspace,
-                      workspace_bytes, stream);
+  return b200_effdet_decode_postprocess_typed(num_levels, hw, A, table_dev, C, B, reinterpret_cast<const void* const*>(pred_boxes),
+                                              B200_DTYPE_F32, reinterpret_cast<const void* const*>(pred_classes), B200_DTYPE_F32,
+                                              out_decoded, max_out, iou_thr, score_thr, metric, out_boxes, out_class_id,
+                                              out_score, out_sel_idx, out_sel_anchor, out_count, workspace, workspace_bytes,
+                                              stream);
 }

@@ -4,11 +4,13 @@
 // B == 1 semantics of the reference applied per image (the reference flattens the batch, tyu:163-166).
 //
 // Kernel 1  yolo_decode_filter_kernel  (HBM-read bound: every head byte is read exactly once)
-//   * each level tensor is treated as a flat array of records of RF = 5+C floats; a warp owns tiles of 32
+//   * each level tensor is treated as a flat array of records of RF = 5+C elements (fp32, bf16 or fp16: the element type
+//     is a template parameter, every element is widened to fp32 exactly as it is read); a warp owns tiles of 32
 //     records staged through its own WarpSlabRing (bulkcopy.cuh: one bulk copy per tile, a plain copy for a level's
 //     ragged tail); 16 warps per SM, each with its own tile in flight;
-//   * lane <-> record; the stride RF between lanes is odd for the 85-float COCO record so the column reads are
-//     bank-conflict free; conf is thresholded first, then the class maximum is found on raw logits and the
+//   * lane <-> record; the stride RF between lanes is odd for the 85-element COCO record, so the fp32 column reads are
+//     bank-conflict free.  With 2-byte elements two lanes three records apart read words 128 apart (85 elements): a
+//     column read takes two shared-memory wavefronts instead of one (DESIGN.md §4); conf is thresholded first, then the class maximum is found on raw logits and the
 //     sigmoid is evaluated only for logits inside a guard band of the maximum (max / first-argmax are taken
 //     in sigmoid space, exactly as tf.reduce_max / tf.argmax of sigmoid(classes) do; detmath's sigmoid is not
 //     monotone at ulp level, see oracle/DETMATH_REPORT.md);
@@ -19,6 +21,8 @@
 //     serves as the NMS tie-break id and as the rank source for `sel_idx`.
 // Kernel 2  yolo_nms_finalize_kernel  (one CTA per image): nms.cuh greedy NMS + gather of the five outputs,
 //   recomputing sigmoid(classes) for the <= max_out selected rows straight from the head tensors.
+// Kernels that read the heads (both above, yolo_classes_kernel) are instantiated per element type; decisions, candidate
+// store and outputs are fp32 whatever the heads are, so a bf16 / fp16 call gives the bits of the fp32 call on heads.float().
 #include <cmath>
 #include "nms.cuh"
 #include "bulkcopy.cuh"
@@ -27,7 +31,7 @@
 #define YD_STAGES 1
 
 struct YoloLevels {
-  const float* head[YD_MAX_LEVELS];
+  const void* head[YD_MAX_LEVELS];   // element type: the kernels' template parameter T
   int h[YD_MAX_LEVELS], w[YD_MAX_LEVELS];
   int rec_per_img[YD_MAX_LEVELS];   // h*w*A
   int anchor_base[YD_MAX_LEVELS];   // flat anchor index of the level's first record within an image
@@ -56,9 +60,10 @@ struct YoloDecodeParams {
 // (oracle/DETMATH_REPORT.md; it is not monotone at ulp level, which is why the band exists).  Otherwise (a few per
 // cent of the records) the whole warp evaluates that record's in-band logits and takes max / first-argmax in sigmoid
 // space, exactly as tf.reduce_max / tf.argmax of sigmoid(classes) do.
-__device__ __forceinline__ void class_max_sigmoid_warp(const float* __restrict__ slab, int RF, int C, bool want, int lane,
+template <typename T>
+__device__ __forceinline__ void class_max_sigmoid_warp(const T* __restrict__ slab, int RF, int C, bool want, int lane,
                                                        float& best_s, int& best_c) {
-  const float* __restrict__ cls = slab + lane * RF + 5;
+  const T* __restrict__ cls = slab + lane * RF + 5;
   bool slow = false;
   float lo = -INFINITY;
   if (want) {
@@ -70,7 +75,7 @@ __device__ __forceinline__ void class_max_sigmoid_warp(const float* __restrict__
     for (; c + 4 <= C; c += 4) {
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
-        const float x = cls[c + k];
+        const float x = elem_f32(cls[c + k]);
         nan_acc = __fmaf_rn(x, 0.0f, nan_acc);            // NaN once any logit is NaN or +-inf
         m2[k] = fmaxf(m2[k], fminf(a[k], x));
         const bool g = x > a[k];                            // strict: the first index of a chain's maximum stays
@@ -79,7 +84,7 @@ __device__ __forceinline__ void class_max_sigmoid_warp(const float* __restrict__
       }
     }
     for (; c < C; ++c) {
-      const float x = cls[c];
+      const float x = elem_f32(cls[c]);
       nan_acc = __fmaf_rn(x, 0.0f, nan_acc);
       m2[0] = fmaxf(m2[0], fminf(a[0], x));
       const bool g = x > a[0];
@@ -110,14 +115,14 @@ __device__ __forceinline__ void class_max_sigmoid_warp(const float* __restrict__
     const int src = __ffs(todo) - 1;
     todo &= todo - 1u;
     const float lo_s = __shfl_sync(0xffffffffu, lo, src);
-    const float* __restrict__ rc = slab + src * RF + 5;
+    const T* __restrict__ rc = slab + src * RF + 5;
     // serial semantics being reproduced: walk c upwards over the in-band logits (x >= lo or NaN); the first one
     // initialises (s, c) even when its sigmoid is NaN; later ones replace it only when s > best
     float ls = 0.0f;
     int lc = 0x7fffffff, lfirst = 0x7fffffff;
     bool lfirst_nan = false;
     for (int c = lane; c < C; c += 32) {
-      const float x = rc[c];
+      const float x = elem_f32(rc[c]);
       if (x >= lo_s || x != x) {
         const float sg = dm_sigmoidf(x);
         if (lfirst == 0x7fffffff) { lfirst = c; lfirst_nan = sg != sg; }
@@ -162,14 +167,15 @@ __device__ __forceinline__ Decoded decode_box(float tx, float ty, float tw, floa
   return d;
 }
 
-template <bool EARLY>   // EARLY: a warp refills its slab before its append (atomic + stores) instead of after it
+// EARLY: a warp refills its slab before its append (atomic + stores) instead of after it; T: element type of the heads
+template <bool EARLY, typename T>
 __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodeParams p) {
   extern __shared__ __align__(128) unsigned char yd_smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   const int warps_per_cta = blockDim.x >> 5;
   const int RF = p.RF;
-  WarpSlabRing<YD_STAGES> ring(yd_smem, RF);
+  WarpSlabRing<YD_STAGES> ring(yd_smem, RF * (int)sizeof(T));
 
   const long long n_tiles = p.lv.tile_base[YD_MAX_LEVELS];
   const long long gwarp = (long long)blockIdx.x * warps_per_cta + warp;
@@ -182,7 +188,7 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
     for (int k = 1; k < YD_MAX_LEVELS; ++k) if (tile >= p.lv.tile_base[k]) l = k;
     const long long rec0 = (tile - p.lv.tile_base[l]) * 32;
     const long long remain = p.lv.total_rec[l] - rec0;
-    ring.issue(s, p.lv.head[l] + rec0 * RF, remain < 32 ? (int)remain : 32, RF);
+    ring.issue(s, static_cast<const T*>(p.lv.head[l]) + rec0 * RF, remain < 32 ? (int)remain : 32, RF);
   };
 
   long long t_issue = gwarp;
@@ -193,13 +199,13 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
   }
   for (long long tile = gwarp; tile < n_tiles; tile += gstride) {
     ring.wait();
-    const float* slab = ring.slab(ring.stage);
+    const T* slab = ring.template slab<T>(ring.stage);
     int l = 0;
 #pragma unroll
     for (int k = 1; k < YD_MAX_LEVELS; ++k) if (tile >= p.lv.tile_base[k]) l = k;
     const long long rec = (tile - p.lv.tile_base[l]) * 32 + lane;
     const bool in_range = rec < p.lv.total_rec[l];
-    const float* r = slab + lane * RF;
+    const T* r = slab + lane * RF;
     bool pass = false;
     int img = 0;
     float score = 0.f, conf = 0.f;
@@ -208,7 +214,7 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
     bool want = false;
     if (in_range) {
       // sigmoid(conf) > conf_thr (tyu:191), decided in logit space outside a narrow band around logit(conf_thr)
-      conf = r[4];
+      conf = elem_f32(r[4]);
       if (conf > p.conf_hi) want = true;
       else if (conf >= p.conf_lo) want = dm_sigmoidf(conf) > p.conf_thr;  // NaN fails both comparisons: not wanted
     }
@@ -221,7 +227,7 @@ __global__ void __launch_bounds__(512, 1) yolo_decode_filter_kernel(YoloDecodePa
       const int cell = p.magic_a ? (int)__umulhi((uint32_t)rin, p.magic_a) : rin, a = rin - cell * p.A;  // rin / A
       // the box itself is decoded by the NMS pass, and only for the candidates it looks at; here only its validity
       // (x2 > x1 and y2 > y1, tyu:163) is needed: certain inside the safe logit range, exact decode otherwise
-      const float tx = r[0], ty = r[1], tw = r[2], th = r[3];
+      const float tx = elem_f32(r[0]), ty = elem_f32(r[1]), tw = elem_f32(r[2]), th = elem_f32(r[3]);
       bool valid = (tw >= p.lv.tmin_w[l][a]) && (tw <= 80.0f) && (th >= p.lv.tmin_h[l][a]) && (th <= 80.0f) && (tx == tx) && (ty == ty);
       if (!valid) {
         const int W = p.lv.w[l], H = p.lv.h[l];
@@ -265,7 +271,8 @@ struct YoloFinalizeParams {
 };
 
 // Decode-on-demand for NMS: candidate `pos` of the image -> its record in the head tensor -> decode_box; the result is
-// written back to the candidate store so that the emitted rows can be copied out afterwards.
+// written back to the candidate store so that the emitted rows can be copied out afterwards.  T: element type of the heads.
+template <typename T>
 struct YoloLazyBox {
   static constexpr bool kKeyCache = true;   // a 416x416 image has ~5 k candidates: its selection passes run from registers
   static constexpr int kMode = B200_NMS_BY_CLASS;
@@ -279,26 +286,26 @@ struct YoloLazyBox {
 #pragma unroll
     for (int j = 1; j < YD_MAX_LEVELS; ++j) if (a_flat >= lv->anchor_base[j]) l = j;
     const int rin = a_flat - lv->anchor_base[l];
-    const float* r = lv->head[l] + ((long long)img * lv->rec_per_img[l] + rin) * RF;
+    const T* r = static_cast<const T*>(lv->head[l]) + ((long long)img * lv->rec_per_img[l] + rin) * RF;
     const int cell = rin / A, a = rin - cell * A;
     const int W = lv->w[l], H = lv->h[l];
     const int gy = cell / W, gx = cell - gy * W;
-    const Decoded d = decode_box(__ldg(r), __ldg(r + 1), __ldg(r + 2), __ldg(r + 3), gx, gy, W, H, lv->anc_w[l][a], lv->anc_h[l][a]);
+    const Decoded d = decode_box(ldg_f32(r), ldg_f32(r + 1), ldg_f32(r + 2), ldg_f32(r + 3), gx, gy, W, H, lv->anc_w[l][a], lv->anc_h[l][a]);
     const float4 b = make_float4(d.x1, d.y1, d.x2, d.y2);
     cand_box[pos] = b;
     return b;
   }
 };
 
-template <int METRIC, int THREADS>
+template <int METRIC, int THREADS, typename T>
 __global__ void __launch_bounds__(THREADS, NMS_THREADS / THREADS) yolo_nms_finalize_kernel(YoloFinalizeParams p) {
   extern __shared__ __align__(16) unsigned char nms_smem[];
   const int img = blockIdx.x;
   const size_t cbase = (size_t)img * p.st.n_img;
   int32_t* pos = p.st.pos + (size_t)img * p.cfg.max_out;
-  YoloLazyBox lazy;
+  YoloLazyBox<T> lazy;
   lazy.lv = &p.lv; lazy.img = img; lazy.A = p.A; lazy.RF = p.RF; lazy.cand_box = p.st.box + cbase;
-  const int kept = nms_run_segment<METRIC, YoloLazyBox, THREADS>(cand_segment(p.st, img, true), p.cfg, pos, nms_smem, nullptr, lazy);
+  const int kept = nms_run_segment<METRIC, YoloLazyBox<T>, THREADS>(cand_segment(p.st, img, true), p.cfg, pos, nms_smem, nullptr, lazy);
   __syncthreads();
   if (threadIdx.x == 0) p.out_count[img] = kept;
   const size_t obase = (size_t)img * p.cfg.max_out;
@@ -322,7 +329,7 @@ __global__ void __launch_bounds__(THREADS, NMS_THREADS / THREADS) yolo_nms_final
 // LPR lanes per row: the kernel is bound by the issue of the deterministic sigmoid (~60 instructions), so the lanes that
 // idle in a row's last round are the cost — 80 classes on 32 lanes waste one round in six, on 16 lanes (two rows per
 // warp) none.
-template <int LPR>
+template <int LPR, typename T>
 __global__ void __launch_bounds__(256) yolo_classes_kernel(YoloFinalizeParams p) {
   constexpr int RPW = 32 / LPR, NJ = 128 / LPR;
   const int sub = threadIdx.x & (LPR - 1);
@@ -336,15 +343,15 @@ __global__ void __launch_bounds__(256) yolo_classes_kernel(YoloFinalizeParams p)
 #pragma unroll
   for (int j = 1; j < YD_MAX_LEVELS; ++j) if ((int)a >= p.lv.anchor_base[j]) l = j;
   const long long rec = (long long)img * p.lv.rec_per_img[l] + ((int)a - p.lv.anchor_base[l]);
-  const float* src = p.lv.head[l] + rec * p.RF + 5;
+  const T* src = static_cast<const T*>(p.lv.head[l]) + rec * p.RF + 5;
   float* dst = p.out_classes + (size_t)row * p.C;
   // the (cold) logits of up to 128 classes are fetched before the first sigmoid starts
   float x[NJ];
 #pragma unroll
-  for (int j = 0; j < NJ; ++j) x[j] = (sub + LPR * j < p.C) ? __ldg(src + sub + LPR * j) : 0.0f;
+  for (int j = 0; j < NJ; ++j) x[j] = (sub + LPR * j < p.C) ? ldg_f32(src + sub + LPR * j) : 0.0f;
 #pragma unroll
   for (int j = 0; j < NJ; ++j) if (sub + LPR * j < p.C) dst[sub + LPR * j] = dm_sigmoidf(x[j]);
-  for (int c = sub + 128; c < p.C; c += LPR) dst[c] = dm_sigmoidf(__ldg(src + c));
+  for (int c = sub + 128; c < p.C; c += LPR) dst[c] = dm_sigmoidf(ldg_f32(src + c));
 }
 
 // ---- dense decode for the stand-alone GetBoxes shim ---------------------------------------------
@@ -375,7 +382,7 @@ __global__ void yolo_decode_dense_kernel(const float* __restrict__ head, long lo
 }
 
 // ---- host side ---------------------------------------------------------------------------------
-static int fill_levels(YoloLevels& lv, const float* const heads[3], const int32_t hw[6], int B, int A, int C,
+static int fill_levels(YoloLevels& lv, const void* const heads[3], const int32_t hw[6], int B, int A, int C,
                        const float* anchors_wh_host, const float* image_wh_host) {
   long long tb = 0;
   int ab = 0;
@@ -409,13 +416,65 @@ extern "C" size_t b200_yolo_decode_nms_workspace_bytes(const int32_t hw[6], int 
   return cand_layout(B, n_img, max_out, true, false).total;
 }
 
-extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t hw[6], int B, int A, int C,
-                                    const float* anchors_wh_host, const float* image_wh_host, float conf_thr,
-                                    float score_thr, float iou_thr, int metric, int max_out, float* out_boxes,
-                                    int32_t* out_class_id, float* out_score, float* out_classes, float* out_conf,
-                                    int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
-                                    void* workspace, size_t workspace_bytes, void* stream_) {
+// The launches of one call, for heads of element type T (the checks and the workspace set-up are done).
+template <typename T>
+static int yd_launch(const YoloDecodeParams& dp, const YoloFinalizeParams& fp, int metric, int warps, size_t smem1,
+                     cudaStream_t stream) {
+  const long long n_tiles = dp.lv.tile_base[YD_MAX_LEVELS];
+  const int grid = WarpSlabRing<YD_STAGES>::grid(n_tiles, warps, b200_sm_count());
+  // Refilling a warp's slab before its append keeps one more copy in flight: -3 % for the call on its own at any size, and
+  // for the fused evaluation step at 512 images; at 64 images per GPU the same step is 3 % SLOWER with it (the filter then
+  // takes DRAM bandwidth from the loss chain that shares the GPU, and that chain is the longer one there).  Long streams
+  // (>= 32 tiles per warp) refill early, short ones late.
+  if (n_tiles >= 32ll * grid * warps) {
+    B200_CUDA(cudaFuncSetAttribute(yolo_decode_filter_kernel<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+    yolo_decode_filter_kernel<true, T><<<grid, warps * 32, smem1, stream>>>(dp);
+  } else {
+    B200_CUDA(cudaFuncSetAttribute(yolo_decode_filter_kernel<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+    yolo_decode_filter_kernel<false, T><<<grid, warps * 32, smem1, stream>>>(dp);
+  }
+  B200_LAUNCH_CHECK();
+
+  const int B = fp.B, C = fp.C, max_out = fp.cfg.max_out;
+  // one 1024-thread CTA per SM gives the lowest latency; batches that need more than one wave use 512-thread CTAs,
+  // two per SM (the shared-memory footprint allows it up to max_out ~ 500)
+  const size_t smem2 = cand_finalize_smem_bytes(fp.st, max_out);
+  const bool half_ctas = (B > b200_sm_count()) && (2 * (smem2 + 1024) <= 227 * 1024);
+#define YD_LAUNCH(M)                                                                                                   \
+  if (half_ctas) {                                                                                                          \
+    B200_CUDA(cudaFuncSetAttribute(yolo_nms_finalize_kernel<M, 512, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2)); \
+    yolo_nms_finalize_kernel<M, 512, T><<<B, 512, smem2, stream>>>(fp);                                                      \
+  } else {                                                                                                                  \
+    B200_CUDA(cudaFuncSetAttribute(yolo_nms_finalize_kernel<M, NMS_THREADS, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2)); \
+    yolo_nms_finalize_kernel<M, NMS_THREADS, T><<<B, NMS_THREADS, smem2, stream>>>(fp);                                      \
+  }
+  // the YOLO metrics only (the entry refuses the others)
+  switch (metric) {
+    case B200_METRIC_YOLO_IOU: { YD_LAUNCH(B200_METRIC_YOLO_IOU); } break;
+    case B200_METRIC_YOLO_DIOU: { YD_LAUNCH(B200_METRIC_YOLO_DIOU); } break;
+    default: { YD_LAUNCH(B200_METRIC_YOLO_CIOU); } break;
+  }
+#undef YD_LAUNCH
+  B200_LAUNCH_CHECK();
+  if (fp.out_classes) {
+    const long long rows = (long long)B * max_out;
+    // half a warp per row when that leaves fewer idle lanes in the last round (80 classes: 5 x 16 against 3 x 32)
+    // (a few hundred rows are latency-bound: a full warp per row has the shorter chain)
+    if (rows >= 16384 && ((C + 15) / 16) * 16 < ((C + 31) / 32) * 32) yolo_classes_kernel<16, T><<<(int)((rows + 15) / 16), 256, 0, stream>>>(fp);
+    else yolo_classes_kernel<32, T><<<(int)((rows + 7) / 8), 256, 0, stream>>>(fp);
+    B200_LAUNCH_CHECK();
+  }
+  return B200_OK;
+}
+
+extern "C" int b200_yolo_decode_nms_typed(const void* const heads[3], int head_dtype, const int32_t hw[6], int B, int A, int C,
+                                          const float* anchors_wh_host, const float* image_wh_host, float conf_thr,
+                                          float score_thr, float iou_thr, int metric, int max_out, float* out_boxes,
+                                          int32_t* out_class_id, float* out_score, float* out_classes, float* out_conf,
+                                          int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
+                                          void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  B200_REQUIRE(b200_dtype_ok(head_dtype), B200_ERR_BAD_ARG, "b200_yolo_decode_nms: head_dtype %d is not a B200_DTYPE_* code", head_dtype);
   B200_REQUIRE(heads && hw && anchors_wh_host && image_wh_host, B200_ERR_BAD_ARG, "b200_yolo_decode_nms: null argument");
   B200_REQUIRE(B >= 0 && A >= 1 && A <= 8 && C >= 1 && C <= 1019, B200_ERR_BAD_ARG,
                "b200_yolo_decode_nms: unsupported shape B=%d A=%d C=%d", B, A, C);
@@ -449,30 +508,15 @@ extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t h
     dp.conf_lo = (float)(t - d); dp.conf_hi = (float)(t + d);
   }
   dp.st = cand_bind(ws, wsb, out_sel_idx != nullptr);
-  B200_CUDA(cudaMemsetAsync(wsb, 0, ws.zeroed(out_sel_idx != nullptr), stream));
-
   using Ring = WarpSlabRing<YD_STAGES>;
+  const int rec_bytes = dp.RF * b200_dtype_bytes(head_dtype);
   int warps = 16;  // one tile in flight per warp; the warps of an SM overlap each other's loads
-  while (warps > 1 && Ring::smem_bytes(warps, dp.RF) > 200 * 1024) warps >>= 1;
+  while (warps > 1 && Ring::smem_bytes(warps, rec_bytes) > 200 * 1024) warps >>= 1;
   // a single image has fewer tiles than the GPU has warp slots: spread them (one warp per scheduler finishes its tile sooner)
   while (warps > 2 && dp.lv.tile_base[YD_MAX_LEVELS] <= (long long)(warps / 2) * b200_sm_count()) warps >>= 1;
-  const size_t smem1 = Ring::smem_bytes(warps, dp.RF);
+  const size_t smem1 = Ring::smem_bytes(warps, rec_bytes);
   B200_REQUIRE(smem1 <= 220 * 1024, B200_ERR_UNSUPPORTED, "b200_yolo_decode_nms: record too large (C=%d)", C);
-
-  const long long n_tiles = dp.lv.tile_base[YD_MAX_LEVELS];
-  const int grid = Ring::grid(n_tiles, warps, b200_sm_count());
-  // Refilling a warp's slab before its append keeps one more copy in flight: -3 % for the call on its own at any size, and
-  // for the fused evaluation step at 512 images; at 64 images per GPU the same step is 3 % SLOWER with it (the filter then
-  // takes DRAM bandwidth from the loss chain that shares the GPU, and that chain is the longer one there).  Long streams
-  // (>= 32 tiles per warp) refill early, short ones late.
-  if (n_tiles >= 32ll * grid * warps) {
-    B200_CUDA(cudaFuncSetAttribute(yolo_decode_filter_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-    yolo_decode_filter_kernel<true><<<grid, warps * 32, smem1, stream>>>(dp);
-  } else {
-    B200_CUDA(cudaFuncSetAttribute(yolo_decode_filter_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-    yolo_decode_filter_kernel<false><<<grid, warps * 32, smem1, stream>>>(dp);
-  }
-  B200_LAUNCH_CHECK();
+  B200_CUDA(cudaMemsetAsync(wsb, 0, ws.zeroed(out_sel_idx != nullptr), stream));
 
   YoloFinalizeParams fp;
   fp.lv = dp.lv; fp.B = B; fp.A = A; fp.C = C; fp.RF = dp.RF; fp.st = dp.st;
@@ -480,30 +524,19 @@ extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t h
   fp.cfg.use_score_thr = 0; fp.cfg.max_out = max_out;
   fp.out_boxes = out_boxes; fp.out_cls = out_class_id; fp.out_score = out_score; fp.out_classes = out_classes;
   fp.out_conf = out_conf; fp.out_sel_idx = out_sel_idx; fp.out_sel_anchor = out_sel_anchor; fp.out_count = out_count;
-  // one 1024-thread CTA per SM gives the lowest latency; batches that need more than one wave use 512-thread CTAs,
-  // two per SM (the shared-memory footprint allows it up to max_out ~ 500)
-  const size_t smem2 = cand_finalize_smem_bytes(fp.st, max_out);
-  const bool half_ctas = (B > b200_sm_count()) && (2 * (smem2 + 1024) <= 227 * 1024);
-#define YD_LAUNCH(M)                                                                                                   \
-  if (half_ctas) {                                                                                                          \
-    B200_CUDA(cudaFuncSetAttribute(yolo_nms_finalize_kernel<M, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2)); \
-    yolo_nms_finalize_kernel<M, 512><<<B, 512, smem2, stream>>>(fp);                                                         \
-  } else {                                                                                                                  \
-    B200_CUDA(cudaFuncSetAttribute(yolo_nms_finalize_kernel<M, NMS_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2)); \
-    yolo_nms_finalize_kernel<M, NMS_THREADS><<<B, NMS_THREADS, smem2, stream>>>(fp);                                         \
-  }
-  NMS_DISPATCH_METRIC(metric, YD_LAUNCH)
-#undef YD_LAUNCH
-  B200_LAUNCH_CHECK();
-  if (out_classes) {
-    const long long rows = (long long)B * max_out;
-    // half a warp per row when that leaves fewer idle lanes in the last round (80 classes: 5 x 16 against 3 x 32)
-    // (a few hundred rows are latency-bound: a full warp per row has the shorter chain)
-    if (rows >= 16384 && ((C + 15) / 16) * 16 < ((C + 31) / 32) * 32) yolo_classes_kernel<16><<<(int)((rows + 15) / 16), 256, 0, stream>>>(fp);
-    else yolo_classes_kernel<32><<<(int)((rows + 7) / 8), 256, 0, stream>>>(fp);
-    B200_LAUNCH_CHECK();
-  }
+  B200_DISPATCH_DTYPE(head_dtype, T, return yd_launch<T>(dp, fp, metric, warps, smem1, stream))
   return B200_OK;
+}
+
+extern "C" int b200_yolo_decode_nms(const float* const heads[3], const int32_t hw[6], int B, int A, int C,
+                                    const float* anchors_wh_host, const float* image_wh_host, float conf_thr,
+                                    float score_thr, float iou_thr, int metric, int max_out, float* out_boxes,
+                                    int32_t* out_class_id, float* out_score, float* out_classes, float* out_conf,
+                                    int32_t* out_sel_idx, int32_t* out_sel_anchor, int32_t* out_count,
+                                    void* workspace, size_t workspace_bytes, void* stream_) {
+  return b200_yolo_decode_nms_typed(reinterpret_cast<const void* const*>(heads), B200_DTYPE_F32, hw, B, A, C, anchors_wh_host, image_wh_host, conf_thr,
+                                    score_thr, iou_thr, metric, max_out, out_boxes, out_class_id, out_score, out_classes,
+                                    out_conf, out_sel_idx, out_sel_anchor, out_count, workspace, workspace_bytes, stream_);
 }
 
 extern "C" int b200_yolo_decode_dense(const float* head, int B, int H, int W, int A, int C,
