@@ -442,6 +442,8 @@ def main():
 
     if any(want(n) for n in ("c1_half", "c3_half_post", "c4_half")):
         _half_heads(args, dev, g, anc, tyu, Anchors, synth, report, wrap, want)
+    if want("c2_half_train"):
+        _half_train(args, dev, g, anc, tyu, DataGenerator, synth, report, wrap)
 
 
 def _half_heads(args, dev, g, anc, tyu, Anchors, synth, report, wrap, want):
@@ -526,6 +528,94 @@ def _half_heads(args, dev, g, anc, tyu, Anchors, synth, report, wrap, want):
             [rel, cls], call, n_anchor * (81 * 4 + 16 + 16), n_anchor * (81 * 2 + 8 + 16), same)
         del rel, cls
         torch.cuda.empty_cache()
+
+
+def _half_train(args, dev, g, anc, tyu, DataGenerator, synth, report, wrap):
+    """The YOLO training step from box lists (GetLossFromBoxesAndGrad, 'ciou') on YOLOv4 608 B=64 heads in fp32, bf16
+    and fp16, each writing its gradient in the heads' type (fp16 with a device loss scale), against "bf16 cast to fp32,
+    fp32 call, gradients cast back to bf16" (what a mixed-precision user does with an fp32-only loss).  Beside them a
+    dense GetLossAndGrad pair and a forward-only GetLossFromBoxes pair.  The heads hold bf16 values that fp16 also holds
+    exactly, so every arm's loss and parts have the same bits and every gradient is round(g32 * s) of the fp32 arm's
+    g32: asserted before anything is timed.  7 windows per arm, alternating, the order rotated window by window."""
+    import torch
+    card = _card()
+    batch, image, C = 64, 608, 80
+    grids = synth.yolo_grids(image)
+    rec = sum(s * s * 3 for s in grids)
+    f32 = []
+    for s in grids:
+        # N(0, 1) logits as the headline's heads (synth.yolo_heads), rounded to bf16
+        x = torch.randn((batch, s, s, 3 * (5 + C)), device=dev, generator=g).to(torch.bfloat16).float()
+        x[x.abs() < 1e-4] = 0.0   # below fp16's normal range a bf16 value may not be exact in fp16
+        f32.append(x)
+    heads = {"fp32": f32, "bf16": [t.to(torch.bfloat16) for t in f32], "fp16": [t.to(torch.float16) for t in f32]}
+    assert all(torch.equal(a.float(), b) for k in ("bf16", "fp16") for a, b in zip(heads[k], f32))
+    rng = np.random.default_rng(20261018 + 2)
+    boxes, classes, off = (torch.from_numpy(a).to(dev) for a in synth.gt_batch(rng, batch, (image, image), max_boxes=100))
+    y_true = DataGenerator(C, anc, (image, image)).GetTargetsBatch(classes, boxes, off)
+    scale = torch.full((1,), 1024.0, dtype=torch.float32, device=dev)   # fp16 loss scale, read on the device
+    box_args = (classes, boxes, off)
+    kw = dict(iou_thresh=0.5, iou_type="ciou", return_parts=True)
+
+    def train(h, **gkw):
+        return tyu.GetLossFromBoxesAndGrad(*box_args, h, (image, image), anc, C, **kw, **gkw)
+
+    def cast_then_fp32():
+        loss, parts, grads = train([t.float() for t in heads["bf16"]])
+        return loss, parts, [t.to(torch.bfloat16) for t in grads]
+
+    def dense(h):
+        loss, parts, grads = tyu._loss_call(y_true, h, (image, image), anc, 0.5, "ciou", 0, return_parts=True, with_grad=True,
+                                            grad_dtype=h[0].dtype)
+        return loss, parts, grads
+
+    fns = {
+        "fp32": lambda: train(heads["fp32"]),
+        "bf16": lambda: train(heads["bf16"], grad_dtype=torch.bfloat16),
+        "fp16_scaled": lambda: train(heads["fp16"], grad_dtype=torch.float16, grad_scale=scale),
+        "bf16_cast_then_fp32": cast_then_fp32,
+        "dense_fp32": lambda: dense(heads["fp32"]),
+        "dense_bf16": lambda: dense(heads["bf16"]),
+        "forward_fp32": lambda: tyu.GetLossFromBoxes(*box_args, heads["fp32"], (image, image), anc, C, **kw),
+        "forward_bf16": lambda: tyu.GetLossFromBoxes(*box_args, heads["bf16"], (image, image), anc, C, **kw),
+    }
+    def same(a, b):   # bit equality, NaN positions equal (payloads not compared)
+        a, b = a.float(), b.float()
+        return torch.equal(torch.isnan(a), torch.isnan(b)) and torch.equal(torch.nan_to_num(a).view(torch.int32),
+                                                                           torch.nan_to_num(b).view(torch.int32))
+
+    def check(name, got, ref, s, dt):
+        assert same(got[0], ref[0]) and same(got[1], ref[1]), "%s: loss bits differ from the fp32 arm" % name
+        for a, b in zip(got[2], ref[2]):
+            assert a.dtype == dt and same(a, (b if s is None else b * s).to(dt)), "%s: gradient bits differ" % name
+
+    ref = fns["fp32"]()
+    check("bf16", fns["bf16"](), ref, None, torch.bfloat16)
+    check("fp16_scaled", fns["fp16_scaled"](), ref, 1024.0, torch.float16)
+    check("bf16_cast_then_fp32", fns["bf16_cast_then_fp32"](), ref, None, torch.bfloat16)
+    dref = fns["dense_fp32"]()
+    check("dense_bf16", fns["dense_bf16"](), dref, None, torch.bfloat16)
+    fref, fh = fns["forward_fp32"](), fns["forward_bf16"]()
+    assert same(fh[0], fref[0]) and same(fh[1], fref[1]), "forward: loss bits differ between the arms"
+    del ref, dref, fref, fh
+    fns = {k: wrap(f) for k, f in fns.items()}
+    steps, n_win = max(args.steps, 20), 7
+    times = {k: [] for k in fns}
+    order = list(fns)
+    for w in range(n_win):
+        for k in order[w % len(order):] + order[:w % len(order)]:
+            times[k].append(timed(fns[k], steps, args.warmup))
+    ms = {k: float(np.median(v)) for k, v in times.items()}
+    elems = rec * (5 + C)
+    report("c2_half_train", "YOLOv4 608 B=64 GetLossFromBoxesAndGrad('ciou') from bf16 / fp16 heads, gradient in the heads' type; "
+           "arms bit-identical (asserted); median of %d alternating windows of %d steps" % (n_win, steps), batch, ms["bf16"],
+           elems * 4,
+           dict(card, arms_ms=ms,
+                algorithmic_bytes_per_image_by_type={"fp32": elems * 8, "half": elems * 4,
+                                             "what": "y_pred read (dense equivalent) + gradient written"},
+                speedup_bf16_vs_cast_then_fp32=ms["bf16_cast_then_fp32"] / ms["bf16"],
+                speedup_bf16_vs_fp32=ms["fp32"] / ms["bf16"], speedup_fp16_vs_fp32=ms["fp32"] / ms["fp16_scaled"],
+                window_ms={k: [round(t, 5) for t in v] for k, v in times.items()}, outputs_bit_identical=True))
 
 
 if __name__ == "__main__":

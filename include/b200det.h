@@ -45,9 +45,10 @@ enum {
   B200_METRIC_COUNT = 7
 };
 
-/* Element type of the head tensors that the *_typed post-processing entries read.  bf16 and fp16 heads (Keras
- * mixed_bfloat16 / mixed_float16, torch autocast) are read in place and widened to fp32 exactly on load: every output
- * is bit-identical to the fp32 entry on the widened tensors.  Outputs, decoded boxes and workspaces stay fp32. */
+/* Element type of the head tensors that the *_typed post-processing and YOLO loss entries read.  bf16 and fp16 heads
+ * (Keras mixed_bfloat16 / mixed_float16, torch autocast) are read in place and widened to fp32 exactly on load: every
+ * output is bit-identical to the fp32 entry on the widened tensors.  Outputs, decoded boxes and workspaces stay fp32,
+ * except the gradient of the typed YOLO loss entries, which is written in the element type the caller asks for. */
 enum { B200_DTYPE_F32 = 0, B200_DTYPE_BF16 = 1, B200_DTYPE_F16 = 2 };
 
 /* NMS survivor predicate. */
@@ -142,6 +143,13 @@ int b200_yolo_loss(const float* const y_true[3], const float* const y_pred[3], c
                    int C, const float* anchors_wh_host, const float* image_wh_host, float iou_thresh, int metric,
                    int variant, float batch_divisor, float* out_parts, float* out_loss, unsigned char* out_ignore,
                    void* workspace, size_t workspace_bytes, void* stream);
+/* b200_yolo_loss on y_pred of element type pred_dtype (B200_DTYPE_*; all three levels share it).  y_true, out_ignore,
+ * parts, loss and the workspace stay fp32 and the same size; b200_yolo_loss is the B200_DTYPE_F32 case.  Every argument
+ * is checked before anything is enqueued. */
+int b200_yolo_loss_typed(const float* const y_true[3], const void* const y_pred[3], int pred_dtype, const int32_t hw[6],
+                         int B, int A, int C, const float* anchors_wh_host, const float* image_wh_host, float iou_thresh,
+                         int metric, int variant, float batch_divisor, float* out_parts, float* out_loss,
+                         unsigned char* out_ignore, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Measurement hook: b200_yolo_loss restricted to a subset of its four launches (bit 0 object scan, 1 GT preparation,
  * 2 ignore mask + object terms, 3 finalize); the workspace carries the state, stages must be issued in order. */
@@ -159,6 +167,19 @@ int b200_yolo_loss_grad(const float* const y_true[3], const float* const y_pred[
                         int C, const float* anchors_wh_host, const float* image_wh_host, float iou_thresh, int metric,
                         int variant, float batch_divisor, float* out_parts, float* out_loss, float* const out_grad[3],
                         void* workspace, size_t workspace_bytes, void* stream);
+/* b200_yolo_loss_grad on y_pred of element type pred_dtype, writing out_grad (16-byte aligned levels) in element type
+ * grad_dtype (B200_DTYPE_*, each shared by the three levels).  Each gradient element is round(g * s) with one rounding
+ * to nearest even (fp16 overflow gives +-inf), where g is the fp32 gradient of b200_yolo_loss_grad on the widened
+ * y_pred and s = *grad_scale_dev: a device fp32 scalar, e.g. a loss scale (torch GradScaler._scale, a Keras
+ * LossScaleOptimizer variable through DLPack), so the call stays free of host synchronisation and graph-capturable with
+ * a scale that changes between steps.  grad_scale_dev NULL: no multiply (s = 1).  The scale is meant to be finite and
+ * positive: the zero elements are stored as +0 without the multiply.  b200_yolo_loss_grad is the (F32, F32, NULL) case;
+ * every argument is checked before anything is enqueued. */
+int b200_yolo_loss_grad_typed(const float* const y_true[3], const void* const y_pred[3], int pred_dtype, const int32_t hw[6],
+                              int B, int A, int C, const float* anchors_wh_host, const float* image_wh_host, float iou_thresh,
+                              int metric, int variant, float batch_divisor, float* out_parts, float* out_loss,
+                              void* const out_grad[3], int grad_dtype, const float* grad_scale_dev, void* workspace,
+                              size_t workspace_bytes, void* stream);
 
 /* Sparse-target fusion (SURVEY §8f N3; an API extension, no reference signature): DataGenerator.GetTargets
  * (datasets/coco_dataset.py:185-285) followed by GetLoss (utils/tf_yolo_utils.py:6-127) without materialising the
@@ -173,6 +194,13 @@ int b200_yolo_loss_from_boxes(const float* boxes, const int32_t* classes, const 
                               float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
                               float* out_loss, unsigned char* out_ignore, void* workspace, size_t workspace_bytes,
                               void* stream);
+/* b200_yolo_loss_from_boxes on y_pred of element type pred_dtype, as b200_yolo_loss_typed is to b200_yolo_loss. */
+int b200_yolo_loss_from_boxes_typed(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
+                                    const float* assign_anchors_wh_host, const void* const y_pred[3], int pred_dtype,
+                                    const int32_t hw[6], int B, int A, int C, const float* anchors_wh_host,
+                                    const float* image_wh_host, float iou_thresh, int metric, int variant, float batch_divisor,
+                                    float* out_parts, float* out_loss, unsigned char* out_ignore, void* workspace,
+                                    size_t workspace_bytes, void* stream);
 
 /* b200_yolo_loss_from_boxes forward + the analytic backward of b200_yolo_loss_grad, still without a dense y_true:
  * out_grad[l] (B,H_l,W_l,A*(5+C)), 16-byte aligned, = d loss / d y_pred[l] for an upstream gradient of 1, bit-identical
@@ -185,6 +213,15 @@ int b200_yolo_loss_from_boxes_grad(const float* boxes, const int32_t* classes, c
                                    float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
                                    float* out_loss, float* const out_grad[3], void* workspace, size_t workspace_bytes,
                                    void* stream);
+/* b200_yolo_loss_from_boxes_grad on y_pred of element type pred_dtype, the gradient in element type grad_dtype scaled by
+ * *grad_scale_dev, as b200_yolo_loss_grad_typed is to b200_yolo_loss_grad. */
+int b200_yolo_loss_from_boxes_grad_typed(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
+                                         const float* assign_anchors_wh_host, const void* const y_pred[3], int pred_dtype,
+                                         const int32_t hw[6], int B, int A, int C, const float* anchors_wh_host,
+                                         const float* image_wh_host, float iou_thresh, int metric, int variant,
+                                         float batch_divisor, float* out_parts, float* out_loss, void* const out_grad[3],
+                                         int grad_dtype, const float* grad_scale_dev, void* workspace, size_t workspace_bytes,
+                                         void* stream);
 
 /* DataGenerator.GetTargets (datasets/coco_dataset.py:185-285), batched: boxes [total,4] pixel corners
  * x1,y1,x2,y2, classes [total] int32, offsets [B+1] int32 (all device).  targets[l]: (B,H_l,W_l,A,5+C), zeroed

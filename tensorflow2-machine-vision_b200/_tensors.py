@@ -29,26 +29,32 @@ def to_cuda(x, dtype=torch.float32):
     return t.contiguous()
 
 
-# element-type codes of the C ABI (B200_DTYPE_*) for the head dtypes the post-processing reads in place
+# element-type codes of the C ABI (B200_DTYPE_*) for the head dtypes the post-processing and the YOLO loss read in place
 DTYPE_F32 = 0
 _HALF_CODES = {torch.bfloat16: 1, torch.float16: 2}
+DTYPE_CODES = {torch.float32: DTYPE_F32, **_HALF_CODES}
 
 
-def to_cuda_heads(xs):
+def to_cuda_heads(xs, keep_pinned=False):
     """The levels of one head family (YOLO heads, EfficientDet box tensors or class logits) -> (contiguous CUDA tensors,
     B200_DTYPE_* code).  A family that is all bf16 or all fp16 stays in its type: the kernels widen each element to fp32
     exactly, so the results are those of the fp32 call on the widened tensors, without a cast pass or an fp32 copy.
-    Any other family is cast to fp32 as to_cuda does."""
+    Any other family is cast to fp32 as to_cuda does.  keep_pinned: the caller's torch tensors in page-locked host memory
+    (is_pinned_host_f32) that already have the family's type are returned as they are, for kernels that read them in
+    place."""
+    require_cuda()
     ts = [_as_tensor(x) for x in xs]
     code = _HALF_CODES.get(ts[0].dtype) if ts else None
-    if code is not None and all(t.dtype == ts[0].dtype for t in ts):
-        return [to_cuda(t, t.dtype) for t in ts], code
-    return [to_cuda(t) for t in ts], DTYPE_F32
+    if code is None or not all(t.dtype == ts[0].dtype for t in ts):
+        code = DTYPE_F32
+    dtype = ts[0].dtype if code != DTYPE_F32 else torch.float32
+    keep = lambda x, t: keep_pinned and t is x and t.dtype == dtype and is_pinned_host_f32(t)
+    return [t if keep(x, t) else to_cuda(t, dtype) for x, t in zip(xs, ts)], code
 
 
 def is_pinned_host_f32(x):
-    """A contiguous fp32 torch tensor in page-locked host memory: device kernels can read it in place (UVA)."""
-    return (isinstance(x, torch.Tensor) and not x.is_cuda and x.dtype == torch.float32 and x.is_contiguous()
+    """A contiguous fp32, bf16 or fp16 torch tensor in page-locked host memory: device kernels can read it in place (UVA)."""
+    return (isinstance(x, torch.Tensor) and not x.is_cuda and x.dtype in DTYPE_CODES and x.is_contiguous()
             and x.is_pinned() and torch.cuda.is_available())
 
 

@@ -154,20 +154,56 @@ def GetNMSBoxes(y1, y2, y3, anchors_wh, image_wh, classes_num,
   return pick(r['boxes']), pick(r['classes_id']), pick(r['scores']), pick(r['classes']), pick(r['confidence'])
 
 
+def _pred_levels(y_pred, with_grad):
+  '''y_pred of the loss -> (3 tensors, B200_DTYPE_* code).  All three levels bf16, or all fp16, are read in place in their
+  type (the loss, parts, ignore mask and fp32 gradient are bit-identical to the call on y.float()); any other mix is cast
+  to fp32.  y_pred in pinned host memory is consumed in place by the forward (unified addressing): the forward kernels
+  need only the five box/conf logits of every record and the object records, ~6 % of the tensor, so fetching those
+  sectors over PCIe beats copying the whole tensor first (9.2 -> 3.1 ms at 608x608 batch 64).  The backward pass needs
+  device tensors.'''
+  if len(y_pred) != 3:
+    raise ValueError('y_pred must hold 3 levels')
+  return T.to_cuda_heads(y_pred, keep_pinned=not with_grad)
+
+
+def _grad_code(grad_dtype):
+  '''B200_DTYPE_* code of a gradient dtype (checked before anything touches the device).'''
+  code = T.DTYPE_CODES.get(grad_dtype)
+  if code is None:
+    raise ValueError('grad_dtype must be torch.float32, torch.bfloat16 or torch.float16, not %r' % (grad_dtype,))
+  return code
+
+
+def _grad_out(yp, grad_dtype, grad_scale):
+  '''The gradient tensors (shaped like y_pred, of grad_dtype) and the scale tensor (1-element fp32 on y_pred's device, or
+  None) of a backward call, and the gradient's B200_DTYPE_* code.'''
+  code = _grad_code(grad_dtype)
+  dev = yp[0].device
+  if grad_scale is not None and not isinstance(grad_scale, torch.Tensor):
+    grad_scale = torch.full((1,), float(grad_scale), dtype=torch.float32, device=dev)
+  if grad_scale is not None and (grad_scale.dtype != torch.float32 or grad_scale.numel() != 1 or grad_scale.device != dev):
+    raise ValueError('grad_scale must be a 1-element float32 tensor on %s, or a Python float' % dev)
+  grads = [torch.empty(t.shape, dtype=grad_dtype, device=dev) for t in yp]
+  return grads, code, grad_scale
+
+
 def _loss_call(y_true, y_pred, image_wh, anchors_wh, iou_thresh, iou_type, variant, batch_divisor=None,
-               return_parts=False, workspace=None, ignore_out=None, with_grad=False, exchange=None, defer_collect=False):
+               return_parts=False, workspace=None, ignore_out=None, with_grad=False, exchange=None, defer_collect=False,
+               grad_dtype=torch.float32, grad_scale=None):
   """exchange: a runtime.PeerExchange (the 12 terms are summed over the ranks inside the finalize kernel, NVLink peer
   stores) or a runtime.NcclExchange (b200_allreduce_loss + b200_yolo_loss_combine behind the loss); batch_divisor must
   then be the GLOBAL batch.  Forward only.  defer_collect (PeerExchange only): the call ends with the publish half of the
-  exchange and returns this rank's own terms; exchange.collect_yolo(parts, loss) on another stream finishes it."""
+  exchange and returns this rank's own terms; exchange.collect_yolo(parts, loss) on another stream finishes it.
+  y_pred: see _pred_levels; a PeerExchange call reads fp32 only (half levels are cast)."""
   lib = _lib.load()
   if len(y_true) != 3 or len(y_pred) != 3:
     raise ValueError('y_true and y_pred must each hold 3 levels')
+  if with_grad:
+    _grad_code(grad_dtype)
   yt = [T.to_cuda(t) for t in y_true]
-  # y_pred in pinned host memory is consumed in place (unified addressing): the forward kernels need only the five
-  # box/conf logits of every record and the object records, ~6 % of the tensor, so fetching those sectors over PCIe
-  # beats copying the whole tensor first (9.2 -> 3.1 ms at 608x608 batch 64).  The backward pass needs device tensors.
-  yp = [t if (not with_grad and T.is_pinned_host_f32(t)) else T.to_cuda(t) for t in y_pred]
+  yp, pdt = _pred_levels(y_pred, with_grad)
+  if pdt != T.DTYPE_F32 and exchange is not None and hasattr(exchange, 'mailboxes'):
+    yp, pdt = [T.to_cuda(t) for t in yp], T.DTYPE_F32   # the fused-exchange entries read fp32 heads
   anc = T.host_floats(anchors_wh)
   if anc.size % 6 != 0:
     raise ValueError('anchors_wh must be (3, anchors_num, 2)')
@@ -191,12 +227,12 @@ def _loss_call(y_true, y_pred, image_wh, anchors_wh, iou_thresh, iou_type, varia
     workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
   div = float(B if batch_divisor is None else batch_divisor)
   if with_grad:
-    grads = [torch.empty_like(t) for t in yp]
+    grads, gdt, scale = _grad_out(yp, grad_dtype, grad_scale)
     gp = (ctypes.c_void_p * 3)(*[t.data_ptr() for t in grads])
-    _lib.check(lib.b200_yolo_loss_grad(tp, pp, hw, B, A, RF - 5, anc.ctypes.data_as(ctypes.c_void_p),
-                                       img.ctypes.data_as(ctypes.c_void_p), float(iou_thresh),
-                                       _lib.METRIC_YOLO[iou_type], variant, div, T.ptr(parts), T.ptr(loss), gp,
-                                       T.ptr(workspace), ws_bytes, T.stream_ptr()), 'GetLoss')
+    _lib.check(lib.b200_yolo_loss_grad_typed(tp, pp, pdt, hw, B, A, RF - 5, anc.ctypes.data_as(ctypes.c_void_p),
+                                             img.ctypes.data_as(ctypes.c_void_p), float(iou_thresh),
+                                             _lib.METRIC_YOLO[iou_type], variant, div, T.ptr(parts), T.ptr(loss), gp, gdt,
+                                             T.ptr(scale), T.ptr(workspace), ws_bytes, T.stream_ptr()), 'GetLoss')
     return loss, parts, grads
   if exchange is not None and hasattr(exchange, 'mailboxes'):
     rank, world, boxes_ = exchange.args()
@@ -206,10 +242,10 @@ def _loss_call(y_true, y_pred, image_wh, anchors_wh, iou_thresh, iou_type, varia
                                      variant, div, T.ptr(parts), T.ptr(loss), T.ptr(workspace), ws_bytes, rank, world, boxes_,
                                      T.stream_ptr()), 'GetLoss (data parallel)')
     return (loss, parts) if return_parts else loss
-  _lib.check(lib.b200_yolo_loss(tp, pp, hw, B, A, RF - 5, anc.ctypes.data_as(ctypes.c_void_p),
-                                img.ctypes.data_as(ctypes.c_void_p), float(iou_thresh), _lib.METRIC_YOLO[iou_type],
-                                variant, div, T.ptr(parts), T.ptr(loss), T.ptr(ignore_out), T.ptr(workspace), ws_bytes,
-                                T.stream_ptr()),
+  _lib.check(lib.b200_yolo_loss_typed(tp, pp, pdt, hw, B, A, RF - 5, anc.ctypes.data_as(ctypes.c_void_p),
+                                      img.ctypes.data_as(ctypes.c_void_p), float(iou_thresh), _lib.METRIC_YOLO[iou_type],
+                                      variant, div, T.ptr(parts), T.ptr(loss), T.ptr(ignore_out), T.ptr(workspace), ws_bytes,
+                                      T.stream_ptr()),
              'GetLoss')
   if exchange is not None:  # NCCL transport: all-reduce the 12 terms in place, then the reference's order of additions
     exchange.allreduce_(parts)
@@ -253,7 +289,8 @@ def GetLossFromBoxes(classes, boxes, offsets, y_pred, image_wh, anchors_wh, clas
 
 
 def GetLossFromBoxesAndGrad(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_num, iou_thresh=0.5, iou_type='iou',
-                            target_anchors=None, batch_divisor=None, return_parts=False, workspace=None):
+                            target_anchors=None, batch_divisor=None, return_parts=False, workspace=None,
+                            grad_dtype=torch.float32, grad_scale=None):
   '''GetLossFromBoxes plus d loss / d y_pred (list of 3 tensors shaped like y_pred) for an upstream gradient of 1: the
   training step of the sparse-target path.  Gradients bit-identical to
   GetLossAndGrad(DataGenerator(classes_num, target_anchors, image_wh).GetTargetsBatch(classes, boxes, offsets), y_pred, ...).
@@ -261,21 +298,27 @@ def GetLossFromBoxesAndGrad(classes, boxes, offsets, y_pred, image_wh, anchors_w
 
   Data parallel: each rank passes its own images with batch_divisor = the global batch.  The gradients need no exchange;
   the (3,4) parts go through combine_loss_parts (or any all-reduce + b200_yolo_loss_combine) for the global loss.
-  Wrap with tf.custom_gradient (INTEGRATION.md §3).'''
+  Wrap with tf.custom_gradient (INTEGRATION.md §3).
+
+  Mixed precision: y_pred levels that are all bf16 or all fp16 are read in place.  grad_dtype (torch.float32, the
+  default, torch.bfloat16 or torch.float16) is the type the gradients are written in, each element rounded once from
+  g * grad_scale, where g is the fp32 gradient of the call on y.float().  grad_scale: None (no multiply), a 1-element
+  float32 tensor on the device (e.g. a loss scale that changes between steps: no host synchronisation, graph
+  capturable) or a Python float.'''
   assert iou_type in ['iou','diou','ciou']
   loss, parts, grads = _boxes_call(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_num, iou_thresh, iou_type,
-                                   target_anchors, batch_divisor, workspace, with_grad=True)
+                                   target_anchors, batch_divisor, workspace, with_grad=True, grad_dtype=grad_dtype,
+                                   grad_scale=grad_scale)
   return (loss, parts, grads) if return_parts else (loss, grads)
 
 
 def _boxes_call(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_num, iou_thresh, iou_type, target_anchors,
-                batch_divisor, workspace, ignore_out=None, with_grad=False):
+                batch_divisor, workspace, ignore_out=None, with_grad=False, grad_dtype=torch.float32, grad_scale=None):
   '''Argument checks and marshalling of the sparse-target entries.  Returns (loss, parts, grads or None).'''
   lib = _lib.load()
-  # pinned host predictions are read in place by the forward; the backward needs device tensors
-  yp = [t if (not with_grad and T.is_pinned_host_f32(t)) else T.to_cuda(t) for t in y_pred]
-  if len(yp) != 3:
-    raise ValueError('y_pred must hold 3 levels')
+  if with_grad:
+    _grad_code(grad_dtype)
+  yp, pdt = _pred_levels(y_pred, with_grad)
   boxes = T.to_cuda(boxes).reshape(-1, 4)
   classes = T.to_cuda(classes, torch.int32).reshape(-1)
   offsets = T.to_cuda(offsets, torch.int32).reshape(-1)
@@ -303,19 +346,21 @@ def _boxes_call(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_n
     workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
   div = float(B if batch_divisor is None else batch_divisor)
   if with_grad:
-    grads = [torch.empty_like(t) for t in yp]
+    grads, gdt, scale = _grad_out(yp, grad_dtype, grad_scale)
     gp = (ctypes.c_void_p * 3)(*[t.data_ptr() for t in grads])
-    _lib.check(lib.b200_yolo_loss_from_boxes_grad(T.ptr(boxes), T.ptr(classes), T.ptr(offsets), total,
-                                                  tanc.ctypes.data_as(ctypes.c_void_p), pp, hw, B, A, RF - 5,
-                                                  anc.ctypes.data_as(ctypes.c_void_p), img.ctypes.data_as(ctypes.c_void_p),
-                                                  float(iou_thresh), _lib.METRIC_YOLO[iou_type], 0, div, T.ptr(parts), T.ptr(loss),
-                                                  gp, T.ptr(workspace), workspace.numel(), T.stream_ptr()), 'GetLossFromBoxesAndGrad')
+    _lib.check(lib.b200_yolo_loss_from_boxes_grad_typed(T.ptr(boxes), T.ptr(classes), T.ptr(offsets), total,
+                                                        tanc.ctypes.data_as(ctypes.c_void_p), pp, pdt, hw, B, A, RF - 5,
+                                                        anc.ctypes.data_as(ctypes.c_void_p), img.ctypes.data_as(ctypes.c_void_p),
+                                                        float(iou_thresh), _lib.METRIC_YOLO[iou_type], 0, div, T.ptr(parts),
+                                                        T.ptr(loss), gp, gdt, T.ptr(scale), T.ptr(workspace), workspace.numel(),
+                                                        T.stream_ptr()), 'GetLossFromBoxesAndGrad')
     return loss, parts, grads
-  _lib.check(lib.b200_yolo_loss_from_boxes(T.ptr(boxes), T.ptr(classes), T.ptr(offsets), total,
-                                           tanc.ctypes.data_as(ctypes.c_void_p), pp, hw, B, A, RF - 5,
-                                           anc.ctypes.data_as(ctypes.c_void_p), img.ctypes.data_as(ctypes.c_void_p),
-                                           float(iou_thresh), _lib.METRIC_YOLO[iou_type], 0, div, T.ptr(parts), T.ptr(loss),
-                                           T.ptr(ignore_out), T.ptr(workspace), workspace.numel(), T.stream_ptr()), 'GetLossFromBoxes')
+  _lib.check(lib.b200_yolo_loss_from_boxes_typed(T.ptr(boxes), T.ptr(classes), T.ptr(offsets), total,
+                                                 tanc.ctypes.data_as(ctypes.c_void_p), pp, pdt, hw, B, A, RF - 5,
+                                                 anc.ctypes.data_as(ctypes.c_void_p), img.ctypes.data_as(ctypes.c_void_p),
+                                                 float(iou_thresh), _lib.METRIC_YOLO[iou_type], 0, div, T.ptr(parts), T.ptr(loss),
+                                                 T.ptr(ignore_out), T.ptr(workspace), workspace.numel(), T.stream_ptr()),
+             'GetLossFromBoxes')
   return loss, parts, None
 
 
@@ -344,7 +389,7 @@ def LossAndNMSBoxesBatch(y_true, y_pred, image_wh, anchors_wh, classes_num, iou_
   loss_anchors_wh: the anchors GetLoss takes when they differ in units from the ones GetNMSBoxes takes (default: the same).
   '''
   assert iou_type in ['iou','diou','ciou'] and nms_iou_type in ['iou','diou','ciou']
-  heads = [T.to_cuda(t) for t in y_pred]
+  heads, _ = T.to_cuda_heads(y_pred)   # bf16 / fp16 heads stay in their type for both branches
   dev = heads[0].device
   main = torch.cuda.current_stream(dev)
   side = _side_stream(dev)
@@ -409,7 +454,7 @@ def EvalStepFromBoxes(classes, boxes, offsets, y_pred, image_wh, anchors_wh, cla
   combine_loss_parts; the mAP is per image and needs no exchange.  CUDA-graph capturable.'''
   from .mAP import Get_mAP_padded
   assert iou_type in ['iou','diou','ciou'] and nms_iou_type in ['iou','diou','ciou']
-  heads = [T.to_cuda(t) for t in y_pred]
+  heads, _ = T.to_cuda_heads(y_pred)   # bf16 / fp16 heads stay in their type for both branches
   dev = heads[0].device
   main = torch.cuda.current_stream(dev)
   side = _side_stream(dev)
@@ -428,11 +473,14 @@ def EvalStepFromBoxes(classes, boxes, offsets, y_pred, image_wh, anchors_wh, cla
   return (loss, parts, r, m_ap) if return_parts else (loss, r, m_ap)
 
 
-def GetLossAndGrad(y_true, y_pred, image_wh, anchors_wh, iou_thresh=0.5, iou_type='iou'):
+def GetLossAndGrad(y_true, y_pred, image_wh, anchors_wh, iou_thresh=0.5, iou_type='iou', grad_dtype=torch.float32,
+                   grad_scale=None):
   '''GetLoss plus d loss / d y_pred (list of 3 tensors shaped like y_pred) for an upstream gradient of 1 —
-  what tf.GradientTape derives from the reference's GetLoss.  Wrap with tf.custom_gradient (INTEGRATION.md §3).'''
+  what tf.GradientTape derives from the reference's GetLoss.  Wrap with tf.custom_gradient (INTEGRATION.md §3).
+  Mixed precision (bf16 / fp16 y_pred, grad_dtype, grad_scale): as GetLossFromBoxesAndGrad.'''
   assert iou_type in ['iou','diou','ciou']
-  loss, _, grads = _loss_call(y_true, y_pred, image_wh, anchors_wh, iou_thresh, iou_type, 0, with_grad=True)
+  loss, _, grads = _loss_call(y_true, y_pred, image_wh, anchors_wh, iou_thresh, iou_type, 0, with_grad=True,
+                              grad_dtype=grad_dtype, grad_scale=grad_scale)
   return loss, grads
 
 

@@ -39,7 +39,8 @@ enum { YL_VARIANT_TF_YOLO_UTILS = 0, YL_VARIANT_KERAS_YOLO3 = 1 };
 
 struct YlLevels {
   const float* y_true[YL_LEVELS];
-  const float* y_pred[YL_LEVELS];
+  const void* y_pred[YL_LEVELS];       // element type pred_dtype; the kernels that read it are instantiated per type (TP)
+  int pred_dtype;                      // B200_DTYPE_*, shared by the three levels
   int h[YL_LEVELS], w[YL_LEVELS], rec_per_img[YL_LEVELS], anchor_base[YL_LEVELS];
   int chunks_per_img[YL_LEVELS];
   int cta_base[YL_LEVELS + 1];
@@ -209,6 +210,7 @@ __global__ void __launch_bounds__(YL_CHUNK) yolo_loss_scan_kernel(YlParams p) {
 // 4*YL_TERM_SPLIT.
 #define YL_TERM_SPLIT 16
 
+template <typename TP>
 __device__ __forceinline__ void yl_terms_body(const YlParams& p, int cta, double (*s_acc)[3]) {
   const int l = cta / (p.B * YL_TERM_SPLIT);
   const int rem = cta - l * (p.B * YL_TERM_SPLIT);
@@ -216,7 +218,7 @@ __device__ __forceinline__ void yl_terms_body(const YlParams& p, int cta, double
   const int rpi = p.lv.rec_per_img[l];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const float* yt = p.sp_t ? nullptr : p.lv.y_true[l] + ((size_t)img * rpi) * p.RF;
-  const float* yp = p.lv.y_pred[l] + ((size_t)img * rpi) * p.RF;
+  const TP* yp = static_cast<const TP*>(p.lv.y_pred[l]) + ((size_t)img * rpi) * p.RF;
   const int n = p.gt_count[img * YL_LEVELS + l];
   const size_t gbase = (size_t)img * p.n_img + p.lv.anchor_base[l];
   double a_xy = 0.0, a_wh = 0.0, a_cls = 0.0;
@@ -224,7 +226,7 @@ __device__ __forceinline__ void yl_terms_body(const YlParams& p, int cta, double
   for (int k = split * (YL_ICHUNK / 32) + warp; k < n; k += YL_TERM_SPLIT * (YL_ICHUNK / 32)) {
     const int r = p.obj_index[gbase + k];
     const float* t = yt + (size_t)r * p.RF;
-    const float* q = yp + (size_t)r * p.RF;
+    const TP* q = yp + (size_t)r * p.RF;
     float obj, tx, ty, tw, th;
     int sp_class = -1;
     if (p.sp_t) {  // the record the dense scatter would have written: obj = 1, one-hot class (cds:246-262)
@@ -246,7 +248,7 @@ __device__ __forceinline__ void yl_terms_body(const YlParams& p, int cta, double
       const float gs = lane == 0 ? (float)W : (float)H;
       float raw = DM_SUB(DM_MUL(tv, gs), g);
       if (p.variant == YL_VARIANT_TF_YOLO_UTILS) raw = DM_MUL(obj, raw);  // tyu:44 (absent in yolo_loss.py:120)
-      e_xy = DM_MUL(os, dm_bce_logits(raw, __ldg(q + lane)));
+      e_xy = DM_MUL(os, dm_bce_logits(raw, ldg_f32(q + lane)));
     } else if (lane < 4) {
       const int a = r - (r / p.A) * p.A;
       const float tv = lane == 2 ? tw : th;
@@ -255,13 +257,13 @@ __device__ __forceinline__ void yl_terms_body(const YlParams& p, int cta, double
       float num = DM_MUL(tv, im);
       if (p.variant == YL_VARIANT_TF_YOLO_UTILS) num = DM_ADD(num, 1e-8f);  // tyu:48
       const float raw = dm_logf(DM_DIV(num, an));
-      const float d = DM_SUB(raw, __ldg(q + lane));
+      const float d = DM_SUB(raw, ldg_f32(q + lane));
       e_wh = DM_MUL(DM_MUL(os, 0.5f), DM_MUL(d, d));
     }
     if (p.sp_t) {
-      for (int c = 5 + lane; c < p.RF; c += 32) e_cls += DM_MUL(obj, dm_bce_logits((c - 5 == sp_class) ? 1.0f : 0.0f, __ldg(q + c)));
+      for (int c = 5 + lane; c < p.RF; c += 32) e_cls += DM_MUL(obj, dm_bce_logits((c - 5 == sp_class) ? 1.0f : 0.0f, ldg_f32(q + c)));
     } else {
-      for (int c = 5 + lane; c < p.RF; c += 32) e_cls += DM_MUL(obj, dm_bce_logits(__ldg(t + c), __ldg(q + c)));
+      for (int c = 5 + lane; c < p.RF; c += 32) e_cls += DM_MUL(obj, dm_bce_logits(__ldg(t + c), ldg_f32(q + c)));
     }
     e_xy = warp_sum(e_xy); e_wh = warp_sum(e_wh); e_cls = warp_sum(e_cls);
     if (lane == 0) { a_xy += (double)e_xy; a_wh += (double)e_wh; a_cls += (double)e_cls; }
@@ -316,6 +318,51 @@ __device__ __forceinline__ void yl_rotate5(const float4 lo, const float4 hi, int
   const float a0 = s1 ? lo.y : lo.x, a1 = s1 ? lo.z : lo.y, a2 = s1 ? lo.w : lo.z, a3 = s1 ? hi.x : lo.w;
   const float a4 = s1 ? hi.y : hi.x, a5 = s1 ? hi.z : hi.y, a6 = s1 ? hi.w : hi.z;
   tx = s2 ? a2 : a0; ty = s2 ? a3 : a1; tw = s2 ? a4 : a2; th = s2 ? a5 : a3; pobj = s2 ? a6 : a4;
+}
+
+// A 2-byte element (low 16 bits of b) widened to fp32: exact, the value heads.float() holds
+template <typename TP> __device__ __forceinline__ float yl_widen16(uint32_t b);
+template <> __device__ __forceinline__ float yl_widen16<__nv_bfloat16>(uint32_t b) { return __uint_as_float(b << 16); }
+template <> __device__ __forceinline__ float yl_widen16<__half>(uint32_t b) { return __half2float(__ushort_as_half((unsigned short)b)); }
+
+// The same for 2-byte elements: a 16-byte chunk holds 8 of them, the record starts sh = 0..7 elements into lo, and hi is
+// needed (and loaded) only when sh >= 4.  The chunks travel as the bit patterns of two float4.  Word rotate by sh / 2
+// with two select stages, then a 16-bit funnel shift for odd sh.
+template <typename TP>
+__device__ __forceinline__ void yl_rotate5h(const float4 lo, const float4 hi, int sh, float& tx, float& ty, float& tw, float& th,
+                                            float& pobj) {
+  const uint32_t w0 = __float_as_uint(lo.x), w1 = __float_as_uint(lo.y), w2 = __float_as_uint(lo.z), w3 = __float_as_uint(lo.w);
+  const uint32_t w4 = __float_as_uint(hi.x), w5 = __float_as_uint(hi.y);
+  const bool s1 = sh & 2, s2 = sh & 4;
+  const uint32_t a0 = s1 ? w1 : w0, a1 = s1 ? w2 : w1, a2 = s1 ? w3 : w2, a3 = s1 ? w4 : w3, a4 = s1 ? w5 : w4;
+  const uint32_t b0 = s2 ? a2 : a0, b1 = s2 ? a3 : a1, b2 = s2 ? a4 : a2;
+  const uint32_t f = (sh & 1) ? 16u : 0u;
+  const uint32_t c0 = __funnelshift_r(b0, b1, f), c1 = __funnelshift_r(b1, b2, f), c2 = b2 >> f;
+  tx = yl_widen16<TP>(c0); ty = yl_widen16<TP>(c0 >> 16); tw = yl_widen16<TP>(c1); th = yl_widen16<TP>(c1 >> 16);
+  pobj = yl_widen16<TP>(c2);
+}
+
+// The five logits of a record from the two 16-byte chunks that cover them (lo = chunk f0 / per, hi = the next one, with
+// per = 16 / sizeof(TP) elements per chunk).  fp32: sh = f0 & 3, both chunks always inside the record (RF >= 8).
+template <typename TP>
+__device__ __forceinline__ void yl_five(const float4 lo, const float4 hi, int sh, float& tx, float& ty, float& tw, float& th,
+                                        float& pobj) {
+  if constexpr (sizeof(TP) == 4) yl_rotate5(lo, hi, sh, tx, ty, tw, th, pobj);
+  else yl_rotate5h<TP>(lo, hi, sh, tx, ty, tw, th, pobj);
+}
+
+// 2-byte elements: the second chunk of the record at element f0 is needed iff its five values cross into it, and may be
+// loaded iff it ends inside the level (total elements): with RF < 16 it reaches past the record, so for the last records
+// of a level it can reach past the tensor.  Such a record takes five scalar loads instead (yl_load5_scalar).
+template <typename TP>
+__device__ __forceinline__ bool yl_hi_needed(size_t f0) { return sizeof(TP) == 4 || (f0 & 7) >= 4; }
+template <typename TP>
+__device__ __forceinline__ bool yl_hi_inside(size_t f0, size_t total) { return sizeof(TP) == 4 || ((f0 >> 3) + 2) * 8 <= total; }
+
+template <typename TP>
+__device__ __forceinline__ void yl_load5_scalar(const TP* q, float& tx, float& ty, float& tw, float& th, float& pobj) {
+  tx = elem_f32(__ldcg(q)); ty = elem_f32(__ldcg(q + 1)); tw = elem_f32(__ldcg(q + 2)); th = elem_f32(__ldcg(q + 3));
+  pobj = elem_f32(__ldcg(q + 4));
 }
 
 // One record's object_loss = obj*bce + (1-obj)*bce*ignore (tyu:114).  Also writes the record's ignore byte and
@@ -493,9 +540,10 @@ __device__ __forceinline__ bool yl_pair_hits(const YlParams& p, int l, int rin, 
   return yl_box_hits(p, pb, yl_regular(pb), c, x);
 }
 
-// The single-kernel form.  Where a level is 16-byte aligned and a record holds at least 8 floats, two neighbouring lanes
+// The single-kernel form.  Where a level is 16-byte aligned and a record holds at least 8 elements, two neighbouring lanes
 // fetch the five logits of a record with one request (see the load section): what bounds the kernel when y_pred is read
-// in place from pinned host memory over PCIe.  Other levels load the five floats one by one.
+// in place from pinned host memory over PCIe.  Other levels load the five elements one by one.
+template <typename TP>
 __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(YlParams p) {
   __shared__ float4 s_t[YL_ICHUNK];
   __shared__ uint32_t s_q[YL_QCAP];
@@ -506,7 +554,7 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
   const int n_icta = (int)gridDim.x - n_term_cta;
   if ((int)blockIdx.x >= n_icta) {  // block-uniform
     __shared__ double s_tacc[YL_ICHUNK / 32][3];
-    yl_terms_body(p, blockIdx.x - n_icta, s_tacc);
+    yl_terms_body<TP>(p, blockIdx.x - n_icta, s_tacc);
     return;
   }
   const int icta = blockIdx.x;
@@ -520,8 +568,10 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
   const float4* gbox = p.gt_box + (size_t)img * p.n_img + p.lv.anchor_base[l];
   const float4* gaux = p.gt_aux + (size_t)img * p.n_img + p.lv.anchor_base[l];
   float obj = 0.f, tx = 0.f, ty = 0.f, tw = 0.f, th = 0.f, pobj = 0.f;
-  // block-uniform.  The two aligned 16-byte loads cover floats [f0 & ~3, (f0 & ~3) + 8): inside the tensor only when a
-  // record holds at least 8 floats (C >= 3); narrower records take the scalar path
+  // block-uniform.  The two aligned 16-byte loads cover elements [f0 & ~(per-1), (f0 & ~(per-1)) + 2 per), per = 16 /
+  // sizeof(TP): for fp32 inside the tensor only when a record holds at least 8 floats (C >= 3); narrower records take the
+  // scalar path.  2-byte elements load the second chunk only where yl_hi_needed / yl_hi_inside allow
+  constexpr int per = 16 / (int)sizeof(TP);
   const bool aligned = ((reinterpret_cast<uintptr_t>(p.lv.y_pred[l]) & 15) == 0) && (p.RF >= 8);
   if (active) obj = yl_obj(p, img, p.lv.anchor_base[l] + rin);
   if (aligned) {
@@ -530,13 +580,15 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
     // record costs one memory request (one 128-byte line, 1-2 sectors) instead of two — this halves the request count,
     // which is what bounds the kernel when y_pred is read in place from pinned host memory over PCIe
     const float4* base = reinterpret_cast<const float4*>(p.lv.y_pred[l]);
+    const size_t total = (size_t)p.B * rpi * p.RF;
     const int sub = lane & 1, rsel = lane >> 1;
     float4 ld[2];
 #pragma unroll
     for (int t = 0; t < 2; ++t) {
       const int rin_t = chunk * YL_ICHUNK + warp * 32 + 16 * t + rsel;
+      const size_t f0_t = ((size_t)img * rpi + rin_t) * p.RF;
       ld[t] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (rin_t < rpi) ld[t] = __ldcg(base + ((((size_t)img * rpi + rin_t) * p.RF) >> 2) + sub);
+      if (rin_t < rpi && (sub == 0 || (yl_hi_needed<TP>(f0_t) && yl_hi_inside<TP>(f0_t, total)))) ld[t] = __ldcg(base + f0_t / per + sub);
     }
     // lane r takes the pair loaded by lanes 2(r mod 16), 2(r mod 16)+1 of instruction r / 16
     const int src = (lane & 15) << 1;
@@ -549,10 +601,13 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
       return lane >= 16 ? v[1] : v[0];
     };
     const float4 lo = take(src), hi = take(src + 1);
-    if (active) yl_rotate5(lo, hi, (int)((((size_t)img * rpi + rin) * p.RF) & 3), tx, ty, tw, th, pobj);
+    const size_t f0 = ((size_t)img * rpi + rin) * p.RF;
+    if (active) {
+      if (yl_hi_needed<TP>(f0) && !yl_hi_inside<TP>(f0, total)) yl_load5_scalar(static_cast<const TP*>(p.lv.y_pred[l]) + f0, tx, ty, tw, th, pobj);
+      else yl_five<TP>(lo, hi, (int)(f0 % per), tx, ty, tw, th, pobj);
+    }
   } else if (active) {
-    const float* q = p.lv.y_pred[l] + ((size_t)img * rpi + rin) * p.RF;
-    tx = __ldcg(q); ty = __ldcg(q + 1); tw = __ldcg(q + 2); th = __ldcg(q + 3); pobj = __ldcg(q + 4);
+    yl_load5_scalar(static_cast<const TP*>(p.lv.y_pred[l]) + ((size_t)img * rpi + rin) * p.RF, tx, ty, tw, th, pobj);
   }
   bool hit = false;  // some GT with metric >= thr (or NaN)
   if (n_gt > 0) {    // block-uniform
@@ -610,13 +665,14 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
 #define YL_FIXED_ONE 4294967296.0  // 2^32
 
 // 10 CTAs per SM (48 registers, no spills): the fastest headline step of 8, 10, 12 and 16 (profiles/r02_ab_measurements.txt)
+template <typename TP>
 __global__ void __launch_bounds__(YL_ICHUNK, 10) yolo_loss_ignore_lean_kernel(YlParams p) {
   __shared__ double s_acc[YL_ICHUNK / 32];
   const int n_term_cta = YL_LEVELS * p.B * YL_TERM_SPLIT;
   const int n_icta = (int)gridDim.x - n_term_cta;
   if ((int)blockIdx.x >= n_icta) {  // block-uniform
     __shared__ double s_tacc[YL_ICHUNK / 32][3];
-    yl_terms_body(p, blockIdx.x - n_icta, s_tacc);
+    yl_terms_body<TP>(p, blockIdx.x - n_icta, s_tacc);
     return;
   }
   const int icta = blockIdx.x;
@@ -632,11 +688,20 @@ __global__ void __launch_bounds__(YL_ICHUNK, 10) yolo_loss_ignore_lean_kernel(Yl
   float obj = 0.f, tx = 0.f, ty = 0.f, tw = 0.f, th = 0.f, pobj = 0.f;
   if (active) {
     obj = yl_obj(p, img, p.lv.anchor_base[l] + rin);
-    // tx,ty,tw,th,conf sit at float offset f0; two aligned 16-byte loads cover them (L1 bypass)
+    // tx,ty,tw,th,conf sit at element offset f0; two aligned 16-byte loads cover them (L1 bypass).  2-byte elements: one
+    // chunk unless the five cross into the next (yl_hi_needed), five scalar loads where that chunk would leave the level
+    constexpr int per = 16 / (int)sizeof(TP);
     const size_t f0 = ((size_t)img * rpi + rin) * p.RF;
-    const float4 lo = __ldcg(reinterpret_cast<const float4*>(p.lv.y_pred[l]) + (f0 >> 2));
-    const float4 hi = __ldcg(reinterpret_cast<const float4*>(p.lv.y_pred[l]) + (f0 >> 2) + 1);
-    yl_rotate5(lo, hi, (int)(f0 & 3), tx, ty, tw, th, pobj);
+    const float4* base = reinterpret_cast<const float4*>(p.lv.y_pred[l]);
+    if (!yl_hi_needed<TP>(f0)) {
+      yl_five<TP>(__ldcg(base + f0 / per), make_float4(0.f, 0.f, 0.f, 0.f), (int)(f0 % per), tx, ty, tw, th, pobj);
+    } else if (yl_hi_inside<TP>(f0, (size_t)p.B * rpi * p.RF)) {
+      const float4 lo = __ldcg(base + f0 / per);
+      const float4 hi = __ldcg(base + f0 / per + 1);
+      yl_five<TP>(lo, hi, (int)(f0 % per), tx, ty, tw, th, pobj);
+    } else {
+      yl_load5_scalar(static_cast<const TP*>(p.lv.y_pred[l]) + f0, tx, ty, tw, th, pobj);
+    }
   }
   bool pending = false;  // some (record, GT) pair survives the rejects: K4b-exact decides
   if (n_gt > 0) {        // block-uniform
@@ -661,6 +726,7 @@ __global__ void __launch_bounds__(YL_ICHUNK, 10) yolo_loss_ignore_lean_kernel(Yl
 // the exact pass over the queued records: HALF a warp per record (two records in flight per warp: the pass is a chain of
 // dependent loads per record — queue entry, record, GT list — so it is bound by how many records are in flight, not by
 // lanes: an (image, level) has ~17 GTs on average, one or two rounds of 16), `gwarp` of `nwarps` warps
+template <typename TP>
 __device__ __forceinline__ void yl_exact_pass(const YlParams& p, unsigned int gwarp, unsigned int nwarps) {
   const int lane = threadIdx.x & 31;
   const int half = lane >> 4, sub = lane & 15;
@@ -676,8 +742,8 @@ __device__ __forceinline__ void yl_exact_pass(const YlParams& p, unsigned int gw
     for (int k = 1; k < YL_LEVELS; ++k) if (ain >= p.lv.anchor_base[k]) l = k;
     const int rin = ain - p.lv.anchor_base[l];
     const int rpi = p.lv.rec_per_img[l];
-    const float* rec = p.lv.y_pred[l] + ((size_t)img * rpi + rin) * p.RF;
-    const float tx = __ldg(rec), ty = __ldg(rec + 1), tw = __ldg(rec + 2), th = __ldg(rec + 3), pobj = __ldg(rec + 4);
+    const TP* rec = static_cast<const TP*>(p.lv.y_pred[l]) + ((size_t)img * rpi + rin) * p.RF;
+    const float tx = ldg_f32(rec), ty = ldg_f32(rec + 1), tw = ldg_f32(rec + 2), th = ldg_f32(rec + 3), pobj = ldg_f32(rec + 4);
     const float obj = yl_obj(p, img, ain);
     const int n_gt = valid ? p.gt_count[img * YL_LEVELS + l] : 0;
     const float4* gbox = p.gt_box + (size_t)img * p.n_img + p.lv.anchor_base[l];
@@ -705,8 +771,9 @@ __device__ __forceinline__ void yl_exact_pass(const YlParams& p, unsigned int gw
   }
 }
 
+template <typename TP>
 __global__ void __launch_bounds__(128) yolo_loss_ignore_exact_kernel(YlParams p) {
-  yl_exact_pass(p, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), gridDim.x * (blockDim.x >> 5));
+  yl_exact_pass<TP>(p, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), gridDim.x * (blockDim.x >> 5));
 }
 
 // K4c: YL_FIN_CTAS CTAs each reduce an interleaved share of the per-CTA partials in fp64 (fixed assignment, fixed
@@ -729,10 +796,11 @@ struct YlFinalize {
 // With `exact` (split form of the ignore pass) the launch is wider than YL_FIN_CTAS: every CTA first resolves its share of
 // the queued records (K4b-exact inside this launch: no third kernel on the step's critical path), the first YL_FIN_CTAS
 // CTAs also reduce their slices, and the ticket counts ALL CTAs.
+template <typename TP>
 __global__ void __launch_bounds__(YL_FIN_THREADS) yolo_loss_finalize_kernel(YlFinalize f, YlParams p, int exact) {
   __shared__ double s_red[YL_FIN_THREADS / 32][12];
   __shared__ bool s_last;
-  if (exact) yl_exact_pass(p, blockIdx.x * (YL_FIN_THREADS / 32) + (threadIdx.x >> 5), gridDim.x * (YL_FIN_THREADS / 32));
+  if (exact) yl_exact_pass<TP>(p, blockIdx.x * (YL_FIN_THREADS / 32) + (threadIdx.x >> 5), gridDim.x * (YL_FIN_THREADS / 32));
   if ((int)blockIdx.x >= YL_FIN_CTAS) {   // block-uniform: exact-pass-only CTAs just take a ticket
     __syncthreads();
     if (threadIdx.x == 0) { __threadfence(); s_last = (atomicAdd(f.ticket, 1u) == gridDim.x - 1); }
@@ -807,18 +875,37 @@ __global__ void __launch_bounds__(YL_FIN_THREADS) yolo_loss_finalize_kernel(YlFi
 // The gradient tensor is dense like y_pred (7.7 MB/image at 608x608) but only the conf channel of every record and
 // the full record of object cells are non-zero: one streaming write pass (conf values saved by the forward ignore
 // kernel, 4 bytes/record) plus one warp per object record.
+//
+// The gradient is written in the caller's type TG (fp32, bf16 or fp16): each element is round_TG(g * s), one rounding
+// to nearest even of today's fp32 value g times the device scale s (*grad_scale; NULL: no multiply, so the fp32
+// instantiations keep their bits).  The zero stream stays +0 for any finite positive s.
 struct YlGradDense {
-  float* grad[YL_LEVELS];
+  void* grad[YL_LEVELS];
   const float* conf_grad[YL_LEVELS];
-  unsigned long long quads[YL_LEVELS];     // cumulative number of 4-record groups per level
-  unsigned long long records[YL_LEVELS];   // records per level (the last records % 4 are written by scalar stores)
+  unsigned long long quads[YL_LEVELS];     // cumulative number of 16 / sizeof(TG)-record groups per level
+  unsigned long long records[YL_LEVELS];   // records per level (the records past the last whole group: scalar stores)
+  const float* scale;                      // device fp32 scalar or null
   int RF;
 };
 
-// Four records = RF float4, always 16-byte aligned: a warp writes one such group per iteration (ceil(RF/32) 16-byte
+__device__ __forceinline__ float yl_scaled(float g, const float* scale) { return scale ? g * __ldg(scale) : g; }
+template <typename TG> __device__ __forceinline__ TG yl_round(float v);
+template <> __device__ __forceinline__ float yl_round<float>(float v) { return v; }
+template <> __device__ __forceinline__ __nv_bfloat16 yl_round<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __half yl_round<__half>(float v) { return __float2half_rn(v); }
+template <typename TG> __device__ __forceinline__ uint32_t yl_bits16(float v) {
+  const TG h = yl_round<TG>(v);
+  return (uint32_t)*reinterpret_cast<const unsigned short*>(&h);
+}
+
+// fp32: four records = RF float4, always 16-byte aligned: a warp writes one such group per iteration (ceil(RF/32) 16-byte
 // stores per lane), all zeros except the four conf channels, whose values are fetched by lanes 0-3 beforehand.  No
-// index division, no load -> store dependency on the streaming path.
+// index division, no load -> store dependency on the streaming path.  2-byte TG: eight records = RF 16-byte chunks, the
+// eight conf values staged in shared memory; a chunk holds at most two conf channels (RF >= 5), found with one division.
+template <typename TG>
 __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g) {
+  constexpr int kRec = 16 / (int)sizeof(TG);   // records per group
+  __shared__ float s_conf[256 / 32][8];
   const int lane = threadIdx.x & 31;
   const unsigned long long total = g.quads[YL_LEVELS - 1];
   const unsigned long long wstride = (unsigned long long)gridDim.x * (blockDim.x >> 5);
@@ -827,10 +914,31 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g
     // explicit selects: indexing the kernel-parameter arrays with a runtime level would copy them to local memory
     unsigned long long q = w;
     const float* cg = g.conf_grad[0];
-    float* gr = g.grad[0];
-    if (w >= g.quads[1]) { q = w - g.quads[1]; cg = g.conf_grad[2]; gr = g.grad[2]; }
-    else if (w >= g.quads[0]) { q = w - g.quads[0]; cg = g.conf_grad[1]; gr = g.grad[1]; }
-    const float mine = (lane < 4) ? __ldg(cg + q * 4ull + lane) : 0.0f;
+    TG* gr = static_cast<TG*>(g.grad[0]);
+    if (w >= g.quads[1]) { q = w - g.quads[1]; cg = g.conf_grad[2]; gr = static_cast<TG*>(g.grad[2]); }
+    else if (w >= g.quads[0]) { q = w - g.quads[0]; cg = g.conf_grad[1]; gr = static_cast<TG*>(g.grad[1]); }
+    if constexpr (kRec == 8) {
+      float* sc = s_conf[threadIdx.x >> 5];
+      __syncwarp();
+      if (lane < 8) sc[lane] = yl_scaled(__ldg(cg + q * 8ull + lane), g.scale);
+      __syncwarp();
+      uint4* dst = reinterpret_cast<uint4*>(gr) + q * (unsigned long long)RF;
+      for (int j = lane; j < RF; j += 32) {
+        // chunk j holds elements 8j..8j+7; record r's conf channel is element r*RF + 4.  The first record whose conf
+        // channel is >= 8j sits at p0 = r*RF + 4 - 8j, the next one RF further
+        const int x0 = 8 * j - 4;
+        const int r = x0 > 0 ? (x0 + RF - 1) / RF : 0;
+        const int p0 = r * RF - x0, p1 = p0 + RF;
+        const uint32_t b0 = p0 < 8 ? yl_bits16<TG>(sc[min(r, 7)]) : 0u, b1 = p1 < 8 ? yl_bits16<TG>(sc[min(r + 1, 7)]) : 0u;
+        uint32_t wd[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+          wd[k] = ((p0 >> 1) == k ? b0 << (16 * (p0 & 1)) : 0u) | ((p1 >> 1) == k ? b1 << (16 * (p1 & 1)) : 0u);
+        __stcs(dst + j, make_uint4(wd[0], wd[1], wd[2], wd[3]));
+      }
+      continue;
+    }
+    const float mine = (lane < 4) ? yl_scaled(__ldg(cg + q * 4ull + lane), g.scale) : 0.0f;
     const float c0 = __shfl_sync(0xffffffffu, mine, 0), c1 = __shfl_sync(0xffffffffu, mine, 1);
     const float c2 = __shfl_sync(0xffffffffu, mine, 2), c3 = __shfl_sync(0xffffffffu, mine, 3);
     float4* dst = reinterpret_cast<float4*>(gr) + q * (unsigned long long)RF;
@@ -850,11 +958,12 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g
   if (blockIdx.x == 0) {
 #pragma unroll
     for (int l = 0; l < YL_LEVELS; ++l) {
-      const unsigned long long r0 = g.records[l] & ~3ull, n_tail = (g.records[l] - r0) * (unsigned long long)RF;
+      const unsigned long long r0 = g.records[l] & ~(unsigned long long)(kRec - 1), n_tail = (g.records[l] - r0) * (unsigned long long)RF;
       for (unsigned long long t = threadIdx.x; t < n_tail; t += blockDim.x) {
         const unsigned long long rec = r0 + t / (unsigned long long)RF;
         const int c = (int)(t % (unsigned long long)RF);
-        g.grad[l][r0 * (unsigned long long)RF + t] = (c == 4) ? g.conf_grad[l][rec] : 0.0f;
+        static_cast<TG*>(g.grad[l])[r0 * (unsigned long long)RF + t] =
+            yl_round<TG>((c == 4) ? yl_scaled(g.conf_grad[l][rec], g.scale) : 0.0f);
       }
     }
   }
@@ -866,24 +975,24 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g
 // dense scatter would have written (obj = 1, one-hot class row; an out-of-range class id gives an all-zero row, as
 // tf.one_hot); the arithmetic is the dense form's.
 #define YL_GRAD_SPLIT 8
-template <bool kSparse>
-__global__ void __launch_bounds__(256) yolo_loss_grad_objects_kernel(YlParams p, float* g0, float* g1, float* g2) {
+template <bool kSparse, typename TP, typename TG>
+__global__ void __launch_bounds__(256) yolo_loss_grad_objects_kernel(YlParams p, TG* g0, TG* g1, TG* g2, const float* scale) {
   const int pair = blockIdx.x / YL_GRAD_SPLIT, split = blockIdx.x - pair * YL_GRAD_SPLIT;
   const int img = pair / YL_LEVELS, l = pair - img * YL_LEVELS;
-  float* grad = (l == 0 ? g0 : l == 1 ? g1 : g2);
+  TG* grad = (l == 0 ? g0 : l == 1 ? g1 : g2);
   const int n = p.gt_count[img * YL_LEVELS + l];
   const int rpi = p.lv.rec_per_img[l];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int W = p.lv.w[l], H = p.lv.h[l];
   const float* yt = kSparse ? nullptr : p.lv.y_true[l] + ((size_t)img * rpi) * p.RF;
-  const float* yp = p.lv.y_pred[l] + ((size_t)img * rpi) * p.RF;
-  float* gr = grad + ((size_t)img * rpi) * p.RF;
+  const TP* yp = static_cast<const TP*>(p.lv.y_pred[l]) + ((size_t)img * rpi) * p.RF;
+  TG* gr = grad + ((size_t)img * rpi) * p.RF;
   for (int k = split * 8 + warp; k < n; k += 8 * YL_GRAD_SPLIT) {
     const size_t slot = (size_t)img * p.n_img + p.lv.anchor_base[l] + k;
     const int r = p.obj_index[slot];
     const float* t = kSparse ? nullptr : yt + (size_t)r * p.RF;
-    const float* q = yp + (size_t)r * p.RF;
-    float* o = gr + (size_t)r * p.RF;
+    const TP* q = yp + (size_t)r * p.RF;
+    TG* o = gr + (size_t)r * p.RF;
     float obj, tx, ty, tw, th;
     int sp_class = -1;
     if (kSparse) {
@@ -900,16 +1009,17 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_objects_kernel(YlParams p,
       const int gy = cell / W, gx = cell - gy * W;
       float raw = (lane == 0 ? tx * (float)W - (float)gx : ty * (float)H - (float)gy);
       if (p.variant == YL_VARIANT_TF_YOLO_UTILS) raw = obj * raw;
-      o[lane] = os * (dm_sigmoidf(__ldg(q + lane)) - raw);
+      o[lane] = yl_round<TG>(yl_scaled(os * (dm_sigmoidf(ldg_f32(q + lane)) - raw), scale));
     } else if (lane < 4) {
       const int a = r - (r / p.A) * p.A;
       float num = (lane == 2 ? tw * p.img_w : th * p.img_h);
       if (p.variant == YL_VARIANT_TF_YOLO_UTILS) num += 1e-8f;
       const float raw = dm_logf(num / (lane == 2 ? p.lv.anc_w[l][a] : p.lv.anc_h[l][a]));
-      o[lane] = os * (__ldg(q + lane) - raw);
+      o[lane] = yl_round<TG>(yl_scaled(os * (ldg_f32(q + lane) - raw), scale));
     }
     for (int c = 5 + lane; c < p.RF; c += 32)
-      o[c] = (obj * p.inv_div) * (dm_sigmoidf(__ldg(q + c)) - (kSparse ? ((c - 5 == sp_class) ? 1.0f : 0.0f) : __ldg(t + c)));
+      o[c] = yl_round<TG>(yl_scaled((obj * p.inv_div) * (dm_sigmoidf(ldg_f32(q + c)) - (kSparse ? ((c - 5 == sp_class) ? 1.0f : 0.0f) : __ldg(t + c))),
+                                    scale));
   }
 }
 
@@ -1064,12 +1174,29 @@ static YlSparseWs yl_sparse_layout(size_t dense_total, int B, int n_img, int tot
   return w;
 }
 
-static int yolo_loss_impl(const float* const y_true[3], const float* const y_pred[3], const int32_t hw[6], int B,
+// Element types of a call: y_pred (B200_DTYPE_*), the gradient, and the optional device gradient scale
+struct YlTypes { int pred, grad; const float* grad_scale; };
+static const YlTypes kYlF32 = {B200_DTYPE_F32, B200_DTYPE_F32, nullptr};
+
+static const void* const* yl_untyped(const float* const* p) { return reinterpret_cast<const void* const*>(p); }
+static void* const* yl_untyped(float* const* p) { return reinterpret_cast<void* const*>(p); }
+
+// d loss / d y_pred of the object records, y_pred of type TP, gradient of type TG
+template <typename TP, typename TG>
+static void yl_grad_objects(const YlParams& p, bool sparse, void* const out_grad[3], const float* scale, cudaStream_t stream) {
+  TG* g0 = static_cast<TG*>(out_grad[0]);
+  TG* g1 = static_cast<TG*>(out_grad[1]);
+  TG* g2 = static_cast<TG*>(out_grad[2]);
+  if (sparse) yolo_loss_grad_objects_kernel<true, TP, TG><<<p.B * YL_LEVELS * YL_GRAD_SPLIT, 256, 0, stream>>>(p, g0, g1, g2, scale);
+  else yolo_loss_grad_objects_kernel<false, TP, TG><<<p.B * YL_LEVELS * YL_GRAD_SPLIT, 256, 0, stream>>>(p, g0, g1, g2, scale);
+}
+
+static int yolo_loss_impl(const float* const y_true[3], const void* const y_pred[3], const int32_t hw[6], int B,
                           int A, int C, const float* anchors_wh_host, const float* image_wh_host,
                           float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
-                          float* out_loss, unsigned char* out_ignore, float* const out_grad[3], void* workspace,
+                          float* out_loss, unsigned char* out_ignore, void* const out_grad[3], void* workspace,
                           size_t workspace_bytes, void* stream_, const YlSparseIn* sparse = nullptr, int stages = 0xf,
-                          const B200Exchange* xchg = nullptr, int publish_only = 0) {
+                          const B200Exchange* xchg = nullptr, int publish_only = 0, const YlTypes& ty = kYlF32) {
   cudaStream_t stream = (cudaStream_t)stream_;
   B200_REQUIRE((y_true || sparse) && y_pred && hw && anchors_wh_host && image_wh_host && out_loss, B200_ERR_BAD_ARG, "b200_yolo_loss: null argument");
   B200_REQUIRE(B >= 1 && A >= 1 && A <= 8 && C >= 0, B200_ERR_BAD_ARG, "b200_yolo_loss: unsupported shape B=%d A=%d C=%d", B, A, C);
@@ -1093,6 +1220,7 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
     B200_REQUIRE((sparse || y_true[l]) && y_pred[l] && hw[2 * l] > 0 && hw[2 * l + 1] > 0, B200_ERR_BAD_ARG, "b200_yolo_loss: bad level %d", l);
     p.lv.y_true[l] = sparse ? nullptr : y_true[l];
     p.lv.y_pred[l] = y_pred[l];
+    p.lv.pred_dtype = ty.pred;
     for (int a = 0; a < A; ++a) {
       p.lv.anc_w[l][a] = anchors_wh_host[(l * A + a) * 2 + 0];
       p.lv.anc_h[l][a] = anchors_wh_host[(l * A + a) * 2 + 1];
@@ -1130,6 +1258,13 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
   p.gt_count = reinterpret_cast<int32_t*>(wsb + ws.cnt);
   p.partials = reinterpret_cast<double*>(wsb + ws.part);
   p.partials_obj = reinterpret_cast<double*>(wsb + ws.part_obj);
+  YtParams t;
+  if (sparse) {   // checked before anything is enqueued
+    B200_REQUIRE(sparse->total_boxes >= 0 && sparse->offsets && sparse->assign_anchors_wh_host, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: null box arrays");
+    B200_REQUIRE(sparse->total_boxes == 0 || (sparse->boxes && sparse->classes), B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: null box arrays");
+    B200_REQUIRE((reinterpret_cast<uintptr_t>(sparse->boxes) & 15) == 0, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: boxes not 16-byte aligned");
+    B200_REQUIRE(yt_fill_geometry(t, A, C, sparse->assign_anchors_wh_host, image_wh_host, hw) == 0, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: bad geometry");
+  }
   if (stages & 1) B200_CUDA(cudaMemsetAsync(wsb + ws.cnt, 0, ws.cnt_bytes, stream));
   p.pend_queue = reinterpret_cast<uint32_t*>(wsb + ws.pend);
   p.pend_count = reinterpret_cast<unsigned int*>(wsb + ws.cnt) + (size_t)B * YL_LEVELS + 1;
@@ -1138,11 +1273,6 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
   p.scan_ticket = (!sparse && (stages & 3) == 3) ? reinterpret_cast<unsigned int*>(p.obj_fixed + 3) : nullptr;
   p.sp_t = nullptr; p.sp_cls = nullptr; p.obj_bits = nullptr; p.bits_words = 0;
   if (sparse) {
-    B200_REQUIRE(sparse->total_boxes >= 0 && sparse->offsets && sparse->assign_anchors_wh_host, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: null box arrays");
-    B200_REQUIRE(sparse->total_boxes == 0 || (sparse->boxes && sparse->classes), B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: null box arrays");
-    B200_REQUIRE((reinterpret_cast<uintptr_t>(sparse->boxes) & 15) == 0, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: boxes not 16-byte aligned");
-    YtParams t;
-    B200_REQUIRE(yt_fill_geometry(t, A, C, sparse->assign_anchors_wh_host, image_wh_host, hw) == 0, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes: bad geometry");
     t.boxes = sparse->boxes; t.classes = sparse->classes; t.offsets = sparse->offsets; t.B = B; t.total = sparse->total_boxes;
     p.bits_words = sws.bits_words;
     float4* sp_t = reinterpret_cast<float4*>(wsb + sws.sp_t);
@@ -1181,13 +1311,13 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
       // the queue counter and the fixed-point sums are zeroed with the object counts (stage 1); the stage hook may run this
       // pass on its own, repeatedly
       if (!(stages & 1)) B200_CUDA(cudaMemsetAsync(p.pend_count, 0, (size_t)(reinterpret_cast<unsigned char*>(p.obj_fixed + 3) - reinterpret_cast<unsigned char*>(p.pend_count)), stream));
-      yolo_loss_ignore_lean_kernel<<<grid, YL_ICHUNK, 0, stream>>>(p);
+      B200_DISPATCH_DTYPE(ty.pred, TP, yolo_loss_ignore_lean_kernel<TP><<<grid, YL_ICHUNK, 0, stream>>>(p));
       if (!(stages & 8)) {   // no finalize in this call: the exact pass as a launch of its own (the finalize launch carries it otherwise)
         B200_LAUNCH_CHECK();
-        yolo_loss_ignore_exact_kernel<<<1024, 128, 0, stream>>>(p);
+        B200_DISPATCH_DTYPE(ty.pred, TP, yolo_loss_ignore_exact_kernel<TP><<<1024, 128, 0, stream>>>(p));
       }
     } else {
-      yolo_loss_ignore_kernel<<<grid, YL_ICHUNK, 0, stream>>>(p);
+      B200_DISPATCH_DTYPE(ty.pred, TP, yolo_loss_ignore_kernel<TP><<<grid, YL_ICHUNK, 0, stream>>>(p));
     }
     B200_LAUNCH_CHECK();
   }
@@ -1205,30 +1335,49 @@ static int yolo_loss_impl(const float* const y_true[3], const float* const y_pre
   // split form: the finalize launch is widened to 4 CTAs per SM and resolves the queued records first
   int wide = 4 * b200_sm_count();
   if (wide < YL_FIN_CTAS) wide = YL_FIN_CTAS;
-  yolo_loss_finalize_kernel<<<use_split ? wide : YL_FIN_CTAS, YL_FIN_THREADS, 0, stream>>>(f, p, use_split ? 1 : 0);
+  B200_DISPATCH_DTYPE(ty.pred, TP, yolo_loss_finalize_kernel<TP><<<use_split ? wide : YL_FIN_CTAS, YL_FIN_THREADS, 0, stream>>>(f, p, use_split ? 1 : 0));
   B200_LAUNCH_CHECK();
   if (out_grad) {
     YlGradDense g;
     g.RF = p.RF;
+    g.scale = ty.grad_scale;
+    const unsigned long long per_group = 16ull / (unsigned long long)b200_dtype_bytes(ty.grad);   // records per 16-byte-store group
     unsigned long long cum = 0;
     for (int l = 0; l < YL_LEVELS; ++l) {
       g.records[l] = (unsigned long long)B * p.lv.rec_per_img[l];
       g.grad[l] = out_grad[l];
       g.conf_grad[l] = p.conf_grad + (size_t)B * p.lv.anchor_base[l];
-      cum += g.records[l] / 4ull;
+      cum += g.records[l] / per_group;
       g.quads[l] = cum;
     }
-    unsigned long long blocks = (cum + 7) / 8;  // a warp per group of four records
+    unsigned long long blocks = (cum + 7) / 8;  // a warp per group of records
     const unsigned long long cap = (unsigned long long)b200_sm_count() * 64;
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
-    yolo_loss_grad_dense_kernel<<<(int)blocks, 256, 0, stream>>>(g);
+    B200_DISPATCH_DTYPE(ty.grad, TG, yolo_loss_grad_dense_kernel<TG><<<(int)blocks, 256, 0, stream>>>(g));
     B200_LAUNCH_CHECK();
-    if (sparse) yolo_loss_grad_objects_kernel<true><<<B * YL_LEVELS * YL_GRAD_SPLIT, 256, 0, stream>>>(p, out_grad[0], out_grad[1], out_grad[2]);
-    else yolo_loss_grad_objects_kernel<false><<<B * YL_LEVELS * YL_GRAD_SPLIT, 256, 0, stream>>>(p, out_grad[0], out_grad[1], out_grad[2]);
+    B200_DISPATCH_DTYPE(ty.pred, TP, B200_DISPATCH_DTYPE(ty.grad, TG, yl_grad_objects<TP, TG>(p, sparse != nullptr, out_grad, ty.grad_scale, stream)));
     B200_LAUNCH_CHECK();
   }
   return B200_OK;
+}
+
+// The typed entries: y_pred of element type pred_dtype, the gradient of element type grad_dtype (B200_DTYPE_*, each
+// shared by the three levels), scaled by *grad_scale_dev (device fp32, NULL: 1) before its one rounding.  The fp32
+// entries are their (F32, F32, NULL) case.
+#define YL_CHECK_DTYPE(code, who, what) \
+  B200_REQUIRE(b200_dtype_ok(code), B200_ERR_BAD_ARG, "%s: %s %d is not a B200_DTYPE_* code", who, what, code)
+
+extern "C" int b200_yolo_loss_typed(const float* const y_true[3], const void* const y_pred[3], int pred_dtype, const int32_t hw[6],
+                                    int B, int A, int C, const float* anchors_wh_host, const float* image_wh_host,
+                                    float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
+                                    float* out_loss, unsigned char* out_ignore, void* workspace, size_t workspace_bytes,
+                                    void* stream_) {
+  YL_CHECK_DTYPE(pred_dtype, "b200_yolo_loss", "pred_dtype");
+  const YlTypes ty = {pred_dtype, B200_DTYPE_F32, nullptr};
+  return yolo_loss_impl(y_true, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+                        batch_divisor, out_parts, out_loss, out_ignore, nullptr, workspace, workspace_bytes, stream_, nullptr,
+                        0xf, nullptr, 0, ty);
 }
 
 extern "C" int b200_yolo_loss(const float* const y_true[3], const float* const y_pred[3], const int32_t hw[6], int B,
@@ -1236,8 +1385,8 @@ extern "C" int b200_yolo_loss(const float* const y_true[3], const float* const y
                               float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
                               float* out_loss, unsigned char* out_ignore, void* workspace, size_t workspace_bytes,
                               void* stream_) {
-  return yolo_loss_impl(y_true, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
-                        batch_divisor, out_parts, out_loss, out_ignore, nullptr, workspace, workspace_bytes, stream_);
+  return b200_yolo_loss_typed(y_true, yl_untyped(y_pred), B200_DTYPE_F32, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh,
+                              metric, variant, batch_divisor, out_parts, out_loss, out_ignore, workspace, workspace_bytes, stream_);
 }
 
 // Measurement hook: the same call restricted to a subset of its four launches (bit 0 scan, 1 GT prep, 2 ignore + object
@@ -1248,7 +1397,7 @@ extern "C" int b200_yolo_loss_stages(const float* const y_true[3], const float* 
                                      float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
                                      float* out_loss, void* workspace, size_t workspace_bytes, int stages, void* stream_) {
   B200_REQUIRE(stages > 0 && stages <= 0xf, B200_ERR_BAD_ARG, "b200_yolo_loss_stages: stages must be a non-empty subset of 0xf");
-  return yolo_loss_impl(y_true, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+  return yolo_loss_impl(y_true, yl_untyped(y_pred), hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
                         batch_divisor, out_parts, out_loss, nullptr, nullptr, workspace, workspace_bytes, stream_, nullptr, stages);
 }
 
@@ -1258,17 +1407,31 @@ extern "C" size_t b200_yolo_loss_from_boxes_workspace_bytes(const int32_t hw[6],
   return yl_sparse_layout(w.total, B, n_img, total_boxes).total;
 }
 
+extern "C" int b200_yolo_loss_from_boxes_typed(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
+                                               const float* assign_anchors_wh_host, const void* const y_pred[3], int pred_dtype,
+                                               const int32_t hw[6], int B, int A, int C, const float* anchors_wh_host,
+                                               const float* image_wh_host, float iou_thresh, int metric, int variant,
+                                               float batch_divisor, float* out_parts, float* out_loss, unsigned char* out_ignore,
+                                               void* workspace, size_t workspace_bytes, void* stream_) {
+  YL_CHECK_DTYPE(pred_dtype, "b200_yolo_loss_from_boxes", "pred_dtype");
+  YlSparseIn sp;
+  sp.boxes = boxes; sp.classes = classes; sp.offsets = offsets; sp.total_boxes = total_boxes;
+  sp.assign_anchors_wh_host = assign_anchors_wh_host;
+  const YlTypes ty = {pred_dtype, B200_DTYPE_F32, nullptr};
+  return yolo_loss_impl(nullptr, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+                        batch_divisor, out_parts, out_loss, out_ignore, nullptr, workspace, workspace_bytes, stream_, &sp, 0xf,
+                        nullptr, 0, ty);
+}
+
 extern "C" int b200_yolo_loss_from_boxes(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
                                          const float* assign_anchors_wh_host, const float* const y_pred[3], const int32_t hw[6],
                                          int B, int A, int C, const float* anchors_wh_host, const float* image_wh_host,
                                          float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
                                          float* out_loss, unsigned char* out_ignore, void* workspace, size_t workspace_bytes,
                                          void* stream_) {
-  YlSparseIn sp;
-  sp.boxes = boxes; sp.classes = classes; sp.offsets = offsets; sp.total_boxes = total_boxes;
-  sp.assign_anchors_wh_host = assign_anchors_wh_host;
-  return yolo_loss_impl(nullptr, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
-                        batch_divisor, out_parts, out_loss, out_ignore, nullptr, workspace, workspace_bytes, stream_, &sp);
+  return b200_yolo_loss_from_boxes_typed(boxes, classes, offsets, total_boxes, assign_anchors_wh_host, yl_untyped(y_pred),
+                                         B200_DTYPE_F32, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+                                         batch_divisor, out_parts, out_loss, out_ignore, workspace, workspace_bytes, stream_);
 }
 
 // GetGroudTruth of the three levels GetTargets would write, straight from the box lists: rows [total,5], image b's
@@ -1311,18 +1474,50 @@ extern "C" int b200_yolo_ground_truth_from_boxes(const float* boxes, const int32
 
 // b200_yolo_loss_from_boxes plus d loss / d y_pred, as b200_yolo_loss_grad is to b200_yolo_loss.  The workspace of
 // b200_yolo_loss_from_boxes_workspace_bytes already holds the per-record conf gradient the backward reads.
+extern "C" int b200_yolo_loss_from_boxes_grad_typed(const float* boxes, const int32_t* classes, const int32_t* offsets,
+                                                    int total_boxes, const float* assign_anchors_wh_host, const void* const y_pred[3],
+                                                    int pred_dtype, const int32_t hw[6], int B, int A, int C,
+                                                    const float* anchors_wh_host, const float* image_wh_host, float iou_thresh,
+                                                    int metric, int variant, float batch_divisor, float* out_parts, float* out_loss,
+                                                    void* const out_grad[3], int grad_dtype, const float* grad_scale_dev,
+                                                    void* workspace, size_t workspace_bytes, void* stream_) {
+  YL_CHECK_DTYPE(pred_dtype, "b200_yolo_loss_from_boxes_grad", "pred_dtype");
+  YL_CHECK_DTYPE(grad_dtype, "b200_yolo_loss_from_boxes_grad", "grad_dtype");
+  B200_REQUIRE(out_grad, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes_grad: null out_grad");
+  YlSparseIn sp;
+  sp.boxes = boxes; sp.classes = classes; sp.offsets = offsets; sp.total_boxes = total_boxes;
+  sp.assign_anchors_wh_host = assign_anchors_wh_host;
+  const YlTypes ty = {pred_dtype, grad_dtype, grad_scale_dev};
+  return yolo_loss_impl(nullptr, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+                        batch_divisor, out_parts, out_loss, nullptr, out_grad, workspace, workspace_bytes, stream_, &sp, 0xf,
+                        nullptr, 0, ty);
+}
+
 extern "C" int b200_yolo_loss_from_boxes_grad(const float* boxes, const int32_t* classes, const int32_t* offsets, int total_boxes,
                                               const float* assign_anchors_wh_host, const float* const y_pred[3], const int32_t hw[6],
                                               int B, int A, int C, const float* anchors_wh_host, const float* image_wh_host,
                                               float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
                                               float* out_loss, float* const out_grad[3], void* workspace, size_t workspace_bytes,
                                               void* stream_) {
-  B200_REQUIRE(out_grad, B200_ERR_BAD_ARG, "b200_yolo_loss_from_boxes_grad: null out_grad");
-  YlSparseIn sp;
-  sp.boxes = boxes; sp.classes = classes; sp.offsets = offsets; sp.total_boxes = total_boxes;
-  sp.assign_anchors_wh_host = assign_anchors_wh_host;
-  return yolo_loss_impl(nullptr, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
-                        batch_divisor, out_parts, out_loss, nullptr, out_grad, workspace, workspace_bytes, stream_, &sp);
+  return b200_yolo_loss_from_boxes_grad_typed(boxes, classes, offsets, total_boxes, assign_anchors_wh_host, yl_untyped(y_pred),
+                                              B200_DTYPE_F32, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric,
+                                              variant, batch_divisor, out_parts, out_loss, yl_untyped(out_grad), B200_DTYPE_F32,
+                                              nullptr, workspace, workspace_bytes, stream_);
+}
+
+extern "C" int b200_yolo_loss_grad_typed(const float* const y_true[3], const void* const y_pred[3], int pred_dtype,
+                                         const int32_t hw[6], int B, int A, int C, const float* anchors_wh_host,
+                                         const float* image_wh_host, float iou_thresh, int metric, int variant,
+                                         float batch_divisor, float* out_parts, float* out_loss, void* const out_grad[3],
+                                         int grad_dtype, const float* grad_scale_dev, void* workspace, size_t workspace_bytes,
+                                         void* stream_) {
+  YL_CHECK_DTYPE(pred_dtype, "b200_yolo_loss_grad", "pred_dtype");
+  YL_CHECK_DTYPE(grad_dtype, "b200_yolo_loss_grad", "grad_dtype");
+  B200_REQUIRE(out_grad, B200_ERR_BAD_ARG, "b200_yolo_loss_grad: null out_grad");
+  const YlTypes ty = {pred_dtype, grad_dtype, grad_scale_dev};
+  return yolo_loss_impl(y_true, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+                        batch_divisor, out_parts, out_loss, nullptr, out_grad, workspace, workspace_bytes, stream_, nullptr, 0xf,
+                        nullptr, 0, ty);
 }
 
 extern "C" int b200_yolo_loss_grad(const float* const y_true[3], const float* const y_pred[3], const int32_t hw[6],
@@ -1330,9 +1525,9 @@ extern "C" int b200_yolo_loss_grad(const float* const y_true[3], const float* co
                                    float iou_thresh, int metric, int variant, float batch_divisor, float* out_parts,
                                    float* out_loss, float* const out_grad[3], void* workspace, size_t workspace_bytes,
                                    void* stream_) {
-  B200_REQUIRE(out_grad, B200_ERR_BAD_ARG, "b200_yolo_loss_grad: null out_grad");
-  return yolo_loss_impl(y_true, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
-                        batch_divisor, out_parts, out_loss, nullptr, out_grad, workspace, workspace_bytes, stream_);
+  return b200_yolo_loss_grad_typed(y_true, yl_untyped(y_pred), B200_DTYPE_F32, hw, B, A, C, anchors_wh_host, image_wh_host,
+                                   iou_thresh, metric, variant, batch_divisor, out_parts, out_loss, yl_untyped(out_grad),
+                                   B200_DTYPE_F32, nullptr, workspace, workspace_bytes, stream_);
 }
 
 // Data-parallel forms (SURVEY 8e): every rank passes its own images and batch_divisor = the GLOBAL batch; the 12
@@ -1350,7 +1545,7 @@ extern "C" int b200_yolo_loss_dp(const float* const y_true[3], const float* cons
   B200Exchange x;
   const int rc = b200_fill_exchange(x, rank, world, mailboxes, "b200_yolo_loss_dp");
   if (rc != B200_OK) return rc;
-  return yolo_loss_impl(y_true, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+  return yolo_loss_impl(y_true, yl_untyped(y_pred), hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
                         global_batch, out_parts, out_loss, nullptr, nullptr, workspace, workspace_bytes, stream_, nullptr, 0xf, &x);
 }
 
@@ -1366,7 +1561,7 @@ extern "C" int b200_yolo_loss_dp_publish(const float* const y_true[3], const flo
   B200Exchange x;
   const int rc = b200_fill_exchange(x, rank, world, mailboxes, "b200_yolo_loss_dp_publish");
   if (rc != B200_OK) return rc;
-  return yolo_loss_impl(y_true, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+  return yolo_loss_impl(y_true, yl_untyped(y_pred), hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
                         global_batch, out_parts, out_loss, nullptr, nullptr, workspace, workspace_bytes, stream_, nullptr, 0xf, &x, 1);
 }
 
@@ -1382,7 +1577,7 @@ extern "C" int b200_yolo_loss_from_boxes_dp(const float* boxes, const int32_t* c
   YlSparseIn sp;
   sp.boxes = boxes; sp.classes = classes; sp.offsets = offsets; sp.total_boxes = total_boxes;
   sp.assign_anchors_wh_host = assign_anchors_wh_host;
-  return yolo_loss_impl(nullptr, y_pred, hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
+  return yolo_loss_impl(nullptr, yl_untyped(y_pred), hw, B, A, C, anchors_wh_host, image_wh_host, iou_thresh, metric, variant,
                         global_batch, out_parts, out_loss, nullptr, nullptr, workspace, workspace_bytes, stream_, &sp, 0xf, &x);
 }
 
