@@ -19,9 +19,9 @@
 //      Every other call (device-resident y_pred, every level 16-byte aligned, records of >= 8 floats) SPLITS the pass.
 //      K4b-lean (yolo_loss_ignore_lean_kernel, 48 registers, 10 CTAs per SM) streams, applies the same rejects and only
 //      QUEUES the records that some GT might still hit (~1 % of them); K4b-exact resolves the queue (a warp per record) at
-//      the head of the widened K4c launch, its object-loss terms in 2^-32 fixed point so that the sum does not depend on
-//      the order.  The launches of a dense call are then K4a (whose last CTA per (image, level) also does K4a'),
-//      K4b-lean, K4c.
+//      the head of the widened K4c launch, its object-loss terms in exact 2^-32 fixed point so that the sum does not
+//      depend on the order (YlObjSum).  The launches of a dense call are then K4a (whose last CTA per (image, level)
+//      also does K4a'), K4b-lean, K4c.
 //  K4c yolo_loss_finalize_kernel  fixed-order fp64 reduction of the per-CTA partials -> parts[3][4] / batch,
 //      loss = sum_l ((xy+wh)+obj)+cls in fp32 in the reference's order (tyu:120-125).  Deterministic run to run (the object lists are
 //      put into ascending record order by K4a' before anything is summed over them).
@@ -48,6 +48,19 @@ struct YlLevels {
   int obj_cta_base[YL_LEVELS + 1];
   uint32_t magic_w[YL_LEVELS];         // floor(2^32/W)+1
   float anc_w[YL_LEVELS][8], anc_h[YL_LEVELS][8];  // pixels
+};
+
+// Object-loss sum of the exact pass, per level.  A term e in [0, 2^63) is added exactly as T = round(e * 2^32) < 2^95,
+// split into three 32-bit limbs, each added to a 64-bit word of its own: fewer than 2^32 terms cannot carry a word past
+// 2^64, integer sums do not depend on the order (the loss stays bit-reproducible), and the adds need no return value.
+// The words are striped over YL_OBJ_STRIPES copies (by warp) so that the atomics of one level do not all queue on one
+// address.  NaN, +-inf and terms of 2^63 or more go to an fp64 side sum instead, where they propagate as in the single
+// kernel's fp64 partials (order dependent, but only in that regime).  The finalize sums the stripes, joins the limbs
+// into a 128-bit hi:lo and adds hi * 2^32 + lo * 2^-32 + side.
+#define YL_OBJ_STRIPES 32
+struct YlObjSum {
+  unsigned long long limb[YL_OBJ_STRIPES][16];   // [stripe][k * YL_LEVELS + level]: bits 32k .. 32k+31 of T (128 B a stripe)
+  double side[YL_LEVELS];
 };
 
 struct YlParams {
@@ -78,7 +91,7 @@ struct YlParams {
   // split form of the ignore pass (K4b-lean + K4b-exact): records whose filter leaves a (record, GT) pair undecided
   uint32_t* pend_queue;            // [B * n_img] global record ids (img * n_img + anchor_base[l] + rin)
   unsigned int* pend_count;        // number of queued records
-  unsigned long long* obj_fixed;   // [3] object-loss terms of the queued records, 2^-32 fixed point (order-independent sum)
+  YlObjSum* obj_sum;               // object-loss terms of the queued records, per level (order-independent sum)
   double* partials;     // [n_cta]      object_loss partial of each ignore-kernel CTA
   double* partials_obj; // [3*B*YL_TERM_SPLIT,3] xy, wh, cls partials of each terms-kernel CTA (level-major)
 };
@@ -658,11 +671,32 @@ __global__ void __launch_bounds__(YL_ICHUNK, YL_IMINB) yolo_loss_ignore_kernel(Y
 //              mid-kernel CTA barriers.
 //   K4b-exact  a warp per queued record: the exact test (yl_pair_hits, with its own exact rejects) against EVERY ground
 //              truth of the record's (image, level), lanes <-> GTs; writes the record's ignore bit / gradient and adds its
-//              object-loss term to a 2^-32 fixed-point accumulator (integer atomics: the sum is order independent, so
-//              the loss stays bit-reproducible).
+//              object-loss term to the level's YlObjSum (integer atomics: the sum is order independent, so the loss stays
+//              bit-reproducible).
 // A rejected pair is provably below the threshold (DESIGN.md section 6), so "some surviving pair hits" == "some GT hits":
 // the ignore mask is bit-identical to K4b's.
-#define YL_FIXED_ONE 4294967296.0  // 2^32
+#define YL_FIXED_ONE 4294967296.0            // 2^32
+#define YL_FIXED_WORD 18446744073709551616.0  // 2^64
+
+__device__ __forceinline__ void yl_obj_sum_add(YlObjSum* s, unsigned int stripe, int l, float e) {
+  if (e >= 0.0f && e < 9.22337204e18f) {   // 2^63
+    // e * 2^32 is exact in fp64; + 0.5 rounds a fraction half up (e < 2^21), above that v is an integer already
+    double v = (double)e * YL_FIXED_ONE + 0.5;
+    unsigned long long t2 = 0ull;
+    if (v >= YL_FIXED_WORD) {
+      const double vh = floor(v * (1.0 / YL_FIXED_WORD));
+      t2 = (unsigned long long)vh;
+      v -= vh * YL_FIXED_WORD;   // exact: a remainder of doubles
+    }
+    const unsigned long long t = (unsigned long long)v;
+    unsigned long long* w = s->limb[stripe % YL_OBJ_STRIPES];
+    atomicAdd(w + l, t & 0xffffffffull);
+    atomicAdd(w + YL_LEVELS + l, t >> 32);
+    if (t2) atomicAdd(w + 2 * YL_LEVELS + l, t2);
+  } else {
+    atomicAdd(&s->side[l], (double)e);
+  }
+}
 
 // 10 CTAs per SM (48 registers, no spills): the fastest headline step of 8, 10, 12 and 16 (profiles/r02_ab_measurements.txt)
 template <typename TP>
@@ -763,10 +797,7 @@ __device__ __forceinline__ void yl_exact_pass(const YlParams& p, unsigned int gw
       hit = hit || ((bal >> (16 * half)) & 0xffffu) != 0u;
     }
     if (valid && sub == 0) {
-      const float e = yl_record_term(p, l, img, ain, obj, pobj, hit, false);
-      // non-finite terms (NaN / inf logits) cannot be carried in fixed point: they poison the sum through the top bit pattern
-      if (e == e && e < 1.0e9f) atomicAdd(p.obj_fixed + l, (unsigned long long)((double)e * YL_FIXED_ONE + 0.5));
-      else atomicOr(p.obj_fixed + l, 0x8000000000000000ull);
+      yl_obj_sum_add(p.obj_sum, gwarp, l, yl_record_term(p, l, img, ain, obj, pobj, hit, false));
     }
   }
 }
@@ -789,7 +820,7 @@ struct YlFinalize {
   double* slices;          // [YL_FIN_CTAS][12]
   unsigned int* ticket;    // zero on entry; reset by the last CTA
   B200Exchange xchg;       // data parallel: the 12 terms are summed over the ranks inside this kernel (world 1: no-op)
-  const unsigned long long* obj_fixed;  // [3] or null: object-loss terms of the records K4b-exact decided (2^-32 fixed point)
+  const YlObjSum* obj_sum;  // or null: object-loss terms of the records K4b-exact decided
   int publish_only;        // 1: store this rank's terms into the peers' mailboxes and return (b200_yolo_loss_collect_peer finishes)
 };
 
@@ -842,13 +873,30 @@ __global__ void __launch_bounds__(YL_FIN_THREADS) yolo_loss_finalize_kernel(YlFi
   __threadfence();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   if (warp == 0) {
+    // the exact pass's sums: lane i reads stripe i, the warp adds the stripes (integers: any order), and lane 4l+2 keeps
+    // the three limb sums of level l
+    unsigned long long w0 = 0ull, w1 = 0ull, w2 = 0ull;
+    if (f.obj_sum) {
+#pragma unroll 1
+      for (int i = 0; i < 3 * YL_LEVELS; ++i) {
+        unsigned long long x = __ldcg(&f.obj_sum->limb[lane % YL_OBJ_STRIPES][i]);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+        if (i % YL_LEVELS == (lane >> 2)) {
+          if (i < YL_LEVELS) w0 = x;
+          else if (i < 2 * YL_LEVELS) w1 = x;
+          else w2 = x;
+        }
+      }
+    }
     float v = 0.0f;
     if (lane < 12) {
       double s = 0.0;
       for (int g = 0; g < YL_FIN_CTAS; ++g) s += __ldcg(f.slices + g * 12 + lane);
-      if (f.obj_fixed && (lane & 3) == 2) {
-        const unsigned long long fx = __ldcg(f.obj_fixed + (lane >> 2));
-        s += (fx >> 63) ? (double)__longlong_as_double(0x7ff8000000000000ll) : (double)fx * (1.0 / YL_FIXED_ONE);   // top bit = a non-finite term
+      if (f.obj_sum && (lane & 3) == 2) {
+        const unsigned long long lo = w0 + (w1 << 32);
+        const unsigned long long hi = w2 + (w1 >> 32) + (lo < w0 ? 1ull : 0ull);
+        s += ((double)hi * YL_FIXED_ONE + (double)lo * (1.0 / YL_FIXED_ONE)) + __ldcg(&f.obj_sum->side[lane >> 2]);
       }
       v = DM_DIV((float)s, f.batch_divisor);  // reduce_sum(...) / batch_size_float, tyu:120-123
     }
@@ -1135,8 +1183,9 @@ static YlWs yl_layout(const int32_t hw[6], int B, int A, int* n_img_out, YlLevel
   w.n_cta = cta;
   w.n_cta_obj = octa;
   size_t o = 0;
-  // zeroed per call: object counts [B,3], the finalize ticket, the pending-record count (+ pad to 8), 3 fixed-point sums
-  w.cnt_bytes = b200_align_up(sizeof(int32_t) * ((size_t)B * YL_LEVELS + 2), 8) + 3 * sizeof(unsigned long long) + sizeof(unsigned int) * (size_t)B * YL_LEVELS;
+  // zeroed per call: object counts [B,3], the finalize ticket, the pending-record count (+ pad to 8), the exact pass's
+  // object-loss sums, the scan tickets [B,3]
+  w.cnt_bytes = b200_align_up(sizeof(int32_t) * ((size_t)B * YL_LEVELS + 2), 8) + sizeof(YlObjSum) + sizeof(unsigned int) * (size_t)B * YL_LEVELS;
   w.cnt = o; o = b200_align_up(o + w.cnt_bytes, 256);
   w.obj = o; o = b200_align_up(o + sizeof(float) * (size_t)B * n_img, 256);
   w.gt = o; o = b200_align_up(o + sizeof(float4) * (size_t)B * n_img, 256);
@@ -1268,9 +1317,9 @@ static int yolo_loss_impl(const float* const y_true[3], const void* const y_pred
   if (stages & 1) B200_CUDA(cudaMemsetAsync(wsb + ws.cnt, 0, ws.cnt_bytes, stream));
   p.pend_queue = reinterpret_cast<uint32_t*>(wsb + ws.pend);
   p.pend_count = reinterpret_cast<unsigned int*>(wsb + ws.cnt) + (size_t)B * YL_LEVELS + 1;
-  p.obj_fixed = reinterpret_cast<unsigned long long*>(wsb + ws.cnt + b200_align_up(sizeof(int32_t) * ((size_t)B * YL_LEVELS + 2), 8));
+  p.obj_sum = reinterpret_cast<YlObjSum*>(wsb + ws.cnt + b200_align_up(sizeof(int32_t) * ((size_t)B * YL_LEVELS + 2), 8));
   // full dense call: the scan's last CTA per (image, level) prepares the GT list (stage hooks keep K4a' as its own launch)
-  p.scan_ticket = (!sparse && (stages & 3) == 3) ? reinterpret_cast<unsigned int*>(p.obj_fixed + 3) : nullptr;
+  p.scan_ticket = (!sparse && (stages & 3) == 3) ? reinterpret_cast<unsigned int*>(p.obj_sum + 1) : nullptr;
   p.sp_t = nullptr; p.sp_cls = nullptr; p.obj_bits = nullptr; p.bits_words = 0;
   if (sparse) {
     t.boxes = sparse->boxes; t.classes = sparse->classes; t.offsets = sparse->offsets; t.B = B; t.total = sparse->total_boxes;
@@ -1308,9 +1357,9 @@ static int yolo_loss_impl(const float* const y_true[3], const void* const y_pred
     // ~12 k undecided records costs 15.6 us as a launch of its own and rides in the widened finalize launch instead.
     use_split = !host_pred && aligned16 && p.RF >= 8;
     if (use_split) {
-      // the queue counter and the fixed-point sums are zeroed with the object counts (stage 1); the stage hook may run this
+      // the queue counter and the object-loss sums are zeroed with the object counts (stage 1); the stage hook may run this
       // pass on its own, repeatedly
-      if (!(stages & 1)) B200_CUDA(cudaMemsetAsync(p.pend_count, 0, (size_t)(reinterpret_cast<unsigned char*>(p.obj_fixed + 3) - reinterpret_cast<unsigned char*>(p.pend_count)), stream));
+      if (!(stages & 1)) B200_CUDA(cudaMemsetAsync(p.pend_count, 0, (size_t)(reinterpret_cast<unsigned char*>(p.obj_sum + 1) - reinterpret_cast<unsigned char*>(p.pend_count)), stream));
       B200_DISPATCH_DTYPE(ty.pred, TP, yolo_loss_ignore_lean_kernel<TP><<<grid, YL_ICHUNK, 0, stream>>>(p));
       if (!(stages & 8)) {   // no finalize in this call: the exact pass as a launch of its own (the finalize launch carries it otherwise)
         B200_LAUNCH_CHECK();
@@ -1329,7 +1378,7 @@ static int yolo_loss_impl(const float* const y_true[3], const void* const y_pred
   f.slices = reinterpret_cast<double*>(wsb + ws.fin);
   f.ticket = reinterpret_cast<unsigned int*>(wsb + ws.cnt) + (size_t)B * YL_LEVELS;
   f.publish_only = publish_only;
-  f.obj_fixed = p.obj_fixed;   // zero unless K4b-exact ran
+  f.obj_sum = p.obj_sum;   // zero unless K4b-exact ran
   if (xchg) f.xchg = *xchg;
   else { f.xchg.rank = 0; f.xchg.world = 1; for (int r = 0; r < B200_XCHG_MAX_WORLD; ++r) f.xchg.mailbox[r] = nullptr; }
   // split form: the finalize launch is widened to 4 CTAs per SM and resolves the queued records first
