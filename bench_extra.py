@@ -444,6 +444,8 @@ def main():
         _half_heads(args, dev, g, anc, tyu, Anchors, synth, report, wrap, want)
     if want("c2_half_train"):
         _half_train(args, dev, g, anc, tyu, DataGenerator, synth, report, wrap)
+    if want("c3_half_train"):
+        _effdet_half_train(args, dev, g, Anchors, synth, report, wrap)
 
 
 def _half_heads(args, dev, g, anc, tyu, Anchors, synth, report, wrap, want):
@@ -615,6 +617,100 @@ def _half_train(args, dev, g, anc, tyu, DataGenerator, synth, report, wrap):
                                              "what": "y_pred read (dense equivalent) + gradient written"},
                 speedup_bf16_vs_cast_then_fp32=ms["bf16_cast_then_fp32"] / ms["bf16"],
                 speedup_bf16_vs_fp32=ms["fp32"] / ms["bf16"], speedup_fp16_vs_fp32=ms["fp32"] / ms["fp16_scaled"],
+                window_ms={k: [round(t, 5) for t in v] for k, v in times.items()}, outputs_bit_identical=True))
+
+
+
+def _effdet_half_train(args, dev, g, Anchors, synth, report, wrap):
+    """The EfficientDet training step from box lists (get_loss_from_boxes_and_grad) on D0 512 B=128 C=81 heads in fp32,
+    bf16 and fp16, each writing its gradients in the heads' type (fp16 with a device loss scale of 1024), against "bf16
+    cast to fp32, fp32 call, gradients cast back to bf16" (what a mixed-precision user does with an fp32-only loss).
+    Beside them the dense class-id path (generate_targets_batch(class_index=True) + get_loss_and_grad) in bf16 and a
+    forward-only get_loss_from_boxes pair.  Ground truth as in c3_sparse_backward; the heads hold N(0, 1) logits (box
+    outputs N(0, 0.25)) rounded to bf16 values that fp16 also holds exactly, so every arm's loss has the same bits and
+    every gradient is round(g32 * s) of the fp32 arm's g32: asserted before anything is timed.  7 windows per arm,
+    alternating, the order rotated window by window."""
+    import torch
+    from tfmv_b200.ai_models.efficientnet.efficientdet_net_train import (get_loss_and_grad, get_loss_from_boxes,
+                                                                         get_loss_from_boxes_and_grad)
+    card = _card()
+    c = synth.EFFDET_CONFIGS["d0"]
+    batch, C = 128, 81
+    a = Anchors(c["min_level"], c["max_level"], c["image_size"], c["num_scales"], c["aspect_ratios"], c["anchor_scale"])
+    shapes = [tuple(b.shape) for b in a.boxes]
+    n_anchor = sum(s[0] * s[1] * s[2] for s in shapes)
+
+    def values(shape, sd):
+        x = (torch.randn(shape, device=dev, generator=g) * sd).to(torch.bfloat16).float()
+        x[x.abs() < 1e-4] = 0.0   # below fp16's normal range a bf16 value may not be exact in fp16
+        return x
+
+    f32 = ([values((batch,) + s, 0.25) for s in shapes], [values((batch,) + s[:-1] + (C,), 1.0) for s in shapes])
+    heads = {"fp32": f32, "bf16": tuple([t.to(torch.bfloat16) for t in f] for f in f32),
+             "fp16": tuple([t.to(torch.float16) for t in f] for f in f32)}
+    assert all(torch.equal(x.float(), y) for k in ("bf16", "fp16") for f, w in zip(heads[k], f32) for x, y in zip(f, w))
+    rng = np.random.default_rng(20261018 + 3)
+    boxes, classes, off = synth.gt_batch(rng, batch, (c["image_size"][1], c["image_size"][0]), max_boxes=100, order="yxyx")
+    gt = (torch.from_numpy(boxes).to(dev), torch.from_numpy((classes + 1).astype(np.int32)).to(dev), torch.from_numpy(off).to(dev))
+    scale = torch.full((1,), 1024.0, dtype=torch.float32, device=dev)   # fp16 loss scale, read on the device
+
+    def train(h, **gkw):
+        return get_loss_from_boxes_and_grad(a, *gt, *h, **gkw)
+
+    def cast_then_fp32():
+        loss, gb, gc = train(tuple([t.float() for t in f] for f in heads["bf16"]))
+        return loss, tuple(t.to(torch.bfloat16) for t in gb), tuple(t.to(torch.bfloat16) for t in gc)
+
+    def dense(h, **gkw):
+        return get_loss_and_grad(*a.generate_targets_batch(*gt, C, class_index=True), *h, **gkw)
+
+    fns = {
+        "fp32": lambda: train(heads["fp32"]),
+        "bf16": lambda: train(heads["bf16"], grad_dtype=torch.bfloat16),
+        "fp16_scaled": lambda: train(heads["fp16"], grad_dtype=torch.float16, grad_scale=scale),
+        "bf16_cast_then_fp32": cast_then_fp32,
+        "dense_class_id_bf16": lambda: dense(heads["bf16"], grad_dtype=torch.bfloat16),
+        "forward_fp32": lambda: get_loss_from_boxes(a, *gt, *heads["fp32"]),
+        "forward_bf16": lambda: get_loss_from_boxes(a, *gt, *heads["bf16"]),
+    }
+
+    def same(x, y):   # bit equality, NaN positions equal (payloads not compared)
+        x, y = x.float(), y.float()
+        return torch.equal(torch.isnan(x), torch.isnan(y)) and torch.equal(torch.nan_to_num(x).view(torch.int32),
+                                                                           torch.nan_to_num(y).view(torch.int32))
+
+    def check(name, got, ref, s, dt):
+        assert same(got[0], ref[0]), "%s: loss bits differ from the fp32 arm" % name
+        for x, y in zip(got[1] + got[2], ref[1] + ref[2]):
+            assert x.dtype == dt and same(x, (y if s is None else y * s).to(dt)), "%s: gradient bits differ" % name
+
+    ref = fns["fp32"]()
+    check("bf16", fns["bf16"](), ref, None, torch.bfloat16)
+    check("fp16_scaled", fns["fp16_scaled"](), ref, 1024.0, torch.float16)
+    check("bf16_cast_then_fp32", fns["bf16_cast_then_fp32"](), ref, None, torch.bfloat16)
+    check("dense_class_id_bf16", fns["dense_class_id_bf16"](), dense(heads["fp32"]), None, torch.bfloat16)
+    assert same(fns["forward_bf16"](), fns["forward_fp32"]()) and same(fns["forward_fp32"](), ref[0]), \
+        "forward: loss bits differ between the arms"
+    del ref
+    fns = {k: wrap(f) for k, f in fns.items()}
+    steps, n_win = max(args.steps, 20), 7
+    times = {k: [] for k in fns}
+    order = list(fns)
+    for w in range(n_win):
+        for k in order[w % len(order):] + order[:w % len(order)]:
+            times[k].append(timed(fns[k], steps, args.warmup))
+    ms = {k: float(np.median(v)) for k, v in times.items()}
+    # per anchor: logits read + gradient written (C each), box outputs read + gradient written (4 each), one int32 match
+    # written and read
+    by_type = {"fp32": n_anchor * ((2 * C + 8) * 4 + 8), "half": n_anchor * ((2 * C + 8) * 2 + 8)}
+    report("c3_half_train", "EfficientDet-D0 512 B=128 C=81 get_loss_from_boxes_and_grad from bf16 / fp16 heads, gradients in "
+           "the heads' type; arms bit-identical (asserted); median of %d alternating windows of %d steps" % (n_win, steps), batch,
+           ms["bf16"], by_type["half"],
+           dict(card, arms_ms=ms, algorithmic_bytes_per_image_by_type=dict(by_type, what="heads read + gradients written + "
+                                                                           "one int32 match written and read, per anchor"),
+                speedup_bf16_vs_cast_then_fp32=ms["bf16_cast_then_fp32"] / ms["bf16"],
+                speedup_bf16_vs_fp32=ms["fp32"] / ms["bf16"], speedup_fp16_vs_fp32=ms["fp32"] / ms["fp16_scaled"],
+                speedup_forward_bf16_vs_fp32=ms["forward_fp32"] / ms["forward_bf16"],
                 window_ms={k: [round(t, 5) for t in v] for k, v in times.items()}, outputs_bit_identical=True))
 
 

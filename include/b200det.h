@@ -45,10 +45,10 @@ enum {
   B200_METRIC_COUNT = 7
 };
 
-/* Element type of the head tensors that the *_typed post-processing and YOLO loss entries read.  bf16 and fp16 heads
- * (Keras mixed_bfloat16 / mixed_float16, torch autocast) are read in place and widened to fp32 exactly on load: every
- * output is bit-identical to the fp32 entry on the widened tensors.  Outputs, decoded boxes and workspaces stay fp32,
- * except the gradient of the typed YOLO loss entries, which is written in the element type the caller asks for. */
+/* Element type of the head tensors that the *_typed post-processing, YOLO loss and EfficientDet loss entries read.  bf16
+ * and fp16 heads (Keras mixed_bfloat16 / mixed_float16, torch autocast) are read in place and widened to fp32 exactly on
+ * load: every output is bit-identical to the fp32 entry on the widened tensors.  Outputs, decoded boxes and workspaces
+ * stay fp32, except the gradients of the typed loss entries, which are written in the element type the caller asks for. */
 enum { B200_DTYPE_F32 = 0, B200_DTYPE_BF16 = 1, B200_DTYPE_F16 = 2 };
 
 /* NMS survivor predicate. */
@@ -360,6 +360,23 @@ int b200_focal_box_partial_sums_indexed(int num_levels, const unsigned long long
                                         const float* const pred_classes[], float alpha, float gamma, float delta,
                                         float label_smoothing, double* sums_out, void* workspace, size_t workspace_bytes,
                                         void* stream);
+/* b200_focal_box_partial_sums(_indexed) on heads of element type pred_dtype (B200_DTYPE_*), shared by every box level
+ * and every class level.  Targets, masks, sums and the workspace stay as they are; every level's tensors stay 16-byte
+ * aligned.  The kernels keep the fp32 entry's CTA plan and summation order, so sums_out is bit-identical to the fp32 call
+ * on the widened heads.  The fp32 entries are the B200_DTYPE_F32 case; every argument is checked before anything is
+ * enqueued. */
+int b200_focal_box_partial_sums_typed(int num_levels, const unsigned long long* anchors_per_level, int C,
+                                      const float* const true_boxes[], const float* const true_classes[],
+                                      const unsigned char* const true_masks[], const void* const pred_boxes[],
+                                      const void* const pred_classes[], int pred_dtype, float alpha, float gamma, float delta,
+                                      float label_smoothing, double* sums_out, void* workspace, size_t workspace_bytes,
+                                      void* stream);
+int b200_focal_box_partial_sums_indexed_typed(int num_levels, const unsigned long long* anchors_per_level, int C,
+                                              const float* const true_boxes[], const int32_t* const true_class_index[],
+                                              const unsigned char* const true_masks[], const void* const pred_boxes[],
+                                              const void* const pred_classes[], int pred_dtype, float alpha, float gamma,
+                                              float delta, float label_smoothing, double* sums_out, void* workspace,
+                                              size_t workspace_bytes, void* stream);
 int b200_focal_box_finalize(int num_levels, const double* sums, const double* numel_per_level_host, float* out_parts,
                             float* out_loss, float* out_num_positives, void* stream);
 /* Backward of _get_loss (SURVEY §8f N1): grad_classes[l] = d loss / d pred_classes[l], grad_boxes[l] = d loss /
@@ -378,6 +395,25 @@ int b200_focal_box_grad_indexed(int num_levels, const unsigned long long* anchor
                                 float gamma, float delta, float label_smoothing, const double* sums,
                                 const double* numel_per_level_host, float* const grad_boxes[],
                                 float* const grad_classes[], void* stream);
+/* b200_focal_box_grad(_indexed) on heads of element type pred_dtype (shared by both head families), writing grad_boxes /
+ * grad_classes (16-byte aligned levels) in element type grad_dtype (shared by both gradient families).  Each gradient
+ * element is round(g * s) with one rounding to nearest even (fp16 overflow gives +-inf), where g is the fp32 entry's
+ * gradient on the widened heads and s = *grad_scale_dev, a device fp32 scalar such as a loss scale (no host
+ * synchronisation, graph-capturable); grad_scale_dev NULL: no multiply.  The scale multiplies the normalised gradient,
+ * it is not folded into the normalisation.  The fp32 entries are the (F32, F32, NULL) case; every argument is checked
+ * before anything is enqueued. */
+int b200_focal_box_grad_typed(int num_levels, const unsigned long long* anchors_per_level, int C,
+                              const float* const true_boxes[], const float* const true_classes[],
+                              const void* const pred_boxes[], const void* const pred_classes[], int pred_dtype, float alpha,
+                              float gamma, float delta, float label_smoothing, const double* sums,
+                              const double* numel_per_level_host, void* const grad_boxes[], void* const grad_classes[],
+                              int grad_dtype, const float* grad_scale_dev, void* stream);
+int b200_focal_box_grad_indexed_typed(int num_levels, const unsigned long long* anchors_per_level, int C,
+                                      const float* const true_boxes[], const int32_t* const true_class_index[],
+                                      const void* const pred_boxes[], const void* const pred_classes[], int pred_dtype,
+                                      float alpha, float gamma, float delta, float label_smoothing, const double* sums,
+                                      const double* numel_per_level_host, void* const grad_boxes[],
+                                      void* const grad_classes[], int grad_dtype, const float* grad_scale_dev, void* stream);
 
 /* generate_targets + _get_loss and its backward from box lists (SURVEY §8f N3 + N1; an API extension): no dense targets.
  * gt_boxes [total,4] y1,x1,y2,x2 (16-byte aligned), gt_classes [total] int32, gt_offsets [B+1] as for
@@ -402,6 +438,16 @@ int b200_effdet_loss_from_boxes_grad(int num_levels, const int32_t* hw, int A, c
                                      float gamma, float delta, float label_smoothing, const double* numel_per_level_host,
                                      double* sums, float* const grad_boxes[], float* const grad_classes[], void* workspace,
                                      size_t workspace_bytes, void* stream);
+/* b200_effdet_loss_from_boxes_grad on heads of element type pred_dtype, the gradients in element type grad_dtype scaled
+ * by *grad_scale_dev, as b200_focal_box_grad_typed is to b200_focal_box_grad: sums bit-identical to the fp32 call on the
+ * widened heads, each gradient element round(g * s).  The match stage reads no heads and is shared. */
+int b200_effdet_loss_from_boxes_grad_typed(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
+                                           const float* gt_boxes, const int32_t* gt_classes, int total_boxes,
+                                           const void* const pred_boxes[], const void* const pred_classes[], int pred_dtype,
+                                           float alpha, float gamma, float delta, float label_smoothing,
+                                           const double* numel_per_level_host, double* sums, void* const grad_boxes[],
+                                           void* const grad_classes[], int grad_dtype, const float* grad_scale_dev,
+                                           void* workspace, size_t workspace_bytes, void* stream);
 
 /* Serving-path box post-processing (SURVEY §8f N4; views/object_detection.py:70-85): boxes [B,max_rows,4] normalised
  * x1,y1,x2,y2 on the letterboxed image (image_size = (w,h) of the network input, padding = (top,bottom,left,right) of

@@ -74,6 +74,16 @@ SIGNATURES = {
     "b200_effdet_loss_from_boxes_match": (c_i, [c_i, c_p, c_i, c_p, c_i, c_p, c_p, c_i, c_f, c_p, c_p, c_sz, c_p]),
     "b200_effdet_loss_from_boxes_grad": (c_i, [c_i, c_p, c_i, c_p, c_i, c_i, c_p, c_p, c_i, c_p, c_p, c_f, c_f, c_f, c_f, c_p, c_p,
                                                c_p, c_p, c_p, c_sz, c_p]),
+    "b200_focal_box_partial_sums_typed": (c_i, [c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_p, c_i, c_f, c_f, c_f, c_f, c_p, c_p, c_sz,
+                                                c_p]),
+    "b200_focal_box_partial_sums_indexed_typed": (c_i, [c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_p, c_i, c_f, c_f, c_f, c_f, c_p, c_p,
+                                                        c_sz, c_p]),
+    "b200_focal_box_grad_typed": (c_i, [c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_i, c_f, c_f, c_f, c_f, c_p, c_p, c_p, c_p, c_i, c_p,
+                                        c_p]),
+    "b200_focal_box_grad_indexed_typed": (c_i, [c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_i, c_f, c_f, c_f, c_f, c_p, c_p, c_p, c_p, c_i,
+                                                c_p, c_p]),
+    "b200_effdet_loss_from_boxes_grad_typed": (c_i, [c_i, c_p, c_i, c_p, c_i, c_i, c_p, c_p, c_i, c_p, c_p, c_i, c_f, c_f, c_f, c_f,
+                                                     c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_sz, c_p]),
     "b200_row_positions_workspace_bytes": (c_sz, [ctypes.c_longlong]),
     "b200_row_positions": (c_i, [c_p, ctypes.c_longlong, c_p, c_p, c_p, c_sz, c_p]),
     "b200_gather_rows": (c_i, [c_p, c_i, c_p, c_p, ctypes.c_longlong, c_p, c_p]),

@@ -29,7 +29,7 @@ def to_cuda(x, dtype=torch.float32):
     return t.contiguous()
 
 
-# element-type codes of the C ABI (B200_DTYPE_*) for the head dtypes the post-processing and the YOLO loss read in place
+# element-type codes of the C ABI (B200_DTYPE_*) for the head dtypes the post-processing and the losses read in place
 DTYPE_F32 = 0
 _HALF_CODES = {torch.bfloat16: 1, torch.float16: 2}
 DTYPE_CODES = {torch.float32: DTYPE_F32, **_HALF_CODES}
@@ -50,6 +50,27 @@ def to_cuda_heads(xs, keep_pinned=False):
     dtype = ts[0].dtype if code != DTYPE_F32 else torch.float32
     keep = lambda x, t: keep_pinned and t is x and t.dtype == dtype and is_pinned_host_f32(t)
     return [t if keep(x, t) else to_cuda(t, dtype) for x, t in zip(xs, ts)], code
+
+
+def grad_code(grad_dtype):
+    """B200_DTYPE_* code of the gradient dtype of a loss backward call (checked before anything touches the device)."""
+    code = DTYPE_CODES.get(grad_dtype)
+    if code is None:
+        raise ValueError("grad_dtype must be torch.float32, torch.bfloat16 or torch.float16, not %r" % (grad_dtype,))
+    return code
+
+
+def grad_out(heads, grad_dtype, grad_scale):
+    """The gradient tensors of a loss backward call (shaped like `heads`, of grad_dtype), their B200_DTYPE_* code and the
+    scale tensor (1-element fp32 on the heads' device, or None; a Python float is put there)."""
+    code = grad_code(grad_dtype)
+    dev = heads[0].device
+    if grad_scale is not None and not isinstance(grad_scale, torch.Tensor):
+        grad_scale = torch.full((1,), float(grad_scale), dtype=torch.float32, device=dev)
+    if grad_scale is not None and (grad_scale.dtype != torch.float32 or grad_scale.numel() != 1 or grad_scale.device != dev):
+        raise ValueError("grad_scale must be a 1-element float32 tensor on %s, or a Python float" % dev)
+    grads = [torch.empty(t.shape, dtype=grad_dtype, device=dev) for t in heads]
+    return grads, code, grad_scale
 
 
 def is_pinned_host_f32(x):

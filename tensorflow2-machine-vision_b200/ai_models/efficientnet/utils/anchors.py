@@ -340,7 +340,8 @@ class Anchors(object):
     utils.mAP.Get_mAP_padded(boxes, classes, offsets, out, classes_num).'''
     assert iou_type in ('iou', 'giou', 'diou', 'ciou')
     from ..efficientdet_net_train import _from_boxes_args
-    gb, gc, go, rel, cl, B, C = _from_boxes_args(self, boxes, classes, offsets, y_pred_boxes, y_pred_classes)
+    gb, gc, go, rel, cl, _, B, C = _from_boxes_args(self, boxes, classes, offsets, y_pred_boxes, y_pred_classes)
+    rel, cl = [T.to_cuda(t) for t in rel], [T.to_cuda(t) for t in cl]   # the tiled stream reads fp32 heads
     if C < 4 or C > 128:
       # the one-pass stream rebuilds one-hot rows a float4 at a time (C >= 4) and stages 64-anchor tiles of logits in
       # shared memory (C <= 128): other heads take the dense targets — same results

@@ -6,8 +6,23 @@ import torch
 from ... import _lib, _tensors as T
 
 
+def _pred_heads(pred_boxes, pred_classes):
+  '''Box outputs and class logits of the loss (either list may be None or hold None levels) -> (box levels, class levels,
+  B200_DTYPE_* code shared by both).  When every given level is bf16, or every one is fp16, the levels stay in their type
+  and the kernels read them in place: sums and gradients are those of the call on the widened heads (y.float()).  Any
+  other mix, fp32 logits with bf16 boxes included, is cast to fp32.'''
+  pb, pc = list(pred_boxes or []), list(pred_classes or [])
+  given = [k for k, t in enumerate(pb + pc) if t is not None]
+  heads, code = T.to_cuda_heads([(pb + pc)[k] for k in given])
+  out = [None] * (len(pb) + len(pc))
+  for k, h in zip(given, heads):
+    out[k] = h
+  return (out[:len(pb)] if pred_boxes is not None else None), (out[len(pb):] if pred_classes is not None else None), code
+
+
 def _partial_sums(true_boxes, true_classes, true_masks, pred_boxes, pred_classes, alpha, gamma, delta, label_smoothing):
-  '''Levels -> device fp64 sums [2L+1] = focal_l..., huber_l..., positives.  Any of the class / box halves may be None.'''
+  '''Levels -> device fp64 sums [2L+1] = focal_l..., huber_l..., positives.  Any of the class / box halves may be None.
+  Heads: see _pred_heads.'''
   lib = _lib.load()
   L = len(pred_classes) if pred_classes is not None else len(pred_boxes)
   none = [None] * L
@@ -17,8 +32,8 @@ def _partial_sums(true_boxes, true_classes, true_masks, pred_boxes, pred_classes
   indexed = true_classes is not None and any(t is not None and not torch.is_floating_point(torch.as_tensor(t)) for t in true_classes)
   tc = [(T.to_cuda(t, torch.int32) if indexed else T.to_cuda(t)) if t is not None else None for t in (true_classes or none)]
   tm = [T.to_cuda(t, torch.bool) if t is not None else None for t in (true_masks or none)]
-  pb = [T.to_cuda(t) if t is not None else None for t in (pred_boxes or none)]
-  pc = [T.to_cuda(t) if t is not None else None for t in (pred_classes or none)]
+  pb, pc, pdt = _pred_heads(pred_boxes, pred_classes)
+  pb, pc = pb or none, pc or none
   C = next((t.shape[-1] for t in pc if t is not None), 1)
   anchors, numel = [], []
   for l in range(L):
@@ -41,10 +56,9 @@ def _partial_sums(true_boxes, true_classes, true_masks, pred_boxes, pred_classes
   sums = torch.empty((2 * L + 1,), dtype=torch.float64, device=dev)
   ws_bytes = max(int(lib.b200_focal_box_workspace_bytes(L, anc, max(C, 4))), 256)
   ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-  fn = lib.b200_focal_box_partial_sums_indexed if indexed else lib.b200_focal_box_partial_sums
-  _lib.check(fn(L, anc, C, arr(tb), arr(tc), arr(tm), arr(pb), arr(pc), float(alpha),
-                                             float(gamma), float(delta), float(label_smoothing), T.ptr(sums), T.ptr(ws),
-                                             ws_bytes, T.stream_ptr()), 'focal/box loss')
+  fn = lib.b200_focal_box_partial_sums_indexed_typed if indexed else lib.b200_focal_box_partial_sums_typed
+  _lib.check(fn(L, anc, C, arr(tb), arr(tc), arr(tm), arr(pb), arr(pc), pdt, float(alpha), float(gamma), float(delta),
+                float(label_smoothing), T.ptr(sums), T.ptr(ws), ws_bytes, T.stream_ptr()), 'focal/box loss')
   return sums, numel
 
 

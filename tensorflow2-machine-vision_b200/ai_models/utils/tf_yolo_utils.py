@@ -166,27 +166,6 @@ def _pred_levels(y_pred, with_grad):
   return T.to_cuda_heads(y_pred, keep_pinned=not with_grad)
 
 
-def _grad_code(grad_dtype):
-  '''B200_DTYPE_* code of a gradient dtype (checked before anything touches the device).'''
-  code = T.DTYPE_CODES.get(grad_dtype)
-  if code is None:
-    raise ValueError('grad_dtype must be torch.float32, torch.bfloat16 or torch.float16, not %r' % (grad_dtype,))
-  return code
-
-
-def _grad_out(yp, grad_dtype, grad_scale):
-  '''The gradient tensors (shaped like y_pred, of grad_dtype) and the scale tensor (1-element fp32 on y_pred's device, or
-  None) of a backward call, and the gradient's B200_DTYPE_* code.'''
-  code = _grad_code(grad_dtype)
-  dev = yp[0].device
-  if grad_scale is not None and not isinstance(grad_scale, torch.Tensor):
-    grad_scale = torch.full((1,), float(grad_scale), dtype=torch.float32, device=dev)
-  if grad_scale is not None and (grad_scale.dtype != torch.float32 or grad_scale.numel() != 1 or grad_scale.device != dev):
-    raise ValueError('grad_scale must be a 1-element float32 tensor on %s, or a Python float' % dev)
-  grads = [torch.empty(t.shape, dtype=grad_dtype, device=dev) for t in yp]
-  return grads, code, grad_scale
-
-
 def _loss_call(y_true, y_pred, image_wh, anchors_wh, iou_thresh, iou_type, variant, batch_divisor=None,
                return_parts=False, workspace=None, ignore_out=None, with_grad=False, exchange=None, defer_collect=False,
                grad_dtype=torch.float32, grad_scale=None):
@@ -199,7 +178,7 @@ def _loss_call(y_true, y_pred, image_wh, anchors_wh, iou_thresh, iou_type, varia
   if len(y_true) != 3 or len(y_pred) != 3:
     raise ValueError('y_true and y_pred must each hold 3 levels')
   if with_grad:
-    _grad_code(grad_dtype)
+    T.grad_code(grad_dtype)
   yt = [T.to_cuda(t) for t in y_true]
   yp, pdt = _pred_levels(y_pred, with_grad)
   if pdt != T.DTYPE_F32 and exchange is not None and hasattr(exchange, 'mailboxes'):
@@ -227,7 +206,7 @@ def _loss_call(y_true, y_pred, image_wh, anchors_wh, iou_thresh, iou_type, varia
     workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
   div = float(B if batch_divisor is None else batch_divisor)
   if with_grad:
-    grads, gdt, scale = _grad_out(yp, grad_dtype, grad_scale)
+    grads, gdt, scale = T.grad_out(yp, grad_dtype, grad_scale)
     gp = (ctypes.c_void_p * 3)(*[t.data_ptr() for t in grads])
     _lib.check(lib.b200_yolo_loss_grad_typed(tp, pp, pdt, hw, B, A, RF - 5, anc.ctypes.data_as(ctypes.c_void_p),
                                              img.ctypes.data_as(ctypes.c_void_p), float(iou_thresh),
@@ -317,7 +296,7 @@ def _boxes_call(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_n
   '''Argument checks and marshalling of the sparse-target entries.  Returns (loss, parts, grads or None).'''
   lib = _lib.load()
   if with_grad:
-    _grad_code(grad_dtype)
+    T.grad_code(grad_dtype)
   yp, pdt = _pred_levels(y_pred, with_grad)
   boxes = T.to_cuda(boxes).reshape(-1, 4)
   classes = T.to_cuda(classes, torch.int32).reshape(-1)
@@ -346,7 +325,7 @@ def _boxes_call(classes, boxes, offsets, y_pred, image_wh, anchors_wh, classes_n
     workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
   div = float(B if batch_divisor is None else batch_divisor)
   if with_grad:
-    grads, gdt, scale = _grad_out(yp, grad_dtype, grad_scale)
+    grads, gdt, scale = T.grad_out(yp, grad_dtype, grad_scale)
     gp = (ctypes.c_void_p * 3)(*[t.data_ptr() for t in grads])
     _lib.check(lib.b200_yolo_loss_from_boxes_grad_typed(T.ptr(boxes), T.ptr(classes), T.ptr(offsets), total,
                                                         tanc.ctypes.data_as(ctypes.c_void_p), pp, pdt, hw, B, A, RF - 5,

@@ -64,6 +64,29 @@ __device__ __forceinline__ float4 ld4_f32(const H* p) {
   const H* h = reinterpret_cast<const H*>(&u);
   return make_float4(elem_f32(h[0]), elem_f32(h[1]), elem_f32(h[2]), elem_f32(h[3]));
 }
+// Gradient elements in the caller's type (float, __nv_bfloat16, __half): round_elem<TG>(scaled_f32(g, scale)) is
+// g * *scale (no multiply when scale is null) rounded once to nearest even, i.e. (g * s).to(dtype) in torch; fp16
+// overflow gives +-inf.
+__device__ __forceinline__ float scaled_f32(float g, const float* scale) { return scale ? g * __ldg(scale) : g; }
+template <typename TG> __device__ __forceinline__ TG round_elem(float v);
+template <> __device__ __forceinline__ float round_elem<float>(float v) { return v; }
+template <> __device__ __forceinline__ __nv_bfloat16 round_elem<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __half round_elem<__half>(float v) { return __float2half_rn(v); }
+template <typename TG> __device__ __forceinline__ uint32_t round_bits16(float v) {
+  const TG h = round_elem<TG>(v);
+  return (uint32_t)*reinterpret_cast<const unsigned short*>(&h);
+}
+// four consecutive gradient elements at a 4-element boundary, streaming (st.global.cs): one 16-byte store for fp32, one
+// 8-byte store of the four rounded values for the 2-byte types
+template <typename TG>
+__device__ __forceinline__ void st4(TG* p, float4 v) {
+  if constexpr (sizeof(TG) == 4) {
+    __stcs(reinterpret_cast<float4*>(p), v);
+  } else {
+    __stcs(reinterpret_cast<uint2*>(p), make_uint2(round_bits16<TG>(v.x) | (round_bits16<TG>(v.y) << 16),
+                                                   round_bits16<TG>(v.z) | (round_bits16<TG>(v.w) << 16)));
+  }
+}
 #endif
 
 // Runs the statements that follow `T` with T bound to the element type of a B200_DTYPE_* code (checked by the caller).

@@ -17,19 +17,33 @@
 #include "exchange.cuh"
 #include "effdet_focal.cuh"
 #include "effdet_anchor.cuh"
+#include <type_traits>
 
 #define EL_MAX_LEVELS 8
 #define EL_THREADS 256
 
+// Group i (elements 4i..4i+3) of a head or gradient tensor of element type T, addressed as element i of an array of
+// 4-element vectors (float4 / uint2): the address arithmetic of the fp32 kernels' float4 walk for every type.
+template <typename T>
+__device__ __forceinline__ T* el_group(T* base, unsigned long long i) {
+  using V = typename std::conditional<sizeof(T) == 4, float4, uint2>::type;
+  using CV = typename std::conditional<std::is_const<T>::value, const V, V>::type;
+  return reinterpret_cast<T*>(reinterpret_cast<CV*>(base) + i);
+}
+
+// Head tensors (cls_pred, cls_pred_tail, box_pred) are of the kernel's element type TP: fp32, bf16 or fp16, each element
+// widened to fp32 exactly on load.  The CTA plan, the 4-element group of index i, the tail of CTA 0 and the fp32
+// accumulators folded into fp64 every 64 groups are those of the fp32 instance, so every sum has the bits of the fp32
+// call on the widened heads.
 struct ElParams {
   int num_levels;
-  const float4* cls_pred[EL_MAX_LEVELS];
+  const void* cls_pred[EL_MAX_LEVELS];
   const float4* cls_true[EL_MAX_LEVELS];
   const int32_t* cls_index[EL_MAX_LEVELS];     // sparse-target mode: class id per anchor instead of the one-hot tensor
   int C;
   unsigned long long cls_vec[EL_MAX_LEVELS];   // float4 count of the class tensors
-  const float* cls_pred_tail[EL_MAX_LEVELS]; const float* cls_true_tail[EL_MAX_LEVELS]; int cls_tail[EL_MAX_LEVELS];
-  const float4* box_pred[EL_MAX_LEVELS];
+  const void* cls_pred_tail[EL_MAX_LEVELS]; const float* cls_true_tail[EL_MAX_LEVELS]; int cls_tail[EL_MAX_LEVELS];
+  const void* box_pred[EL_MAX_LEVELS];
   const float4* box_true[EL_MAX_LEVELS];
   const unsigned char* mask[EL_MAX_LEVELS];
   unsigned long long anchors[EL_MAX_LEVELS];   // B*H*W*A
@@ -39,7 +53,7 @@ struct ElParams {
 };
 
 // G15: gamma == 1.5 (the reference's value, global_params.py:186) — q^1.5 = q*sqrt(q) without a per-element branch
-template <bool G15>
+template <bool G15, typename TP>
 __global__ void __launch_bounds__(EL_THREADS) focal_box_partials_kernel(ElParams p) {
   __shared__ double s_red[EL_THREADS / 32][3];
   int l = 0;
@@ -50,7 +64,7 @@ __global__ void __launch_bounds__(EL_THREADS) focal_box_partials_kernel(ElParams
   const unsigned long long stride = (unsigned long long)ncta * EL_THREADS;
   float f0 = 0.f, f1 = 0.f;  // two fp32 accumulators per thread, folded into fp64 per thread at the end
   double focal = 0.0;
-  const float4* __restrict__ cp = p.cls_pred[l];
+  const TP* __restrict__ cp = static_cast<const TP*>(p.cls_pred[l]);
   const float4* __restrict__ ct = p.cls_true[l];
   const unsigned long long nv = p.cls_vec[l];
   unsigned long long i = (unsigned long long)cta * EL_THREADS + threadIdx.x;
@@ -62,39 +76,40 @@ __global__ void __launch_bounds__(EL_THREADS) focal_box_partials_kernel(ElParams
     const float oma = 1.0f - p.alpha, hls = 0.5f * p.label_smoothing;
 #pragma unroll 2
     for (; i < nv; i += stride) {
-      const float4 x = __ldcs(cp + i);
+      const float4 x = ld4_f32<true>(el_group(cp, i));
       f0 += el_focal_bg<G15>(x.x, oma, p.gamma, hls) + el_focal_bg<G15>(x.y, oma, p.gamma, hls);
       f1 += el_focal_bg<G15>(x.z, oma, p.gamma, hls) + el_focal_bg<G15>(x.w, oma, p.gamma, hls);
       if ((++it & 63) == 0) { focal += (double)f0 + (double)f1; f0 = f1 = 0.f; }
     }
-    if (cta == 0 && (int)threadIdx.x < p.cls_tail[l]) f0 += el_focal_bg<G15>(p.cls_pred_tail[l][threadIdx.x], oma, p.gamma, hls);
-    const float* __restrict__ logits = reinterpret_cast<const float*>(cp);
+    if (cta == 0 && (int)threadIdx.x < p.cls_tail[l])
+      f0 += el_focal_bg<G15>(elem_f32(static_cast<const TP*>(p.cls_pred_tail[l])[threadIdx.x]), oma, p.gamma, hls);
     const unsigned long long n_anchor = (nv * 4ull + (unsigned long long)p.cls_tail[l]) / (unsigned long long)p.C;
     for (unsigned long long a = (unsigned long long)cta * EL_THREADS + threadIdx.x; a < n_anchor; a += stride) {
       const int cls = __ldg(ci + a);
       if (cls >= 0 && cls < p.C) {  // tf.one_hot: ids outside [0, C) give an all-zero row
-        const float x = __ldg(logits + a * (unsigned long long)p.C + cls);
+        const float x = ldg_f32(cp + a * (unsigned long long)p.C + cls);
         f0 += el_focal<G15>(1.0f, x, p.alpha, p.gamma, p.label_smoothing) - el_focal_bg<G15>(x, oma, p.gamma, hls);
       }
     }
   } else {
 #pragma unroll 2
     for (; i < nv; i += stride) {
-      const float4 x = __ldcs(cp + i);
+      const float4 x = ld4_f32<true>(el_group(cp, i));
       const float4 y = __ldcs(ct + i);
       f0 += el_focal<G15>(y.x, x.x, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.y, x.y, p.alpha, p.gamma, p.label_smoothing);
       f1 += el_focal<G15>(y.z, x.z, p.alpha, p.gamma, p.label_smoothing) + el_focal<G15>(y.w, x.w, p.alpha, p.gamma, p.label_smoothing);
       if ((++it & 63) == 0) { focal += (double)f0 + (double)f1; f0 = f1 = 0.f; }
     }
     if (cta == 0 && (int)threadIdx.x < p.cls_tail[l])
-      f0 += el_focal<G15>(p.cls_true_tail[l][threadIdx.x], p.cls_pred_tail[l][threadIdx.x], p.alpha, p.gamma, p.label_smoothing);
+      f0 += el_focal<G15>(p.cls_true_tail[l][threadIdx.x], elem_f32(static_cast<const TP*>(p.cls_pred_tail[l])[threadIdx.x]), p.alpha,
+                          p.gamma, p.label_smoothing);
   }
   focal += (double)f0 + (double)f1;
   float hub = 0.f;
   unsigned int pos = 0;
   const unsigned long long na = p.anchors[l];
   for (unsigned long long a = (unsigned long long)cta * EL_THREADS + threadIdx.x; a < na; a += stride) {
-    const float4 o = __ldcs(p.box_pred[l] + a);
+    const float4 o = ld4_f32<true>(el_group(static_cast<const TP*>(p.box_pred[l]), a));
     const float4 t = __ldcs(p.box_true[l] + a);
     hub += el_huber(t.x, o.x, p.delta) + el_huber(t.y, o.y, p.delta) + el_huber(t.z, o.z, p.delta) + el_huber(t.w, o.w, p.delta);
     pos += p.mask[l][a] ? 1u : 0u;
@@ -167,19 +182,24 @@ __global__ void __launch_bounds__(32) focal_box_finalize_kernel(ElFinalize f) {
 //   df/dx = af * ( gamma q^(gamma-1) * (-(2y-1) p (1-p)) * ce + mod * (p - y_smoothed) );  scaled by 1/(num_pos*numel_l)
 // box:   d huber/d o = (|e| <= delta ? e : delta sign(e)) for target != 0, scaled by 50/(4 num_pos)
 // num_pos comes from the (all-reduced) partial sums and is a constant of the targets.
+// Heads of element type TP (widened exactly on load), gradients written in type TG: each element is
+// round_elem<TG>(scaled_f32(cs * focal_grad, scale)) (bs * huber_grad for boxes), so the fp32 value is the fp32 call's
+// and the scale is applied after the normalisation, with one rounding.  kScale: a scale pointer was given (the host
+// tests it, so the instances without a scale compile to the unscaled kernel).
 struct ElGradParams {
   int num_levels;
-  const float4* cls_pred[EL_MAX_LEVELS]; const float4* cls_true[EL_MAX_LEVELS]; float4* cls_grad[EL_MAX_LEVELS];
+  const void* cls_pred[EL_MAX_LEVELS]; const float4* cls_true[EL_MAX_LEVELS]; void* cls_grad[EL_MAX_LEVELS];
   const int32_t* cls_index[EL_MAX_LEVELS];  // sparse-target mode: class id per anchor instead of cls_true
   int C;
   unsigned long long cls_vec[EL_MAX_LEVELS];
   int cls_tail[EL_MAX_LEVELS];  // floats after the last whole float4
-  const float4* box_pred[EL_MAX_LEVELS]; const float4* box_true[EL_MAX_LEVELS]; float4* box_grad[EL_MAX_LEVELS];
+  const void* box_pred[EL_MAX_LEVELS]; const float4* box_true[EL_MAX_LEVELS]; void* box_grad[EL_MAX_LEVELS];
   unsigned long long anchors[EL_MAX_LEVELS];
   double numel[EL_MAX_LEVELS];
   int cta_base[EL_MAX_LEVELS + 1];
   float alpha, gamma, delta, label_smoothing;
   const double* sums;  // [2L+1], sums[2L] = positives
+  const float* scale;  // device fp32 gradient scale or null (no multiply)
 };
 
 // The focal derivative and, from the same intermediates, the focal value af*mod*ce (4 MUFU operations for both).
@@ -211,7 +231,9 @@ __device__ __forceinline__ float el_huber_grad(float t, float o, float delta) {
   return fabsf(e) <= delta ? e : copysignf(delta, e);
 }
 
+template <typename TP, typename TG, bool kScale>
 __global__ void __launch_bounds__(EL_THREADS) focal_box_grad_kernel(ElGradParams p) {
+  const float* scale = kScale ? p.scale : nullptr;
   int l = 0;
 #pragma unroll
   for (int k = 1; k < EL_MAX_LEVELS; ++k) if (k < p.num_levels && (int)blockIdx.x >= p.cta_base[k]) l = k;
@@ -226,7 +248,7 @@ __global__ void __launch_bounds__(EL_THREADS) focal_box_grad_kernel(ElGradParams
     const int32_t* __restrict__ ci = p.cls_index[l];
 #pragma unroll 2
     for (unsigned long long i = (unsigned long long)cta * EL_THREADS + threadIdx.x; i < nv; i += stride) {
-      const float4 x = __ldcs(p.cls_pred[l] + i);
+      const float4 x = ld4_f32<true>(el_group(static_cast<const TP*>(p.cls_pred[l]), i));
       float4 y;
       if (ci) {
         // the one-hot row generate_targets would have written: 1 at the anchor's class id, ids outside [0, C) -> zeros
@@ -245,11 +267,11 @@ __global__ void __launch_bounds__(EL_THREADS) focal_box_grad_kernel(ElGradParams
         y = __ldcs(p.cls_true[l] + i);
       }
       float4 g;
-      g.x = cs * el_focal_grad(y.x, x.x, p.alpha, p.gamma, p.label_smoothing);
-      g.y = cs * el_focal_grad(y.y, x.y, p.alpha, p.gamma, p.label_smoothing);
-      g.z = cs * el_focal_grad(y.z, x.z, p.alpha, p.gamma, p.label_smoothing);
-      g.w = cs * el_focal_grad(y.w, x.w, p.alpha, p.gamma, p.label_smoothing);
-      __stcs(p.cls_grad[l] + i, g);
+      g.x = scaled_f32(cs * el_focal_grad(y.x, x.x, p.alpha, p.gamma, p.label_smoothing), scale);
+      g.y = scaled_f32(cs * el_focal_grad(y.y, x.y, p.alpha, p.gamma, p.label_smoothing), scale);
+      g.z = scaled_f32(cs * el_focal_grad(y.z, x.z, p.alpha, p.gamma, p.label_smoothing), scale);
+      g.w = scaled_f32(cs * el_focal_grad(y.w, x.w, p.alpha, p.gamma, p.label_smoothing), scale);
+      st4(el_group(static_cast<TG*>(p.cls_grad[l]), i), g);
     }
     if (cta == 0 && (int)threadIdx.x < p.cls_tail[l]) {
       const unsigned long long e = nv * 4ull + threadIdx.x;
@@ -260,17 +282,18 @@ __global__ void __launch_bounds__(EL_THREADS) focal_box_grad_kernel(ElGradParams
       } else {
         yt = reinterpret_cast<const float*>(p.cls_true[l])[e];
       }
-      reinterpret_cast<float*>(p.cls_grad[l])[e] =
-          cs * el_focal_grad(yt, reinterpret_cast<const float*>(p.cls_pred[l])[e], p.alpha, p.gamma, p.label_smoothing);
+      static_cast<TG*>(p.cls_grad[l])[e] = round_elem<TG>(
+          scaled_f32(cs * el_focal_grad(yt, elem_f32(static_cast<const TP*>(p.cls_pred[l])[e]), p.alpha, p.gamma, p.label_smoothing), scale));
     }
   }
   if (p.box_grad[l]) {
     const unsigned long long na = p.anchors[l];
     for (unsigned long long a = (unsigned long long)cta * EL_THREADS + threadIdx.x; a < na; a += stride) {
-      const float4 o = __ldcs(p.box_pred[l] + a);
+      const float4 o = ld4_f32<true>(el_group(static_cast<const TP*>(p.box_pred[l]), a));
       const float4 t = __ldcs(p.box_true[l] + a);
-      __stcs(p.box_grad[l] + a, make_float4(bs * el_huber_grad(t.x, o.x, p.delta), bs * el_huber_grad(t.y, o.y, p.delta),
-                                             bs * el_huber_grad(t.z, o.z, p.delta), bs * el_huber_grad(t.w, o.w, p.delta)));
+      st4(el_group(static_cast<TG*>(p.box_grad[l]), a),
+          make_float4(scaled_f32(bs * el_huber_grad(t.x, o.x, p.delta), scale), scaled_f32(bs * el_huber_grad(t.y, o.y, p.delta), scale),
+                      scaled_f32(bs * el_huber_grad(t.z, o.z, p.delta), scale), scaled_f32(bs * el_huber_grad(t.w, o.w, p.delta), scale)));
     }
   }
 }
@@ -328,14 +351,20 @@ extern "C" size_t b200_focal_box_workspace_bytes(int num_levels, const unsigned 
   return b200_align_up(sizeof(double) * 3 * (size_t)n, 256);
 }
 
+// The fp32 entries pass their arrays of float pointers as arrays of untyped pointers (same representation).
+#define EL_UNTYPED(a) reinterpret_cast<const void* const*>(a)
+#define EL_UNTYPED_OUT(a) reinterpret_cast<void* const*>(a)
+
 // anchors_per_level[l] = B*H_l*W_l*A of THIS call (local shard); sums_out: device double[2L+1]
 static int el_partial_sums_impl(int num_levels, const unsigned long long* anchors_per_level, int C,
                                 const float* const true_boxes[], const float* const true_classes_dense[],
                                 const int32_t* const true_class_index[], const unsigned char* const true_masks[],
-                                const float* const pred_boxes[], const float* const pred_classes[], float alpha, float gamma,
-                                float delta, float label_smoothing, double* sums_out, void* workspace, size_t workspace_bytes,
-                                void* stream_) {
+                                const void* const pred_boxes[], const void* const pred_classes[], int pred_dtype, float alpha,
+                                float gamma, float delta, float label_smoothing, double* sums_out, void* workspace,
+                                size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  B200_REQUIRE(b200_dtype_ok(pred_dtype), B200_ERR_BAD_ARG, "b200_focal_box_partial_sums: pred_dtype %d is not a B200_DTYPE_* code", pred_dtype);
+  const unsigned long long esize = (unsigned long long)b200_dtype_bytes(pred_dtype);
   B200_REQUIRE(num_levels >= 1 && num_levels <= EL_MAX_LEVELS && C >= 1, B200_ERR_BAD_ARG, "b200_focal_box_partial_sums: bad level count / classes");
   B200_REQUIRE(anchors_per_level && true_boxes && (true_classes_dense || true_class_index) && true_masks && pred_boxes && pred_classes && sums_out,
                B200_ERR_BAD_ARG, "b200_focal_box_partial_sums: null argument");
@@ -357,20 +386,21 @@ static int el_partial_sums_impl(int num_levels, const unsigned long long* anchor
                            reinterpret_cast<uintptr_t>(pred_boxes[l]) | reinterpret_cast<uintptr_t>(pred_classes[l]);
       B200_REQUIRE((al & 15) == 0, B200_ERR_BAD_ARG, "b200_focal_box_partial_sums: level %d tensors must be 16-byte aligned", l);
       elems[l] = has_cls ? anchors_per_level[l] * (unsigned long long)C : 0ull;
-      p.cls_pred[l] = reinterpret_cast<const float4*>(pred_classes[l]);
+      p.cls_pred[l] = pred_classes[l];
       p.cls_true[l] = true_classes_dense ? reinterpret_cast<const float4*>(true_classes[l]) : nullptr;
       p.cls_index[l] = true_classes_dense ? nullptr : reinterpret_cast<const int32_t*>(true_classes[l]);
       p.cls_vec[l] = elems[l] / 4;
       p.cls_tail[l] = (int)(elems[l] - p.cls_vec[l] * 4);
-      p.cls_pred_tail[l] = pred_classes[l] + p.cls_vec[l] * 4;
+      p.cls_pred_tail[l] = static_cast<const char*>(pred_classes[l]) + p.cls_vec[l] * 4 * esize;
       p.cls_true_tail[l] = true_classes_dense ? true_classes_dense[l] + p.cls_vec[l] * 4 : nullptr;
-      p.box_pred[l] = reinterpret_cast<const float4*>(pred_boxes[l]);
+      p.box_pred[l] = pred_boxes[l];
       p.box_true[l] = reinterpret_cast<const float4*>(true_boxes[l]);
       p.mask[l] = true_masks[l];
       p.anchors[l] = has_box ? anchors_per_level[l] : 0ull;
     } else {
-      elems[l] = 0; p.cls_pred[l] = p.cls_true[l] = nullptr; p.cls_index[l] = nullptr; p.cls_vec[l] = 0; p.cls_tail[l] = 0;
-      p.cls_pred_tail[l] = p.cls_true_tail[l] = nullptr; p.box_pred[l] = p.box_true[l] = nullptr; p.mask[l] = nullptr; p.anchors[l] = 0;
+      elems[l] = 0; p.cls_pred[l] = nullptr; p.cls_true[l] = nullptr; p.cls_index[l] = nullptr; p.cls_vec[l] = 0; p.cls_tail[l] = 0;
+      p.cls_pred_tail[l] = nullptr; p.cls_true_tail[l] = nullptr; p.box_pred[l] = nullptr; p.box_true[l] = nullptr; p.mask[l] = nullptr;
+      p.anchors[l] = 0;
     }
   }
   unsigned long long plan[EL_MAX_LEVELS];
@@ -381,8 +411,9 @@ static int el_partial_sums_impl(int num_levels, const unsigned long long* anchor
   p.alpha = alpha; p.gamma = gamma; p.delta = delta; p.label_smoothing = label_smoothing;
   p.partials = static_cast<double*>(workspace);
   B200_CUDA(cudaMemsetAsync(sums_out, 0, sizeof(double) * (2 * num_levels + 1), stream));
-  if (gamma == 1.5f) focal_box_partials_kernel<true><<<n_cta, EL_THREADS, 0, stream>>>(p);
-  else focal_box_partials_kernel<false><<<n_cta, EL_THREADS, 0, stream>>>(p);
+  B200_DISPATCH_DTYPE(pred_dtype, TP,
+                      if (gamma == 1.5f) focal_box_partials_kernel<true, TP><<<n_cta, EL_THREADS, 0, stream>>>(p);
+                      else focal_box_partials_kernel<false, TP><<<n_cta, EL_THREADS, 0, stream>>>(p))
   B200_LAUNCH_CHECK();
   ElReduce r;
   r.partials = p.partials; r.num_levels = num_levels; r.sums = sums_out;
@@ -392,28 +423,54 @@ static int el_partial_sums_impl(int num_levels, const unsigned long long* anchor
   return B200_OK;
 }
 
+extern "C" int b200_focal_box_partial_sums_typed(int num_levels, const unsigned long long* anchors_per_level, int C,
+                                                 const float* const true_boxes[], const float* const true_classes[],
+                                                 const unsigned char* const true_masks[], const void* const pred_boxes[],
+                                                 const void* const pred_classes[], int pred_dtype, float alpha, float gamma,
+                                                 float delta, float label_smoothing, double* sums_out, void* workspace,
+                                                 size_t workspace_bytes, void* stream_) {
+  B200_REQUIRE(true_classes, B200_ERR_BAD_ARG, "b200_focal_box_partial_sums: null argument");
+  return el_partial_sums_impl(num_levels, anchors_per_level, C, true_boxes, true_classes, nullptr, true_masks, pred_boxes,
+                              pred_classes, pred_dtype, alpha, gamma, delta, label_smoothing, sums_out, workspace, workspace_bytes,
+                              stream_);
+}
+
 extern "C" int b200_focal_box_partial_sums(int num_levels, const unsigned long long* anchors_per_level, int C,
                                            const float* const true_boxes[], const float* const true_classes[],
                                            const unsigned char* const true_masks[], const float* const pred_boxes[],
                                            const float* const pred_classes[], float alpha, float gamma, float delta,
                                            float label_smoothing, double* sums_out, void* workspace,
                                            size_t workspace_bytes, void* stream_) {
-  B200_REQUIRE(true_classes, B200_ERR_BAD_ARG, "b200_focal_box_partial_sums: null argument");
-  return el_partial_sums_impl(num_levels, anchors_per_level, C, true_boxes, true_classes, nullptr, true_masks, pred_boxes,
-                              pred_classes, alpha, gamma, delta, label_smoothing, sums_out, workspace, workspace_bytes, stream_);
+  return b200_focal_box_partial_sums_typed(num_levels, anchors_per_level, C, true_boxes, true_classes, true_masks,
+                                           EL_UNTYPED(pred_boxes),
+                                           EL_UNTYPED(pred_classes), B200_DTYPE_F32, alpha, gamma,
+                                           delta, label_smoothing, sums_out, workspace, workspace_bytes, stream_);
 }
 
 // Sparse-target mode (SURVEY §8f N3): true_class_index[l] (B,H,W,A) int32 = the class id whose one-hot row
 // generate_targets would have written (0 for unmatched anchors; out-of-range ids = all-zero row).
+extern "C" int b200_focal_box_partial_sums_indexed_typed(int num_levels, const unsigned long long* anchors_per_level, int C,
+                                                         const float* const true_boxes[], const int32_t* const true_class_index[],
+                                                         const unsigned char* const true_masks[], const void* const pred_boxes[],
+                                                         const void* const pred_classes[], int pred_dtype, float alpha,
+                                                         float gamma, float delta, float label_smoothing, double* sums_out,
+                                                         void* workspace, size_t workspace_bytes, void* stream_) {
+  B200_REQUIRE(true_class_index, B200_ERR_BAD_ARG, "b200_focal_box_partial_sums_indexed: null argument");
+  return el_partial_sums_impl(num_levels, anchors_per_level, C, true_boxes, nullptr, true_class_index, true_masks, pred_boxes,
+                              pred_classes, pred_dtype, alpha, gamma, delta, label_smoothing, sums_out, workspace, workspace_bytes,
+                              stream_);
+}
+
 extern "C" int b200_focal_box_partial_sums_indexed(int num_levels, const unsigned long long* anchors_per_level, int C,
                                                    const float* const true_boxes[], const int32_t* const true_class_index[],
                                                    const unsigned char* const true_masks[], const float* const pred_boxes[],
                                                    const float* const pred_classes[], float alpha, float gamma, float delta,
                                                    float label_smoothing, double* sums_out, void* workspace,
                                                    size_t workspace_bytes, void* stream_) {
-  B200_REQUIRE(true_class_index, B200_ERR_BAD_ARG, "b200_focal_box_partial_sums_indexed: null argument");
-  return el_partial_sums_impl(num_levels, anchors_per_level, C, true_boxes, nullptr, true_class_index, true_masks, pred_boxes,
-                              pred_classes, alpha, gamma, delta, label_smoothing, sums_out, workspace, workspace_bytes, stream_);
+  return b200_focal_box_partial_sums_indexed_typed(num_levels, anchors_per_level, C, true_boxes, true_class_index, true_masks,
+                                                   EL_UNTYPED(pred_boxes),
+                                                   EL_UNTYPED(pred_classes), B200_DTYPE_F32, alpha,
+                                                   gamma, delta, label_smoothing, sums_out, workspace, workspace_bytes, stream_);
 }
 
 // numel_per_level[l] = GLOBAL element count B_global*H*W*A*C of level l (the Keras mean divisor)
@@ -455,10 +512,12 @@ extern "C" int b200_focal_box_finalize_dp(int num_levels, double* sums, const do
 static int el_grad_impl(int num_levels, const unsigned long long* anchors_per_level, int C,
                         const float* const true_boxes[], const float* const true_classes[],
                         const int32_t* const true_class_index[],
-                        const float* const pred_boxes[], const float* const pred_classes[], float alpha,
+                        const void* const pred_boxes[], const void* const pred_classes[], int pred_dtype, float alpha,
                         float gamma, float delta, float label_smoothing, const double* sums,
-                        const double* numel_per_level_host, float* const grad_boxes[],
-                        float* const grad_classes[], void* stream) {
+                        const double* numel_per_level_host, void* const grad_boxes[], void* const grad_classes[],
+                        int grad_dtype, const float* grad_scale_dev, void* stream) {
+  B200_REQUIRE(b200_dtype_ok(pred_dtype), B200_ERR_BAD_ARG, "b200_focal_box_grad: pred_dtype %d is not a B200_DTYPE_* code", pred_dtype);
+  B200_REQUIRE(b200_dtype_ok(grad_dtype), B200_ERR_BAD_ARG, "b200_focal_box_grad: grad_dtype %d is not a B200_DTYPE_* code", grad_dtype);
   B200_REQUIRE(num_levels >= 1 && num_levels <= EL_MAX_LEVELS && C >= 1 && anchors_per_level && sums && numel_per_level_host,
                B200_ERR_BAD_ARG, "b200_focal_box_grad: bad argument");
   B200_REQUIRE(!true_class_index || C >= 4, B200_ERR_UNSUPPORTED, "b200_focal_box_grad_indexed: needs classes_num >= 4");
@@ -478,10 +537,10 @@ static int el_grad_impl(int num_levels, const unsigned long long* anchors_per_le
       const unsigned long long n = anchors_per_level[l] * (unsigned long long)C;
       const uintptr_t al = (true_class_index ? 0 : reinterpret_cast<uintptr_t>(tcl)) | reinterpret_cast<uintptr_t>(pred_classes[l]) | reinterpret_cast<uintptr_t>(grad_classes[l]);
       B200_REQUIRE((al & 15) == 0, B200_ERR_BAD_ARG, "b200_focal_box_grad: level %d class tensors must be 16-byte aligned", l);
-      p.cls_pred[l] = reinterpret_cast<const float4*>(pred_classes[l]);
+      p.cls_pred[l] = pred_classes[l];
       p.cls_true[l] = true_class_index ? nullptr : reinterpret_cast<const float4*>(tcl);
       p.cls_index[l] = true_class_index ? true_class_index[l] : nullptr;
-      p.cls_grad[l] = reinterpret_cast<float4*>(grad_classes[l]);
+      p.cls_grad[l] = grad_classes[l];
       p.cls_vec[l] = n / 4ull;
       p.cls_tail[l] = (int)(n - p.cls_vec[l] * 4ull);
       plan[l] = n;
@@ -490,9 +549,9 @@ static int el_grad_impl(int num_levels, const unsigned long long* anchors_per_le
       B200_REQUIRE(true_boxes && pred_boxes && true_boxes[l] && pred_boxes[l], B200_ERR_BAD_ARG, "b200_focal_box_grad: null box tensors at level %d", l);
       const uintptr_t al = reinterpret_cast<uintptr_t>(true_boxes[l]) | reinterpret_cast<uintptr_t>(pred_boxes[l]) | reinterpret_cast<uintptr_t>(grad_boxes[l]);
       B200_REQUIRE((al & 15) == 0, B200_ERR_BAD_ARG, "b200_focal_box_grad: level %d box tensors must be 16-byte aligned", l);
-      p.box_pred[l] = reinterpret_cast<const float4*>(pred_boxes[l]);
+      p.box_pred[l] = pred_boxes[l];
       p.box_true[l] = reinterpret_cast<const float4*>(true_boxes[l]);
-      p.box_grad[l] = reinterpret_cast<float4*>(grad_boxes[l]);
+      p.box_grad[l] = grad_boxes[l];
       p.anchors[l] = anchors_per_level[l];
       if (plan[l] < anchors_per_level[l] * 4ull) plan[l] = anchors_per_level[l] * 4ull;
     }
@@ -500,9 +559,23 @@ static int el_grad_impl(int num_levels, const unsigned long long* anchors_per_le
   }
   const int n_cta = el_cta_plan(num_levels, plan, p.cta_base);
   p.alpha = alpha; p.gamma = gamma; p.delta = delta; p.label_smoothing = label_smoothing; p.sums = sums;
-  focal_box_grad_kernel<<<n_cta, EL_THREADS, 0, (cudaStream_t)stream>>>(p);
+  p.scale = grad_scale_dev;
+  B200_DISPATCH_DTYPE(pred_dtype, TP, B200_DISPATCH_DTYPE(grad_dtype, TG,
+                      if (grad_scale_dev) focal_box_grad_kernel<TP, TG, true><<<n_cta, EL_THREADS, 0, (cudaStream_t)stream>>>(p);
+                      else focal_box_grad_kernel<TP, TG, false><<<n_cta, EL_THREADS, 0, (cudaStream_t)stream>>>(p)))
   B200_LAUNCH_CHECK();
   return B200_OK;
+}
+
+extern "C" int b200_focal_box_grad_typed(int num_levels, const unsigned long long* anchors_per_level, int C,
+                                         const float* const true_boxes[], const float* const true_classes[],
+                                         const void* const pred_boxes[], const void* const pred_classes[], int pred_dtype,
+                                         float alpha, float gamma, float delta, float label_smoothing, const double* sums,
+                                         const double* numel_per_level_host, void* const grad_boxes[],
+                                         void* const grad_classes[], int grad_dtype, const float* grad_scale_dev, void* stream) {
+  return el_grad_impl(num_levels, anchors_per_level, C, true_boxes, true_classes, nullptr, pred_boxes, pred_classes, pred_dtype,
+                      alpha, gamma, delta, label_smoothing, sums, numel_per_level_host, grad_boxes, grad_classes, grad_dtype,
+                      grad_scale_dev, stream);
 }
 
 extern "C" int b200_focal_box_grad(int num_levels, const unsigned long long* anchors_per_level, int C,
@@ -511,21 +584,36 @@ extern "C" int b200_focal_box_grad(int num_levels, const unsigned long long* anc
                                    float gamma, float delta, float label_smoothing, const double* sums,
                                    const double* numel_per_level_host, float* const grad_boxes[],
                                    float* const grad_classes[], void* stream) {
-  return el_grad_impl(num_levels, anchors_per_level, C, true_boxes, true_classes, nullptr, pred_boxes, pred_classes, alpha, gamma,
-                      delta, label_smoothing, sums, numel_per_level_host, grad_boxes, grad_classes, stream);
+  return el_grad_impl(num_levels, anchors_per_level, C, true_boxes, true_classes, nullptr, EL_UNTYPED(pred_boxes),
+                      EL_UNTYPED(pred_classes), B200_DTYPE_F32, alpha, gamma, delta, label_smoothing, sums, numel_per_level_host,
+                      EL_UNTYPED_OUT(grad_boxes), EL_UNTYPED_OUT(grad_classes), B200_DTYPE_F32, nullptr, stream);
 }
 
 // Sparse-target mode of the backward pass: true_class_index[l] (B,H,W,A) int32 class ids, as
 // b200_focal_box_partial_sums_indexed takes them (the one-hot row is rebuilt in registers).
+extern "C" int b200_focal_box_grad_indexed_typed(int num_levels, const unsigned long long* anchors_per_level, int C,
+                                                 const float* const true_boxes[], const int32_t* const true_class_index[],
+                                                 const void* const pred_boxes[], const void* const pred_classes[], int pred_dtype,
+                                                 float alpha, float gamma, float delta, float label_smoothing, const double* sums,
+                                                 const double* numel_per_level_host, void* const grad_boxes[],
+                                                 void* const grad_classes[], int grad_dtype, const float* grad_scale_dev,
+                                                 void* stream) {
+  B200_REQUIRE(true_class_index, B200_ERR_BAD_ARG, "b200_focal_box_grad_indexed: null argument");
+  return el_grad_impl(num_levels, anchors_per_level, C, true_boxes, nullptr, true_class_index, pred_boxes, pred_classes, pred_dtype,
+                      alpha, gamma, delta, label_smoothing, sums, numel_per_level_host, grad_boxes, grad_classes, grad_dtype,
+                      grad_scale_dev, stream);
+}
+
 extern "C" int b200_focal_box_grad_indexed(int num_levels, const unsigned long long* anchors_per_level, int C,
                                            const float* const true_boxes[], const int32_t* const true_class_index[],
                                            const float* const pred_boxes[], const float* const pred_classes[], float alpha,
                                            float gamma, float delta, float label_smoothing, const double* sums,
                                            const double* numel_per_level_host, float* const grad_boxes[],
                                            float* const grad_classes[], void* stream) {
-  B200_REQUIRE(true_class_index, B200_ERR_BAD_ARG, "b200_focal_box_grad_indexed: null argument");
-  return el_grad_impl(num_levels, anchors_per_level, C, true_boxes, nullptr, true_class_index, pred_boxes, pred_classes, alpha,
-                      gamma, delta, label_smoothing, sums, numel_per_level_host, grad_boxes, grad_classes, stream);
+  return b200_focal_box_grad_indexed_typed(num_levels, anchors_per_level, C, true_boxes, true_class_index, EL_UNTYPED(pred_boxes),
+                                           EL_UNTYPED(pred_classes), B200_DTYPE_F32, alpha, gamma, delta, label_smoothing, sums,
+                                           numel_per_level_host, EL_UNTYPED_OUT(grad_boxes), EL_UNTYPED_OUT(grad_classes),
+                                           B200_DTYPE_F32, nullptr, stream);
 }
 
 // ---- loss and gradient from box lists, stage 2 (SURVEY §8f N3 + N1) --------------------------------------------------
@@ -542,8 +630,8 @@ struct EfbParams {
   const float* gt_boxes;       // [total,4] y1,x1,y2,x2
   const int32_t* gt_classes;   // [total]
   const int32_t* match;        // per anchor: row of gt_boxes or -1; level l at B*anchor_base[l]
-  const float4* cls_pred[EL_MAX_LEVELS]; float4* cls_grad[EL_MAX_LEVELS];
-  const float4* box_pred[EL_MAX_LEVELS]; float4* box_grad[EL_MAX_LEVELS];
+  const void* cls_pred[EL_MAX_LEVELS]; void* cls_grad[EL_MAX_LEVELS];    // heads of type TP, gradients of type TG
+  const void* box_pred[EL_MAX_LEVELS]; void* box_grad[EL_MAX_LEVELS];
   unsigned long long cls_vec[EL_MAX_LEVELS];
   int cls_tail[EL_MAX_LEVELS];
   unsigned long long anchors[EL_MAX_LEVELS];   // B*H*W*A
@@ -552,6 +640,7 @@ struct EfbParams {
   float alpha, gamma, delta, label_smoothing;
   const double* sums;   // sums[2L] = positives (after the caller's all-reduce)
   double* partials;     // [n_cta, 3]
+  const float* scale;   // device fp32 gradient scale or null (no multiply)
 };
 
 // the class id whose one-hot row generate_targets writes for anchor a (anc:131-133: class 0 when unmatched)
@@ -560,7 +649,9 @@ __device__ __forceinline__ int efb_class(const EfbParams& p, const int32_t* matc
   return m >= 0 ? __ldg(p.gt_classes + m) : 0;
 }
 
+template <typename TP, typename TG, bool kScale>
 __global__ void __launch_bounds__(EL_THREADS) effdet_loss_from_boxes_kernel(EfbParams p) {
+  const float* scale = kScale ? p.scale : nullptr;
   __shared__ double s_red[EL_THREADS / 32][2];
   int l = 0;
 #pragma unroll
@@ -577,12 +668,12 @@ __global__ void __launch_bounds__(EL_THREADS) effdet_loss_from_boxes_kernel(EfbP
   float f0 = 0.f, f1 = 0.f;
   double focal = 0.0;
   int it = 0;
-  const float4* __restrict__ cp = p.cls_pred[l];
-  float4* __restrict__ cg = p.cls_grad[l];
+  const TP* __restrict__ cp = static_cast<const TP*>(p.cls_pred[l]);
+  TG* __restrict__ cg = static_cast<TG*>(p.cls_grad[l]);
   const unsigned long long nv = p.cls_vec[l];
 #pragma unroll 2
   for (unsigned long long i = (unsigned long long)cta * EL_THREADS + threadIdx.x; i < nv; i += stride) {
-    const float4 x = __ldcs(cp + i);
+    const float4 x = ld4_f32<true>(el_group(cp, i));
     const unsigned long long e = i * 4ull, a0 = e / (unsigned long long)C;
     const int c0 = (int)(e - a0 * (unsigned long long)C);
     const int id0 = efb_class(p, match, a0);
@@ -595,11 +686,11 @@ __global__ void __launch_bounds__(EL_THREADS) effdet_loss_from_boxes_kernel(EfbP
     }
     float v0, v1, v2, v3;
     float4 g;
-    g.x = cs * el_focal_value_grad(yy[0], x.x, p.alpha, p.gamma, p.label_smoothing, v0);
-    g.y = cs * el_focal_value_grad(yy[1], x.y, p.alpha, p.gamma, p.label_smoothing, v1);
-    g.z = cs * el_focal_value_grad(yy[2], x.z, p.alpha, p.gamma, p.label_smoothing, v2);
-    g.w = cs * el_focal_value_grad(yy[3], x.w, p.alpha, p.gamma, p.label_smoothing, v3);
-    if (cg) __stcs(cg + i, g);
+    g.x = scaled_f32(cs * el_focal_value_grad(yy[0], x.x, p.alpha, p.gamma, p.label_smoothing, v0), scale);
+    g.y = scaled_f32(cs * el_focal_value_grad(yy[1], x.y, p.alpha, p.gamma, p.label_smoothing, v1), scale);
+    g.z = scaled_f32(cs * el_focal_value_grad(yy[2], x.z, p.alpha, p.gamma, p.label_smoothing, v2), scale);
+    g.w = scaled_f32(cs * el_focal_value_grad(yy[3], x.w, p.alpha, p.gamma, p.label_smoothing, v3), scale);
+    if (cg) st4(el_group(cg, i), g);
     f0 += v0 + v1;
     f1 += v2 + v3;
     if ((++it & 63) == 0) { focal += (double)f0 + (double)f1; f0 = f1 = 0.f; }
@@ -608,8 +699,8 @@ __global__ void __launch_bounds__(EL_THREADS) effdet_loss_from_boxes_kernel(EfbP
     const unsigned long long e = nv * 4ull + threadIdx.x, a = e / (unsigned long long)C;
     const float yt = ((int)(e - a * (unsigned long long)C) == efb_class(p, match, a)) ? 1.0f : 0.0f;
     float v;
-    const float g = cs * el_focal_value_grad(yt, reinterpret_cast<const float*>(cp)[e], p.alpha, p.gamma, p.label_smoothing, v);
-    if (cg) reinterpret_cast<float*>(cg)[e] = g;
+    const float g = scaled_f32(cs * el_focal_value_grad(yt, elem_f32(cp[e]), p.alpha, p.gamma, p.label_smoothing, v), scale);
+    if (cg) cg[e] = round_elem<TG>(g);
     f0 += v;
   }
   focal += (double)f0 + (double)f1;
@@ -617,9 +708,9 @@ __global__ void __launch_bounds__(EL_THREADS) effdet_loss_from_boxes_kernel(EfbP
   float hub = 0.f;
   const unsigned long long na = p.anchors[l];
   const unsigned int api = (unsigned int)p.lv.anc_per_img[l];
-  float4* __restrict__ bg = p.box_grad[l];
+  TG* __restrict__ bg = static_cast<TG*>(p.box_grad[l]);
   for (unsigned long long a = (unsigned long long)cta * EL_THREADS + threadIdx.x; a < na; a += stride) {
-    const float4 o = __ldcs(p.box_pred[l] + a);
+    const float4 o = ld4_f32<true>(el_group(static_cast<const TP*>(p.box_pred[l]), a));
     const int m = __ldg(match + a);
     float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
     if (m >= 0) {
@@ -631,8 +722,9 @@ __global__ void __launch_bounds__(EL_THREADS) effdet_loss_from_boxes_kernel(EfbP
       t = ef_encode_box(an.y1, an.x1, an.y2, an.x2, q.x, q.y, q.z, q.w);
     }
     hub += el_huber(t.x, o.x, p.delta) + el_huber(t.y, o.y, p.delta) + el_huber(t.z, o.z, p.delta) + el_huber(t.w, o.w, p.delta);
-    if (bg) __stcs(bg + a, make_float4(bs * el_huber_grad(t.x, o.x, p.delta), bs * el_huber_grad(t.y, o.y, p.delta),
-                                       bs * el_huber_grad(t.z, o.z, p.delta), bs * el_huber_grad(t.w, o.w, p.delta)));
+    if (bg)
+      st4(el_group(bg, a), make_float4(scaled_f32(bs * el_huber_grad(t.x, o.x, p.delta), scale), scaled_f32(bs * el_huber_grad(t.y, o.y, p.delta), scale),
+                                  scaled_f32(bs * el_huber_grad(t.z, o.z, p.delta), scale), scaled_f32(bs * el_huber_grad(t.w, o.w, p.delta), scale)));
   }
   const double v0 = warp_sum_d(focal), v1 = warp_sum_d((double)hub);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -662,16 +754,19 @@ extern "C" size_t b200_effdet_loss_from_boxes_workspace_bytes(int num_levels, co
   return n_img < 0 ? 0 : efb_workspace_bytes(num_levels, n_img, B);
 }
 
-extern "C" int b200_effdet_loss_from_boxes_grad(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
-                                                const float* gt_boxes, const int32_t* gt_classes, int total_boxes,
-                                                const float* const pred_boxes[], const float* const pred_classes[], float alpha,
-                                                float gamma, float delta, float label_smoothing,
-                                                const double* numel_per_level_host, double* sums, float* const grad_boxes[],
-                                                float* const grad_classes[], void* workspace, size_t workspace_bytes,
-                                                void* stream_) {
+extern "C" int b200_effdet_loss_from_boxes_grad_typed(int num_levels, const int32_t* hw, int A, const float* table_dev, int C,
+                                                      int B, const float* gt_boxes, const int32_t* gt_classes, int total_boxes,
+                                                      const void* const pred_boxes[], const void* const pred_classes[],
+                                                      int pred_dtype, float alpha, float gamma, float delta,
+                                                      float label_smoothing, const double* numel_per_level_host, double* sums,
+                                                      void* const grad_boxes[], void* const grad_classes[], int grad_dtype,
+                                                      const float* grad_scale_dev, void* workspace, size_t workspace_bytes,
+                                                      void* stream_) {
   const char* who = "b200_effdet_loss_from_boxes_grad";
   cudaStream_t stream = (cudaStream_t)stream_;
   EfbParams p;
+  B200_REQUIRE(b200_dtype_ok(pred_dtype), B200_ERR_BAD_ARG, "%s: pred_dtype %d is not a B200_DTYPE_* code", who, pred_dtype);
+  B200_REQUIRE(b200_dtype_ok(grad_dtype), B200_ERR_BAD_ARG, "%s: grad_dtype %d is not a B200_DTYPE_* code", who, grad_dtype);
   B200_REQUIRE(hw && table_dev && pred_boxes && pred_classes && numel_per_level_host && sums, B200_ERR_BAD_ARG, "%s: null argument", who);
   const int n_img = ef_fill_levels(p.lv, num_levels, hw, A, table_dev);
   B200_REQUIRE(n_img >= 0, B200_ERR_BAD_ARG, "%s: bad level spec", who);
@@ -693,10 +788,10 @@ extern "C" int b200_effdet_loss_from_boxes_grad(int num_levels, const int32_t* h
     B200_REQUIRE((al & 15) == 0, B200_ERR_BAD_ARG, "%s: level %d tensors must be 16-byte aligned", who, l);
     B200_REQUIRE(numel_per_level_host[l] > 0.0, B200_ERR_BAD_ARG, "%s: numel of level %d must be positive", who, l);
     const unsigned long long na = (unsigned long long)B * (unsigned long long)p.lv.anc_per_img[l], n = na * (unsigned long long)C;
-    p.cls_pred[l] = reinterpret_cast<const float4*>(pred_classes[l]);
-    p.cls_grad[l] = grad_classes ? reinterpret_cast<float4*>(grad_classes[l]) : nullptr;
-    p.box_pred[l] = reinterpret_cast<const float4*>(pred_boxes[l]);
-    p.box_grad[l] = grad_boxes ? reinterpret_cast<float4*>(grad_boxes[l]) : nullptr;
+    p.cls_pred[l] = pred_classes[l];
+    p.cls_grad[l] = grad_classes ? grad_classes[l] : nullptr;
+    p.box_pred[l] = pred_boxes[l];
+    p.box_grad[l] = grad_boxes ? grad_boxes[l] : nullptr;
     p.cls_vec[l] = n / 4ull;
     p.cls_tail[l] = (int)(n - p.cls_vec[l] * 4ull);
     p.anchors[l] = na;
@@ -714,9 +809,12 @@ extern "C" int b200_effdet_loss_from_boxes_grad(int num_levels, const int32_t* h
   p.match = reinterpret_cast<const int32_t*>(wsb);
   p.partials = reinterpret_cast<double*>(wsb + efb_match_bytes(n_img, B));
   p.alpha = alpha; p.gamma = gamma; p.delta = delta; p.label_smoothing = label_smoothing; p.sums = sums;
+  p.scale = grad_scale_dev;
   const int budget = b200_sm_count() * 64;
   const int n_cta = el_cta_plan_budget(num_levels, plan, p.cta_base, budget < EFB_MAX_CTAS ? budget : EFB_MAX_CTAS);
-  effdet_loss_from_boxes_kernel<<<n_cta, EL_THREADS, 0, stream>>>(p);
+  B200_DISPATCH_DTYPE(pred_dtype, TP, B200_DISPATCH_DTYPE(grad_dtype, TG,
+                      if (grad_scale_dev) effdet_loss_from_boxes_kernel<TP, TG, true><<<n_cta, EL_THREADS, 0, stream>>>(p);
+                      else effdet_loss_from_boxes_kernel<TP, TG, false><<<n_cta, EL_THREADS, 0, stream>>>(p)))
   B200_LAUNCH_CHECK();
   ElReduce r;
   r.partials = p.partials; r.num_levels = num_levels; r.sums = sums;
@@ -724,4 +822,18 @@ extern "C" int b200_effdet_loss_from_boxes_grad(int num_levels, const int32_t* h
   focal_box_reduce_kernel<<<num_levels, 256, 0, stream>>>(r);   // sums[0..2L); adds the partials' 0 to sums[2L]
   B200_LAUNCH_CHECK();
   return B200_OK;
+}
+
+extern "C" int b200_effdet_loss_from_boxes_grad(int num_levels, const int32_t* hw, int A, const float* table_dev, int C, int B,
+                                                const float* gt_boxes, const int32_t* gt_classes, int total_boxes,
+                                                const float* const pred_boxes[], const float* const pred_classes[], float alpha,
+                                                float gamma, float delta, float label_smoothing,
+                                                const double* numel_per_level_host, double* sums, float* const grad_boxes[],
+                                                float* const grad_classes[], void* workspace, size_t workspace_bytes,
+                                                void* stream_) {
+  return b200_effdet_loss_from_boxes_grad_typed(num_levels, hw, A, table_dev, C, B, gt_boxes, gt_classes, total_boxes,
+                                                EL_UNTYPED(pred_boxes), EL_UNTYPED(pred_classes), B200_DTYPE_F32, alpha, gamma,
+                                                delta, label_smoothing, numel_per_level_host, sums, EL_UNTYPED_OUT(grad_boxes),
+                                                EL_UNTYPED_OUT(grad_classes), B200_DTYPE_F32, nullptr, workspace, workspace_bytes,
+                                                stream_);
 }

@@ -936,16 +936,6 @@ struct YlGradDense {
   int RF;
 };
 
-__device__ __forceinline__ float yl_scaled(float g, const float* scale) { return scale ? g * __ldg(scale) : g; }
-template <typename TG> __device__ __forceinline__ TG yl_round(float v);
-template <> __device__ __forceinline__ float yl_round<float>(float v) { return v; }
-template <> __device__ __forceinline__ __nv_bfloat16 yl_round<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
-template <> __device__ __forceinline__ __half yl_round<__half>(float v) { return __float2half_rn(v); }
-template <typename TG> __device__ __forceinline__ uint32_t yl_bits16(float v) {
-  const TG h = yl_round<TG>(v);
-  return (uint32_t)*reinterpret_cast<const unsigned short*>(&h);
-}
-
 // fp32: four records = RF float4, always 16-byte aligned: a warp writes one such group per iteration (ceil(RF/32) 16-byte
 // stores per lane), all zeros except the four conf channels, whose values are fetched by lanes 0-3 beforehand.  No
 // index division, no load -> store dependency on the streaming path.  2-byte TG: eight records = RF 16-byte chunks, the
@@ -968,7 +958,7 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g
     if constexpr (kRec == 8) {
       float* sc = s_conf[threadIdx.x >> 5];
       __syncwarp();
-      if (lane < 8) sc[lane] = yl_scaled(__ldg(cg + q * 8ull + lane), g.scale);
+      if (lane < 8) sc[lane] = scaled_f32(__ldg(cg + q * 8ull + lane), g.scale);
       __syncwarp();
       uint4* dst = reinterpret_cast<uint4*>(gr) + q * (unsigned long long)RF;
       for (int j = lane; j < RF; j += 32) {
@@ -977,7 +967,7 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g
         const int x0 = 8 * j - 4;
         const int r = x0 > 0 ? (x0 + RF - 1) / RF : 0;
         const int p0 = r * RF - x0, p1 = p0 + RF;
-        const uint32_t b0 = p0 < 8 ? yl_bits16<TG>(sc[min(r, 7)]) : 0u, b1 = p1 < 8 ? yl_bits16<TG>(sc[min(r + 1, 7)]) : 0u;
+        const uint32_t b0 = p0 < 8 ? round_bits16<TG>(sc[min(r, 7)]) : 0u, b1 = p1 < 8 ? round_bits16<TG>(sc[min(r + 1, 7)]) : 0u;
         uint32_t wd[4];
 #pragma unroll
         for (int k = 0; k < 4; ++k)
@@ -986,7 +976,7 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g
       }
       continue;
     }
-    const float mine = (lane < 4) ? yl_scaled(__ldg(cg + q * 4ull + lane), g.scale) : 0.0f;
+    const float mine = (lane < 4) ? scaled_f32(__ldg(cg + q * 4ull + lane), g.scale) : 0.0f;
     const float c0 = __shfl_sync(0xffffffffu, mine, 0), c1 = __shfl_sync(0xffffffffu, mine, 1);
     const float c2 = __shfl_sync(0xffffffffu, mine, 2), c3 = __shfl_sync(0xffffffffu, mine, 3);
     float4* dst = reinterpret_cast<float4*>(gr) + q * (unsigned long long)RF;
@@ -1011,7 +1001,7 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_dense_kernel(YlGradDense g
         const unsigned long long rec = r0 + t / (unsigned long long)RF;
         const int c = (int)(t % (unsigned long long)RF);
         static_cast<TG*>(g.grad[l])[r0 * (unsigned long long)RF + t] =
-            yl_round<TG>((c == 4) ? yl_scaled(g.conf_grad[l][rec], g.scale) : 0.0f);
+            round_elem<TG>((c == 4) ? scaled_f32(g.conf_grad[l][rec], g.scale) : 0.0f);
       }
     }
   }
@@ -1057,16 +1047,16 @@ __global__ void __launch_bounds__(256) yolo_loss_grad_objects_kernel(YlParams p,
       const int gy = cell / W, gx = cell - gy * W;
       float raw = (lane == 0 ? tx * (float)W - (float)gx : ty * (float)H - (float)gy);
       if (p.variant == YL_VARIANT_TF_YOLO_UTILS) raw = obj * raw;
-      o[lane] = yl_round<TG>(yl_scaled(os * (dm_sigmoidf(ldg_f32(q + lane)) - raw), scale));
+      o[lane] = round_elem<TG>(scaled_f32(os * (dm_sigmoidf(ldg_f32(q + lane)) - raw), scale));
     } else if (lane < 4) {
       const int a = r - (r / p.A) * p.A;
       float num = (lane == 2 ? tw * p.img_w : th * p.img_h);
       if (p.variant == YL_VARIANT_TF_YOLO_UTILS) num += 1e-8f;
       const float raw = dm_logf(num / (lane == 2 ? p.lv.anc_w[l][a] : p.lv.anc_h[l][a]));
-      o[lane] = yl_round<TG>(yl_scaled(os * (ldg_f32(q + lane) - raw), scale));
+      o[lane] = round_elem<TG>(scaled_f32(os * (ldg_f32(q + lane) - raw), scale));
     }
     for (int c = 5 + lane; c < p.RF; c += 32)
-      o[c] = yl_round<TG>(yl_scaled((obj * p.inv_div) * (dm_sigmoidf(ldg_f32(q + c)) - (kSparse ? ((c - 5 == sp_class) ? 1.0f : 0.0f) : __ldg(t + c))),
+      o[c] = round_elem<TG>(scaled_f32((obj * p.inv_div) * (dm_sigmoidf(ldg_f32(q + c)) - (kSparse ? ((c - 5 == sp_class) ? 1.0f : 0.0f) : __ldg(t + c))),
                                     scale));
   }
 }
